@@ -2,6 +2,7 @@
 """bench.py -- megapixel frame-pairs/s of the dense pyramidal LK path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs B] [--impl b200|reference] [--solve fast|exact]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 1920x1080 frame pairs, 3-level Gaussian pyramid, 9x9 window.
 A step is one pass of the whole path (both pyramids + 3 fused LK levels) over a batch of B synthetic
@@ -20,6 +21,10 @@ GPU, for scale), `cpu_baseline`.
 
 `--impl reference` times the reference's own CPU implementation (cpu::gauss_pyramid +
 cpu::calc_optical_flow, compiled unmodified into oracle/_ref/libofref.so) on the host cores.
+
+`--dump-outputs DIR` writes what the headline's last timed step returned, so that two builds can be compared output for
+output (the inputs depend only on the arguments): DIR/flow_level<k>.npy, float32 (pairs, H >> k, W >> k, 2), the residual
+flow of level k for a fixed, seeded sample of the batch's pairs (as many whole pairs as fit in 64 MB; rank 0's batch).
 """
 from __future__ import annotations
 
@@ -324,6 +329,21 @@ def timed_device_steps(env, ctx, prev, nxt, w, h, levels, win, steps, warmup, fl
     pyr = ctx.profile_read(_lib.PROFILE_PYRAMID)
     ctx.profile_enable(False)
     return env.max_over_ranks(ms_total) / steps, launches, lvl, pyr, clocks, flows
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, flows):
+    """Writes a fixed, seeded sample of whole pairs of `flows` (one (n, h, w, 2) tensor per level) to out_dir; returns the
+    sampled pair indices."""
+    n = flows[0].shape[0]
+    per_pair = sum(f[0].numel() * f.element_size() for f in flows)
+    pairs = np.sort(np.random.default_rng(0).choice(n, max(1, min(n, DUMP_BYTES // per_pair)), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, f in enumerate(flows):
+        np.save(os.path.join(out_dir, f"flow_level{k}.npy"), f[pairs.tolist()].cpu().numpy())
+    return pairs.tolist()
 
 
 def roofline_of(level_ms, w, h, level, levels, n_pairs, cum_out, peak):
@@ -820,6 +840,9 @@ def main_b200(args):
                                                                          sampler=sampler)
     launches = int(env.sum_over_ranks(launches))
     value = (W * H / 1e6) * B * world / (ms_step / 1e3)
+    dumped = None
+    if args.dump_outputs and rank == 0:  # before the next measurement reuses `flows`
+        dumped = {"dir": args.dump_outputs, "pairs": dump_outputs(args.dump_outputs, flows)}
 
     # ---- the other solve, same way, fewer steps (rank-local clock is enough for a side record)
     other = SOLVE_EXACT if args.solve == "fast" else SOLVE_FAST
@@ -909,7 +932,7 @@ def main_b200(args):
                                       "double-precision solve, timed in the record named `exact`/`fast` beside the headline",
                         "single_pair_latency_ms": one_ms, "single_pair_latency_ms_cuda_graph": one_graph_ms,
                         "l2": f"inputs exceed L2 ({B * 2 * pitch * H / 1e6:.0f} MB of frames per step, fresh outputs each level)",
-                        "parallelism": f"frame-batch x{world}"},
+                        "parallelism": f"frame-batch x{world}", "dumped_outputs": dumped},
                 "roofline": roofline, other_name: other_rec, "parity": parity, "cpu_baseline": cpu, "e2e": e2e,
                 "e2e_dropin": dropin, "reference_gpu": refgpu, "configs": cfgs, "strips": strips,
                 "gpu_launches": launches, "clocks": clocks}
@@ -936,7 +959,11 @@ def main():
     ap.add_argument("--strips-size", default="7680x4320x4", help="WxHxLEVELS of the row-strip record")
     ap.add_argument("--strips-reps", type=int, default=100)
     ap.add_argument("--refgpu-only", action="store_true", help="(child of the B200 arm) time the reference's own GPU path")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the flows of the headline's last timed step (a seeded sample of "
+                    "whole pairs, at most 64 MB) to DIR/flow_level<k>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.strips_only):
+        ap.error("--dump-outputs applies to the B200 arm's headline (not --impl reference or --strips-only)")
     if args.refgpu_only:
         return main_refgpu(args)
     if args.impl == "reference":

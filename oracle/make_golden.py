@@ -1,14 +1,19 @@
 """Generate tests/golden/ref_gpu_b200.npz by running the UNMODIFIED reference's GPU functions on a B200.
 
-TEST INFRASTRUCTURE ONLY.  Run on the GPU box (oracle/_ref/libofref.so travels there prebuilt; the
-reference sources do not):
+TEST INFRASTRUCTURE ONLY.  Run on a B200 with oracle/_ref/libofref.so built (`make -C oracle ref`):
 
-    gpurun -- 'python oracle/make_golden.py gpurun_out/ref_gpu_b200.npz'
+    python oracle/make_golden.py <out.npz>
 
 then copy the file to tests/golden/.  Inputs are the seeded synthetic frames of orc_make_frame, so
 only the reference's OUTPUTS are stored.  Sizes are launch-valid for the reference's swapped
 <<<block, grid>>> launches (SURVEY.md Q6): width and height multiples of 32 with
 (w/32)*(h/32) <= 1024, at every level that is used.
+
+The file keeps every output bit for bit in a compact form (as plain float32 arrays they take 2.8 MB):
+derivatives as int16 (they are integers), window sums as their difference from the exact integer window
+sums of those derivatives (zero wherever the reference's fp32 accumulation stayed exact), and single-level
+flows as the XOR of their bits with a double-precision solve of those sums (zero wherever both round
+alike).  Tests read it through load(), which returns the reference's arrays under their original names.
 """
 from __future__ import annotations
 
@@ -68,8 +73,75 @@ def main(out_path: str) -> None:
     for k in range(levels):
         g[f"{name}_loop_flow_l{k}"] = flows[k]
     os.makedirs(os.path.dirname(os.path.abspath(out_path)), exist_ok=True)
-    np.savez_compressed(out_path, **g)
+    np.savez_compressed(out_path, **pack(g))
     print(f"wrote {out_path}: {len(g)} arrays, {sum(v.nbytes for v in g.values())} bytes raw")
+
+
+# ------------------------------------------------------------------ storage form (see the module docstring)
+DERIVATIVES = ("ix", "iy", "it1", "it2")
+ENTRY_WIN = 19  # the window gpu::calc_opt_flow hard-codes
+
+
+def _exact_sums(d: dict, win: int) -> np.ndarray:
+    """The five window sums (xx, yy, xy, xt, yt) of int64 derivatives, exact, zero outside the image."""
+    ix, iy, it = d["ix"], d["iy"], d["it2"] - d["it1"]
+    h, w = ix.shape
+    r = win // 2
+    out = []
+    for a in (ix * ix, iy * iy, ix * iy, ix * it, iy * it):
+        c = np.zeros((h + 2 * r + 1, w + 2 * r + 1), np.int64)
+        c[1 + r:1 + r + h, 1 + r:1 + r + w] = a
+        c = c.cumsum(0).cumsum(1)
+        out.append(c[win:, win:] - c[:h, win:] - c[win:, :w] + c[:h, :w])
+    return np.stack(out)
+
+
+def _solve_bits(sums: np.ndarray) -> np.ndarray:
+    """uint32 bits of the 2x2 solve of float32 sums in double precision (a predictor: it need not match exactly)."""
+    a, d, b, xt, yt = sums.astype(np.float64)
+    with np.errstate(all="ignore"):
+        p = 1.0 / (a * d - b * b)
+        flow = np.stack([b * p * yt - d * p * xt, b * p * xt - a * p * yt], axis=-1).astype(np.float32)
+    return flow.view(np.uint32)
+
+
+def unpack(z) -> dict:
+    """Stored form (a mapping of arrays) -> the reference's arrays under their original names."""
+    g = {}
+    for name, *_ in SINGLE:
+        d = {k: z[f"{name}_{k}"].astype(np.int64) for k in DERIVATIVES}
+        g.update({f"{name}_{k}": v.astype(np.float32) for k, v in d.items()})
+        for win in WINDOWS:
+            sums = (_exact_sums(d, win) + z[f"{name}_sums_w{win}_minus_exact"]).astype(np.float32)
+            g[f"{name}_sums_w{win}"] = sums
+            g[f"{name}_flow_w{win}"] = (z[f"{name}_flow_w{win}_xor_solve"] ^ _solve_bits(sums)).view(np.float32)
+        g[f"{name}_entry_flow"] = (z[f"{name}_entry_flow_xor_solve"] ^ _solve_bits(g[f"{name}_sums_w{ENTRY_WIN}"])).view(np.float32)
+    g.update({k: z[k] for k in z.keys() if k.startswith(MULTI[0] + "_")})
+    return g
+
+
+def pack(g: dict) -> dict:
+    """The reference's arrays -> stored form; checks that unpack() gives every bit back."""
+    z = {}
+    for name, *_ in SINGLE:
+        d = {k: g[f"{name}_{k}"].astype(np.int64) for k in DERIVATIVES}
+        z.update({f"{name}_{k}": v.astype(np.int16) for k, v in d.items()})
+        for win in WINDOWS:
+            sums = g[f"{name}_sums_w{win}"]
+            z[f"{name}_sums_w{win}_minus_exact"] = (sums.astype(np.int64) - _exact_sums(d, win)).astype(np.int32)
+            z[f"{name}_flow_w{win}_xor_solve"] = g[f"{name}_flow_w{win}"].view(np.uint32) ^ _solve_bits(sums)
+        z[f"{name}_entry_flow_xor_solve"] = g[f"{name}_entry_flow"].view(np.uint32) ^ _solve_bits(g[f"{name}_sums_w{ENTRY_WIN}"])
+    z.update({k: v for k, v in g.items() if k.startswith(MULTI[0] + "_")})
+    back = unpack(z)
+    assert back.keys() == g.keys(), "stored form does not cover every array"
+    for k, v in g.items():
+        assert back[k].dtype == v.dtype and np.array_equal(back[k].view(np.uint8), v.view(np.uint8)), f"{k} does not round-trip"
+    return z
+
+
+def load(path: str) -> dict:
+    with np.load(path) as z:
+        return unpack(z)
 
 
 if __name__ == "__main__":

@@ -11,7 +11,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle.make_golden import MULTI, SINGLE, WINDOWS
+from oracle.make_golden import MULTI, SINGLE, WINDOWS, load
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_gpu_b200.npz")
@@ -20,7 +20,7 @@ TOL_ABS, TOL_REL = 1e-4, 1e-5
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(GOLDEN)
+    return load(GOLDEN)
 
 
 def compare(got, ref, exact, what, mask=None):

@@ -14,14 +14,43 @@ import os
 import numpy as np
 import pytest
 
-from oracle.make_golden import MULTI, SINGLE, WINDOWS
+from oracle.make_golden import DERIVATIVES, MULTI, SINGLE, WINDOWS, load
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_gpu_b200.npz")
 
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(GOLDEN)
+    return load(GOLDEN)
+
+
+def test_golden_file_decodes(gold):
+    """The stored form of oracle/make_golden.py gives back float32 arrays of the reference's shapes, and what it stores
+    beside them is near zero: a decoding mistake shows here instead of as an oracle mismatch further down."""
+    for name, w, h, *_ in SINGLE:
+        for k in DERIVATIVES:
+            assert gold[f"{name}_{k}"].dtype == np.float32 and gold[f"{name}_{k}"].shape == (h, w)
+        for win in WINDOWS:
+            assert gold[f"{name}_sums_w{win}"].dtype == np.float32 and gold[f"{name}_sums_w{win}"].shape == (5, h, w)
+            assert gold[f"{name}_flow_w{win}"].dtype == np.float32 and gold[f"{name}_flow_w{win}"].shape == (h, w, 2)
+        assert gold[f"{name}_entry_flow"].dtype == np.float32 and gold[f"{name}_entry_flow"].shape == (h, w, 2)
+    name, w, h, levels, *_ = MULTI
+    for k in range(levels):
+        assert gold[f"{name}_loop_flow_l{k}"].dtype == np.float32 and gold[f"{name}_loop_flow_l{k}"].shape == (h >> k, w >> k, 2)
+    for k in range(1, levels):
+        assert gold[f"{name}_pyr_prev_l{k}"].dtype == np.uint8 and gold[f"{name}_pyr_prev_l{k}"].shape == (h >> k, w >> k)
+    with np.load(GOLDEN) as z:
+        for key in z.keys():
+            if key.endswith("_xor_solve"):  # a double-precision solve rounds like the reference's almost everywhere
+                assert (z[key] == 0).mean() > 0.99, key
+            elif key.endswith("_minus_exact") and np.abs(gold[key[:-len("_minus_exact")]]).max() < 2 ** 24:
+                assert not z[key].any(), key  # fp32 accumulation is exact below 2^24
+    # the decoder's window sums against a direct sum over every 5x5 window (case a stays below 2^24 at window 5)
+    ix, iy = gold["a_ix"].astype(np.int64), gold["a_iy"].astype(np.int64)
+    it = (gold["a_it2"] - gold["a_it1"]).astype(np.int64)
+    for k, p in enumerate((ix * ix, iy * iy, ix * iy, ix * it, iy * it)):
+        direct = np.lib.stride_tricks.sliding_window_view(np.pad(p, 2), (5, 5)).sum(axis=(-2, -1))
+        assert np.array_equal(direct, gold["a_sums_w5"][k]), f"sum {k}"
 
 
 def bits_equal(a, b):
