@@ -43,7 +43,10 @@ extern "C" {
  *   EXACT (default): the reference's double-precision operation order; flow bit-identical to the reference's solve.
  *   FAST           : exact 64-bit integer determinant and numerators, each rounded once to float, one hardware
  *                    reciprocal: |du|, |dv| <= 1e-4 px + 1e-5 |ref| per level on identical inputs (measured: a few
- *                    float ulps, < 3e-7 relative); about 20 % less time in the level kernel. */
+ *                    float ulps, < 3e-7 relative); about 20 % less time in the level kernel.  Pixels whose |SIxIy|
+ *                    exceeds 94,906,265 (b*b no longer exact in double: the reference's determinant of a
+ *                    one-dimensional window is then a rounding residue, not 0) take the EXACT sequence and match it
+ *                    bit for bit; windows up to 9 never reach that. */
 #define OFB_SOLVE_EXACT 0
 #define OFB_SOLVE_FAST 1
 
