@@ -18,7 +18,9 @@ OFB_OK, OFB_ERR_INVALID, OFB_ERR_CUDA, OFB_ERR_UNSUPPORTED, OFB_ERR_NOMEM = 0, 1
 WARP_AS_WRITTEN, WARP_NEAREST, WARP_BILINEAR = 0, 1, 2
 SOLVE_EXACT, SOLVE_FAST = 0, 1
 MAX_LEVELS, MAX_WINDOW = 8, 19
-PROFILE_PYRAMID = 100
+PROFILE_PYRAMID, PROFILE_FB_CHECK = 100, 101
+# per-pixel status of the forward-backward consistency check (ofb_fb_check_device)
+FB_CONSISTENT, FB_INCONSISTENT, FB_OUTSIDE, FB_FWD_NONFINITE, FB_BWD_NONFINITE = 0, 1, 2, 3, 4
 
 u8p = C.POINTER(C.c_uint8)
 f32p = C.POINTER(C.c_float)
@@ -56,6 +58,11 @@ SIGNATURES = {
     "ofb_ctx_profile_enable": (C.c_int, [_vp, C.c_int]),
     "ofb_ctx_profile_read": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_ulonglong)]),
     "ofb_flow_pairs_device": (C.c_int, [_vp, C.POINTER(OfbParams), _vp, _vp, _sz, _sz, C.POINTER(_vp), _vp, _vp]),
+    "ofb_fb_check_device": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, _vp, _vp,
+                                      _vp]),
+    "ofb_flow_pairs_fb_device": (C.c_int, [_vp, C.POINTER(OfbParams), _vp, _vp, _sz, _sz, C.c_float, C.c_float, _vp, _vp, _vp,
+                                           _vp, _vp]),
+    "ofb_ctx_reserve_pairs_fb": (C.c_int, [_vp, C.POINTER(OfbParams)]),
     "ofb_pyr_down_device": (C.c_int, [_vp, _vp, _sz, _sz, C.c_int, C.c_int, _vp, _sz, _sz, C.c_int, _vp]),
     "ofb_pyr_down2_device": (C.c_int, [_vp, _vp, _sz, _sz, C.c_int, C.c_int, _vp, _sz, _sz, _vp, _sz, _sz, C.c_int, _vp]),
     "ofb_pyr_down_strip_device": (C.c_int, [_vp, _vp, _sz, C.c_int, C.c_int, C.c_int, _vp, _sz, C.c_int, C.c_int, _vp]),

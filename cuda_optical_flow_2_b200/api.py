@@ -6,7 +6,8 @@ Function names, argument order and meaning follow OptFlowGpu.cuh (reference): `g
 (h, w, 3 interleaved channels); flow is float32 (h, w, 2).  Everything computes on the GPU through
 the C ABI in include/ofb200.h -- there is no CPU path here.
 
-The device-resident entry points (`flow_pairs_device`, `lk_level_device`, `pyr_down_device`) take
+The device-resident entry points (`flow_pairs_device`, `flow_pairs_fb_device`, `fb_check_device`, `lk_level_device`,
+`pyr_down_device`) take
 torch CUDA tensors only as owners of device memory; torch does none of the arithmetic.
 """
 from __future__ import annotations
@@ -112,12 +113,17 @@ class Context:
         p = OfbParams(w, h, levels, win, WARP_BILINEAR, 1.0, n_pairs)
         L.check(self._lib.ofb_ctx_reserve_pairs(self._h, C.byref(p)))
 
+    def reserve_pairs_fb(self, w: int, h: int, levels: int, win: int, n_pairs: int) -> None:
+        """As reserve_pairs, for flow_pairs_fb_device calls of this shape."""
+        p = OfbParams(w, h, levels, win, WARP_BILINEAR, 1.0, n_pairs)
+        L.check(self._lib.ofb_ctx_reserve_pairs_fb(self._h, C.byref(p)))
+
     def profile_enable(self, on: bool = True) -> None:
-        """CUDA-event timing around each fused-LK launch (tag = level) and the pyramid build."""
+        """CUDA-event timing around each fused-LK launch (tag = level), the pyramid build and the forward-backward check."""
         L.check(self._lib.ofb_ctx_profile_enable(self._h, 1 if on else 0))
 
     def profile_read(self, tag: int) -> tuple[float, int]:
-        """(summed milliseconds, number of records) for a tag: a pyramid level or PROFILE_PYRAMID."""
+        """(summed milliseconds, number of records) for a tag: a pyramid level, PROFILE_PYRAMID or PROFILE_FB_CHECK."""
         ms, n = C.c_double(), C.c_ulonglong()
         L.check(self._lib.ofb_ctx_profile_read(self._h, int(tag), C.byref(ms), C.byref(n)))
         return ms.value, n.value
@@ -330,6 +336,49 @@ class Context:
                                                 ptrs, total_flow.data_ptr() if total_flow is not None else None,
                                                 C.c_void_p(stream)))
         return flows
+
+    def fb_check_device(self, fwd, bwd, flow_scale: float = 1.0, alpha: float = 0.01, beta: float = 0.5, status=None,
+                        err2=None, want_err2: bool = False, stream: int = 0):
+        """Forward-backward consistency check of two total-flow fields: fwd / bwd are float32 (n, h, w, 2) CUDA tensors
+        in flow units, flow_scale px per unit.  Returns (status (n, h, w) uint8 of FB_* codes, err2 (n, h, w) float32
+        squared error in px^2 or None); passing `err2` implies want_err2."""
+        import torch
+
+        if fwd.dtype != torch.float32 or fwd.dim() != 4 or fwd.shape[3] != 2 or fwd.shape != bwd.shape or \
+                not (fwd.is_contiguous() and bwd.is_contiguous()):
+            raise ValueError("fwd/bwd must be contiguous float32 (n, h, w, 2) CUDA tensors of equal shape")
+        n, h, w, _ = fwd.shape
+        if status is None:
+            status = torch.empty((n, h, w), dtype=torch.uint8, device=fwd.device)
+        if err2 is None and want_err2:
+            err2 = torch.empty((n, h, w), dtype=torch.float32, device=fwd.device)
+        L.check(self._lib.ofb_fb_check_device(self._h, fwd.data_ptr(), bwd.data_ptr(), w, h, n, C.c_float(flow_scale),
+                                              C.c_float(alpha), C.c_float(beta), status.data_ptr(),
+                                              err2.data_ptr() if err2 is not None else None, C.c_void_p(stream)))
+        return status, err2
+
+    def flow_pairs_fb_device(self, prev, next, w: int, levels: int, win: int, warp_mode: int = WARP_BILINEAR,
+                             flow_scale: float = 1.0, alpha: float = 0.01, beta: float = 0.5, want_err2: bool = False,
+                             stream: int = 0):
+        """Flow prev->next and next->prev from one pyramid build, and their forward-backward check.  prev/next as in
+        flow_pairs_device.  Returns (fwd_total, bwd_total, status, err2 or None): the totals (n, h, w, 2) as
+        flow_pairs_device's total_flow, status (n, h, w) uint8 FB_* codes."""
+        import torch
+
+        if prev.dtype != torch.uint8 or prev.dim() != 3 or not prev.is_contiguous() or prev.shape != next.shape:
+            raise ValueError("prev/next must be contiguous uint8 (n, h, pitch) CUDA tensors of equal shape")
+        n, h, pitch = prev.shape
+        dev = prev.device
+        fwd = torch.empty((n, h, w, 2), dtype=torch.float32, device=dev)
+        bwd = torch.empty((n, h, w, 2), dtype=torch.float32, device=dev)
+        status = torch.empty((n, h, w), dtype=torch.uint8, device=dev)
+        err2 = torch.empty((n, h, w), dtype=torch.float32, device=dev) if want_err2 else None
+        p = OfbParams(w, h, levels, win, warp_mode, flow_scale, n)
+        L.check(self._lib.ofb_flow_pairs_fb_device(self._h, C.byref(p), prev.data_ptr(), next.data_ptr(), pitch, pitch * h,
+                                                   C.c_float(alpha), C.c_float(beta), fwd.data_ptr(), bwd.data_ptr(),
+                                                   status.data_ptr(), err2.data_ptr() if err2 is not None else None,
+                                                   C.c_void_p(stream)))
+        return fwd, bwd, status, err2
 
     def pyr_down_device(self, src, sw: int, dst=None, stream: int = 0):
         """src: torch.uint8 (n, sh, pitch) -> dst (n, sh>>1, pitch_d)."""

@@ -2,6 +2,7 @@
 #include "host_extract.hpp"
 #include "ofb_common.cuh"
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -211,13 +212,19 @@ static int prof_end(ofb_ctx *c, cudaStream_t st)
     return OFB_OK;
 }
 
-static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, uint8_t *base, const uint8_t *prev0,
-                            const uint8_t *next0, size_t pitch0, size_t istride0, float *const *flow_levels,
-                            float *total_flow, cudaStream_t st)
+// Level-0 frames and the pyramid levels built from them, both frames of every pair.
+struct PairLevels {
+    const uint8_t *prev[OFB_MAX_LEVELS], *next[OFB_MAX_LEVELS];
+    size_t pitch[OFB_MAX_LEVELS], istr[OFB_MAX_LEVELS];
+};
+
+// Pyramids of both frames: levels 1..L-1 into the plan's regions of `base`, one launch per one or two steps.
+static int build_pyramids(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, uint8_t *base, const uint8_t *prev0,
+                          const uint8_t *next0, size_t pitch0, size_t istride0, PairLevels *lv, cudaStream_t st)
 {
     const int L = p->levels, n = p->n_pairs;
-    const uint8_t *pp[OFB_MAX_LEVELS], *pn[OFB_MAX_LEVELS];
-    size_t pitch[OFB_MAX_LEVELS], istr[OFB_MAX_LEVELS];
+    const uint8_t **pp = lv->prev, **pn = lv->next;
+    size_t *pitch = lv->pitch, *istr = lv->istr;
     pp[0] = prev0;
     pn[0] = next0;
     pitch[0] = pitch0;
@@ -251,6 +258,16 @@ static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl,
         int rc = prof_end(c, st);
         if (rc) return rc;
     }
+    return OFB_OK;
+}
+
+// The coarse-to-fine loop of main.cu:256-262 on built pyramids: prev / next are the two frames' levels (swapped for
+// the backward direction), cum[k] (k = 1..L-2) the regions where warped levels materialise their cumulative flow.
+static int run_levels(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, const uint8_t *const *pp, const uint8_t *const *pn,
+                      const size_t *pitch, const size_t *istr, float *const *flow_levels, float *const *cum, float *total_flow,
+                      cudaStream_t st)
+{
+    const int L = p->levels, n = p->n_pairs;
     // Which warped levels materialise their cumulative flow.  Level 1 need not when level 0 composes it on the fly from
     // flow_1 and cum_2 (lk_level_kernel<..., COMP>): 8 bytes per pixel less to write at level 1, whose kernel is bound by
     // exactly those stores.  Composition needs even sizes (no clamped coarse indices), TMA-able rows and a per-pixel warp
@@ -265,7 +282,7 @@ static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl,
     }();
     if (L >= 3 && !total_flow && allow_compose && p->warp_mode != OFB_WARP_AS_WRITTEN) {
         const bool even = !((pl.w[0] | pl.h[0] | pl.w[1] | pl.h[1] | pl.w[2]) & 1);
-        const float *c2 = (2 == L - 1) ? flow_levels[2] : reinterpret_cast<const float *>(base + pl.off_cum[2]);
+        const float *c2 = (2 == L - 1) ? flow_levels[2] : cum[2];
         const bool aligned = !((reinterpret_cast<uintptr_t>(flow_levels[1]) | reinterpret_cast<uintptr_t>(c2)) & 15);
         if (even && aligned) {
             comp[0] = true;
@@ -295,25 +312,85 @@ static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl,
         if (k < L - 1) {
             // cum_{k+1}: the coarsest level's cumulative flow is its residual flow; a level that did not materialise its
             // own hands over its residual flow together with its parent's cumulative flow
-            a.cum_in = (k + 1 == L - 1 || comp[k]) ? flow_levels[k + 1] : reinterpret_cast<const float *>(base + pl.off_cum[k + 1]);
+            a.cum_in = (k + 1 == L - 1 || comp[k]) ? flow_levels[k + 1] : cum[k + 1];
             a.cum_w = pl.w[k + 1];
             a.cum_h_global = pl.h[k + 1];
             a.cum_y_off = 0;
             a.cum_h_local = pl.h[k + 1];
             a.cum_pair_stride = (size_t)pl.w[k + 1] * pl.h[k + 1];
             if (comp[k]) {
-                a.cum2_in = (k + 2 == L - 1) ? flow_levels[k + 2] : reinterpret_cast<const float *>(base + pl.off_cum[k + 2]);
+                a.cum2_in = (k + 2 == L - 1) ? flow_levels[k + 2] : cum[k + 2];
                 a.cum2_pair_stride = (size_t)pl.w[k + 2] * pl.h[k + 2];
             }
         }
         if (k == 0) a.cum_out = total_flow;
-        else if (k <= L - 2 && mat[k]) a.cum_out = reinterpret_cast<float *>(base + pl.off_cum[k]);
+        else if (k <= L - 2 && mat[k]) a.cum_out = cum[k];
         int rc = prof_begin(c, k, st);
         if (rc) return rc;
         rc = launch_lk_level(a, st, &c->launches);
         if (rc) return rc;
         rc = prof_end(c, st);
         if (rc) return rc;
+    }
+    return OFB_OK;
+}
+
+// ofb_flow_pairs_device and the batched host entry point: both pyramids, then the level loop.
+static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, uint8_t *base, const uint8_t *prev0,
+                            const uint8_t *next0, size_t pitch0, size_t istride0, float *const *flow_levels,
+                            float *total_flow, cudaStream_t st)
+{
+    PairLevels lv;
+    int rc = build_pyramids(c, p, pl, base, prev0, next0, pitch0, istride0, &lv, st);
+    if (rc) return rc;
+    float *cum[OFB_MAX_LEVELS] = {};
+    for (int k = 1; k <= p->levels - 2; k++) cum[k] = reinterpret_cast<float *>(base + pl.off_cum[k]);
+    return run_levels(c, p, pl, lv.prev, lv.next, lv.pitch, lv.istr, flow_levels, cum, total_flow, st);
+}
+
+// Workspace of the forward-backward call: the regions of plan_pairs (both pyramids, the forward direction's cumulative
+// flow), then the residual flow of every level of both directions and the backward direction's cumulative flow.
+struct PairFbPlan {
+    PairPlan pl;
+    size_t off_flow[2][OFB_MAX_LEVELS], off_cum_b[OFB_MAX_LEVELS];
+    size_t bytes = 0;
+};
+
+static void plan_pairs_fb(const ofb_params *p, PairFbPlan *fp)
+{
+    Carver cv;
+    plan_pairs(p, &fp->pl, &cv);
+    for (int d = 0; d < 2; d++)
+        for (int k = 0; k < p->levels; k++) fp->off_flow[d][k] = cv.take((size_t)fp->pl.w[k] * fp->pl.h[k] * 8 * p->n_pairs);
+    for (int k = 0; k < p->levels; k++) {
+        fp->off_cum_b[k] = (size_t)-1;
+        if (k >= 1 && k <= p->levels - 2) fp->off_cum_b[k] = cv.take((size_t)fp->pl.w[k] * fp->pl.h[k] * 8 * p->n_pairs);
+    }
+    fp->bytes = cv.off;
+}
+
+static int check_fb_args(float flow_scale, float alpha, float beta)
+{
+    if (!(std::isfinite(flow_scale) && flow_scale > 0.0f)) {
+        set_error("flow_scale %g must be finite and > 0", (double)flow_scale);
+        return OFB_ERR_INVALID;
+    }
+    if (!(std::isfinite(alpha) && alpha >= 0.0f && std::isfinite(beta) && beta >= 0.0f)) {
+        set_error("alpha %g / beta %g must be finite and >= 0", (double)alpha, (double)beta);
+        return OFB_ERR_INVALID;
+    }
+    return OFB_OK;
+}
+
+static int check_fb_buffers(const float *fwd, const float *bwd, const uint8_t *status, const float *err2)
+{
+    if (!fwd || !bwd || !status) {
+        set_error("NULL flow or status pointer");
+        return OFB_ERR_INVALID;
+    }
+    if (((reinterpret_cast<uintptr_t>(fwd) | reinterpret_cast<uintptr_t>(bwd)) & 7) || (reinterpret_cast<uintptr_t>(err2) & 3)) {
+        set_error("flow fields must be 8-byte aligned, err2 4-byte aligned");
+        return OFB_ERR_INVALID;
     }
     return OFB_OK;
 }
@@ -613,6 +690,80 @@ int ofb_ctx_reserve_pairs(ofb_ctx *c, const ofb_params *p)
     PairPlan pl;
     plan_pairs(p, &pl, &cv);
     return ws_reserve(c, pl.bytes);
+}
+
+int ofb_fb_check_device(ofb_ctx *c, const float *fwd_d, const float *bwd_d, int w, int h, int n_pairs, float flow_scale,
+                        float alpha, float beta, uint8_t *status_d, float *err2_d, void *stream)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_fb_args(flow_scale, alpha, beta);
+    if (rc) return rc;
+    if ((rc = check_fb_buffers(fwd_d, bwd_d, status_d, err2_d))) return rc;
+    OFB_GUARD(c);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = prof_begin(c, OFB_PROFILE_FB_CHECK, st))) return rc;
+    if ((rc = launch_fb_check(fwd_d, bwd_d, w, h, n_pairs, flow_scale, alpha, beta, status_d, err2_d, st, &c->launches))) return rc;
+    return prof_end(c, st);
+}
+
+int ofb_flow_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d, size_t pitch_bytes,
+                             size_t image_stride_bytes, float alpha, float beta, float *fwd_total_d, float *bwd_total_d,
+                             uint8_t *status_d, float *err2_d, void *stream)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_params(p);
+    if (rc) return rc;
+    if ((rc = check_fb_args(p->flow_scale, alpha, beta))) return rc;
+    if ((rc = check_fb_buffers(fwd_total_d, bwd_total_d, status_d, err2_d))) return rc;
+    if (!prev_d || !next_d) {
+        set_error("NULL frame pointer");
+        return OFB_ERR_INVALID;
+    }
+    if (pitch_bytes < (size_t)p->w || (p->n_pairs > 1 && image_stride_bytes < pitch_bytes * (size_t)p->h)) {
+        set_error("pitch %zu / image stride %zu too small for %dx%d", pitch_bytes, image_stride_bytes, p->w, p->h);
+        return OFB_ERR_INVALID;
+    }
+    if (p->n_pairs > 65535) { // (before anything is enqueued: the level kernels and the check take at most this many)
+        set_error("at most 65535 pairs per call (got %d)", p->n_pairs);
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    PairFbPlan fp;
+    plan_pairs_fb(p, &fp);
+    rc = ws_reserve(c, fp.bytes);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = ws_acquire(c, st))) return rc;
+    uint8_t *base = c->ws;
+    PairLevels lv;
+    if ((rc = build_pyramids(c, p, fp.pl, base, prev_d, next_d, pitch_bytes, image_stride_bytes, &lv, st))) return rc;
+    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS] = {};
+    for (int k = 0; k < p->levels; k++) {
+        for (int d = 0; d < 2; d++) flow[d][k] = reinterpret_cast<float *>(base + fp.off_flow[d][k]);
+        if (k >= 1 && k <= p->levels - 2) {
+            cum[0][k] = reinterpret_cast<float *>(base + fp.pl.off_cum[k]);
+            cum[1][k] = reinterpret_cast<float *>(base + fp.off_cum_b[k]);
+        }
+    }
+    if ((rc = run_levels(c, p, fp.pl, lv.prev, lv.next, lv.pitch, lv.istr, flow[0], cum[0], fwd_total_d, st))) return rc;
+    if ((rc = run_levels(c, p, fp.pl, lv.next, lv.prev, lv.pitch, lv.istr, flow[1], cum[1], bwd_total_d, st))) return rc;
+    if ((rc = prof_begin(c, OFB_PROFILE_FB_CHECK, st))) return rc;
+    if ((rc = launch_fb_check(fwd_total_d, bwd_total_d, p->w, p->h, p->n_pairs, p->flow_scale, alpha, beta, status_d, err2_d, st,
+                              &c->launches)))
+        return rc;
+    if ((rc = prof_end(c, st))) return rc;
+    return ws_release(c, st);
+}
+
+int ofb_ctx_reserve_pairs_fb(ofb_ctx *c, const ofb_params *p)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_params(p);
+    if (rc) return rc;
+    OFB_GUARD(c);
+    PairFbPlan fp;
+    plan_pairs_fb(p, &fp);
+    return ws_reserve(c, fp.bytes);
 }
 
 int ofb_pyr_down_device(ofb_ctx *c, const uint8_t *src_d, size_t src_pitch, size_t src_image_stride, int sw, int sh,

@@ -153,6 +153,10 @@ int launch_inverse_f32(const float *sxx, const float *syy, const float *sxy, con
 int launch_compose_cum(const float *flow_k, const float *cum_coarser, int w, int h, int n_pairs, float *cum_out,
                        cudaStream_t stream, unsigned long long *launches);
 
+// ---- forward-backward consistency check (fb_check.cu) ---------------------------------------
+int launch_fb_check(const float *fwd, const float *bwd, int w, int h, int n_pairs, float flow_scale, float alpha, float beta,
+                    uint8_t *status, float *err2, cudaStream_t stream, unsigned long long *launches);
+
 int launch_grayscale(const uint8_t *src_c3, int w, int h, uint8_t *dst_c3, uint8_t *dst_planar, size_t dst_pitch,
                      cudaStream_t stream, unsigned long long *launches);
 int launch_bilateral(const uint8_t *src, const uint8_t *gray, size_t pitch, int channels, int w, int h, int ww, int wh,

@@ -326,6 +326,40 @@ int ofb_flow_arrows_host(ofb_ctx *ctx, float *const *flow_pyramid_h, int w, int 
                          int *arrows_xyxy, int max_arrows, int *n_arrows);
 int ofb_write_flo(const char *path, const float *flow_h, int w, int h);
 
+/* ---- forward-backward consistency check; the reference has no counterpart -----------------------------------------
+ * Which flow values can be trusted: flow prev->next (f) and next->prev (b) should cancel where a pixel is visible in
+ * both frames.  Per pixel (i, j), with s = flow_scale (px per flow unit, the ofb_params value), in this order:
+ *   f = fwd[i][j] not finite                                         -> OFB_FB_FWD_NONFINITE (e.g. a det == 0 window, Q3)
+ *   du = s*f.u, dv = s*f.v; !(|du| < 32768 && |dv| < 32768)           -> OFB_FB_OUTSIDE
+ *   X = j*256 + rint(du*256), Y = i*256 + rint(dv*256) (half to even, the bilinear warp's 1/256-px rounding);
+ *   X or Y outside [0, (w-1)*256] / [0, (h-1)*256]                   -> OFB_FB_OUTSIDE (the target leaves the frame)
+ *   b = bilinear sample of bwd at (X/256, Y/256); a tap with weight 0 is not read; a read tap not finite
+ *                                                                    -> OFB_FB_BWD_NONFINITE
+ *   err2 = |s*(f + b)|^2, mag2 = |s*f|^2 + |s*b|^2 (px^2); err2 finite and err2 <= alpha*mag2 + beta
+ *                                                                    -> OFB_FB_CONSISTENT, else OFB_FB_INCONSISTENT
+ * (Sundaram, Brox and Keutzer 2010; alpha = 0.01, beta = 0.5 px^2 are the usual values.)  Every multiply and add is
+ * rounded separately, without fma: the result does not depend on the compiler.  err2 (optional) receives the value
+ * above for CONSISTENT / INCONSISTENT pixels and NaN for the others.  Flow fields are (u, v) float pairs in the
+ * library's layout, pairs back to back (n_pairs*h*w*2 floats, 8-byte aligned); status is n_pairs*h*w bytes; err2
+ * n_pairs*h*w floats (4-byte aligned) or NULL.  At most 65535 pairs per call and 32768 x 32768 pixels. */
+#define OFB_FB_CONSISTENT 0
+#define OFB_FB_INCONSISTENT 1
+#define OFB_FB_OUTSIDE 2
+#define OFB_FB_FWD_NONFINITE 3
+#define OFB_FB_BWD_NONFINITE 4
+/* The check alone, on any two total-flow fields (e.g. the caller's own).  flow_scale > 0, alpha >= 0, beta >= 0. */
+int ofb_fb_check_device(ofb_ctx *ctx, const float *fwd_d, const float *bwd_d, int w, int h, int n_pairs, float flow_scale,
+                        float alpha, float beta, uint8_t *status_d, float *err2_d, void *stream);
+/* Both directions of every pair plus the check.  The pyramids of both frames are built once (one launch, as in
+ * ofb_flow_pairs_device); the level loop runs prev->next, then next->prev on the same pyramids.  fwd_total_d /
+ * bwd_total_d (required, n_pairs*h*w*2 floats) receive the level-0 compositions (main.cu:136-147), bit-identical to
+ * ofb_flow_pairs_device(prev, next) / ofb_flow_pairs_device(next, prev) with total_flow_d.  The residual pyramids of
+ * both directions live in the context workspace.  p->flow_scale is the check's s and must be > 0. */
+int ofb_flow_pairs_fb_device(ofb_ctx *ctx, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d,
+                             size_t pitch_bytes, size_t image_stride_bytes, float alpha, float beta, float *fwd_total_d,
+                             float *bwd_total_d, uint8_t *status_d, float *err2_d, void *stream);
+int ofb_ctx_reserve_pairs_fb(ofb_ctx *ctx, const ofb_params *p); /* workspace for the call above (CUDA graph capture) */
+
 /* Pinned host memory helpers for callers without a CUDA runtime of their own. */
 int ofb_host_alloc(void **ptr, size_t bytes);
 int ofb_host_free(void *ptr);
@@ -335,9 +369,11 @@ int ofb_ctx_launch_count(const ofb_ctx *ctx, unsigned long long *count);
 
 /* In-situ kernel timing for the roofline report.  While enabled, ofb_flow_pairs_device/_host put a
  * CUDA-event pair (on the stream the work is launched on) around every fused-LK launch, tagged with
- * its pyramid level, and around the pyramid build, tagged OFB_PROFILE_PYRAMID.  _enable(on) also
+ * its pyramid level, and around the pyramid build, tagged OFB_PROFILE_PYRAMID; the forward-backward entry points
+ * also around the check kernel, tagged OFB_PROFILE_FB_CHECK.  _enable(on) also
  * discards earlier records.  _read waits for the tagged events and returns their summed duration. */
 #define OFB_PROFILE_PYRAMID 100
+#define OFB_PROFILE_FB_CHECK 101
 int ofb_ctx_profile_enable(ofb_ctx *ctx, int on);
 int ofb_ctx_profile_read(ofb_ctx *ctx, int tag, double *ms_sum, unsigned long long *n_records);
 
