@@ -94,7 +94,10 @@ static int launch_one(const LkLevelArgs &a, cudaStream_t stream, unsigned long l
         const char *envw = getenv("OFB_LK_TAIL_WAVES"); // ... and the length of the tail in tenths of a wave
         const int shift = env ? atoi(env) : 2;
         const int slots = n_sm * C::MIN_BLOCKS;
-        const int tail_pairs = ((slots + strips - 1) / strips * (envw ? atoi(envw) : 10) + 9) / 10;
+        int tail_pairs = ((slots + strips - 1) / strips * (envw ? atoi(envw) : 10) + 9) / 10;
+        // grid z = n + ((1 << shift) - 1) * tail_pairs must stay within the hardware's 65535: near that many pairs the
+        // tail shrinks, and at 65535 it is off
+        if (shift > 0 && shift <= 4) tail_pairs = std::min(tail_pairs, (65535 - a.n_pairs) / ((1 << shift) - 1));
         if (shift > 0 && shift <= 4 && nby == 1 && a.npush == 0 && a.nwait == 0 && out_rows >= (2 * C::CH << shift) &&
             tail_pairs > 0 && (long long)a.n_pairs * strips >= 4ll * slots && tail_pairs < a.n_pairs) {
             tail_shift = shift;

@@ -667,6 +667,10 @@ int ofb_flow_pairs_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev_d
         set_error("pitch %zu / image stride %zu too small for %dx%d", pitch_bytes, image_stride_bytes, p->w, p->h);
         return OFB_ERR_INVALID;
     }
+    if (p->n_pairs > 65535) { // (before the workspace grows: the level kernels take at most this many)
+        set_error("at most 65535 pairs per call (got %d)", p->n_pairs);
+        return OFB_ERR_INVALID;
+    }
     OFB_GUARD(c);
     Carver cv;
     PairPlan pl;

@@ -108,7 +108,8 @@ int ofb_c3_extract_host(const unsigned char *src_c3, unsigned char *dst_planar, 
  *   flow_levels_d[k]: out, RESIDUAL flow of level k (what the reference leaves in
  *                     optFlowPyramid[k]); n_pairs * (h>>k) * (w>>k) * 2 floats.
  *   total_flow_d    : optional out (may be NULL), the composition rule of main.cu:136-147 at
- *                     level 0: sum_k 2^k * flow_k[i>>k, j>>k]; n_pairs * h * w * 2 floats. */
+ *                     level 0: sum_k 2^k * flow_k[i>>k, j>>k]; n_pairs * h * w * 2 floats.
+ * At most 65535 pairs per call (as ofb_lk_level_device and ofb_flow_pairs_fb_device). */
 int ofb_flow_pairs_device(ofb_ctx *ctx, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d,
                           size_t pitch_bytes, size_t image_stride_bytes, float *const *flow_levels_d,
                           float *total_flow_d, void *stream);
@@ -139,7 +140,8 @@ int ofb_pyr_down_strip_device(ofb_ctx *ctx, const uint8_t *src_d, size_t src_pit
  *   cum_in_d : cumulative flow of the next-coarser level ((w>>1) x (h>>1) float2 per pair:
  *              cum_{k+1} = flow_{k+1} + 2*cum_{k+2}[i>>1, j>>1]); NULL for the coarsest level
  *              (not warped, OptFlowGpu.cu:1918).
- *   flow_out_d: residual flow of this level.  cum_out_d: optional, 2*cum_in[i>>1,j>>1] + flow. */
+ *   flow_out_d: residual flow of this level.  cum_out_d: optional, 2*cum_in[i>>1,j>>1] + flow.
+ *   n_pairs: at most 65535. */
 int ofb_lk_level_device(ofb_ctx *ctx, const uint8_t *prev_d, const uint8_t *next_d, size_t pitch_bytes,
                         size_t image_stride_bytes, int w, int h, int n_pairs, int win, int warp_mode, float flow_scale,
                         const float *cum_in_d, float *flow_out_d, float *cum_out_d, void *stream);
