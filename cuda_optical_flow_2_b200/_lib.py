@@ -62,6 +62,9 @@ SIGNATURES = {
                                       _vp]),
     "ofb_flow_pairs_fb_device": (C.c_int, [_vp, C.POINTER(OfbParams), _vp, _vp, _sz, _sz, C.c_float, C.c_float, _vp, _vp, _vp,
                                            _vp, _vp]),
+    "ofb_flow_pairs_fb_host": (C.c_int, [_vp, C.POINTER(OfbParams), u8p, u8p, C.c_int, C.c_float, C.c_float, f32p, f32p, u8p,
+                                         f32p]),
+    "ofb_stream_push_bgr_host_fb": (C.c_int, [_vp, u8p, C.c_float, C.c_float, C.POINTER(f32p), f32p, f32p, u8p, f32p, i32p]),
     "ofb_ctx_reserve_pairs_fb": (C.c_int, [_vp, C.POINTER(OfbParams)]),
     "ofb_pyr_down_device": (C.c_int, [_vp, _vp, _sz, _sz, C.c_int, C.c_int, _vp, _sz, _sz, C.c_int, _vp]),
     "ofb_pyr_down2_device": (C.c_int, [_vp, _vp, _sz, _sz, C.c_int, C.c_int, _vp, _sz, _sz, _vp, _sz, _sz, C.c_int, _vp]),

@@ -8,7 +8,8 @@ the C ABI in include/ofb200.h -- there is no CPU path here.
 
 The device-resident entry points (`flow_pairs_device`, `flow_pairs_fb_device`, `fb_check_device`, `lk_level_device`,
 `pyr_down_device`) take
-torch CUDA tensors only as owners of device memory; torch does none of the arithmetic.
+torch CUDA tensors only as owners of device memory; torch does none of the arithmetic.  The forward-backward check also
+runs on host batches (`flow_pairs_fb_host`) and on the frame stream (`FrameStream.push_fb`).
 """
 from __future__ import annotations
 
@@ -40,8 +41,27 @@ def _ptrs(arrs: Sequence[np.ndarray], t):
     return (t * len(arrs))(*[a.ctypes.data_as(t) for a in arrs])
 
 
+def _optp(a: Optional[np.ndarray], t):
+    return a.ctypes.data_as(t) if a is not None else None
+
+
 def align_up(v: int, a: int) -> int:
     return (v + a - 1) // a * a
+
+
+def _batch_shape(prev: np.ndarray, next: np.ndarray) -> tuple[int, int, int, int]:
+    """(channels, n, h, w) of a host batch: (n, h, w) planar gray or (n, h, w, 3) reference layout."""
+    if prev.ndim == 4:
+        if prev.shape[3] != 3:
+            raise ValueError("4-d input must be (n, h, w, 3)")
+        channels, (n, h, w) = 3, prev.shape[:3]
+    elif prev.ndim == 3:
+        channels, (n, h, w) = 1, prev.shape
+    else:
+        raise ValueError("prev must be (n,h,w) or (n,h,w,3)")
+    if next.shape != prev.shape:
+        raise ValueError("prev and next differ in shape")
+    return channels, n, h, w
 
 
 class Context:
@@ -300,16 +320,7 @@ class Context:
                               out: Optional[np.ndarray] = None) -> np.ndarray:
         """As flow_pairs_host, but only the level-0 composition of main.cu:136-147 (the total flow, (n, h, w, 2))
         leaves the device: 8 bytes per pixel over PCIe instead of 10.5."""
-        if prev.ndim == 4:
-            if prev.shape[3] != 3:
-                raise ValueError("4-d input must be (n, h, w, 3)")
-            channels, (n, h, w) = 3, prev.shape[:3]
-        elif prev.ndim == 3:
-            channels, (n, h, w) = 1, prev.shape
-        else:
-            raise ValueError("prev must be (n,h,w) or (n,h,w,3)")
-        if next.shape != prev.shape:
-            raise ValueError("prev and next differ in shape")
+        channels, n, h, w = _batch_shape(prev, next)
         p = OfbParams(w, h, levels, win, warp_mode, flow_scale, n)
         if out is None:
             out = np.empty((n, h, w, 2), np.float32)
@@ -317,6 +328,24 @@ class Context:
                                                  _u8(next).ctypes.data_as(L.u8p), channels, None,
                                                  _f32(out).ctypes.data_as(L.f32p)))
         return out
+
+    def flow_pairs_fb_host(self, prev: np.ndarray, next: np.ndarray, levels: int, win: int, warp_mode: int = WARP_BILINEAR,
+                           flow_scale: float = 1.0, alpha: float = 0.01, beta: float = 0.5, want_bwd: bool = False,
+                           want_err2: bool = False):
+        """flow_pairs_fb_device for host batches: prev/next as in total_flow_pairs_host.  Returns numpy arrays
+        (fwd_total (n, h, w, 2), bwd_total or None, status (n, h, w) uint8 FB_* codes, err2 (n, h, w) or None); the
+        outputs not asked for are not downloaded."""
+        channels, n, h, w = _batch_shape(prev, next)
+        p = OfbParams(w, h, levels, win, warp_mode, flow_scale, n)
+        fwd = np.empty((n, h, w, 2), np.float32)
+        bwd = np.empty((n, h, w, 2), np.float32) if want_bwd else None
+        status = np.empty((n, h, w), np.uint8)
+        err2 = np.empty((n, h, w), np.float32) if want_err2 else None
+        L.check(self._lib.ofb_flow_pairs_fb_host(self._h, C.byref(p), _u8(prev).ctypes.data_as(L.u8p),
+                                                 _u8(next).ctypes.data_as(L.u8p), channels, C.c_float(alpha), C.c_float(beta),
+                                                 fwd.ctypes.data_as(L.f32p), _optp(bwd, L.f32p), status.ctypes.data_as(L.u8p),
+                                                 _optp(err2, L.f32p)))
+        return fwd, bwd, status, err2
 
     # ---------------------------------------------------------------- device-resident API
     def flow_pairs_device(self, prev, next, w: int, levels: int, win: int, warp_mode: int = WARP_BILINEAR,
@@ -463,6 +492,28 @@ class FrameStream:
         L.check(self._lib.ofb_stream_push_bgr_host(self._h, _u8(frame_bgr).ctypes.data_as(L.u8p), ptrs,
                                                    total.ctypes.data_as(L.f32p) if want_total else None, C.byref(has)))
         return (flows, total) if has.value else None
+
+    def push_fb(self, frame_bgr: np.ndarray, alpha: float = 0.01, beta: float = 0.5, want_levels: bool = False,
+                want_bwd: bool = False, want_err2: bool = False):
+        """push with the forward-backward check: returns None for the first frame, else a dict with `fwd_total` (h, w, 2),
+        `status` (h, w) uint8 FB_* codes and, as asked, `levels` (the forward residual flows, level 0 first), `bwd_total`
+        (h, w, 2) and `err2` (h, w).  Mixes freely with push on one stream."""
+        if frame_bgr.shape != (self.h, self.w, 3):
+            raise ValueError("frame must be (h, w, 3) uint8")
+        out = {"fwd_total": np.empty((self.h, self.w, 2), np.float32), "status": np.empty((self.h, self.w), np.uint8)}
+        if want_levels:
+            out["levels"] = [np.empty((self.h >> k, self.w >> k, 2), np.float32) for k in range(self.levels)]
+        if want_bwd:
+            out["bwd_total"] = np.empty((self.h, self.w, 2), np.float32)
+        if want_err2:
+            out["err2"] = np.empty((self.h, self.w), np.float32)
+        ptrs = _ptrs(out["levels"], L.f32p) if want_levels else None
+        has = C.c_int(0)
+        L.check(self._lib.ofb_stream_push_bgr_host_fb(self._h, _u8(frame_bgr).ctypes.data_as(L.u8p), C.c_float(alpha),
+                                                      C.c_float(beta), ptrs, out["fwd_total"].ctypes.data_as(L.f32p),
+                                                      _optp(out.get("bwd_total"), L.f32p), out["status"].ctypes.data_as(L.u8p),
+                                                      _optp(out.get("err2"), L.f32p), C.byref(has)))
+        return out if has.value else None
 
     def close(self):
         if getattr(self, "_h", None):

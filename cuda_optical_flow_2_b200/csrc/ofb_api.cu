@@ -395,6 +395,141 @@ static int check_fb_buffers(const float *fwd, const float *bwd, const uint8_t *s
     return OFB_OK;
 }
 
+// The check kernel with its OFB_PROFILE_FB_CHECK record.
+static int run_fb_check(ofb_ctx *c, const float *fwd, const float *bwd, int w, int h, int n_pairs, float flow_scale, float alpha,
+                        float beta, uint8_t *status, float *err2, cudaStream_t st)
+{
+    int rc = prof_begin(c, OFB_PROFILE_FB_CHECK, st);
+    if (rc) return rc;
+    if ((rc = launch_fb_check(fwd, bwd, w, h, n_pairs, flow_scale, alpha, beta, status, err2, st, &c->launches))) return rc;
+    return prof_end(c, st);
+}
+
+// The device-side body of ofb_flow_pairs_fb_device and ofb_flow_pairs_fb_host: both pyramids once, the level loop
+// prev->next and then next->prev on them, the check.  `base` holds the regions of `fp`.
+static int run_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const PairFbPlan &fp, uint8_t *base, const uint8_t *prev0,
+                               const uint8_t *next0, size_t pitch0, size_t istride0, float alpha, float beta, float *fwd_total,
+                               float *bwd_total, uint8_t *status, float *err2, cudaStream_t st)
+{
+    PairLevels lv;
+    int rc = build_pyramids(c, p, fp.pl, base, prev0, next0, pitch0, istride0, &lv, st);
+    if (rc) return rc;
+    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS] = {};
+    for (int k = 0; k < p->levels; k++) {
+        for (int d = 0; d < 2; d++) flow[d][k] = reinterpret_cast<float *>(base + fp.off_flow[d][k]);
+        if (k >= 1 && k <= p->levels - 2) {
+            cum[0][k] = reinterpret_cast<float *>(base + fp.pl.off_cum[k]);
+            cum[1][k] = reinterpret_cast<float *>(base + fp.off_cum_b[k]);
+        }
+    }
+    if ((rc = run_levels(c, p, fp.pl, lv.prev, lv.next, lv.pitch, lv.istr, flow[0], cum[0], fwd_total, st))) return rc;
+    if ((rc = run_levels(c, p, fp.pl, lv.next, lv.prev, lv.pitch, lv.istr, flow[1], cum[1], bwd_total, st))) return rc;
+    return run_fb_check(c, fwd_total, bwd_total, p->w, p->h, p->n_pairs, p->flow_scale, alpha, beta, status, err2, st);
+}
+
+// One sub-batch of the batched host entry points: pairs [first, first + p.n_pairs) of the call, whose level-0 frames have
+// been uploaded into prev0 / next0 inside the lane's workspace region B; its work goes on the lane's stream st.
+struct HostSub {
+    ofb_params p;
+    int first;
+    uint8_t *B;
+    const uint8_t *prev0, *next0;
+    size_t pitch0, istride0;
+    cudaStream_t st;
+};
+
+// The sub-batch pipeline of the batched host entry points (ofb_flow_pairs_host / _ex and ofb_flow_pairs_fb_host), with
+// host input in the layout of `channels`.  plan_lane(sub, &cv) lays out the caller's regions of a lane's workspace after the
+// level-0 frames and returns the lane's end offset; run_sub(HostSub) enqueues a sub-batch's compute and downloads.
+template <class PlanLane, class RunSub>
+static int host_pipeline(ofb_ctx *c, const ofb_params *p, const unsigned char *prev_h, const unsigned char *next_h, int channels,
+                         PlanLane plan_lane, RunSub run_sub)
+{
+    // Software pipeline over sub-batches on OFB_LANES streams: while one lane downloads its flow the
+    // other uploads and computes, so the PCIe directions and the SMs overlap (with pinned host memory).
+    // Sub-batches are kept small (at least eight per lane when the batch allows): the first upload and the last
+    // download are the part of the pipeline nothing overlaps, and a 1080p pair already is 12 MB in and 22 MB out.
+    const int n = p->n_pairs;
+    const int LANES = c->lanes;
+    int sub = n / (8 * LANES);
+    if (sub < 1) sub = 1;
+    if (sub > 8) sub = 8;
+    if (c->sub_pairs > 0) sub = c->sub_pairs < n ? c->sub_pairs : n;
+    const size_t pitch0 = align_up((size_t)p->w, 64), istride0 = pitch0 * (size_t)p->h;
+    const size_t c3 = (size_t)p->w * p->h * 3;
+    size_t lane_bytes = 0;
+    size_t off_p0, off_n0, off_c3 = 0;
+    {
+        Carver cv;
+        off_p0 = cv.take(istride0 * sub);
+        off_n0 = cv.take(istride0 * sub);
+        if (channels == 3) off_c3 = cv.take(c3 * sub * 2);
+        lane_bytes = align_up(plan_lane(sub, &cv), 256);
+    }
+    int rc = ws_reserve(c, lane_bytes * LANES);
+    if (rc) return rc;
+    // 3-channel input with host threads: channel 0 is extracted on the host into pinned planar staging buffers (one
+    // prev + one next buffer per lane) and only those bytes are uploaded (host_extract.cpp)
+    const bool host_extract = channels == 3 && c->host_threads > 0;
+    const size_t frame_px = (size_t)p->w * p->h, stage_lane = 2 * frame_px * sub;
+    bool stage_used[OFB_LANES] = {};
+    if (host_extract) {
+        if (!c->pool) {
+            try {
+                c->pool = new ofb::HostPool(c->host_threads);
+            } catch (...) {
+                set_error("flow_pairs_host: could not start %d host threads", c->host_threads);
+                return OFB_ERR_NOMEM;
+            }
+        }
+        if (c->stage_bytes < stage_lane * LANES) {
+            if (c->stage) OFB_CUDA_TRY(cudaFreeHost(c->stage));
+            c->stage = nullptr;
+            c->stage_bytes = 0;
+            OFB_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&c->stage), stage_lane * LANES, cudaHostAllocDefault));
+            c->stage_bytes = stage_lane * LANES;
+        }
+        for (int lane = 0; lane < LANES; lane++)
+            if (!c->stage_ev[lane]) OFB_CUDA_TRY(cudaEventCreateWithFlags(&c->stage_ev[lane], cudaEventDisableTiming));
+    }
+    for (int lane = 0; lane < LANES; lane++)
+        if ((rc = ws_acquire(c, c->lane_stream[lane]))) return rc;
+    for (int first = 0, sb = 0; first < n; first += sub, sb++) {
+        const int lane = sb % LANES;
+        const int cnt = (n - first < sub) ? n - first : sub;
+        cudaStream_t st = c->lane_stream[lane];
+        uint8_t *B = c->ws + lane_bytes * lane;
+        if (channels == 1) {
+            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_p0, pitch0, prev_h + (size_t)first * p->w * p->h, (size_t)p->w, (size_t)p->w,
+                                           (size_t)p->h * cnt, cudaMemcpyHostToDevice, st));
+            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_n0, pitch0, next_h + (size_t)first * p->w * p->h, (size_t)p->w, (size_t)p->w,
+                                           (size_t)p->h * cnt, cudaMemcpyHostToDevice, st));
+        } else if (host_extract) {
+            uint8_t *sp = c->stage + stage_lane * lane, *sn = sp + frame_px * sub;
+            if (stage_used[lane]) OFB_CUDA_TRY(cudaEventSynchronize(c->stage_ev[lane])); // the lane's previous upload has left the buffers
+            ofb::c3_extract_pair_sets(c->pool, prev_h + c3 * first, next_h + c3 * first, sp, sn, frame_px * cnt);
+            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_p0, pitch0, sp, (size_t)p->w, (size_t)p->w, (size_t)p->h * cnt,
+                                           cudaMemcpyHostToDevice, st));
+            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_n0, pitch0, sn, (size_t)p->w, (size_t)p->w, (size_t)p->h * cnt,
+                                           cudaMemcpyHostToDevice, st));
+            OFB_CUDA_TRY(cudaEventRecord(c->stage_ev[lane], st));
+            stage_used[lane] = true;
+        } else {
+            OFB_CUDA_TRY(cudaMemcpyAsync(B + off_c3, prev_h + c3 * first, c3 * cnt, cudaMemcpyHostToDevice, st));
+            OFB_CUDA_TRY(cudaMemcpyAsync(B + off_c3 + c3 * sub, next_h + c3 * first, c3 * cnt, cudaMemcpyHostToDevice, st));
+            rc = launch_c3_to_planar(B + off_c3, p->w, p->h, cnt, B + off_p0, pitch0, istride0, st, &c->launches);
+            if (rc) return rc;
+            rc = launch_c3_to_planar(B + off_c3 + c3 * sub, p->w, p->h, cnt, B + off_n0, pitch0, istride0, st, &c->launches);
+            if (rc) return rc;
+        }
+        HostSub s{*p, first, B, B + off_p0, B + off_n0, pitch0, istride0, st};
+        s.p.n_pairs = cnt;
+        if ((rc = run_sub(s))) return rc;
+    }
+    for (int lane = 0; lane < LANES; lane++) OFB_CUDA_TRY(cudaStreamSynchronize(c->lane_stream[lane]));
+    return OFB_OK;
+}
+
 } // namespace ofb
 
 using namespace ofb;
@@ -704,10 +839,7 @@ int ofb_fb_check_device(ofb_ctx *c, const float *fwd_d, const float *bwd_d, int 
     if (rc) return rc;
     if ((rc = check_fb_buffers(fwd_d, bwd_d, status_d, err2_d))) return rc;
     OFB_GUARD(c);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if ((rc = prof_begin(c, OFB_PROFILE_FB_CHECK, st))) return rc;
-    if ((rc = launch_fb_check(fwd_d, bwd_d, w, h, n_pairs, flow_scale, alpha, beta, status_d, err2_d, st, &c->launches))) return rc;
-    return prof_end(c, st);
+    return run_fb_check(c, fwd_d, bwd_d, w, h, n_pairs, flow_scale, alpha, beta, status_d, err2_d, static_cast<cudaStream_t>(stream));
 }
 
 int ofb_flow_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d, size_t pitch_bytes,
@@ -738,24 +870,9 @@ int ofb_flow_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const uint8_t *pre
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if ((rc = ws_acquire(c, st))) return rc;
-    uint8_t *base = c->ws;
-    PairLevels lv;
-    if ((rc = build_pyramids(c, p, fp.pl, base, prev_d, next_d, pitch_bytes, image_stride_bytes, &lv, st))) return rc;
-    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS] = {};
-    for (int k = 0; k < p->levels; k++) {
-        for (int d = 0; d < 2; d++) flow[d][k] = reinterpret_cast<float *>(base + fp.off_flow[d][k]);
-        if (k >= 1 && k <= p->levels - 2) {
-            cum[0][k] = reinterpret_cast<float *>(base + fp.pl.off_cum[k]);
-            cum[1][k] = reinterpret_cast<float *>(base + fp.off_cum_b[k]);
-        }
-    }
-    if ((rc = run_levels(c, p, fp.pl, lv.prev, lv.next, lv.pitch, lv.istr, flow[0], cum[0], fwd_total_d, st))) return rc;
-    if ((rc = run_levels(c, p, fp.pl, lv.next, lv.prev, lv.pitch, lv.istr, flow[1], cum[1], bwd_total_d, st))) return rc;
-    if ((rc = prof_begin(c, OFB_PROFILE_FB_CHECK, st))) return rc;
-    if ((rc = launch_fb_check(fwd_total_d, bwd_total_d, p->w, p->h, p->n_pairs, p->flow_scale, alpha, beta, status_d, err2_d, st,
-                              &c->launches)))
+    if ((rc = run_pairs_fb_device(c, p, fp, c->ws, prev_d, next_d, pitch_bytes, image_stride_bytes, alpha, beta, fwd_total_d,
+                                  bwd_total_d, status_d, err2_d, st)))
         return rc;
-    if ((rc = prof_end(c, st))) return rc;
     return ws_release(c, st);
 }
 
@@ -1134,114 +1251,41 @@ static int flow_pairs_host_impl(ofb_ctx *c, const ofb_params *p, const unsigned 
         return OFB_ERR_INVALID;
     }
     OFB_GUARD(c);
-    // Software pipeline over sub-batches on OFB_LANES streams: while one lane downloads its flow the
-    // other uploads and computes, so the PCIe directions and the SMs overlap (with pinned host memory).
-    // Sub-batches are kept small (at least eight per lane when the batch allows): the first upload and the last
-    // download are the part of the pipeline nothing overlaps, and a 1080p pair already is 12 MB in and 22 MB out.
-    const int n = p->n_pairs;
-    const int LANES = c->lanes;
-    int sub = n / (8 * LANES);
-    if (sub < 1) sub = 1;
-    if (sub > 8) sub = 8;
-    if (c->sub_pairs > 0) sub = c->sub_pairs < n ? c->sub_pairs : n;
-    ofb_params ps = *p;
-    ps.n_pairs = sub;
-    const size_t pitch0 = align_up((size_t)p->w, 64), istride0 = pitch0 * (size_t)p->h;
-    const size_t c3 = (size_t)p->w * p->h * 3;
-    size_t lane_bytes = 0;
-    size_t off_p0, off_n0, off_c3 = 0, off_flow[OFB_MAX_LEVELS], off_total = 0, plan_base;
+    size_t off_flow[OFB_MAX_LEVELS], off_total = 0, plan_base = 0;
     PairPlan pl;
-    {
-        Carver cv;
-        off_p0 = cv.take(istride0 * sub);
-        off_n0 = cv.take(istride0 * sub);
-        if (channels == 3) off_c3 = cv.take(c3 * sub * 2);
-        for (int k = 0; k < p->levels; k++) off_flow[k] = cv.take((size_t)(p->w >> k) * (p->h >> k) * 8 * sub);
-        if (total_flow_h) off_total = cv.take((size_t)p->w * p->h * 8 * sub);
-        plan_base = cv.off;
+    auto plan_lane = [&](int sub, Carver *cv) {
+        for (int k = 0; k < p->levels; k++) off_flow[k] = cv->take((size_t)(p->w >> k) * (p->h >> k) * 8 * sub);
+        if (total_flow_h) off_total = cv->take((size_t)p->w * p->h * 8 * sub);
+        plan_base = cv->off;
+        ofb_params ps = *p;
+        ps.n_pairs = sub;
         Carver cv2;
         plan_pairs(&ps, &pl, &cv2);
-        lane_bytes = align_up(plan_base + pl.bytes, 256);
-    }
-    rc = ws_reserve(c, lane_bytes * LANES);
-    if (rc) return rc;
-    // 3-channel input with host threads: channel 0 is extracted on the host into pinned planar staging buffers (one
-    // prev + one next buffer per lane) and only those bytes are uploaded (host_extract.cpp)
-    const bool host_extract = channels == 3 && c->host_threads > 0;
-    const size_t frame_px = (size_t)p->w * p->h, stage_lane = 2 * frame_px * sub;
-    bool stage_used[OFB_LANES] = {};
-    if (host_extract) {
-        if (!c->pool) {
-            try {
-                c->pool = new ofb::HostPool(c->host_threads);
-            } catch (...) {
-                set_error("flow_pairs_host: could not start %d host threads", c->host_threads);
-                return OFB_ERR_NOMEM;
-            }
-        }
-        if (c->stage_bytes < stage_lane * LANES) {
-            if (c->stage) OFB_CUDA_TRY(cudaFreeHost(c->stage));
-            c->stage = nullptr;
-            c->stage_bytes = 0;
-            OFB_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&c->stage), stage_lane * LANES, cudaHostAllocDefault));
-            c->stage_bytes = stage_lane * LANES;
-        }
-        for (int lane = 0; lane < LANES; lane++)
-            if (!c->stage_ev[lane]) OFB_CUDA_TRY(cudaEventCreateWithFlags(&c->stage_ev[lane], cudaEventDisableTiming));
-    }
-    for (int lane = 0; lane < LANES; lane++)
-        if ((rc = ws_acquire(c, c->lane_stream[lane]))) return rc;
-    for (int first = 0, sb = 0; first < n; first += sub, sb++) {
-        const int lane = sb % LANES;
-        const int cnt = (n - first < sub) ? n - first : sub;
-        cudaStream_t st = c->lane_stream[lane];
-        uint8_t *B = c->ws + lane_bytes * lane;
-        ofb_params pc = *p;
-        pc.n_pairs = cnt;
-        if (channels == 1) {
-            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_p0, pitch0, prev_h + (size_t)first * p->w * p->h, (size_t)p->w, (size_t)p->w,
-                                           (size_t)p->h * cnt, cudaMemcpyHostToDevice, st));
-            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_n0, pitch0, next_h + (size_t)first * p->w * p->h, (size_t)p->w, (size_t)p->w,
-                                           (size_t)p->h * cnt, cudaMemcpyHostToDevice, st));
-        } else if (host_extract) {
-            uint8_t *sp = c->stage + stage_lane * lane, *sn = sp + frame_px * sub;
-            if (stage_used[lane]) OFB_CUDA_TRY(cudaEventSynchronize(c->stage_ev[lane])); // the lane's previous upload has left the buffers
-            ofb::c3_extract_pair_sets(c->pool, prev_h + c3 * first, next_h + c3 * first, sp, sn, frame_px * cnt);
-            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_p0, pitch0, sp, (size_t)p->w, (size_t)p->w, (size_t)p->h * cnt,
-                                           cudaMemcpyHostToDevice, st));
-            OFB_CUDA_TRY(cudaMemcpy2DAsync(B + off_n0, pitch0, sn, (size_t)p->w, (size_t)p->w, (size_t)p->h * cnt,
-                                           cudaMemcpyHostToDevice, st));
-            OFB_CUDA_TRY(cudaEventRecord(c->stage_ev[lane], st));
-            stage_used[lane] = true;
-        } else {
-            OFB_CUDA_TRY(cudaMemcpyAsync(B + off_c3, prev_h + c3 * first, c3 * cnt, cudaMemcpyHostToDevice, st));
-            OFB_CUDA_TRY(cudaMemcpyAsync(B + off_c3 + c3 * sub, next_h + c3 * first, c3 * cnt, cudaMemcpyHostToDevice, st));
-            rc = launch_c3_to_planar(B + off_c3, p->w, p->h, cnt, B + off_p0, pitch0, istride0, st, &c->launches);
-            if (rc) return rc;
-            rc = launch_c3_to_planar(B + off_c3 + c3 * sub, p->w, p->h, cnt, B + off_n0, pitch0, istride0, st, &c->launches);
-            if (rc) return rc;
-        }
+        return plan_base + pl.bytes;
+    };
+    auto run_sub = [&](const HostSub &s) -> int {
+        const int cnt = s.p.n_pairs;
         float *flow_d[OFB_MAX_LEVELS];
-        for (int k = 0; k < p->levels; k++) flow_d[k] = reinterpret_cast<float *>(B + off_flow[k]);
-        float *total_d = total_flow_h ? reinterpret_cast<float *>(B + off_total) : nullptr;
+        for (int k = 0; k < p->levels; k++) flow_d[k] = reinterpret_cast<float *>(s.B + off_flow[k]);
+        float *total_d = total_flow_h ? reinterpret_cast<float *>(s.B + off_total) : nullptr;
         // (one level: the total flow is the residual flow, the kernel has nothing to compose)
-        rc = run_pairs_device(c, &pc, pl, B + plan_base, B + off_p0, B + off_n0, pitch0, istride0, flow_d,
-                              p->levels > 1 ? total_d : nullptr, st);
+        int rc = run_pairs_device(c, &s.p, pl, s.B + plan_base, s.prev0, s.next0, s.pitch0, s.istride0, flow_d,
+                                  p->levels > 1 ? total_d : nullptr, s.st);
         if (rc) return rc;
         for (int k = p->levels - 1; k >= 0; k--) {
             if (!flow_levels_h || !flow_levels_h[k]) continue;
             const size_t per_pair = (size_t)(p->w >> k) * (p->h >> k) * 2; // floats
-            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k] + per_pair * first, flow_d[k], per_pair * 4 * cnt,
-                                         cudaMemcpyDeviceToHost, st));
+            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k] + per_pair * s.first, flow_d[k], per_pair * 4 * cnt,
+                                         cudaMemcpyDeviceToHost, s.st));
         }
         if (total_flow_h) {
             const size_t per_pair = (size_t)p->w * p->h * 2;
-            OFB_CUDA_TRY(cudaMemcpyAsync(total_flow_h + per_pair * first, p->levels > 1 ? total_d : flow_d[0], per_pair * 4 * cnt,
-                                         cudaMemcpyDeviceToHost, st));
+            OFB_CUDA_TRY(cudaMemcpyAsync(total_flow_h + per_pair * s.first, p->levels > 1 ? total_d : flow_d[0], per_pair * 4 * cnt,
+                                         cudaMemcpyDeviceToHost, s.st));
         }
-    }
-    for (int lane = 0; lane < LANES; lane++) OFB_CUDA_TRY(cudaStreamSynchronize(c->lane_stream[lane]));
-    return OFB_OK;
+        return OFB_OK;
+    };
+    return host_pipeline(c, p, prev_h, next_h, channels, plan_lane, run_sub);
 }
 
 int ofb_flow_pairs_host(ofb_ctx *c, const ofb_params *p, const unsigned char *prev_h, const unsigned char *next_h,
@@ -1264,6 +1308,50 @@ int ofb_flow_pairs_host_ex(ofb_ctx *c, const ofb_params *p, const unsigned char 
                            int channels, float *const *flow_levels_h, float *total_flow_h)
 {
     return flow_pairs_host_impl(c, p, prev_h, next_h, channels, flow_levels_h, total_flow_h);
+}
+
+int ofb_flow_pairs_fb_host(ofb_ctx *c, const ofb_params *p, const unsigned char *prev_h, const unsigned char *next_h, int channels,
+                           float alpha, float beta, float *fwd_total_h, float *bwd_total_h, uint8_t *status_h, float *err2_h)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_params(p);
+    if (rc) return rc;
+    if ((rc = check_fb_args(p->flow_scale, alpha, beta))) return rc;
+    if (!prev_h || !next_h || !fwd_total_h || !status_h || (channels != 1 && channels != 3)) {
+        set_error("flow_pairs_fb_host: bad arguments (NULL frame, fwd_total_h or status_h, or channels %d)", channels);
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    // a lane: both totals, status and err2 of a sub-batch, then the workspace of ofb_flow_pairs_fb_device
+    size_t off_fwd = 0, off_bwd = 0, off_status = 0, off_err2 = 0, plan_base = 0;
+    PairFbPlan fp;
+    auto plan_lane = [&](int sub, Carver *cv) {
+        const size_t px = (size_t)p->w * p->h * sub;
+        off_fwd = cv->take(px * 8);
+        off_bwd = cv->take(px * 8);
+        off_status = cv->take(px);
+        if (err2_h) off_err2 = cv->take(px * 4);
+        plan_base = cv->off;
+        ofb_params ps = *p;
+        ps.n_pairs = sub;
+        plan_pairs_fb(&ps, &fp);
+        return plan_base + fp.bytes;
+    };
+    auto run_sub = [&](const HostSub &s) -> int {
+        float *fwd = reinterpret_cast<float *>(s.B + off_fwd), *bwd = reinterpret_cast<float *>(s.B + off_bwd);
+        uint8_t *status = s.B + off_status;
+        float *err2 = err2_h ? reinterpret_cast<float *>(s.B + off_err2) : nullptr;
+        int rc = run_pairs_fb_device(c, &s.p, fp, s.B + plan_base, s.prev0, s.next0, s.pitch0, s.istride0, alpha, beta, fwd, bwd,
+                                     status, err2, s.st);
+        if (rc) return rc;
+        const size_t px = (size_t)p->w * p->h, at = px * s.first, cnt = s.p.n_pairs;
+        OFB_CUDA_TRY(cudaMemcpyAsync(fwd_total_h + 2 * at, fwd, px * 8 * cnt, cudaMemcpyDeviceToHost, s.st));
+        if (bwd_total_h) OFB_CUDA_TRY(cudaMemcpyAsync(bwd_total_h + 2 * at, bwd, px * 8 * cnt, cudaMemcpyDeviceToHost, s.st));
+        OFB_CUDA_TRY(cudaMemcpyAsync(status_h + at, status, px * cnt, cudaMemcpyDeviceToHost, s.st));
+        if (err2_h) OFB_CUDA_TRY(cudaMemcpyAsync(err2_h + at, err2, px * 4 * cnt, cudaMemcpyDeviceToHost, s.st));
+        return OFB_OK;
+    };
+    return host_pipeline(c, p, prev_h, next_h, channels, plan_lane, run_sub);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1514,7 +1602,145 @@ struct ofb_stream {
     size_t pitch[OFB_MAX_LEVELS] = {}, off_pyr[2][OFB_MAX_LEVELS] = {}, off_bgr = 0, off_gray = 0, off_lut = 0;
     size_t off_flow[OFB_MAX_LEVELS] = {}, off_cum[OFB_MAX_LEVELS] = {}, off_total = 0;
     int cur = 0; // which pyramid receives the next frame
+    // The forward-backward check (ofb_stream_push_bgr_host_fb), set up by its first call: the backward direction's residual
+    // flow, interior cumulative flow and total, status and err2 in one allocation, and a second stream with two events
+    // on which the backward level loop runs alongside the forward one.
+    uint8_t *fb_mem = nullptr;
+    size_t off_bflow[OFB_MAX_LEVELS] = {}, off_bcum[OFB_MAX_LEVELS] = {}, off_btotal = 0, off_status = 0, off_err2 = 0;
+    cudaStream_t fb_stream = nullptr;
+    cudaEvent_t fb_fork = nullptr, fb_join = nullptr;
 };
+
+namespace ofb {
+
+// Upload, grayscale (main.cu:232), bilateral pre-filter (main.cu:240) and pyramid (main.cu:250) of a new frame into the
+// stream's current pyramid, on the context stream.
+static int stream_new_frame(ofb_stream *s, const unsigned char *frame_bgr)
+{
+    ofb_ctx *c = s->ctx;
+    const ofb_params &p = s->p;
+    cudaStream_t st = c->stream;
+    uint8_t *B = s->mem;
+    const int cur = s->cur;
+    OFB_CUDA_TRY(cudaMemcpyAsync(B + s->off_bgr, frame_bgr, (size_t)p.w * p.h * 3, cudaMemcpyHostToDevice, st));
+    uint8_t *lvl0 = B + s->off_pyr[cur][0];
+    int rc = launch_grayscale(B + s->off_bgr, p.w, p.h, nullptr, s->bil_win ? B + s->off_gray : lvl0, s->pitch[0], st,
+                              &c->launches);
+    if (rc) return rc;
+    if (s->bil_win) {
+        rc = launch_bilateral(B + s->off_gray, B + s->off_gray, s->pitch[0], 1, p.w, p.h, s->bil_win, s->bil_win, s->sig_s,
+                              s->sig_b, reinterpret_cast<double *>(B + s->off_lut), lvl0, s->pitch[0], st, &c->launches);
+        if (rc) return rc;
+    }
+    for (int k = 1; k < p.levels;) { // main.cu:250; two steps per launch where two are left
+        const bool two = pyr_fuse_enabled() && k + 1 < p.levels;
+        rc = launch_pyr_roll(B + s->off_pyr[cur][k - 1], s->pitch[k - 1], s->pitch[k - 1] * (size_t)(p.h >> (k - 1)), p.w >> (k - 1),
+                             p.h >> (k - 1), B + s->off_pyr[cur][k], s->pitch[k], s->pitch[k] * (size_t)(p.h >> k),
+                             two ? B + s->off_pyr[cur][k + 1] : nullptr, two ? s->pitch[k + 1] : 0,
+                             two ? s->pitch[k + 1] * (size_t)(p.h >> (k + 1)) : 0, 1, st, &c->launches, nullptr, nullptr, nullptr,
+                             c->sm_count);
+        if (rc) return rc;
+        k += two ? 2 : 1;
+    }
+    return OFB_OK;
+}
+
+// The buffers, stream and events of the check (see ofb_stream::fb_mem); nothing once they exist.
+static int stream_fb_setup(ofb_stream *s)
+{
+    if (s->fb_mem) return OFB_OK;
+    if (!s->fb_stream) OFB_CUDA_TRY(cudaStreamCreateWithFlags(&s->fb_stream, cudaStreamNonBlocking));
+    if (!s->fb_fork) OFB_CUDA_TRY(cudaEventCreateWithFlags(&s->fb_fork, cudaEventDisableTiming));
+    if (!s->fb_join) OFB_CUDA_TRY(cudaEventCreateWithFlags(&s->fb_join, cudaEventDisableTiming));
+    const ofb_params &p = s->p;
+    Carver cv;
+    for (int k = 0; k < p.levels; k++) {
+        s->off_bflow[k] = cv.take((size_t)(p.w >> k) * (p.h >> k) * 8);
+        if (k >= 1 && k <= p.levels - 2) s->off_bcum[k] = cv.take((size_t)(p.w >> k) * (p.h >> k) * 8);
+    }
+    const size_t px = (size_t)p.w * p.h;
+    s->off_btotal = cv.take(px * 8);
+    s->off_status = cv.take(px);
+    s->off_err2 = cv.take(px * 4);
+    cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&s->fb_mem), cv.off);
+    if (e != cudaSuccess) {
+        s->fb_mem = nullptr;
+        set_error("stream forward-backward cudaMalloc(%zu) failed: %s", cv.off, cudaGetErrorString(e));
+        cudaGetLastError();
+        return OFB_ERR_NOMEM;
+    }
+    return OFB_OK;
+}
+
+// Backward level loop on the stream's second CUDA stream, concurrently with the forward one (OFB_FB_SERIAL=1: after it, on the
+// context stream; a developer switch for A/B measurements).
+static bool fb_serial()
+{
+    static const bool on = [] {
+        const char *e = getenv("OFB_FB_SERIAL");
+        return e && e[0] == '1';
+    }();
+    return on;
+}
+
+// Both directions on the stream's two pyramids, with the level loop of ofb_flow_pairs_fb_device, then the check and the
+// downloads, on the context stream.  The two loops read only the pyramids and write disjoint buffers: forked after the
+// pyramid and joined before the check, the backward one runs beside the forward one and shortens the chain of one pair's
+// small kernels.
+static int stream_fb_pair(ofb_stream *s, float alpha, float beta, float *const *flow_levels_h, float *fwd_total_h,
+                          float *bwd_total_h, uint8_t *status_h, float *err2_h)
+{
+    ofb_ctx *c = s->ctx;
+    const ofb_params &p = s->p;
+    const int L = p.levels;
+    cudaStream_t st = c->stream;
+    uint8_t *B = s->mem, *F = s->fb_mem;
+    PairPlan pl; // (run_levels reads the level sizes from it)
+    pl.L = L;
+    size_t istr[OFB_MAX_LEVELS];
+    const uint8_t *prv_lv[OFB_MAX_LEVELS], *cur_lv[OFB_MAX_LEVELS];
+    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS] = {};
+    for (int k = 0; k < L; k++) {
+        pl.w[k] = p.w >> k;
+        pl.h[k] = p.h >> k;
+        istr[k] = s->pitch[k] * (size_t)pl.h[k];
+        prv_lv[k] = B + s->off_pyr[s->cur ^ 1][k];
+        cur_lv[k] = B + s->off_pyr[s->cur][k];
+        flow[0][k] = reinterpret_cast<float *>(B + s->off_flow[k]);
+        flow[1][k] = reinterpret_cast<float *>(F + s->off_bflow[k]);
+        if (k >= 1 && k <= L - 2) {
+            cum[0][k] = reinterpret_cast<float *>(B + s->off_cum[k]);
+            cum[1][k] = reinterpret_cast<float *>(F + s->off_bcum[k]);
+        }
+    }
+    float *fwd = reinterpret_cast<float *>(B + s->off_total), *bwd = reinterpret_cast<float *>(F + s->off_btotal);
+    auto backward = [&](cudaStream_t bst) { return run_levels(c, &p, pl, cur_lv, prv_lv, s->pitch, istr, flow[1], cum[1], bwd, bst); };
+    const bool fork = !fb_serial();
+    int rc;
+    if (fork) {
+        OFB_CUDA_TRY(cudaEventRecord(s->fb_fork, st));
+        OFB_CUDA_TRY(cudaStreamWaitEvent(s->fb_stream, s->fb_fork, 0));
+        if ((rc = backward(s->fb_stream))) return rc;
+        OFB_CUDA_TRY(cudaEventRecord(s->fb_join, s->fb_stream));
+    }
+    if ((rc = run_levels(c, &p, pl, prv_lv, cur_lv, s->pitch, istr, flow[0], cum[0], fwd, st))) return rc;
+    if (fork) OFB_CUDA_TRY(cudaStreamWaitEvent(st, s->fb_join, 0));
+    else if ((rc = backward(st))) return rc;
+    uint8_t *status = F + s->off_status;
+    float *err2 = err2_h ? reinterpret_cast<float *>(F + s->off_err2) : nullptr;
+    if ((rc = run_fb_check(c, fwd, bwd, p.w, p.h, 1, p.flow_scale, alpha, beta, status, err2, st))) return rc;
+    for (int k = L - 1; k >= 0; k--)
+        if (flow_levels_h && flow_levels_h[k])
+            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k], flow[0][k], (size_t)pl.w[k] * pl.h[k] * 8, cudaMemcpyDeviceToHost, st));
+    const size_t px = (size_t)p.w * p.h;
+    OFB_CUDA_TRY(cudaMemcpyAsync(fwd_total_h, fwd, px * 8, cudaMemcpyDeviceToHost, st));
+    if (bwd_total_h) OFB_CUDA_TRY(cudaMemcpyAsync(bwd_total_h, bwd, px * 8, cudaMemcpyDeviceToHost, st));
+    OFB_CUDA_TRY(cudaMemcpyAsync(status_h, status, px, cudaMemcpyDeviceToHost, st));
+    if (err2_h) OFB_CUDA_TRY(cudaMemcpyAsync(err2_h, err2, px * 4, cudaMemcpyDeviceToHost, st));
+    return OFB_OK;
+}
+
+} // namespace ofb
 
 extern "C" {
 
@@ -1590,6 +1816,13 @@ int ofb_stream_destroy(ofb_stream *s)
         if (g.ok) {
             cudaStreamSynchronize(s->ctx->stream);
             if (s->mem) cudaFree(s->mem);
+            if (s->fb_stream) {
+                cudaStreamSynchronize(s->fb_stream);
+                cudaStreamDestroy(s->fb_stream);
+            }
+            if (s->fb_mem) cudaFree(s->fb_mem);
+            if (s->fb_fork) cudaEventDestroy(s->fb_fork);
+            if (s->fb_join) cudaEventDestroy(s->fb_join);
         }
     }
     delete s;
@@ -1621,27 +1854,8 @@ int ofb_stream_push_bgr_host(ofb_stream *s, const unsigned char *frame_bgr, floa
     uint8_t *B = s->mem;
     const int cur = s->cur, prv = cur ^ 1;
     if (has_flow) *has_flow = 0;
-    // upload, grayscale (main.cu:232), bilateral pre-filter (main.cu:240) into level 0 of the current pyramid
-    OFB_CUDA_TRY(cudaMemcpyAsync(B + s->off_bgr, frame_bgr, (size_t)p.w * p.h * 3, cudaMemcpyHostToDevice, st));
-    uint8_t *lvl0 = B + s->off_pyr[cur][0];
-    int rc = launch_grayscale(B + s->off_bgr, p.w, p.h, nullptr, s->bil_win ? B + s->off_gray : lvl0, s->pitch[0], st,
-                              &c->launches);
+    int rc = stream_new_frame(s, frame_bgr);
     if (rc) return rc;
-    if (s->bil_win) {
-        rc = launch_bilateral(B + s->off_gray, B + s->off_gray, s->pitch[0], 1, p.w, p.h, s->bil_win, s->bil_win, s->sig_s,
-                              s->sig_b, reinterpret_cast<double *>(B + s->off_lut), lvl0, s->pitch[0], st, &c->launches);
-        if (rc) return rc;
-    }
-    for (int k = 1; k < p.levels;) { // main.cu:250; two steps per launch where two are left
-        const bool two = pyr_fuse_enabled() && k + 1 < p.levels;
-        rc = launch_pyr_roll(B + s->off_pyr[cur][k - 1], s->pitch[k - 1], s->pitch[k - 1] * (size_t)(p.h >> (k - 1)), p.w >> (k - 1),
-                             p.h >> (k - 1), B + s->off_pyr[cur][k], s->pitch[k], s->pitch[k] * (size_t)(p.h >> k),
-                             two ? B + s->off_pyr[cur][k + 1] : nullptr, two ? s->pitch[k + 1] : 0,
-                             two ? s->pitch[k + 1] * (size_t)(p.h >> (k + 1)) : 0, 1, st, &c->launches, nullptr, nullptr, nullptr,
-                             c->sm_count);
-        if (rc) return rc;
-        k += two ? 2 : 1;
-    }
     if (s->frames > 0) {
         for (int k = p.levels - 1; k >= 0; k--) { // main.cu:256-262
             LkLevelArgs a{};
@@ -1677,6 +1891,37 @@ int ofb_stream_push_bgr_host(ofb_stream *s, const unsigned char *frame_bgr, floa
     }
     OFB_CUDA_TRY(cudaStreamSynchronize(st));
     s->cur = prv; // main.cu:270-272: the current pyramid becomes the previous one
+    s->frames++;
+    return OFB_OK;
+}
+
+int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, float alpha, float beta, float *const *flow_levels_h,
+                                float *fwd_total_h, float *bwd_total_h, uint8_t *status_h, float *err2_h, int *has_flow)
+{
+    if (!s || !frame_bgr || !fwd_total_h || !status_h) {
+        set_error("stream_push_fb: NULL stream, frame, fwd_total_h or status_h");
+        return OFB_ERR_INVALID;
+    }
+    ofb_ctx *c = s->ctx;
+    const ofb_params &p = s->p;
+    int rc = check_fb_args(p.flow_scale, alpha, beta);
+    if (rc) return rc;
+    OFB_GUARD(c);
+    // (before anything is enqueued: a failed set-up leaves the sequence where it was)
+    if ((rc = stream_fb_setup(s))) return rc;
+    cudaStream_t st = c->stream;
+    if (has_flow) *has_flow = 0;
+    if ((rc = stream_new_frame(s, frame_bgr))) return rc;
+    if (s->frames > 0) {
+        if ((rc = stream_fb_pair(s, alpha, beta, flow_levels_h, fwd_total_h, bwd_total_h, status_h, err2_h))) {
+            // (a failure after the fork: the backward loop may still read the pyramid the next push overwrites)
+            cudaStreamSynchronize(s->fb_stream);
+            return rc;
+        }
+        if (has_flow) *has_flow = 1;
+    }
+    OFB_CUDA_TRY(cudaStreamSynchronize(st));
+    s->cur ^= 1;
     s->frames++;
     return OFB_OK;
 }

@@ -361,6 +361,28 @@ int ofb_flow_pairs_fb_device(ofb_ctx *ctx, const ofb_params *p, const uint8_t *p
                              size_t pitch_bytes, size_t image_stride_bytes, float alpha, float beta, float *fwd_total_d,
                              float *bwd_total_d, uint8_t *status_d, float *err2_d, void *stream);
 int ofb_ctx_reserve_pairs_fb(ofb_ctx *ctx, const ofb_params *p); /* workspace for the call above (CUDA graph capture) */
+/* The same with HOST buffers, synchronous: frames as in ofb_flow_pairs_host_ex (channels = 1: planar gray, 3: the
+ * reference layout, channel 0 read; ofb_ctx_set_host_threads applies), through its sub-batch pipeline, so that uploads,
+ * compute and downloads of different sub-batches overlap (pinned host memory makes the copies asynchronous; pageable
+ * memory works too).  Each sub-batch runs what ofb_flow_pairs_fb_device runs; every output is bit-identical to that call
+ * on the same frames.  fwd_total_h (n_pairs*h*w*2 floats) and status_h (n_pairs*h*w bytes) are required; bwd_total_h
+ * (n_pairs*h*w*2 floats) and err2_h (n_pairs*h*w floats) may be NULL and are then not downloaded.  Arguments are checked as
+ * there: p->flow_scale > 0, alpha >= 0, beta >= 0. */
+int ofb_flow_pairs_fb_host(ofb_ctx *ctx, const ofb_params *p, const unsigned char *prev_h, const unsigned char *next_h,
+                           int channels, float alpha, float beta, float *fwd_total_h, float *bwd_total_h, uint8_t *status_h,
+                           float *err2_h);
+/* The check on a frame sequence (ofb_stream): ofb_stream_push_bgr_host's upload, grayscale, optional bilateral filter and
+ * pyramid of the new frame, then the flow previous->current and current->previous on the two pyramids the stream keeps,
+ * the check and the downloads.  Every output is bit-identical to ofb_flow_pairs_fb_device on the two preprocessed frames.
+ * fwd_total_h and status_h are required (h*w*2 floats, h*w bytes); flow_levels_h (forward residual flow, NULL or with NULL
+ * entries as in ofb_flow_pairs_host_ex), bwd_total_h and err2_h may be NULL.  The first push only primes the pyramid
+ * (*has_flow = 0, nothing written).  Pushes with and without the check may be mixed on one stream.  The backward level loop
+ * runs on a second CUDA stream of the sequence, beside the forward one; the buffers of the backward direction, that
+ * stream and its events are created by the first call (OFB_ERR_NOMEM, with the sequence left where it was, if the device
+ * memory cannot be had), so a sequence that never runs the check uses no more device memory than before. */
+int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, float alpha, float beta,
+                                float *const *flow_levels_h, float *fwd_total_h, float *bwd_total_h, uint8_t *status_h,
+                                float *err2_h, int *has_flow);
 
 /* Pinned host memory helpers for callers without a CUDA runtime of their own. */
 int ofb_host_alloc(void **ptr, size_t bytes);
