@@ -21,6 +21,7 @@ MAX_LEVELS, MAX_WINDOW = 8, 19
 PROFILE_PYRAMID, PROFILE_FB_CHECK = 100, 101
 # per-pixel status of the forward-backward consistency check (ofb_fb_check_device)
 FB_CONSISTENT, FB_INCONSISTENT, FB_OUTSIDE, FB_FWD_NONFINITE, FB_BWD_NONFINITE = 0, 1, 2, 3, 4
+FB_UNCHECKED = 5  # row strips only: a tap the check needs lies outside the backward rows the rank holds
 
 u8p = C.POINTER(C.c_uint8)
 f32p = C.POINTER(C.c_float)
@@ -108,6 +109,11 @@ SIGNATURES = {
     "ofb_strips_peer_connect": (C.c_int, [_vp, _vp]),
     "ofb_strips_peer_arena": (C.c_int, [_vp, C.POINTER(_vp)]),
     "ofb_strips_peer_connect_local": (C.c_int, [_vp, C.POINTER(_vp)]),
+    "ofb_strips_create_fb": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
+                                       C.c_int, _vp, C.POINTER(_vp)]),
+    "ofb_strips_run_fb_device": (C.c_int, [_vp, _vp, _vp, _sz, C.c_float, C.c_float, C.c_int, _vp]),
+    "ofb_strips_run_fb_phase_device": (C.c_int, [_vp, _vp, _vp, _sz, C.c_float, C.c_float, C.c_int, C.c_int, _vp]),
+    "ofb_strips_fb_result": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
     "ofb_conv_3ch_1ch_u8_u8_host": (C.c_int, [_vp, u8p, C.c_int, C.c_int, u8p, f32p, C.c_int, C.c_int]),
     "ofb_debug_view_host_u8c3": (C.c_int, [_vp, u8p, u8p, C.c_int, C.c_int, C.c_int, C.c_int, u8p]),
     "ofb_compose_flow_host": (C.c_int, [_vp, C.POINTER(f32p), C.c_int, C.c_int, C.c_int, C.c_int, f32p]),

@@ -156,6 +156,11 @@ int launch_compose_cum(const float *flow_k, const float *cum_coarser, int w, int
 // ---- forward-backward consistency check (fb_check.cu) ---------------------------------------
 int launch_fb_check(const float *fwd, const float *bwd, int w, int h, int n_pairs, float flow_scale, float alpha, float beta,
                     uint8_t *status, float *err2, cudaStream_t stream, unsigned long long *launches);
+// row strips (strips.cu): own rows [y0, y0 + rows) against backward rows [b0, b1); bit 2 of *flag for UNCHECKED pixels
+int launch_fb_check_strip(const float *fwd, const float *bwd_rows, int w, int h, int y0, int rows, int b0, int b1, float flow_scale,
+                          float alpha, float beta, uint8_t *status, float *err2, int *flag, cudaStream_t stream,
+                          unsigned long long *launches);
+int preload_fb_check_strip();
 
 int launch_grayscale(const uint8_t *src_c3, int w, int h, uint8_t *dst_c3, uint8_t *dst_planar, size_t dst_pitch,
                      cudaStream_t stream, unsigned long long *launches);

@@ -22,6 +22,7 @@
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <mutex>
 #include <new>
@@ -97,7 +98,15 @@ struct LevelStrip {
 };
 struct StripPlan {
     int W, H, levels, win, world, reach, r, img_halo;
+    int fb_reach = -1; // >= 0: handle of ofb_strips_create_fb (checked pairs); level-0 backward rows beyond the own rows held
     std::vector<int> coarse_bounds;
+    // rows [lo, hi) of the level-0 backward total flow that `rank`'s check holds
+    void fb_rows(int rank, int *lo, int *hi) const
+    {
+        const LevelStrip s = level(0, rank);
+        *lo = std::max(0, s.y0 - fb_reach);
+        *hi = std::min(H, s.y1 + fb_reach + 1);
+    }
     LevelStrip level(int k, int rank) const
     {
         const int sh = levels - 1 - k;
@@ -138,19 +147,28 @@ struct StripPlan {
 };
 
 // ---- peer-memory transport ------------------------------------------------------------------------------------
-// Arena of one rank: [prev level 0][next level 0][cum_in level 0 .. L-2][flags].  Every rank can compute every other
-// rank's layout from the plan, so a peer address is (peer arena base) + (offset computed here).
+// Arena of one rank: [prev level 0][next level 0][cum_in level 0 .. L-2][flags]; a handle that runs checked pairs also has
+// [cum_in_b level 0 .. L-2][fbh: held rows of the backward total flow] before the flags.  Every rank can compute every
+// other rank's layout from the plan, so a peer address is (peer arena base) + (offset computed here).
 constexpr int PEER_MAX_SEG = 8;   // copy segments per exchange (prev + next rows per destination)
 constexpr int PEER_MAX_DST = 4;   // ranks one exchange sends to / receives from
 struct ArenaLayout {
-    size_t prev0, next0, cum_in[OFB_MAX_LEVELS], flags, bytes;
+    size_t prev0, next0, cum_in[OFB_MAX_LEVELS], cum_in_b[OFB_MAX_LEVELS], fbh, flags, bytes;
+    // Exchanges of a pair: 0 = level-0 images, 1 .. L-1 = forward cumulative flow; a checked pair adds L .. 2L-2 = backward
+    // cumulative flow and 2L-1 = backward total rows for the check.  nx = L (plain handle) or 2L.
+    int world, nx;
     // flags (unsigned): arrive[x * world + src] = epoch of the last exchange x that src completed into this arena;
-    //                   done[src] at L * world + src = last epoch rank src finished reading what this rank pushed;
-    //                   counter[x] at (L + 1) * world + x: blocks of this rank's push kernel that have finished (local);
-    //                   pairs at (L + 1) * world + L: pairs this rank has completed (local).  The epoch of a pair is
+    //                   done[src] at nx * world + src = last epoch rank src finished reading what this rank pushed;
+    //                   counter[x] at (nx + 1) * world + x: blocks of this rank's push kernel that have finished (local);
+    //                   pairs at (nx + 1) * world + nx: pairs this rank has completed (local).  The epoch of a pair is
     //                   pairs + 1, read from here by the kernels, so that a captured CUDA graph of one pair replays;
     //                   fused[2 * x + d] after that: CTAs of the level kernel that have pushed their rows of exchange x to
     //                   target d (local; the halo push fused into the level kernels).
+    size_t arrive(int x, int src) const { return (size_t)x * world + src; }
+    size_t done(int src) const { return (size_t)nx * world + src; }
+    size_t counter(int x) const { return (size_t)(nx + 1) * world + x; }
+    size_t pairs() const { return (size_t)(nx + 1) * world + nx; }
+    size_t fused(int x) const { return pairs() + 1 + 2 * (size_t)x; }
 };
 static ArenaLayout arena_layout(const StripPlan &pl, int rank)
 {
@@ -166,7 +184,16 @@ static ArenaLayout arena_layout(const StripPlan &pl, int rank)
     a.prev0 = take(pitch0 * (v[0].eb1 - v[0].eb0));
     a.next0 = take(pitch0 * (v[0].eb1 - v[0].eb0));
     for (int k = 0; k < pl.levels; k++) a.cum_in[k] = take((size_t)(v[k].w >> 1) * std::max(v[k].cy1 - v[k].cy0, 1) * 8);
-    a.flags = take(((size_t)(pl.levels + 1) * pl.world + pl.levels + 1 + 2 * (size_t)pl.levels) * sizeof(unsigned));
+    a.world = pl.world;
+    a.nx = pl.levels;
+    if (pl.fb_reach >= 0) {
+        for (int k = 0; k < pl.levels; k++) a.cum_in_b[k] = take((size_t)(v[k].w >> 1) * std::max(v[k].cy1 - v[k].cy0, 1) * 8);
+        int lo, hi;
+        pl.fb_rows(rank, &lo, &hi);
+        a.fbh = take((size_t)v[0].w * (hi - lo) * 8);
+        a.nx = 2 * pl.levels;
+    }
+    a.flags = take((a.pairs() + 1 + 2 * (size_t)a.nx) * sizeof(unsigned));
     a.bytes = off;
     return a;
 }
@@ -311,6 +338,13 @@ struct ofb_strips {
     std::vector<void *> ipc_opened;
     bool peers_connected = false;
     std::vector<int> done_from;             // ranks this one pushes to: they write done[rank] into this arena (teardown waits for it)
+    // checked pairs (ofb_strips_create_fb): the backward direction's buffers, laid out like the forward ones
+    std::vector<float *> flow_b, cum_in_b, cum_dst_b; // cum_dst_b[0]: level 0's rows inside fbh
+    float *fbh = nullptr;                   // backward total flow, rows [hy0, hy1) of level 0 (in the arena)
+    int hy0 = 0, hy1 = 0;
+    uint8_t *status = nullptr;              // own rows [y0, y1) of level 0
+    float *err2 = nullptr;
+    std::vector<int> fb_sources;            // ranks whose own rows lie in [hy0, hy1): they push check rows to this one
 };
 
 namespace {
@@ -321,6 +355,8 @@ int dev_alloc(ofb_strips *st, void **p, size_t bytes)
     st->allocs.push_back(*p);
     return OFB_OK;
 }
+// pixels of the own rows of level 0
+inline size_t s_own_px(const ofb_strips *st) { return (size_t)st->s[0].w * (st->s[0].y1 - st->s[0].y0); }
 // rows [lo, hi) that `owner` owns and `peer`'s buffer [b0, b1) holds
 inline bool overlap(int own0, int own1, int b0, int b1, int *lo, int *hi)
 {
@@ -345,8 +381,8 @@ inline unsigned *flag_ptr(uint8_t *arena, const ArenaLayout &lay, size_t index)
 int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, const std::vector<int> &sources, cudaStream_t q,
                   unsigned long long *launches, bool do_push = true, bool do_wait = true)
 {
-    const int world = st->plan.world, L = st->plan.levels, me = st->rank;
-    unsigned *pairs = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * world + L);
+    const int me = st->rank;
+    unsigned *pairs = flag_ptr(st->arena, st->lay, st->lay.pairs());
     if (do_push && !sends.empty()) {
         PeerPushArgs a{};
         size_t total = 0;
@@ -358,19 +394,19 @@ int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, con
             a.seg[a.nseg++] = PeerSeg{sd.src, st->peer_arena[sd.peer] + sd.dst_off, sd.bytes};
             total += sd.bytes;
             bool seen = false;
-            for (int d = 0; d < a.ndst; d++) seen |= a.arrive[d] == flag_ptr(st->peer_arena[sd.peer], st->peer_lay[sd.peer], (size_t)x * world + me);
+            for (int d = 0; d < a.ndst; d++) seen |= a.arrive[d] == flag_ptr(st->peer_arena[sd.peer], st->peer_lay[sd.peer], st->peer_lay[sd.peer].arrive(x, me));
             if (!seen) {
                 if (a.ndst == PEER_MAX_DST) {
                     set_error("strips: exchange %d sends to more than %d ranks", x, PEER_MAX_DST);
                     return OFB_ERR_UNSUPPORTED;
                 }
-                a.arrive[a.ndst] = flag_ptr(st->peer_arena[sd.peer], st->peer_lay[sd.peer], (size_t)x * world + me);
-                a.done_local[a.ndst] = flag_ptr(st->arena, st->lay, (size_t)L * world + sd.peer);
+                a.arrive[a.ndst] = flag_ptr(st->peer_arena[sd.peer], st->peer_lay[sd.peer], st->peer_lay[sd.peer].arrive(x, me));
+                a.done_local[a.ndst] = flag_ptr(st->arena, st->lay, st->lay.done(sd.peer));
                 a.ndst++;
                 if (std::find(st->done_from.begin(), st->done_from.end(), sd.peer) == st->done_from.end()) st->done_from.push_back(sd.peer);
             }
         }
-        a.counter = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * world + x);
+        a.counter = flag_ptr(st->arena, st->lay, st->lay.counter(x));
         a.pairs = pairs;
         a.err = st->overflow;
         const unsigned blocks = (unsigned)std::min<size_t>(64, std::max<size_t>(1, total / (256 * 64)));
@@ -385,7 +421,7 @@ int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, con
                 set_error("strips: exchange %d receives from more than %d ranks", x, PEER_MAX_DST);
                 return OFB_ERR_UNSUPPORTED;
             }
-            w.flag[w.n++] = flag_ptr(st->arena, st->lay, (size_t)x * world + src);
+            w.flag[w.n++] = flag_ptr(st->arena, st->lay, st->lay.arrive(x, src));
         }
         w.pairs = pairs;
         w.err = st->overflow;
@@ -448,13 +484,20 @@ int ofb_strips_nccl_unique_id(void *id128)
     return OFB_OK;
 }
 
-int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                      int reach, const void *nccl_id128, ofb_strips **out)
+} // extern "C"
+
+// ofb_strips_create (fb_reach < 0) and ofb_strips_create_fb
+static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
+                              int reach, int fb_reach, const void *nccl_id128, ofb_strips **out)
 {
     if (!ctx || !out || w < 1 || h < 1 || levels < 1 || levels > OFB_MAX_LEVELS || (win & 1) == 0 || win < 3 ||
         win > OFB_MAX_WINDOW || world < 1 || rank < 0 || rank >= world || reach < 0) {
         set_error("strips_create: bad arguments");
         return OFB_ERR_INVALID;
+    }
+    if (fb_reach >= 0 && world > 1 && nccl_id128) {
+        set_error("strips_create_fb: checked pairs run on the peer-memory transport (nccl_id128 = NULL) or on one rank");
+        return OFB_ERR_UNSUPPORTED;
     }
     if (warp_mode == OFB_WARP_AS_WRITTEN && levels > 1) {
         set_error("OFB_WARP_AS_WRITTEN needs pixel (0,0) of every coarser level: not available on strips");
@@ -479,6 +522,7 @@ int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_
     st->flow_scale = flow_scale;
     StripPlan &pl = st->plan;
     pl.W = w, pl.H = h, pl.levels = levels, pl.win = win, pl.world = world, pl.reach = reach;
+    pl.fb_reach = fb_reach;
     pl.r = win / 2;
     // image halo: 3x3 stencil + window radius + one row of even-row alignment + warp reach + bilinear tap
     pl.img_halo = pl.r + 2 + reach + 2;
@@ -520,6 +564,33 @@ int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_
         st->cum.push_back(static_cast<float *>(p));
         st->cum_in.push_back(reinterpret_cast<float *>(st->arena + st->lay.cum_in[k]));
     }
+    if (fb_reach >= 0) {
+        pl.fb_rows(rank, &st->hy0, &st->hy1);
+        st->fbh = reinterpret_cast<float *>(st->arena + st->lay.fbh);
+        for (int peer = 0; peer < world; peer++) {
+            const LevelStrip ps = pl.level(0, peer);
+            int lo, hi;
+            if (peer != rank && overlap(ps.y0, ps.y1, st->hy0, st->hy1, &lo, &hi)) st->fb_sources.push_back(peer);
+        }
+        const size_t own = s_own_px(st);
+        void *p = nullptr;
+        if (rc == OFB_OK) rc = dev_alloc(st, &p, own);
+        st->status = static_cast<uint8_t *>(p);
+        p = nullptr;
+        if (rc == OFB_OK) rc = dev_alloc(st, &p, own * 4);
+        st->err2 = static_cast<float *>(p);
+        for (int k = 0; k < levels && rc == OFB_OK; k++) {
+            const LevelStrip s = st->s[k];
+            if ((rc = dev_alloc(st, &p, (size_t)s.w * (s.eb1 - s.eb0) * 8))) break;
+            st->flow_b.push_back(static_cast<float *>(p));
+            st->cum_in_b.push_back(reinterpret_cast<float *>(st->arena + st->lay.cum_in_b[k]));
+        }
+        for (int k = 0; k < levels && rc == OFB_OK; k++) {
+            const LevelStrip &s = st->s[k];
+            st->cum_dst_b.push_back(k == 0 ? st->fbh + ((ptrdiff_t)s.eb0 - st->hy0) * (ptrdiff_t)s.w * 2
+                                           : st->cum_in_b[k - 1] + ((ptrdiff_t)s.eb0 - st->s[k - 1].cy0) * (ptrdiff_t)s.w * 2);
+        }
+    }
     for (int k = 0; k < levels && rc == OFB_OK; k++) {
         // buffer row b of level k is global row eb0 + b; row g of cum_in[k-1] sits at (g - cy0) * w
         float *dst = st->cum[k];
@@ -558,6 +629,7 @@ int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_
     // launch, which must not happen behind a kernel that waits for a neighbour
     if (rc == OFB_OK) rc = preload_lk_level(win);
     if (rc == OFB_OK) rc = preload_pyramid();
+    if (rc == OFB_OK && fb_reach >= 0) rc = preload_fb_check_strip();
     if (rc == OFB_OK) {
         cudaFuncAttributes fa;
         if (cudaFuncGetAttributes(&fa, peer_push_kernel) != cudaSuccess || cudaFuncGetAttributes(&fa, peer_wait_kernel) != cudaSuccess ||
@@ -583,6 +655,24 @@ int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_
     }
     *out = st;
     return OFB_OK;
+}
+
+extern "C" {
+
+int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
+                      int reach, const void *nccl_id128, ofb_strips **out)
+{
+    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, -1, nccl_id128, out);
+}
+
+int ofb_strips_create_fb(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
+                         int reach, int fb_reach, const void *nccl_id128, ofb_strips **out)
+{
+    if (fb_reach < 0 || !(std::isfinite(flow_scale) && flow_scale > 0.0f)) {
+        set_error("strips_create_fb: fb_reach %d must be >= 0 and flow_scale %g finite and > 0", fb_reach, (double)flow_scale);
+        return OFB_ERR_INVALID;
+    }
+    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, fb_reach, nccl_id128, out);
 }
 
 // ---- peer-memory transport: set-up -------------------------------------------------------------------------------
@@ -641,6 +731,11 @@ bool is_neighbour(const ofb_strips *st, int peer)
     for (int k = 0; k + 1 < pl.levels; k++) {
         const LevelStrip up = st->s[k + 1], sk = st->s[k], pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
         if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi) || overlap(pu.y0, pu.y1, sk.cy0, sk.cy1, &lo, &hi)) return true;
+    }
+    if (pl.fb_reach >= 0) { // backward total rows for the check, in either direction
+        int plo, phi;
+        pl.fb_rows(peer, &plo, &phi);
+        if (overlap(s.y0, s.y1, plo, phi, &lo, &hi) || overlap(ps.y0, ps.y1, st->hy0, st->hy1, &lo, &hi)) return true;
     }
     return false;
 }
@@ -705,10 +800,9 @@ int ofb_strips_destroy(ofb_strips *st)
             cudaDeviceSynchronize();
             if (st->plan.world > 1 && st->peers_connected && !st->comm && !st->done_from.empty()) {
                 PeerDrainArgs d{};
-                const int L = st->plan.levels, world = st->plan.world;
                 for (int dst : st->done_from)
-                    if (d.n < 2 * PEER_MAX_DST) d.flag[d.n++] = flag_ptr(st->arena, st->lay, (size_t)L * world + dst);
-                d.pairs = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * world + L);
+                    if (d.n < 2 * PEER_MAX_DST) d.flag[d.n++] = flag_ptr(st->arena, st->lay, st->lay.done(dst));
+                d.pairs = flag_ptr(st->arena, st->lay, st->lay.pairs());
                 d.err = st->overflow;
                 peer_drain_kernel<<<1, 32>>>(d);
                 cudaDeviceSynchronize();
@@ -786,19 +880,198 @@ int ofb_strips_set_fused(ofb_strips *st, int on)
     return OFB_OK;
 }
 
+} // extern "C"
+
+namespace {
+// The coarse-to-fine level loop of one direction of a pair: forward (prev -> next) or, in a checked pair, backward
+// (next -> prev on the same pyramid, with its own residual-flow buffers, cum_in regions and exchanges).  Level k's
+// neighbours' cumulative-flow rows arrive by exchange xb + L - 1 - k; the loop's phases start at pb (see
+// strips_run_impl).  In the backward loop of a checked pair level 0 writes the backward total into fbh, and -- fused
+// form, at most two targets -- its kernel also pushes the rows the neighbours' checks need (*check_pushed).
+int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream_t q, int phase, std::vector<int> &all_sources,
+                  bool *check_pushed, unsigned long long *launches)
+{
+    auto on = [phase](int ph) { return phase < 0 || phase == ph; };
+    const StripPlan &pl = st->plan;
+    const bool peer_mode = pl.world > 1 && !st->comm;
+    const int L = pl.levels, me = st->rank;
+    const int pb = bwd ? 2 * L - 1 : 0, xb = bwd ? L - 1 : 0;
+    const std::vector<float *> &flow = bwd ? st->flow_b : st->flow, &cum_in = bwd ? st->cum_in_b : st->cum_in;
+    const std::vector<float *> &cum_dst = bwd ? st->cum_dst_b : st->cum_dst;
+    auto peer_cum_in = [&](int peer, int k) { return bwd ? st->peer_lay[peer].cum_in_b[k] : st->peer_lay[peer].cum_in[k]; };
+    // coarse to fine: rows [cy0, cy1) of cum_{k+1} into cum_in[k] (own part copied, the rest received), then the level
+    bool pushed_by_kernel = false; // the exchange that feeds the level at hand was pushed by the previous (coarser) level's kernel
+    for (int k = L - 1; k >= 0; k--) {
+        const LevelStrip &s = st->s[k];
+        struct WaitSrc {
+            int peer, crow_lo, crow_hi;
+        } wait_src[2] = {};
+        int nwait = 0;
+        bool wait_in_kernel = false;
+        const int j = L - 1 - k; // this level's step of the loop
+        if (k < L - 1) {
+            const LevelStrip &up = st->s[k + 1];
+            // level k+1 wrote its own rows of cum_{k+1} straight into cum_in[k] (cum_dst); the neighbours' rows follow
+            const float *src = cum_dst[k + 1]; // buffer-row indexing of level k+1 (origin up.eb0)
+            const size_t rowf = (size_t)up.w * 2;  // floats per row
+            int lo, hi;
+            if (n) {
+                OFB_NCCL_TRY(n->GroupStart());
+                for (int peer = 0; peer < pl.world; peer++) {
+                    if (peer == me) continue;
+                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
+                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
+                        OFB_NCCL_TRY(n->Send(src + (size_t)(lo - up.eb0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer, st->comm, q));
+                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) // the peer's cum rows I need
+                        OFB_NCCL_TRY(n->Recv(cum_in[k] + (size_t)(lo - s.cy0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer,
+                                             st->comm, q));
+                }
+                OFB_NCCL_TRY(n->GroupEnd());
+            }
+            if (peer_mode) {
+                std::vector<PeerSend> sends;
+                std::vector<int> sources;
+                for (int peer = 0; peer < pl.world; peer++) {
+                    if (peer == me) continue;
+                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
+                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
+                        sends.push_back({peer, src + (size_t)(lo - up.eb0) * rowf, peer_cum_in(peer, k) + (size_t)(lo - pk.cy0) * rowf * 4,
+                                         (size_t)(hi - lo) * rowf * 4});
+                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) { // the peer's cum rows I need
+                        sources.push_back(peer);
+                        add_unique(all_sources, peer);
+                        if (nwait < 2) wait_src[nwait] = {peer, lo - s.cy0, hi - s.cy0};
+                        nwait++;
+                    }
+                }
+                // Fused form: level k+1's kernel has already pushed my rows (pushed_by_kernel, previous iteration) and this
+                // level's kernel waits for the neighbours' flags itself; the copy / wait kernels remain for what does not
+                // fit the kernel's two slots (strips thinner than the halo).
+                wait_in_kernel = st->fused && nwait >= 1 && nwait <= 2;
+                int rc = peer_exchange(st, xb + j, sends, sources, q, launches, on(pb + 2 * j) && !pushed_by_kernel,
+                                       on(pb + 2 * j + 1) && !wait_in_kernel);
+                if (rc) return rc;
+            }
+        }
+        // what THIS level's kernel pushes: my rows of cum_k that the neighbours' level k-1 needs (exchange xb + L - k), or,
+        // at level 0 of the backward loop of a checked pair, my rows of the backward total their checks need (2L - 1)
+        LkLevelArgs::PeerPush push[2] = {};
+        int npush = 0, xn = 0;
+        pushed_by_kernel = false;
+        if (peer_mode && st->fused && (k >= 1 || (bwd && checked))) {
+            int cnt = 0, lo, hi;
+            xn = k >= 1 ? xb + L - k : 2 * L - 1;
+            for (int peer = 0; peer < pl.world; peer++) {
+                if (peer == me) continue;
+                int plo, phi;
+                if (k >= 1) { // the peer's finer level reads rows [cy0, cy1) of cum_k
+                    const LevelStrip pf = pl.level(k - 1, peer);
+                    plo = pf.cy0, phi = pf.cy1;
+                } else {
+                    pl.fb_rows(peer, &plo, &phi);
+                }
+                if (!overlap(s.y0, s.y1, plo, phi, &lo, &hi)) continue;
+                if (cnt < 2 && st->peer_arena[peer]) {
+                    const ArenaLayout &pa = st->peer_lay[peer];
+                    push[cnt].dst = reinterpret_cast<float *>(st->peer_arena[peer] + (k >= 1 ? peer_cum_in(peer, k - 1) : pa.fbh)) +
+                                    ((ptrdiff_t)s.eb0 - plo) * (ptrdiff_t)s.w * 2;
+                    push[cnt].row_lo = lo - s.eb0;
+                    push[cnt].row_hi = hi - s.eb0;
+                    push[cnt].flag = flag_ptr(st->peer_arena[peer], pa, pa.arrive(xn, me));
+                    push[cnt].done = flag_ptr(st->arena, st->lay, st->lay.done(peer));
+                    add_unique(st->done_from, peer);
+                }
+                cnt++;
+            }
+            if (cnt >= 1 && cnt <= 2) {
+                npush = cnt;
+                pushed_by_kernel = true;
+            }
+        }
+        if (k == 0 && bwd) *check_pushed = pushed_by_kernel;
+        if (!on(pb + 2 * j + 1)) continue;
+        LkLevelArgs a{};
+        a.prev = bwd ? st->next[k] : st->prev[k];
+        a.next = bwd ? st->prev[k] : st->next[k];
+        a.pitch = st->pitch[k];
+        a.image_stride = a.pitch * (size_t)(s.eb1 - s.eb0);
+        a.w = s.w;
+        a.h_local = s.eb1 - s.eb0;
+        a.y_off = s.eb0;
+        a.h_global = s.h;
+        a.out_y0 = s.y0 - s.eb0;
+        a.out_y1 = s.y1 - s.eb0;
+        a.n_pairs = 1;
+        a.win = pl.win;
+        a.warp_mode = st->warp_mode;
+        a.flow_scale = st->flow_scale;
+        a.cum_in = k < L - 1 ? cum_in[k] : nullptr;
+        a.cum_w = s.w >> 1;
+        a.cum_h_global = s.h >> 1;
+        a.cum_y_off = s.cy0;
+        a.cum_h_local = std::max(s.cy1 - s.cy0, 1);
+        a.cum_pair_stride = 0;
+        a.flow_out = flow[k];
+        // every level but the finest feeds the next one; level 0 writes the total flow (always in a checked pair)
+        const bool want_cum = k > 0 || checked || (L > 1 && st->want_total);
+        a.cum_out = want_cum ? cum_dst[k] : nullptr;
+        a.flow_pair_stride = 0;
+        a.reach_overflow = st->overflow;
+        a.sm_count = ctx_sm_count(st->ctx);
+        a.solve_fast = ctx_solve_fast(st->ctx);
+        if (npush > 0 && a.cum_out) {
+            a.npush = npush;
+            a.push[0] = push[0];
+            a.push[1] = push[1];
+            a.push_counter = flag_ptr(st->arena, st->lay, st->lay.fused(xn));
+        }
+        if (wait_in_kernel) {
+            a.nwait = nwait;
+            for (int d = 0; d < nwait; d++)
+                a.wait[d] = {flag_ptr(st->arena, st->lay, st->lay.arrive(xb + j, wait_src[d].peer)), wait_src[d].crow_lo, wait_src[d].crow_hi};
+        }
+        a.epoch_src = flag_ptr(st->arena, st->lay, st->lay.pairs());
+        int rc = launch_lk_level(a, q, launches);
+        if (rc) return rc;
+    }
+    return OFB_OK;
+}
+} // namespace
+
 // One pair: own rows of level 0 in, residual (and cumulative) flow of the own rows of every level out, all
 // asynchronous on `stream`.  prev_own_d / next_own_d: rows [y0, y1) of level 0, planar u8 with `pitch` bytes per row.
+// fb != NULL: a checked pair (handles of ofb_strips_create_fb): the backward level loop on the same pyramid, the exchange
+// of the backward total rows the neighbours' checks sample, and the check of the own rows.
 //
-// `phase` < 0: the whole pair.  Otherwise one of its 2L phases (peer-memory transport only), so that a host can interleave
+// `phase` < 0: the whole pair.  Otherwise one of its phases (peer-memory transport only), so that a host can interleave
 // the ranks of ONE process on ONE stream in an order in which no kernel ever waits for a later one:
 //   phase 0      own-row upload, push of the level-0 image rows (exchange 0)
 //   phase 1      wait for exchange 0, pyramid, coarsest level L-1
 //   phase 2j     push of the cumulative-flow rows of level L-j (exchange j),            j = 1 .. L-1
-//   phase 2j+1   wait for exchange j, level L-1-j; after level 0 the end-of-pair handshake
-static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, void *stream, int phase)
+//   phase 2j+1   wait for exchange j, level L-1-j; after level 0 of a plain pair the end-of-pair handshake
+// and in a checked pair (4L + 1 phases):
+//   phase 2L         backward coarsest level L-1
+//   phase 2L+2j-1    push of the backward cumulative-flow rows of level L-j (exchange L-1+j), j = 1 .. L-1
+//   phase 2L+2j      wait for exchange L-1+j, backward level L-1-j
+//   phase 4L-1       push of the backward total rows the neighbours' checks sample (exchange 2L-1)
+//   phase 4L         wait for exchange 2L-1, the check, the end-of-pair handshake
+struct FbRun {
+    float alpha, beta;
+    int want_err2;
+};
+static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, void *stream, int phase,
+                           const FbRun *fb = nullptr)
 {
     if (!st || !prev_own_d || !next_own_d) {
         set_error("strips_run: bad arguments");
+        return OFB_ERR_INVALID;
+    }
+    if (fb && st->plan.fb_reach < 0) {
+        set_error("strips_run_fb: the handle was not created by ofb_strips_create_fb");
+        return OFB_ERR_INVALID;
+    }
+    if (fb && !(std::isfinite(fb->alpha) && fb->alpha >= 0.0f && std::isfinite(fb->beta) && fb->beta >= 0.0f)) {
+        set_error("strips_run_fb: alpha %g / beta %g must be finite and >= 0", (double)fb->alpha, (double)fb->beta);
         return OFB_ERR_INVALID;
     }
     OFB_STRIPS_GUARD(st);
@@ -812,13 +1085,14 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
         return OFB_ERR_INVALID;
     }
     NcclApi *n = pl.world > 1 && !peer_mode ? nccl() : nullptr;
-    if (phase >= 0 && (n || phase >= 2 * pl.levels)) {
-        set_error("strips_run_phase: phase %d of %d (phases exist for the peer-memory transport and one rank only)", phase, 2 * pl.levels);
+    const int L = pl.levels, me = st->rank;
+    const int nphase = fb ? 4 * L + 1 : 2 * L;
+    if (phase >= 0 && (n || phase >= nphase)) {
+        set_error("strips_run_phase: phase %d of %d (phases exist for the peer-memory transport and one rank only)", phase, nphase);
         return OFB_ERR_INVALID;
     }
     unsigned long long *launches = ctx_launch_counter(st->ctx);
-    const int L = pl.levels, me = st->rank;
-    std::vector<int> all_sources; // every rank that pushes to me during the pair
+    std::vector<int> all_sources = st->fb_sources; // every rank that pushes to me during a pair of either kind
     if (pitch < (size_t)pl.W) {
         set_error("strips_run: pitch %zu smaller than the width %d", pitch, pl.W);
         return OFB_ERR_INVALID;
@@ -884,141 +1158,45 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
                                        d.eb1, q, launches, 2, st->img_stride[k], st->img_stride[k + 1]);
         if (rc) return rc;
     }
-    // coarse to fine: rows [cy0, cy1) of cum_{k+1} into cum_in[k] (own part copied, the rest received), then the level
-    bool pushed_by_kernel = false; // the exchange that feeds the level at hand was pushed by the previous (coarser) level's kernel
-    for (int k = L - 1; k >= 0; k--) {
-        const LevelStrip &s = st->s[k];
-        struct WaitSrc {
-            int peer, crow_lo, crow_hi;
-        } wait_src[2] = {};
-        int nwait = 0;
-        bool wait_in_kernel = false;
-        if (k < L - 1) {
-            const LevelStrip &up = st->s[k + 1];
-            // level k+1 wrote its own rows of cum_{k+1} straight into cum_in[k] (cum_dst); the neighbours' rows follow
-            const float *src = st->cum_dst[k + 1]; // buffer-row indexing of level k+1 (origin up.eb0)
-            const size_t rowf = (size_t)up.w * 2;  // floats per row
-            int lo, hi;
-            if (n) {
-                OFB_NCCL_TRY(n->GroupStart());
-                for (int peer = 0; peer < pl.world; peer++) {
-                    if (peer == me) continue;
-                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
-                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
-                        OFB_NCCL_TRY(n->Send(src + (size_t)(lo - up.eb0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer, st->comm, q));
-                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) // the peer's cum rows I need
-                        OFB_NCCL_TRY(n->Recv(st->cum_in[k] + (size_t)(lo - s.cy0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer,
-                                             st->comm, q));
-                }
-                OFB_NCCL_TRY(n->GroupEnd());
-            }
-            if (peer_mode) {
-                std::vector<PeerSend> sends;
-                std::vector<int> sources;
-                for (int peer = 0; peer < pl.world; peer++) {
-                    if (peer == me) continue;
-                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
-                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
-                        sends.push_back({peer, src + (size_t)(lo - up.eb0) * rowf, st->peer_lay[peer].cum_in[k] + (size_t)(lo - pk.cy0) * rowf * 4,
-                                         (size_t)(hi - lo) * rowf * 4});
-                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) { // the peer's cum rows I need
-                        sources.push_back(peer);
-                        add_unique(all_sources, peer);
-                        if (nwait < 2) wait_src[nwait] = {peer, lo - s.cy0, hi - s.cy0};
-                        nwait++;
-                    }
-                }
-                const int x = L - 1 - k; // exchanges 1 .. L-1
-                // Fused form: level k+1's kernel has already pushed my rows (pushed_by_kernel, previous iteration) and this
-                // level's kernel waits for the neighbours' flags itself; the copy / wait kernels remain for what does not
-                // fit the kernel's two slots (strips thinner than the halo).
-                wait_in_kernel = st->fused && nwait >= 1 && nwait <= 2;
-                int rc = peer_exchange(st, x, sends, sources, q, launches, on(2 * x) && !pushed_by_kernel, on(2 * x + 1) && !wait_in_kernel);
-                if (rc) return rc;
-            }
-        }
-        // what THIS level's kernel pushes: my rows of cum_k that the neighbours' level k-1 needs (exchange L-k)
-        LkLevelArgs::PeerPush push[2] = {};
-        int npush = 0;
-        pushed_by_kernel = false;
-        if (peer_mode && st->fused && k >= 1) {
-            int cnt = 0, lo, hi;
+    bool check_pushed = false;
+    int rc = strips_levels(st, false, fb != nullptr, n, q, phase, all_sources, &check_pushed, launches);
+    if (rc) return rc;
+    if (fb) {
+        if ((rc = strips_levels(st, true, true, n, q, phase, all_sources, &check_pushed, launches))) return rc;
+        // exchange 2L-1: my own rows of the backward total that the neighbours' checks sample (unless level 0's kernel pushed
+        // them), then the wait for the rows I sample
+        if (peer_mode) {
+            const LevelStrip &s = st->s[0];
+            const size_t rowf = (size_t)s.w * 2;
+            std::vector<PeerSend> sends;
             for (int peer = 0; peer < pl.world; peer++) {
-                if (peer == me) continue;
-                const LevelStrip pf = pl.level(k - 1, peer); // the peer's finer level reads rows [cy0, cy1) of cum_k
-                if (!overlap(s.y0, s.y1, pf.cy0, pf.cy1, &lo, &hi)) continue;
-                if (cnt < 2 && st->peer_arena[peer]) {
-                    const int xn = L - k;
-                    push[cnt].dst = reinterpret_cast<float *>(st->peer_arena[peer] + st->peer_lay[peer].cum_in[k - 1]) +
-                                    ((ptrdiff_t)s.eb0 - pf.cy0) * (ptrdiff_t)s.w * 2;
-                    push[cnt].row_lo = lo - s.eb0;
-                    push[cnt].row_hi = hi - s.eb0;
-                    push[cnt].flag = flag_ptr(st->peer_arena[peer], st->peer_lay[peer], (size_t)xn * pl.world + me);
-                    push[cnt].done = flag_ptr(st->arena, st->lay, (size_t)L * pl.world + peer);
-                    if (std::find(st->done_from.begin(), st->done_from.end(), peer) == st->done_from.end()) st->done_from.push_back(peer);
-                }
-                cnt++;
+                int plo, phi, lo, hi;
+                pl.fb_rows(peer, &plo, &phi);
+                if (peer != me && overlap(s.y0, s.y1, plo, phi, &lo, &hi))
+                    sends.push_back({peer, st->fbh + (size_t)(lo - st->hy0) * rowf, st->peer_lay[peer].fbh + (size_t)(lo - plo) * rowf * 4,
+                                     (size_t)(hi - lo) * rowf * 4});
             }
-            if (cnt >= 1 && cnt <= 2) {
-                npush = cnt;
-                pushed_by_kernel = true;
-            }
+            if ((rc = peer_exchange(st, 2 * L - 1, sends, st->fb_sources, q, launches, on(4 * L - 1) && !check_pushed, on(4 * L))))
+                return rc;
         }
-        if (!on(2 * (L - 1 - k) + 1)) continue;
-        LkLevelArgs a{};
-        a.prev = st->prev[k];
-        a.next = st->next[k];
-        a.pitch = st->pitch[k];
-        a.image_stride = a.pitch * (size_t)(s.eb1 - s.eb0);
-        a.w = s.w;
-        a.h_local = s.eb1 - s.eb0;
-        a.y_off = s.eb0;
-        a.h_global = s.h;
-        a.out_y0 = s.y0 - s.eb0;
-        a.out_y1 = s.y1 - s.eb0;
-        a.n_pairs = 1;
-        a.win = pl.win;
-        a.warp_mode = st->warp_mode;
-        a.flow_scale = st->flow_scale;
-        a.cum_in = k < L - 1 ? st->cum_in[k] : nullptr;
-        a.cum_w = s.w >> 1;
-        a.cum_h_global = s.h >> 1;
-        a.cum_y_off = s.cy0;
-        a.cum_h_local = std::max(s.cy1 - s.cy0, 1);
-        a.cum_pair_stride = 0;
-        a.flow_out = st->flow[k];
-        const bool want_cum = k > 0 || (L > 1 && st->want_total); // every level but the finest feeds the next one
-        a.cum_out = want_cum ? st->cum_dst[k] : nullptr;
-        a.flow_pair_stride = 0;
-        a.reach_overflow = st->overflow;
-        a.sm_count = ctx_sm_count(st->ctx);
-        a.solve_fast = ctx_solve_fast(st->ctx);
-        if (npush > 0 && a.cum_out) {
-            a.npush = npush;
-            a.push[0] = push[0];
-            a.push[1] = push[1];
-            a.push_counter = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * pl.world + L + 1 + 2 * (size_t)(L - k));
+        if (on(4 * L)) {
+            const LevelStrip &s = st->s[0];
+            if ((rc = launch_fb_check_strip(st->cum[0] + (size_t)(s.y0 - s.eb0) * s.w * 2, st->fbh, s.w, s.h, s.y0, s.y1 - s.y0, st->hy0,
+                                            st->hy1, st->flow_scale, fb->alpha, fb->beta, st->status, fb->want_err2 ? st->err2 : nullptr,
+                                            st->overflow, q, launches)))
+                return rc;
         }
-        if (wait_in_kernel) {
-            a.nwait = nwait;
-            const int x = L - 1 - k;
-            for (int d = 0; d < nwait; d++)
-                a.wait[d] = {flag_ptr(st->arena, st->lay, (size_t)x * pl.world + wait_src[d].peer), wait_src[d].crow_lo, wait_src[d].crow_hi};
-        }
-        a.epoch_src = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * pl.world + L);
-        int rc = launch_lk_level(a, q, launches);
-        if (rc) return rc;
     }
-    if (peer_mode && on(2 * L - 1)) { // the rows my neighbours pushed have been used: they may push the next pair's
+    if (peer_mode && on(nphase - 1)) { // the rows my neighbours pushed have been used: they may push the next pair's
         PeerDoneArgs d{};
         for (int src : all_sources) {
             if (d.n == 2 * PEER_MAX_DST) {
                 set_error("strips: more than %d ranks push to this one", 2 * PEER_MAX_DST);
                 return OFB_ERR_UNSUPPORTED;
             }
-            d.flag[d.n++] = flag_ptr(st->peer_arena[src], st->peer_lay[src], (size_t)L * pl.world + me);
+            d.flag[d.n++] = flag_ptr(st->peer_arena[src], st->peer_lay[src], st->peer_lay[src].done(me));
         }
-        d.pairs = flag_ptr(st->arena, st->lay, (size_t)(L + 1) * pl.world + L);
+        d.pairs = flag_ptr(st->arena, st->lay, st->lay.pairs());
         peer_done_kernel<<<1, 32, 0, q>>>(d);
         OFB_CUDA_TRY(cudaGetLastError());
         if (launches) ++*launches;
@@ -1029,6 +1207,8 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
     }
     return OFB_OK;
 }
+
+extern "C" {
 
 int ofb_strips_run_device(ofb_strips *st, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, void *stream)
 {
@@ -1043,6 +1223,39 @@ int ofb_strips_run_phase_device(ofb_strips *st, const uint8_t *prev_own_d, const
         return OFB_ERR_INVALID;
     }
     return strips_run_impl(st, prev_own_d, next_own_d, pitch, stream, phase);
+}
+
+int ofb_strips_run_fb_device(ofb_strips *st, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha, float beta,
+                             int want_err2, void *stream)
+{
+    const FbRun fb{alpha, beta, want_err2};
+    return strips_run_impl(st, prev_own_d, next_own_d, pitch, stream, -1, &fb);
+}
+
+int ofb_strips_run_fb_phase_device(ofb_strips *st, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha,
+                                   float beta, int want_err2, int phase, void *stream)
+{
+    if (phase < 0) {
+        set_error("strips_run_fb_phase: phase %d", phase);
+        return OFB_ERR_INVALID;
+    }
+    const FbRun fb{alpha, beta, want_err2};
+    return strips_run_impl(st, prev_own_d, next_own_d, pitch, stream, phase, &fb);
+}
+
+int ofb_strips_fb_result(const ofb_strips *st, float **fwd_total_own_d, float **bwd_total_own_d, uint8_t **status_own_d,
+                         float **err2_own_d)
+{
+    if (!st || st->plan.fb_reach < 0) {
+        set_error("strips_fb_result: NULL handle, or one not created by ofb_strips_create_fb");
+        return OFB_ERR_INVALID;
+    }
+    const LevelStrip &s = st->s[0];
+    if (fwd_total_own_d) *fwd_total_own_d = st->cum[0] + (size_t)(s.y0 - s.eb0) * s.w * 2;
+    if (bwd_total_own_d) *bwd_total_own_d = st->fbh + (size_t)(s.y0 - st->hy0) * s.w * 2;
+    if (status_own_d) *status_own_d = st->status;
+    if (err2_own_d) *err2_own_d = st->err2;
+    return OFB_OK;
 }
 
 // Synchronises the stream and reports whether a warp sample reached past the exchanged halo rows (the result is

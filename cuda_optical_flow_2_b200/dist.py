@@ -379,10 +379,14 @@ class NativeStrips:
     from C++ on one stream.  transport "nccl": the halo rows move by NCCL send/recv between the ranks' buffers;
     "peer": by the sender's copy kernel straight into the receiver's memory over NVLink (CUDA IPC), epoch flags instead
     of a collective; "local": peer memory between ranks living in this process (connect_local, tests).
-    `torch.distributed` is used once, to hand round the NCCL unique id or the IPC handles."""
+    `torch.distributed` is used once, to hand round the NCCL unique id or the IPC handles.
+
+    fb_reach (an int >= 0) makes a handle that can also run checked pairs (run_fb: the forward-backward consistency check
+    of Context.flow_pairs_fb_device on the strips; peer or local transport, or world 1): a rank's check may sample
+    backward rows up to fb_reach rows beyond its own."""
 
     def __init__(self, ctx, w: int, h: int, levels: int, win: int, world: int, rank: int, device, warp_mode: int = WARP_BILINEAR,
-                 flow_scale: float = 1.0, reach: int = 16, transport: str = "nccl"):
+                 flow_scale: float = 1.0, reach: int = 16, transport: str = "nccl", fb_reach: Optional[int] = None):
         import ctypes as C
 
         import torch
@@ -393,6 +397,7 @@ class NativeStrips:
             raise ValueError(f"unknown strip transport {transport!r}")
         self.torch, self.C, self.L, self.lib, self.ctx = torch, C, L, L.load(), ctx
         self.w, self.h, self.levels, self.dev, self.world, self.rank = w, h, levels, device, world, rank
+        self.flow_scale = flow_scale
         self._transport = transport
         idbuf = torch.zeros(128, dtype=torch.uint8)
         use_nccl = world > 1 and transport == "nccl"
@@ -407,8 +412,14 @@ class NativeStrips:
             dist.broadcast(idbuf, 0)
         raw = (C.c_ubyte * 128)(*idbuf.cpu().tolist())
         hnd = C.c_void_p()
-        L.check(self.lib.ofb_strips_create(ctx._h, w, h, levels, win, warp_mode, C.c_float(flow_scale), world, rank, reach,
-                                           C.cast(raw, C.c_void_p) if use_nccl else None, C.byref(hnd)))
+        nccl_id = C.cast(raw, C.c_void_p) if use_nccl else None
+        self.fb_reach = fb_reach
+        if fb_reach is None:
+            L.check(self.lib.ofb_strips_create(ctx._h, w, h, levels, win, warp_mode, C.c_float(flow_scale), world, rank, reach,
+                                               nccl_id, C.byref(hnd)))
+        else:
+            L.check(self.lib.ofb_strips_create_fb(ctx._h, w, h, levels, win, warp_mode, C.c_float(flow_scale), world, rank, reach,
+                                                  int(fb_reach), nccl_id, C.byref(hnd)))
         self._h = hnd
         if world > 1 and transport == "peer":
             import torch.distributed as dist
@@ -485,14 +496,57 @@ class NativeStrips:
             for ns, (pin, nin) in zip(ranks, inputs):
                 ns.run_phase(pin, nin, phase, stream)
 
-    def check(self, stream: int = 0) -> None:
-        """Synchronises; raises if any pair since the last check went wrong (the flag is sticky), and clears the flag."""
+    def run_fb(self, prev_own, next_own, alpha: float = 0.01, beta: float = 0.5, want_err2: bool = False, stream: int = 0) -> None:
+        """One checked pair (a handle made with fb_reach): both directions on one pyramid build, then the check of the own
+        rows; results in own_fb()."""
+        self.L.check(self.lib.ofb_strips_run_fb_device(self._h, prev_own.data_ptr(), next_own.data_ptr(), prev_own.stride(0),
+                                                       self.C.c_float(alpha), self.C.c_float(beta), 1 if want_err2 else 0,
+                                                       self.C.c_void_p(stream)))
+
+    def run_fb_phase(self, prev_own, next_own, phase: int, alpha: float = 0.01, beta: float = 0.5, want_err2: bool = False,
+                     stream: int = 0) -> None:
+        """One of the 4 * levels + 1 phases of a checked pair; see run_local_sequenced_fb."""
+        self.L.check(self.lib.ofb_strips_run_fb_phase_device(self._h, prev_own.data_ptr(), next_own.data_ptr(), prev_own.stride(0),
+                                                             self.C.c_float(alpha), self.C.c_float(beta), 1 if want_err2 else 0,
+                                                             int(phase), self.C.c_void_p(stream)))
+
+    @staticmethod
+    def run_local_sequenced_fb(ranks, inputs, alpha: float = 0.01, beta: float = 0.5, want_err2: bool = False,
+                               stream: int = 0) -> None:
+        """run_local_sequenced for a checked pair."""
+        for phase in range(4 * ranks[0].levels + 1):
+            for ns, (pin, nin) in zip(ranks, inputs):
+                ns.run_fb_phase(pin, nin, phase, alpha, beta, want_err2, stream)
+
+    def own_fb(self):
+        """Torch views (no copy) of the own rows of level 0 after a checked pair: (forward total (rows, w, 2), backward
+        total (rows, w, 2), status (rows, w) uint8 FB_* codes, err2 (rows, w); err2 is written only by pairs run with
+        want_err2)."""
+        C = self.C
+        f, b, s, e = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_void_p()
+        self.L.check(self.lib.ofb_strips_fb_result(self._h, C.byref(f), C.byref(b), C.byref(s), C.byref(e)))
+        y0, y1 = self.own_rows(0)
+        rows = y1 - y0
+
+        class _H:
+            __cuda_array_interface__ = {"shape": (rows * self.w,), "typestr": "|u1", "data": (s.value, False), "version": 3}
+
+        status = self.torch.as_tensor(_H(), device=self.dev).view(rows, self.w)
+        return (_device_view(self.torch, f.value, (rows, self.w, 2), self.dev),
+                _device_view(self.torch, b.value, (rows, self.w, 2), self.dev), status,
+                _device_view(self.torch, e.value, (rows, self.w), self.dev))
+
+    def check(self, stream: int = 0, allow_unchecked: bool = False) -> None:
+        """Synchronises; raises if any pair since the last check went wrong (the flag is sticky), and clears the flag.
+        allow_unchecked: accept checked pairs with FB_UNCHECKED pixels (their other outputs are still exact)."""
         v = self.C.c_int()
         self.L.check(self.lib.ofb_strips_check(self._h, self.C.c_void_p(stream), self.C.byref(v)))
         if v.value & 2:
             raise RuntimeError("a neighbour's halo rows did not arrive (peer-memory transport timed out)")
         if v.value & 1:
             raise RuntimeError("a warp sample reached past the exchanged halo rows: raise `reach`")
+        if v.value & 4 and not allow_unchecked:
+            raise RuntimeError("the check needed backward flow rows beyond those held (FB_UNCHECKED pixels): raise `fb_reach`")
 
     def own_flow(self, level: int, total: bool = False):
         """A torch view (no copy) of the own rows of the residual (or cumulative) flow of `level`."""

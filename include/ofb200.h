@@ -261,8 +261,10 @@ int ofb_stream_destroy(ofb_stream *s);
  *   ofb_strips_nccl_unique_id : rank 0 makes the 128-byte id, the application broadcasts it (any transport)
  *   ofb_strips_create         : collective over all ranks when a NCCL id is given (ncclCommInitRank)
  *   ofb_strips_check          : synchronises; *overflow bit 0 = a warp sample reached past the halo rows, bit 1 = a
- *                               neighbour's rows did not arrive within 4 s (peer-memory transport).  The flag is sticky:
- *                               it covers every pair since the previous check, which clears it
+ *                               neighbour's rows did not arrive within 4 s (peer-memory transport), bit 2 = a checked
+ *                               pair's check needed a backward tap outside the rows the rank holds (OFB_FB_UNCHECKED
+ *                               pixels: raise fb_reach).  The flag is sticky: it covers every pair since the previous
+ *                               check, which clears it
  *   ofb_strips_run_phase_device: one of the 2 * levels phases of a pair (peer-memory transport): 0 = upload + push of the
  *                               level-0 image rows; 1 = wait, pyramid, coarsest level; 2j = push of the cumulative flow of
  *                               level L-j; 2j+1 = wait, level L-1-j (j = 1 .. L-1).  A host that runs several ranks in ONE
@@ -295,6 +297,45 @@ int ofb_strips_peer_handle(ofb_strips *s, void *blob128);
 int ofb_strips_peer_connect(ofb_strips *s, const void *blobs_world_x_128);
 int ofb_strips_peer_arena(ofb_strips *s, void **arena_d);
 int ofb_strips_peer_connect_local(ofb_strips *s, void *const *arenas_d);
+
+/* ---- forward-backward consistency check on row strips (a checked pair) --------------------------------------------
+ * The check of ofb_flow_pairs_fb_device on one pair cut into row strips.  A checked pair runs the forward level loop as
+ * ofb_strips_run_device does (level 0 always writes the total flow), then the backward level loop (next -> prev) on the
+ * pyramid the rank has already built (no second image exchange), then exchanges the backward total rows the neighbours'
+ * checks sample and checks the own rows [y0, y1) of level 0.  All of it is enqueued on one stream without host
+ * synchronisation, so a checked pair can be captured as a CUDA graph.
+ *   ofb_strips_create_fb : the arguments of ofb_strips_create plus fb_reach >= 0, the level-0 rows beyond its own rows a
+ *                          rank's check may sample: it holds backward total rows [max(0, y0 - fb_reach), min(h, y1 +
+ *                          fb_reach + 1)).  The arena also holds the backward direction's regions, so a handle that runs
+ *                          checked pairs is created this way (before ofb_strips_peer_handle / _connect).  flow_scale > 0.
+ *                          Peer-memory transport or world == 1 only: world > 1 with a NCCL id is OFB_ERR_UNSUPPORTED
+ *                          (nothing allocated).  Plain pairs (ofb_strips_run_device) run on it unchanged, and plain and
+ *                          checked pairs may alternate; all ranks must be created with the same fb_reach.
+ *   ofb_strips_run_fb_device : one checked pair; alpha >= 0, beta >= 0 as in ofb_flow_pairs_fb_device; want_err2 = 0 leaves
+ *                          the err2 buffer untouched.  Bad arguments are refused before anything is enqueued.
+ *   ofb_strips_run_fb_phase_device : one of its 4L + 1 phases (L = levels; ranks of one process on one stream, as
+ *                          ofb_strips_run_phase_device):
+ *                            0 .. 2L-1   the forward phases of ofb_strips_run_phase_device, without the handshake
+ *                            2L          backward coarsest level L-1
+ *                            2L+2j-1     push of the backward cumulative flow of level L-j        (j = 1 .. L-1)
+ *                            2L+2j       wait, backward level L-1-j                               (j = 1 .. L-1)
+ *                            4L-1        push of the own backward total rows the neighbours' checks sample
+ *                            4L          wait, the check, the end-of-pair handshake
+ *   ofb_strips_fb_result : device pointers to the own rows [y0, y1) of level 0: forward total, backward total (2 floats
+ *                          per pixel), status (1 byte) and err2 (1 float) per pixel.
+ * Status: that of ofb_fb_check_device, except that a pixel whose whole-frame status would read backward taps
+ * (CONSISTENT, INCONSISTENT, BWD_NONFINITE) and has a tap of non-zero weight outside the rows held is OFB_FB_UNCHECKED
+ * (err2 NaN; bit 2 of ofb_strips_check).  FWD_NONFINITE and OUTSIDE read no tap and are never replaced.  Unless
+ * ofb_strips_check reports bit 0 or bit 2, every output is bit-identical to rows [y0, y1) of ofb_flow_pairs_fb_device on
+ * the whole frame with the same parameters and solve mode. */
+int ofb_strips_create_fb(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
+                         int reach, int fb_reach, const void *nccl_id128, ofb_strips **out);
+int ofb_strips_run_fb_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha,
+                             float beta, int want_err2, void *stream);
+int ofb_strips_run_fb_phase_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha,
+                                   float beta, int want_err2, int phase, void *stream);
+int ofb_strips_fb_result(const ofb_strips *s, float **fwd_total_own_d, float **bwd_total_own_d, uint8_t **status_own_d,
+                         float **err2_own_d);
 
 /* ---- debug derivative views: showTest (main.cu:19-92) without the windows ------------------------------------------
  * ofb_conv_3ch_1ch_u8_u8_host replaces gpu::conv_3ch_1ch_tiled (OptFlowGpu.cuh; OptFlowGpu.cu:741-766, kernel
@@ -349,6 +390,7 @@ int ofb_write_flo(const char *path, const float *flow_h, int w, int h);
 #define OFB_FB_OUTSIDE 2
 #define OFB_FB_FWD_NONFINITE 3
 #define OFB_FB_BWD_NONFINITE 4
+#define OFB_FB_UNCHECKED 5 /* row strips only (ofb_strips_run_fb_device): a tap the check needs lies outside the rows held */
 /* The check alone, on any two total-flow fields (e.g. the caller's own).  flow_scale > 0, alpha >= 0, beta >= 0. */
 int ofb_fb_check_device(ofb_ctx *ctx, const float *fwd_d, const float *bwd_d, int w, int h, int n_pairs, float flow_scale,
                         float alpha, float beta, uint8_t *status_d, float *err2_d, void *stream);
