@@ -185,6 +185,55 @@ int launch_lk_level(const LkLevelArgs &a, cudaStream_t stream, unsigned long lon
     }
 }
 
+LkLevelArgs lk_args_frame(const uint8_t *prev, const uint8_t *next, size_t pitch, size_t image_stride, int w, int h, int n_pairs,
+                          int win, int warp_mode, float flow_scale, float *flow_out, int sm_count, int solve_fast)
+{
+    LkLevelArgs a{};
+    a.prev = prev;
+    a.next = next;
+    a.pitch = pitch;
+    a.image_stride = image_stride;
+    a.w = w;
+    a.h_local = a.h_global = h;
+    a.y_off = 0;
+    a.out_y0 = 0;
+    a.out_y1 = h;
+    a.n_pairs = n_pairs;
+    a.win = win;
+    a.warp_mode = warp_mode;
+    a.flow_scale = flow_scale;
+    a.flow_out = flow_out;
+    a.flow_pair_stride = (size_t)w * h;
+    a.sm_count = sm_count;
+    a.solve_fast = solve_fast;
+    return a;
+}
+
+LkLevelArgs lk_args_strip(const uint8_t *prev, const uint8_t *next, size_t pitch, int w, int h_local, int y_off, int h_global,
+                          int out_y0, int out_y1, int win, int warp_mode, float flow_scale, float *flow_out, int sm_count,
+                          int solve_fast)
+{
+    LkLevelArgs a{};
+    a.prev = prev;
+    a.next = next;
+    a.pitch = pitch;
+    a.image_stride = pitch * (size_t)h_local;
+    a.w = w;
+    a.h_local = h_local;
+    a.y_off = y_off;
+    a.h_global = h_global;
+    a.out_y0 = out_y0;
+    a.out_y1 = out_y1;
+    a.n_pairs = 1;
+    a.win = win;
+    a.warp_mode = warp_mode;
+    a.flow_scale = flow_scale;
+    a.flow_out = flow_out;
+    a.sm_count = sm_count;
+    a.solve_fast = solve_fast;
+    return a;
+}
+
 template <int WIN> int preload_lk_win(); // lk_win.cu
 int preload_lk_level(int win)
 {

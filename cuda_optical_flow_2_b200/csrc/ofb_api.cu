@@ -160,8 +160,6 @@ static int check_params(const ofb_params *p)
 // Pyramids of both frames + coarse-to-fine LK, everything device resident.  `base` is the
 // context workspace region reserved for this call.
 struct PairPlan {
-    int L = 0;
-    int w[OFB_MAX_LEVELS], h[OFB_MAX_LEVELS];
     size_t pitch[OFB_MAX_LEVELS], istride[OFB_MAX_LEVELS];
     size_t off_prev[OFB_MAX_LEVELS], off_next[OFB_MAX_LEVELS], off_cum[OFB_MAX_LEVELS];
     size_t bytes = 0;
@@ -179,18 +177,16 @@ static bool pyr_fuse_enabled()
 
 static void plan_pairs(const ofb_params *p, PairPlan *pl, Carver *cv)
 {
-    pl->L = p->levels;
     for (int k = 0; k < p->levels; k++) {
-        pl->w[k] = p->w >> k;
-        pl->h[k] = p->h >> k;
-        pl->pitch[k] = align_up((size_t)pl->w[k], 64);
-        pl->istride[k] = pl->pitch[k] * (size_t)pl->h[k];
+        const int wk = p->w >> k, hk = p->h >> k;
+        pl->pitch[k] = align_up((size_t)wk, 64);
+        pl->istride[k] = pl->pitch[k] * (size_t)hk;
         pl->off_prev[k] = pl->off_next[k] = pl->off_cum[k] = (size_t)-1;
         if (k >= 1) {
             pl->off_prev[k] = cv->take(pl->istride[k] * p->n_pairs);
             pl->off_next[k] = cv->take(pl->istride[k] * p->n_pairs);
         }
-        if (k >= 1 && k <= p->levels - 2) pl->off_cum[k] = cv->take((size_t)pl->w[k] * pl->h[k] * 8 * p->n_pairs);
+        if (k >= 1 && k <= p->levels - 2) pl->off_cum[k] = cv->take((size_t)wk * hk * 8 * p->n_pairs);
     }
     pl->bytes = cv->off;
 }
@@ -218,56 +214,58 @@ struct PairLevels {
     size_t pitch[OFB_MAX_LEVELS], istr[OFB_MAX_LEVELS];
 };
 
-// Pyramids of both frames: levels 1..L-1 into the plan's regions of `base`, one launch per one or two steps.
-static int build_pyramids(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, uint8_t *base, const uint8_t *prev0,
-                          const uint8_t *next0, size_t pitch0, size_t istride0, PairLevels *lv, cudaStream_t st)
+// Levels 1..L-1 of one image set (b == NULL) or two, n images of w x h each, from their level 0, with the
+// OFB_PROFILE_PYRAMID record: one launch per one or two pyramid steps, both sets in it when the grid allows.
+static int build_pyramid_levels(ofb_ctx *c, int w, int h, int L, const uint8_t *const *a, const uint8_t *const *b,
+                                const size_t *pitch, const size_t *istr, int n, cudaStream_t st)
 {
-    const int L = p->levels, n = p->n_pairs;
-    const uint8_t **pp = lv->prev, **pn = lv->next;
-    size_t *pitch = lv->pitch, *istr = lv->istr;
-    pp[0] = prev0;
-    pn[0] = next0;
-    pitch[0] = pitch0;
-    istr[0] = istride0;
-    if (L > 1) {
-        int rc = prof_begin(c, OFB_PROFILE_PYRAMID, st);
-        if (rc) return rc;
-    }
-    for (int k = 1; k < L; k++) {
-        pp[k] = base + pl.off_prev[k];
-        pn[k] = base + pl.off_next[k];
-        pitch[k] = pl.pitch[k];
-        istr[k] = pl.istride[k];
-    }
-    const bool one = 2 * n <= 65535; // grid.z limit: both frames of every pair in one launch
+    if (L < 2) return OFB_OK;
+    int rc = prof_begin(c, OFB_PROFILE_PYRAMID, st);
+    if (rc) return rc;
+    const bool joint = b && 2 * n <= 65535; // grid.z limit: both sets in one launch
+    auto lv = [](const uint8_t *const *set, int k) { return const_cast<uint8_t *>(set[k]); };
     for (int k = 1; k < L;) {
         // two pyramid steps per launch where two are left (level k is then never read back), else one
         const bool two = pyr_fuse_enabled() && k + 1 < L;
-        for (int f = 0; f < (one ? 1 : 2); f++) {
-            const uint8_t *const *src = f ? pn : pp;
-            int rc = launch_pyr_roll(src[k - 1], pitch[k - 1], istr[k - 1], pl.w[k - 1], pl.h[k - 1], const_cast<uint8_t *>(src[k]),
-                                     pitch[k], istr[k], two ? const_cast<uint8_t *>(src[k + 1]) : nullptr, two ? pitch[k + 1] : 0,
-                                     two ? istr[k + 1] : 0, n, st, &c->launches, one ? pn[k - 1] : nullptr,
-                                     one ? const_cast<uint8_t *>(pn[k]) : nullptr,
-                                     one && two ? const_cast<uint8_t *>(pn[k + 1]) : nullptr, c->sm_count);
+        for (int f = 0; f < (b && !joint ? 2 : 1); f++) {
+            const uint8_t *const *src = f ? b : a;
+            rc = launch_pyr_roll(src[k - 1], pitch[k - 1], istr[k - 1], w >> (k - 1), h >> (k - 1), lv(src, k), pitch[k], istr[k],
+                                 two ? lv(src, k + 1) : nullptr, two ? pitch[k + 1] : 0, two ? istr[k + 1] : 0, n, st, &c->launches,
+                                 joint ? b[k - 1] : nullptr, joint ? lv(b, k) : nullptr, joint && two ? lv(b, k + 1) : nullptr,
+                                 c->sm_count);
             if (rc) return rc;
         }
         k += two ? 2 : 1;
     }
-    if (L > 1) {
-        int rc = prof_end(c, st);
-        if (rc) return rc;
-    }
-    return OFB_OK;
+    return prof_end(c, st);
 }
 
-// The coarse-to-fine loop of main.cu:256-262 on built pyramids: prev / next are the two frames' levels (swapped for
-// the backward direction), cum[k] (k = 1..L-2) the regions where warped levels materialise their cumulative flow.
-static int run_levels(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, const uint8_t *const *pp, const uint8_t *const *pn,
-                      const size_t *pitch, const size_t *istr, float *const *flow_levels, float *const *cum, float *total_flow,
-                      cudaStream_t st)
+// Pyramids of both frames: levels 1..L-1 into the plan's regions of `base`.
+static int build_pyramids(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, uint8_t *base, const uint8_t *prev0,
+                          const uint8_t *next0, size_t pitch0, size_t istride0, PairLevels *lv, cudaStream_t st)
+{
+    lv->prev[0] = prev0;
+    lv->next[0] = next0;
+    lv->pitch[0] = pitch0;
+    lv->istr[0] = istride0;
+    for (int k = 1; k < p->levels; k++) {
+        lv->prev[k] = base + pl.off_prev[k];
+        lv->next[k] = base + pl.off_next[k];
+        lv->pitch[k] = pl.pitch[k];
+        lv->istr[k] = pl.istride[k];
+    }
+    return build_pyramid_levels(c, p->w, p->h, p->levels, lv->prev, lv->next, lv->pitch, lv->istr, p->n_pairs, st);
+}
+
+// The coarse-to-fine loop of main.cu:256-262 on built pyramids, prev -> next or (backward) next -> prev; cum[k]
+// (k = 1..L-2) are the regions where warped levels materialise their cumulative flow.
+static int run_levels(ofb_ctx *c, const ofb_params *p, const PairLevels &lv, bool backward, float *const *flow_levels,
+                      float *const *cum, float *total_flow, cudaStream_t st)
 {
     const int L = p->levels, n = p->n_pairs;
+    const uint8_t *const *pp = backward ? lv.next : lv.prev, *const *pn = backward ? lv.prev : lv.next;
+    auto W = [p](int k) { return p->w >> k; };
+    auto H = [p](int k) { return p->h >> k; };
     // Which warped levels materialise their cumulative flow.  Level 1 need not when level 0 composes it on the fly from
     // flow_1 and cum_2 (lk_level_kernel<..., COMP>): 8 bytes per pixel less to write at level 1, whose kernel is bound by
     // exactly those stores.  Composition needs even sizes (no clamped coarse indices), TMA-able rows and a per-pixel warp
@@ -281,7 +279,7 @@ static int run_levels(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, const
         return !(e && e[0] == '1');
     }();
     if (L >= 3 && !total_flow && allow_compose && p->warp_mode != OFB_WARP_AS_WRITTEN) {
-        const bool even = !((pl.w[0] | pl.h[0] | pl.w[1] | pl.h[1] | pl.w[2]) & 1);
+        const bool even = !((W(0) | H(0) | W(1) | H(1) | W(2)) & 1);
         const float *c2 = (2 == L - 1) ? flow_levels[2] : cum[2];
         const bool aligned = !((reinterpret_cast<uintptr_t>(flow_levels[1]) | reinterpret_cast<uintptr_t>(c2)) & 15);
         if (even && aligned) {
@@ -290,37 +288,20 @@ static int run_levels(ofb_ctx *c, const ofb_params *p, const PairPlan &pl, const
         }
     }
     for (int k = L - 1; k >= 0; k--) {
-        LkLevelArgs a{};
-        a.prev = pp[k];
-        a.next = pn[k];
-        a.pitch = pitch[k];
-        a.image_stride = istr[k];
-        a.w = pl.w[k];
-        a.h_local = pl.h[k];
-        a.y_off = 0;
-        a.h_global = pl.h[k];
-        a.out_y0 = 0;
-        a.out_y1 = pl.h[k];
-        a.n_pairs = n;
-        a.win = p->win;
-        a.warp_mode = p->warp_mode;
-        a.flow_scale = p->flow_scale;
-        a.flow_out = flow_levels[k];
-        a.flow_pair_stride = (size_t)pl.w[k] * pl.h[k];
-        a.sm_count = c->sm_count;
-        a.solve_fast = c->solve_fast;
+        LkLevelArgs a = lk_args_frame(pp[k], pn[k], lv.pitch[k], lv.istr[k], W(k), H(k), n, p->win, p->warp_mode, p->flow_scale,
+                                      flow_levels[k], c->sm_count, c->solve_fast);
         if (k < L - 1) {
             // cum_{k+1}: the coarsest level's cumulative flow is its residual flow; a level that did not materialise its
             // own hands over its residual flow together with its parent's cumulative flow
             a.cum_in = (k + 1 == L - 1 || comp[k]) ? flow_levels[k + 1] : cum[k + 1];
-            a.cum_w = pl.w[k + 1];
-            a.cum_h_global = pl.h[k + 1];
+            a.cum_w = W(k + 1);
+            a.cum_h_global = H(k + 1);
             a.cum_y_off = 0;
-            a.cum_h_local = pl.h[k + 1];
-            a.cum_pair_stride = (size_t)pl.w[k + 1] * pl.h[k + 1];
+            a.cum_h_local = H(k + 1);
+            a.cum_pair_stride = (size_t)W(k + 1) * H(k + 1);
             if (comp[k]) {
                 a.cum2_in = (k + 2 == L - 1) ? flow_levels[k + 2] : cum[k + 2];
-                a.cum2_pair_stride = (size_t)pl.w[k + 2] * pl.h[k + 2];
+                a.cum2_pair_stride = (size_t)W(k + 2) * H(k + 2);
             }
         }
         if (k == 0) a.cum_out = total_flow;
@@ -345,7 +326,7 @@ static int run_pairs_device(ofb_ctx *c, const ofb_params *p, const PairPlan &pl,
     if (rc) return rc;
     float *cum[OFB_MAX_LEVELS] = {};
     for (int k = 1; k <= p->levels - 2; k++) cum[k] = reinterpret_cast<float *>(base + pl.off_cum[k]);
-    return run_levels(c, p, pl, lv.prev, lv.next, lv.pitch, lv.istr, flow_levels, cum, total_flow, st);
+    return run_levels(c, p, lv, false, flow_levels, cum, total_flow, st);
 }
 
 // Workspace of the forward-backward call: the regions of plan_pairs (both pyramids, the forward direction's cumulative
@@ -360,13 +341,35 @@ static void plan_pairs_fb(const ofb_params *p, PairFbPlan *fp)
 {
     Carver cv;
     plan_pairs(p, &fp->pl, &cv);
+    auto bytes = [p](int k) { return (size_t)(p->w >> k) * (p->h >> k) * 8 * p->n_pairs; };
     for (int d = 0; d < 2; d++)
-        for (int k = 0; k < p->levels; k++) fp->off_flow[d][k] = cv.take((size_t)fp->pl.w[k] * fp->pl.h[k] * 8 * p->n_pairs);
+        for (int k = 0; k < p->levels; k++) fp->off_flow[d][k] = cv.take(bytes(k));
     for (int k = 0; k < p->levels; k++) {
         fp->off_cum_b[k] = (size_t)-1;
-        if (k >= 1 && k <= p->levels - 2) fp->off_cum_b[k] = cv.take((size_t)fp->pl.w[k] * fp->pl.h[k] * 8 * p->n_pairs);
+        if (k >= 1 && k <= p->levels - 2) fp->off_cum_b[k] = cv.take(bytes(k));
     }
     fp->bytes = cv.off;
+}
+
+// The frames of the device entry points: `ptrs_ok` (their non-NULL pointers, `null_msg` otherwise), pitch, image stride,
+// and the pair count, before the workspace grows or anything is enqueued: the level kernels and the check take at most
+// 65535 pairs.
+static int check_device_frames(const ofb_params *p, bool ptrs_ok, const char *null_msg, size_t pitch_bytes,
+                               size_t image_stride_bytes)
+{
+    if (!ptrs_ok) {
+        set_error("%s", null_msg);
+        return OFB_ERR_INVALID;
+    }
+    if (pitch_bytes < (size_t)p->w || (p->n_pairs > 1 && image_stride_bytes < pitch_bytes * (size_t)p->h)) {
+        set_error("pitch %zu / image stride %zu too small for %dx%d", pitch_bytes, image_stride_bytes, p->w, p->h);
+        return OFB_ERR_INVALID;
+    }
+    if (p->n_pairs > 65535) {
+        set_error("at most 65535 pairs per call (got %d)", p->n_pairs);
+        return OFB_ERR_INVALID;
+    }
+    return OFB_OK;
 }
 
 static int check_fb_args(float flow_scale, float alpha, float beta)
@@ -422,8 +425,8 @@ static int run_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const PairFbPlan
             cum[1][k] = reinterpret_cast<float *>(base + fp.off_cum_b[k]);
         }
     }
-    if ((rc = run_levels(c, p, fp.pl, lv.prev, lv.next, lv.pitch, lv.istr, flow[0], cum[0], fwd_total, st))) return rc;
-    if ((rc = run_levels(c, p, fp.pl, lv.next, lv.prev, lv.pitch, lv.istr, flow[1], cum[1], bwd_total, st))) return rc;
+    if ((rc = run_levels(c, p, lv, false, flow[0], cum[0], fwd_total, st))) return rc;
+    if ((rc = run_levels(c, p, lv, true, flow[1], cum[1], bwd_total, st))) return rc;
     return run_fb_check(c, fwd_total, bwd_total, p->w, p->h, p->n_pairs, p->flow_scale, alpha, beta, status, err2, st);
 }
 
@@ -789,23 +792,14 @@ int ofb_flow_pairs_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev_d
     OFB_CHECK_CTX(c);
     int rc = check_params(p);
     if (rc) return rc;
-    if (!prev_d || !next_d || !flow_levels_d) {
-        set_error("NULL frame or flow pointer");
-        return OFB_ERR_INVALID;
-    }
+    if ((rc = check_device_frames(p, prev_d && next_d && flow_levels_d, "NULL frame or flow pointer", pitch_bytes,
+                                  image_stride_bytes)))
+        return rc;
     for (int k = 0; k < p->levels; k++)
         if (!flow_levels_d[k]) {
             set_error("flow_levels_d[%d] is NULL", k);
             return OFB_ERR_INVALID;
         }
-    if (pitch_bytes < (size_t)p->w || (p->n_pairs > 1 && image_stride_bytes < pitch_bytes * (size_t)p->h)) {
-        set_error("pitch %zu / image stride %zu too small for %dx%d", pitch_bytes, image_stride_bytes, p->w, p->h);
-        return OFB_ERR_INVALID;
-    }
-    if (p->n_pairs > 65535) { // (before the workspace grows: the level kernels take at most this many)
-        set_error("at most 65535 pairs per call (got %d)", p->n_pairs);
-        return OFB_ERR_INVALID;
-    }
     OFB_GUARD(c);
     Carver cv;
     PairPlan pl;
@@ -851,18 +845,7 @@ int ofb_flow_pairs_fb_device(ofb_ctx *c, const ofb_params *p, const uint8_t *pre
     if (rc) return rc;
     if ((rc = check_fb_args(p->flow_scale, alpha, beta))) return rc;
     if ((rc = check_fb_buffers(fwd_total_d, bwd_total_d, status_d, err2_d))) return rc;
-    if (!prev_d || !next_d) {
-        set_error("NULL frame pointer");
-        return OFB_ERR_INVALID;
-    }
-    if (pitch_bytes < (size_t)p->w || (p->n_pairs > 1 && image_stride_bytes < pitch_bytes * (size_t)p->h)) {
-        set_error("pitch %zu / image stride %zu too small for %dx%d", pitch_bytes, image_stride_bytes, p->w, p->h);
-        return OFB_ERR_INVALID;
-    }
-    if (p->n_pairs > 65535) { // (before anything is enqueued: the level kernels and the check take at most this many)
-        set_error("at most 65535 pairs per call (got %d)", p->n_pairs);
-        return OFB_ERR_INVALID;
-    }
+    if ((rc = check_device_frames(p, prev_d && next_d, "NULL frame pointer", pitch_bytes, image_stride_bytes))) return rc;
     OFB_GUARD(c);
     PairFbPlan fp;
     plan_pairs_fb(p, &fp);
@@ -938,32 +921,15 @@ int ofb_lk_level_device(ofb_ctx *c, const uint8_t *prev_d, const uint8_t *next_d
         return OFB_ERR_INVALID;
     }
     OFB_GUARD(c);
-    LkLevelArgs a{};
-    a.prev = prev_d;
-    a.next = next_d;
-    a.pitch = pitch_bytes;
-    a.image_stride = image_stride_bytes;
-    a.w = w;
-    a.h_local = h;
-    a.y_off = 0;
-    a.h_global = h;
-    a.out_y0 = 0;
-    a.out_y1 = h;
-    a.n_pairs = n_pairs;
-    a.win = win;
-    a.warp_mode = warp_mode;
-    a.flow_scale = flow_scale;
+    LkLevelArgs a = lk_args_frame(prev_d, next_d, pitch_bytes, image_stride_bytes, w, h, n_pairs, win, warp_mode, flow_scale,
+                                  flow_out_d, c->sm_count, c->solve_fast);
     a.cum_in = cum_in_d;
     a.cum_w = w >> 1;
     a.cum_h_global = h >> 1;
     a.cum_y_off = 0;
     a.cum_h_local = h >> 1;
     a.cum_pair_stride = (size_t)(w >> 1) * (h >> 1);
-    a.flow_out = flow_out_d;
     a.cum_out = cum_out_d;
-    a.flow_pair_stride = (size_t)w * h;
-    a.sm_count = c->sm_count;
-    a.solve_fast = c->solve_fast;
     if (cum_in_d && ((w >> 1) < 1 || (h >> 1) < 1)) {
         set_error("level %dx%d has no coarser level", w, h);
         return OFB_ERR_INVALID;
@@ -990,33 +956,15 @@ int ofb_lk_level_strip_device(ofb_ctx *c, const uint8_t *prev_d, const uint8_t *
         return OFB_ERR_INVALID;
     }
     OFB_GUARD(c);
-    LkLevelArgs a{};
-    a.prev = prev_d;
-    a.next = next_d;
-    a.pitch = pitch_bytes;
-    a.image_stride = pitch_bytes * (size_t)h_local;
-    a.w = w;
-    a.h_local = h_local;
-    a.y_off = y_off;
-    a.h_global = h_global;
-    a.out_y0 = out_y0;
-    a.out_y1 = out_y1;
-    a.n_pairs = 1;
-    a.win = win;
-    a.warp_mode = warp_mode;
-    a.flow_scale = flow_scale;
+    LkLevelArgs a = lk_args_strip(prev_d, next_d, pitch_bytes, w, h_local, y_off, h_global, out_y0, out_y1, win, warp_mode,
+                                  flow_scale, flow_out_d, c->sm_count, c->solve_fast);
     a.cum_in = cum_in_d;
     a.cum_w = w >> 1;
     a.cum_h_global = h_global >> 1;
     a.cum_y_off = cum_y_off;
     a.cum_h_local = cum_h_local;
-    a.cum_pair_stride = 0;
-    a.flow_out = flow_out_d;
     a.cum_out = cum_out_d;
-    a.flow_pair_stride = 0;
     a.reach_overflow = reach_overflow_d;
-    a.sm_count = c->sm_count;
-    a.solve_fast = c->solve_fast;
     return launch_lk_level(a, static_cast<cudaStream_t>(stream), &c->launches);
 }
 
@@ -1127,26 +1075,12 @@ int ofb_calc_opt_flow_host_u8c3(ofb_ctx *c, const unsigned char *prev, const uns
             cum_in = reinterpret_cast<const float *>(B + off_cum[k]);
         }
     }
-    LkLevelArgs a{};
-    a.prev = B + off_p;
-    a.next = B + off_n;
-    a.pitch = pitch;
-    a.image_stride = pitch * h;
-    a.w = w;
-    a.h_local = h;
-    a.h_global = h;
-    a.out_y1 = h;
-    a.n_pairs = 1;
-    a.win = win;
-    a.warp_mode = warp_mode;
-    a.flow_scale = flow_scale;
+    LkLevelArgs a = lk_args_frame(B + off_p, B + off_n, pitch, pitch * h, w, h, 1, win, warp_mode, flow_scale,
+                                  reinterpret_cast<float *>(B + off_flow), c->sm_count, c->solve_fast);
     a.cum_in = cum_in;
     a.cum_w = w >> 1;
     a.cum_h_global = h >> 1;
     a.cum_h_local = h >> 1;
-    a.flow_out = reinterpret_cast<float *>(B + off_flow);
-    a.sm_count = c->sm_count;
-    a.solve_fast = c->solve_fast;
     rc = launch_lk_level(a, st, &c->launches);
     if (rc) return rc;
     OFB_CUDA_TRY(cudaMemcpyAsync(optFlowPyramid[level], B + off_flow, (size_t)w * h * 8, cudaMemcpyDeviceToHost, st));
@@ -1600,7 +1534,7 @@ struct ofb_stream {
     int frames = 0;
     uint8_t *mem = nullptr; // all device buffers of the stream in one allocation
     size_t pitch[OFB_MAX_LEVELS] = {}, off_pyr[2][OFB_MAX_LEVELS] = {}, off_bgr = 0, off_gray = 0, off_lut = 0;
-    size_t off_flow[OFB_MAX_LEVELS] = {}, off_cum[OFB_MAX_LEVELS] = {}, off_total = 0;
+    size_t off_flow[OFB_MAX_LEVELS] = {}, off_cum[OFB_MAX_LEVELS] = {}, off_total = 0; // off_cum: levels 1..L-2
     int cur = 0; // which pyramid receives the next frame
     // The forward-backward check (ofb_stream_push_bgr_host_fb), set up by its first call: the backward direction's residual
     // flow, interior cumulative flow and total, status and err2 in one allocation, and a second stream with two events
@@ -1613,6 +1547,30 @@ struct ofb_stream {
 
 namespace ofb {
 
+// The stream's two pyramids as a pair: the previous frame's and the current one's.
+static PairLevels stream_pair_levels(const ofb_stream *s)
+{
+    PairLevels lv;
+    for (int k = 0; k < s->p.levels; k++) {
+        lv.prev[k] = s->mem + s->off_pyr[s->cur ^ 1][k];
+        lv.next[k] = s->mem + s->off_pyr[s->cur][k];
+        lv.pitch[k] = s->pitch[k];
+        lv.istr[k] = s->pitch[k] * (size_t)(s->p.h >> k);
+    }
+    return lv;
+}
+
+// The residual flow of every level and the cumulative flow of levels 1..L-2 of one direction (bwd: in the check's
+// allocation).
+static void stream_flow(const ofb_stream *s, bool bwd, float **flow, float **cum)
+{
+    uint8_t *B = bwd ? s->fb_mem : s->mem;
+    for (int k = 0; k < s->p.levels; k++) {
+        flow[k] = reinterpret_cast<float *>(B + (bwd ? s->off_bflow[k] : s->off_flow[k]));
+        cum[k] = k >= 1 && k <= s->p.levels - 2 ? reinterpret_cast<float *>(B + (bwd ? s->off_bcum[k] : s->off_cum[k])) : nullptr;
+    }
+}
+
 // Upload, grayscale (main.cu:232), bilateral pre-filter (main.cu:240) and pyramid (main.cu:250) of a new frame into the
 // stream's current pyramid, on the context stream.
 static int stream_new_frame(ofb_stream *s, const unsigned char *frame_bgr)
@@ -1621,9 +1579,9 @@ static int stream_new_frame(ofb_stream *s, const unsigned char *frame_bgr)
     const ofb_params &p = s->p;
     cudaStream_t st = c->stream;
     uint8_t *B = s->mem;
-    const int cur = s->cur;
+    const PairLevels lv = stream_pair_levels(s);
+    uint8_t *lvl0 = const_cast<uint8_t *>(lv.next[0]);
     OFB_CUDA_TRY(cudaMemcpyAsync(B + s->off_bgr, frame_bgr, (size_t)p.w * p.h * 3, cudaMemcpyHostToDevice, st));
-    uint8_t *lvl0 = B + s->off_pyr[cur][0];
     int rc = launch_grayscale(B + s->off_bgr, p.w, p.h, nullptr, s->bil_win ? B + s->off_gray : lvl0, s->pitch[0], st,
                               &c->launches);
     if (rc) return rc;
@@ -1632,16 +1590,23 @@ static int stream_new_frame(ofb_stream *s, const unsigned char *frame_bgr)
                               s->sig_b, reinterpret_cast<double *>(B + s->off_lut), lvl0, s->pitch[0], st, &c->launches);
         if (rc) return rc;
     }
-    for (int k = 1; k < p.levels;) { // main.cu:250; two steps per launch where two are left
-        const bool two = pyr_fuse_enabled() && k + 1 < p.levels;
-        rc = launch_pyr_roll(B + s->off_pyr[cur][k - 1], s->pitch[k - 1], s->pitch[k - 1] * (size_t)(p.h >> (k - 1)), p.w >> (k - 1),
-                             p.h >> (k - 1), B + s->off_pyr[cur][k], s->pitch[k], s->pitch[k] * (size_t)(p.h >> k),
-                             two ? B + s->off_pyr[cur][k + 1] : nullptr, two ? s->pitch[k + 1] : 0,
-                             two ? s->pitch[k + 1] * (size_t)(p.h >> (k + 1)) : 0, 1, st, &c->launches, nullptr, nullptr, nullptr,
-                             c->sm_count);
-        if (rc) return rc;
-        k += two ? 2 : 1;
+    return build_pyramid_levels(c, p.w, p.h, p.levels, lv.next, nullptr, lv.pitch, lv.istr, 1, st);
+}
+
+// One push of either kind: the new frame into the current pyramid; from the second frame on, `pair()` enqueues the pair's
+// work and downloads.  Once they are done the current pyramid becomes the previous one (main.cu:270-272).
+template <class Pair> static int stream_push(ofb_stream *s, const unsigned char *frame_bgr, int *has_flow, Pair pair)
+{
+    if (has_flow) *has_flow = 0;
+    int rc = stream_new_frame(s, frame_bgr);
+    if (rc) return rc;
+    if (s->frames > 0) {
+        if ((rc = pair())) return rc;
+        if (has_flow) *has_flow = 1;
     }
+    OFB_CUDA_TRY(cudaStreamSynchronize(s->ctx->stream));
+    s->cur ^= 1;
+    s->frames++;
     return OFB_OK;
 }
 
@@ -1692,29 +1657,14 @@ static int stream_fb_pair(ofb_stream *s, float alpha, float beta, float *const *
 {
     ofb_ctx *c = s->ctx;
     const ofb_params &p = s->p;
-    const int L = p.levels;
     cudaStream_t st = c->stream;
     uint8_t *B = s->mem, *F = s->fb_mem;
-    PairPlan pl; // (run_levels reads the level sizes from it)
-    pl.L = L;
-    size_t istr[OFB_MAX_LEVELS];
-    const uint8_t *prv_lv[OFB_MAX_LEVELS], *cur_lv[OFB_MAX_LEVELS];
-    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS] = {};
-    for (int k = 0; k < L; k++) {
-        pl.w[k] = p.w >> k;
-        pl.h[k] = p.h >> k;
-        istr[k] = s->pitch[k] * (size_t)pl.h[k];
-        prv_lv[k] = B + s->off_pyr[s->cur ^ 1][k];
-        cur_lv[k] = B + s->off_pyr[s->cur][k];
-        flow[0][k] = reinterpret_cast<float *>(B + s->off_flow[k]);
-        flow[1][k] = reinterpret_cast<float *>(F + s->off_bflow[k]);
-        if (k >= 1 && k <= L - 2) {
-            cum[0][k] = reinterpret_cast<float *>(B + s->off_cum[k]);
-            cum[1][k] = reinterpret_cast<float *>(F + s->off_bcum[k]);
-        }
-    }
+    const PairLevels lv = stream_pair_levels(s);
+    float *flow[2][OFB_MAX_LEVELS], *cum[2][OFB_MAX_LEVELS];
+    stream_flow(s, false, flow[0], cum[0]);
+    stream_flow(s, true, flow[1], cum[1]);
     float *fwd = reinterpret_cast<float *>(B + s->off_total), *bwd = reinterpret_cast<float *>(F + s->off_btotal);
-    auto backward = [&](cudaStream_t bst) { return run_levels(c, &p, pl, cur_lv, prv_lv, s->pitch, istr, flow[1], cum[1], bwd, bst); };
+    auto backward = [&](cudaStream_t bst) { return run_levels(c, &p, lv, true, flow[1], cum[1], bwd, bst); };
     const bool fork = !fb_serial();
     int rc;
     if (fork) {
@@ -1723,15 +1673,15 @@ static int stream_fb_pair(ofb_stream *s, float alpha, float beta, float *const *
         if ((rc = backward(s->fb_stream))) return rc;
         OFB_CUDA_TRY(cudaEventRecord(s->fb_join, s->fb_stream));
     }
-    if ((rc = run_levels(c, &p, pl, prv_lv, cur_lv, s->pitch, istr, flow[0], cum[0], fwd, st))) return rc;
+    if ((rc = run_levels(c, &p, lv, false, flow[0], cum[0], fwd, st))) return rc;
     if (fork) OFB_CUDA_TRY(cudaStreamWaitEvent(st, s->fb_join, 0));
     else if ((rc = backward(st))) return rc;
     uint8_t *status = F + s->off_status;
     float *err2 = err2_h ? reinterpret_cast<float *>(F + s->off_err2) : nullptr;
     if ((rc = run_fb_check(c, fwd, bwd, p.w, p.h, 1, p.flow_scale, alpha, beta, status, err2, st))) return rc;
-    for (int k = L - 1; k >= 0; k--)
+    for (int k = p.levels - 1; k >= 0; k--)
         if (flow_levels_h && flow_levels_h[k])
-            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k], flow[0][k], (size_t)pl.w[k] * pl.h[k] * 8, cudaMemcpyDeviceToHost, st));
+            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k], flow[0][k], (size_t)(p.w >> k) * (p.h >> k) * 8, cudaMemcpyDeviceToHost, st));
     const size_t px = (size_t)p.w * p.h;
     OFB_CUDA_TRY(cudaMemcpyAsync(fwd_total_h, fwd, px * 8, cudaMemcpyDeviceToHost, st));
     if (bwd_total_h) OFB_CUDA_TRY(cudaMemcpyAsync(bwd_total_h, bwd, px * 8, cudaMemcpyDeviceToHost, st));
@@ -1781,7 +1731,7 @@ int ofb_stream_create(ofb_ctx *c, const ofb_params *p, int bil_win, double bil_s
         s->off_pyr[0][k] = cv.take(s->pitch[k] * hk);
         s->off_pyr[1][k] = cv.take(s->pitch[k] * hk);
         s->off_flow[k] = cv.take((size_t)wk * hk * 8);
-        s->off_cum[k] = cv.take((size_t)wk * hk * 8);
+        if (k >= 1 && k <= p->levels - 2) s->off_cum[k] = cv.take((size_t)wk * hk * 8);
     }
     s->off_gray = cv.take(s->pitch[0] * p->h);
     s->off_total = cv.take((size_t)p->w * p->h * 8);
@@ -1850,49 +1800,18 @@ int ofb_stream_push_bgr_host(ofb_stream *s, const unsigned char *frame_bgr, floa
             }
     }
     OFB_GUARD(c);
-    cudaStream_t st = c->stream;
-    uint8_t *B = s->mem;
-    const int cur = s->cur, prv = cur ^ 1;
-    if (has_flow) *has_flow = 0;
-    int rc = stream_new_frame(s, frame_bgr);
-    if (rc) return rc;
-    if (s->frames > 0) {
-        for (int k = p.levels - 1; k >= 0; k--) { // main.cu:256-262
-            LkLevelArgs a{};
-            a.prev = B + s->off_pyr[prv][k];
-            a.next = B + s->off_pyr[cur][k];
-            a.pitch = s->pitch[k];
-            a.image_stride = s->pitch[k] * (size_t)(p.h >> k);
-            a.w = p.w >> k;
-            a.h_local = a.h_global = p.h >> k;
-            a.out_y1 = p.h >> k;
-            a.n_pairs = 1;
-            a.win = p.win;
-            a.warp_mode = p.warp_mode;
-            a.flow_scale = p.flow_scale;
-            a.flow_out = reinterpret_cast<float *>(B + s->off_flow[k]);
-            a.sm_count = c->sm_count;
-            a.solve_fast = c->solve_fast;
-            if (k < p.levels - 1) {
-                a.cum_in = reinterpret_cast<const float *>(k + 1 == p.levels - 1 ? B + s->off_flow[k + 1] : B + s->off_cum[k + 1]);
-                a.cum_w = p.w >> (k + 1);
-                a.cum_h_global = a.cum_h_local = p.h >> (k + 1);
-            }
-            if (k == 0) a.cum_out = total_flow_h ? reinterpret_cast<float *>(B + s->off_total) : nullptr;
-            else if (k <= p.levels - 2) a.cum_out = reinterpret_cast<float *>(B + s->off_cum[k]);
-            rc = launch_lk_level(a, st, &c->launches);
-            if (rc) return rc;
-            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k], B + s->off_flow[k], (size_t)(p.w >> k) * (p.h >> k) * 8,
-                                         cudaMemcpyDeviceToHost, st));
-        }
-        if (total_flow_h)
-            OFB_CUDA_TRY(cudaMemcpyAsync(total_flow_h, B + s->off_total, (size_t)p.w * p.h * 8, cudaMemcpyDeviceToHost, st));
-        if (has_flow) *has_flow = 1;
-    }
-    OFB_CUDA_TRY(cudaStreamSynchronize(st));
-    s->cur = prv; // main.cu:270-272: the current pyramid becomes the previous one
-    s->frames++;
-    return OFB_OK;
+    return stream_push(s, frame_bgr, has_flow, [&]() -> int {
+        cudaStream_t st = c->stream;
+        float *flow[OFB_MAX_LEVELS], *cum[OFB_MAX_LEVELS];
+        stream_flow(s, false, flow, cum);
+        float *total = total_flow_h ? reinterpret_cast<float *>(s->mem + s->off_total) : nullptr;
+        int rc = run_levels(c, &p, stream_pair_levels(s), false, flow, cum, total, st);
+        if (rc) return rc;
+        for (int k = p.levels - 1; k >= 0; k--)
+            OFB_CUDA_TRY(cudaMemcpyAsync(flow_levels_h[k], flow[k], (size_t)(p.w >> k) * (p.h >> k) * 8, cudaMemcpyDeviceToHost, st));
+        if (total_flow_h) OFB_CUDA_TRY(cudaMemcpyAsync(total_flow_h, total, (size_t)p.w * p.h * 8, cudaMemcpyDeviceToHost, st));
+        return OFB_OK;
+    });
 }
 
 int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, float alpha, float beta, float *const *flow_levels_h,
@@ -1902,28 +1821,17 @@ int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, f
         set_error("stream_push_fb: NULL stream, frame, fwd_total_h or status_h");
         return OFB_ERR_INVALID;
     }
-    ofb_ctx *c = s->ctx;
-    const ofb_params &p = s->p;
-    int rc = check_fb_args(p.flow_scale, alpha, beta);
+    int rc = check_fb_args(s->p.flow_scale, alpha, beta);
     if (rc) return rc;
-    OFB_GUARD(c);
+    OFB_GUARD(s->ctx);
     // (before anything is enqueued: a failed set-up leaves the sequence where it was)
     if ((rc = stream_fb_setup(s))) return rc;
-    cudaStream_t st = c->stream;
-    if (has_flow) *has_flow = 0;
-    if ((rc = stream_new_frame(s, frame_bgr))) return rc;
-    if (s->frames > 0) {
-        if ((rc = stream_fb_pair(s, alpha, beta, flow_levels_h, fwd_total_h, bwd_total_h, status_h, err2_h))) {
-            // (a failure after the fork: the backward loop may still read the pyramid the next push overwrites)
-            cudaStreamSynchronize(s->fb_stream);
-            return rc;
-        }
-        if (has_flow) *has_flow = 1;
-    }
-    OFB_CUDA_TRY(cudaStreamSynchronize(st));
-    s->cur ^= 1;
-    s->frames++;
-    return OFB_OK;
+    return stream_push(s, frame_bgr, has_flow, [&]() -> int {
+        int rc = stream_fb_pair(s, alpha, beta, flow_levels_h, fwd_total_h, bwd_total_h, status_h, err2_h);
+        // (a failure after the fork: the backward loop may still read the pyramid the next push overwrites)
+        if (rc) cudaStreamSynchronize(s->fb_stream);
+        return rc;
+    });
 }
 
 } // extern "C"

@@ -120,6 +120,15 @@ struct LkLevelArgs {
     const unsigned *epoch_src;
 };
 int launch_lk_level(const LkLevelArgs &a, cudaStream_t stream, unsigned long long *launches);
+// The level's geometry and solve, everything else zero; callers add the coarser flow, cum_out and the peer fields.
+// Whole frames: n_pairs images of w x h, every row produced.
+LkLevelArgs lk_args_frame(const uint8_t *prev, const uint8_t *next, size_t pitch, size_t image_stride, int w, int h, int n_pairs,
+                          int win, int warp_mode, float flow_scale, float *flow_out, int sm_count, int solve_fast);
+// One row strip of one pair: rows [y_off, y_off + h_local) of a level of height h_global held, local rows
+// [out_y0, out_y1) produced.
+LkLevelArgs lk_args_strip(const uint8_t *prev, const uint8_t *next, size_t pitch, int w, int h_local, int y_off, int h_global,
+                          int out_y0, int out_y1, int win, int warp_mode, float flow_scale, float *flow_out, int sm_count,
+                          int solve_fast);
 int preload_lk_level(int win); // loads the window's kernels now instead of at their first launch
 int preload_pyramid();
 

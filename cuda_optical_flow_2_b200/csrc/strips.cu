@@ -198,6 +198,29 @@ static ArenaLayout arena_layout(const StripPlan &pl, int rank)
     return a;
 }
 
+// Exchange x of a pair moves rows of one level from the ranks that own them into the window of that level other ranks'
+// buffers hold.  `rank`'s own rows [*o0, *o1) and window [*w0, *w1): x = 0 level-0 image rows into the image buffers;
+// x = j or L-1+j (backward), j = 1 .. L-1, cumulative flow of level L-j into the cum_in rows of level L-1-j; x = 2L-1
+// level-0 backward total rows into the rows the check holds.
+static void exchange_rows(const StripPlan &pl, int x, int rank, int *o0, int *o1, int *w0, int *w1)
+{
+    const int L = pl.levels;
+    if (x == 0 || x == 2 * L - 1) {
+        const LevelStrip s = pl.strips(rank)[0];
+        *o0 = s.y0, *o1 = s.y1;
+        if (x == 0) *w0 = s.eb0, *w1 = s.eb1;
+        else pl.fb_rows(rank, w0, w1);
+        return;
+    }
+    const int j = x < L ? x : x - (L - 1);
+    const LevelStrip own = pl.level(L - j, rank), fine = pl.level(L - 1 - j, rank);
+    *o0 = own.y0, *o1 = own.y1, *w0 = fine.cy0, *w1 = fine.cy1;
+}
+// Rows [lo, hi) of one exchange between this rank and `peer`; the receiving rank's buffer starts at global row `base`.
+struct HaloRows {
+    int peer, lo, hi, base;
+};
+
 struct PeerSeg {
     const void *src;
     void *dst; // inside a peer's arena
@@ -319,7 +342,8 @@ struct ofb_strips {
     float flow_scale = 1.0f;
     ncclComm_t comm = nullptr;
     std::vector<LevelStrip> s;                 // this rank's strip per level
-    std::vector<LevelStrip> peer0;             // every rank's level-0 strip (for the one image exchange)
+    // the halo-row table, per exchange x in [0, lay.nx) (numbering: ArenaLayout): rows this rank sends and receives
+    std::vector<std::vector<HaloRows>> send, recv;
     std::vector<size_t> pitch;                 // image pitch per level
     std::vector<uint8_t *> prev, next;         // [eb0, eb1) rows
     std::vector<float *> flow, cum, cum_in;    // flow / cum: buffer rows (origin eb0); cum_in[k]: rows [cy0, cy1) of cum_{k+1}
@@ -338,13 +362,13 @@ struct ofb_strips {
     std::vector<void *> ipc_opened;
     bool peers_connected = false;
     std::vector<int> done_from;             // ranks this one pushes to: they write done[rank] into this arena (teardown waits for it)
+    std::vector<int> sources;               // ranks that push to this one, in a pair of either kind: told when their rows are used
     // checked pairs (ofb_strips_create_fb): the backward direction's buffers, laid out like the forward ones
     std::vector<float *> flow_b, cum_in_b, cum_dst_b; // cum_dst_b[0]: level 0's rows inside fbh
     float *fbh = nullptr;                   // backward total flow, rows [hy0, hy1) of level 0 (in the arena)
     int hy0 = 0, hy1 = 0;
     uint8_t *status = nullptr;              // own rows [y0, y1) of level 0
     float *err2 = nullptr;
-    std::vector<int> fb_sources;            // ranks whose own rows lie in [hy0, hy1): they push check rows to this one
 };
 
 namespace {
@@ -376,10 +400,10 @@ inline unsigned *flag_ptr(uint8_t *arena, const ArenaLayout &lay, size_t index)
 {
     return reinterpret_cast<unsigned *>(arena + lay.flags) + index;
 }
-// Exchange x of the pair with epoch `epoch`: push `sends`, then wait for the ranks in `sources`.
+// Exchange x of the pair: push `sends`, then wait for the ranks this one receives rows from (recv[x]).
 // (do_push / do_wait: the two halves, which ofb_strips_run_phase_device enqueues separately.)
-int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, const std::vector<int> &sources, cudaStream_t q,
-                  unsigned long long *launches, bool do_push = true, bool do_wait = true)
+int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, cudaStream_t q, unsigned long long *launches, bool do_push,
+                  bool do_wait)
 {
     const int me = st->rank;
     unsigned *pairs = flag_ptr(st->arena, st->lay, st->lay.pairs());
@@ -403,7 +427,6 @@ int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, con
                 a.arrive[a.ndst] = flag_ptr(st->peer_arena[sd.peer], st->peer_lay[sd.peer], st->peer_lay[sd.peer].arrive(x, me));
                 a.done_local[a.ndst] = flag_ptr(st->arena, st->lay, st->lay.done(sd.peer));
                 a.ndst++;
-                if (std::find(st->done_from.begin(), st->done_from.end(), sd.peer) == st->done_from.end()) st->done_from.push_back(sd.peer);
             }
         }
         a.counter = flag_ptr(st->arena, st->lay, st->lay.counter(x));
@@ -414,14 +437,14 @@ int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, con
         OFB_CUDA_TRY(cudaGetLastError());
         if (launches) ++*launches;
     }
-    if (do_wait && !sources.empty()) {
+    if (do_wait && !st->recv[x].empty()) {
         PeerWaitArgs w{};
-        for (int src : sources) {
+        for (const HaloRows &e : st->recv[x]) {
             if (w.n == PEER_MAX_DST) {
                 set_error("strips: exchange %d receives from more than %d ranks", x, PEER_MAX_DST);
                 return OFB_ERR_UNSUPPORTED;
             }
-            w.flag[w.n++] = flag_ptr(st->arena, st->lay, st->lay.arrive(x, src));
+            w.flag[w.n++] = flag_ptr(st->arena, st->lay, st->lay.arrive(x, e.peer));
         }
         w.pairs = pairs;
         w.err = st->overflow;
@@ -530,9 +553,29 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
     pl.coarse_bounds.push_back(hc);
     int rc = OFB_OK;
     st->s = pl.strips(rank);
-    for (int peer = 0; peer < world; peer++) st->peer0.push_back(pl.strips(peer)[0]);
     // what neighbours write into (level-0 image rows, coarser cumulative-flow rows, flags): one allocation, the arena
     st->lay = arena_layout(pl, rank);
+    // The halo-row table.  Sender and receiver lists come from the same exchange_rows, so they agree; the backward
+    // exchanges repeat the forward ones.  The end-of-pair handshake and the teardown drain cover every rank that can
+    // push to / be pushed to by this one in either kind of pair.
+    st->send.assign(st->lay.nx, {});
+    st->recv.assign(st->lay.nx, {});
+    for (int x = 0; x < st->lay.nx; x++) {
+        int m0, m1, mw0, mw1;
+        exchange_rows(pl, x, rank, &m0, &m1, &mw0, &mw1);
+        for (int peer = 0; peer < world; peer++) {
+            int p0, p1, pw0, pw1, lo, hi;
+            if (peer == rank) continue;
+            exchange_rows(pl, x, peer, &p0, &p1, &pw0, &pw1);
+            if (overlap(m0, m1, pw0, pw1, &lo, &hi)) st->send[x].push_back({peer, lo, hi, pw0});
+            if (overlap(p0, p1, mw0, mw1, &lo, &hi)) st->recv[x].push_back({peer, lo, hi, mw0});
+        }
+        for (const HaloRows &e : st->send[x]) add_unique(st->done_from, e.peer);
+    }
+    if (fb_reach >= 0) // (the check-row senders first: the handshake kernel's flags keep their order)
+        for (const HaloRows &e : st->recv[2 * levels - 1]) add_unique(st->sources, e.peer);
+    for (int x = 0; x < st->lay.nx; x++)
+        for (const HaloRows &e : st->recv[x]) add_unique(st->sources, e.peer);
     {
         void *p = nullptr;
         rc = dev_alloc(st, &p, st->lay.bytes);
@@ -567,11 +610,6 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
     if (fb_reach >= 0) {
         pl.fb_rows(rank, &st->hy0, &st->hy1);
         st->fbh = reinterpret_cast<float *>(st->arena + st->lay.fbh);
-        for (int peer = 0; peer < world; peer++) {
-            const LevelStrip ps = pl.level(0, peer);
-            int lo, hi;
-            if (peer != rank && overlap(ps.y0, ps.y1, st->hy0, st->hy1, &lo, &hi)) st->fb_sources.push_back(peer);
-        }
         const size_t own = s_own_px(st);
         void *p = nullptr;
         if (rc == OFB_OK) rc = dev_alloc(st, &p, own);
@@ -724,20 +762,8 @@ namespace {
 // ranks whose buffers I write into, or that write into mine, at any exchange
 bool is_neighbour(const ofb_strips *st, int peer)
 {
-    const StripPlan &pl = st->plan;
-    int lo, hi;
-    const LevelStrip &s = st->s[0], &ps = st->peer0[peer];
-    if (overlap(s.y0, s.y1, ps.eb0, ps.eb1, &lo, &hi) || overlap(ps.y0, ps.y1, s.eb0, s.eb1, &lo, &hi)) return true;
-    for (int k = 0; k + 1 < pl.levels; k++) {
-        const LevelStrip up = st->s[k + 1], sk = st->s[k], pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
-        if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi) || overlap(pu.y0, pu.y1, sk.cy0, sk.cy1, &lo, &hi)) return true;
-    }
-    if (pl.fb_reach >= 0) { // backward total rows for the check, in either direction
-        int plo, phi;
-        pl.fb_rows(peer, &plo, &phi);
-        if (overlap(s.y0, s.y1, plo, phi, &lo, &hi) || overlap(ps.y0, ps.y1, st->hy0, st->hy1, &lo, &hi)) return true;
-    }
-    return false;
+    return std::find(st->done_from.begin(), st->done_from.end(), peer) != st->done_from.end() ||
+           std::find(st->sources.begin(), st->sources.end(), peer) != st->sources.end();
 }
 int finish_connect(ofb_strips *st)
 {
@@ -888,8 +914,8 @@ namespace {
 // neighbours' cumulative-flow rows arrive by exchange xb + L - 1 - k; the loop's phases start at pb (see
 // strips_run_impl).  In the backward loop of a checked pair level 0 writes the backward total into fbh, and -- fused
 // form, at most two targets -- its kernel also pushes the rows the neighbours' checks need (*check_pushed).
-int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream_t q, int phase, std::vector<int> &all_sources,
-                  bool *check_pushed, unsigned long long *launches)
+int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream_t q, int phase, bool *check_pushed,
+                  unsigned long long *launches)
 {
     auto on = [phase](int ph) { return phase < 0 || phase == ph; };
     const StripPlan &pl = st->plan;
@@ -903,122 +929,68 @@ int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream
     bool pushed_by_kernel = false; // the exchange that feeds the level at hand was pushed by the previous (coarser) level's kernel
     for (int k = L - 1; k >= 0; k--) {
         const LevelStrip &s = st->s[k];
-        struct WaitSrc {
-            int peer, crow_lo, crow_hi;
-        } wait_src[2] = {};
-        int nwait = 0;
+        const int j = L - 1 - k, x = xb + j; // this level's step of the loop, and the exchange that feeds it
         bool wait_in_kernel = false;
-        const int j = L - 1 - k; // this level's step of the loop
         if (k < L - 1) {
             const LevelStrip &up = st->s[k + 1];
             // level k+1 wrote its own rows of cum_{k+1} straight into cum_in[k] (cum_dst); the neighbours' rows follow
             const float *src = cum_dst[k + 1]; // buffer-row indexing of level k+1 (origin up.eb0)
             const size_t rowf = (size_t)up.w * 2;  // floats per row
-            int lo, hi;
             if (n) {
                 OFB_NCCL_TRY(n->GroupStart());
-                for (int peer = 0; peer < pl.world; peer++) {
-                    if (peer == me) continue;
-                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
-                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
-                        OFB_NCCL_TRY(n->Send(src + (size_t)(lo - up.eb0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer, st->comm, q));
-                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) // the peer's cum rows I need
-                        OFB_NCCL_TRY(n->Recv(cum_in[k] + (size_t)(lo - s.cy0) * rowf, (size_t)(hi - lo) * rowf * 4, NCCL_UINT8, peer,
-                                             st->comm, q));
-                }
+                for (const HaloRows &e : st->send[x])
+                    OFB_NCCL_TRY(n->Send(src + (size_t)(e.lo - up.eb0) * rowf, (size_t)(e.hi - e.lo) * rowf * 4, NCCL_UINT8, e.peer, st->comm, q));
+                for (const HaloRows &e : st->recv[x])
+                    OFB_NCCL_TRY(n->Recv(cum_in[k] + (size_t)(e.lo - e.base) * rowf, (size_t)(e.hi - e.lo) * rowf * 4, NCCL_UINT8, e.peer,
+                                         st->comm, q));
                 OFB_NCCL_TRY(n->GroupEnd());
             }
             if (peer_mode) {
                 std::vector<PeerSend> sends;
-                std::vector<int> sources;
-                for (int peer = 0; peer < pl.world; peer++) {
-                    if (peer == me) continue;
-                    const LevelStrip pk = pl.level(k, peer), pu = pl.level(k + 1, peer);
-                    if (overlap(up.y0, up.y1, pk.cy0, pk.cy1, &lo, &hi)) // my cum rows the peer needs
-                        sends.push_back({peer, src + (size_t)(lo - up.eb0) * rowf, peer_cum_in(peer, k) + (size_t)(lo - pk.cy0) * rowf * 4,
-                                         (size_t)(hi - lo) * rowf * 4});
-                    if (overlap(pu.y0, pu.y1, s.cy0, s.cy1, &lo, &hi)) { // the peer's cum rows I need
-                        sources.push_back(peer);
-                        add_unique(all_sources, peer);
-                        if (nwait < 2) wait_src[nwait] = {peer, lo - s.cy0, hi - s.cy0};
-                        nwait++;
-                    }
-                }
+                for (const HaloRows &e : st->send[x])
+                    sends.push_back({e.peer, src + (size_t)(e.lo - up.eb0) * rowf, peer_cum_in(e.peer, k) + (size_t)(e.lo - e.base) * rowf * 4,
+                                     (size_t)(e.hi - e.lo) * rowf * 4});
                 // Fused form: level k+1's kernel has already pushed my rows (pushed_by_kernel, previous iteration) and this
                 // level's kernel waits for the neighbours' flags itself; the copy / wait kernels remain for what does not
                 // fit the kernel's two slots (strips thinner than the halo).
-                wait_in_kernel = st->fused && nwait >= 1 && nwait <= 2;
-                int rc = peer_exchange(st, xb + j, sends, sources, q, launches, on(pb + 2 * j) && !pushed_by_kernel,
-                                       on(pb + 2 * j + 1) && !wait_in_kernel);
+                wait_in_kernel = st->fused && !st->recv[x].empty() && st->recv[x].size() <= 2;
+                int rc = peer_exchange(st, x, sends, q, launches, on(pb + 2 * j) && !pushed_by_kernel, on(pb + 2 * j + 1) && !wait_in_kernel);
                 if (rc) return rc;
             }
         }
-        // what THIS level's kernel pushes: my rows of cum_k that the neighbours' level k-1 needs (exchange xb + L - k), or,
-        // at level 0 of the backward loop of a checked pair, my rows of the backward total their checks need (2L - 1)
+        // what THIS level's kernel pushes: my rows of cum_k that the neighbours' level k-1 needs (exchange x + 1), or, at
+        // level 0 of the backward loop of a checked pair, my rows of the backward total their checks need (2L - 1)
         LkLevelArgs::PeerPush push[2] = {};
-        int npush = 0, xn = 0;
+        int npush = 0;
+        const int xn = k >= 1 ? x + 1 : 2 * L - 1;
         pushed_by_kernel = false;
-        if (peer_mode && st->fused && (k >= 1 || (bwd && checked))) {
-            int cnt = 0, lo, hi;
-            xn = k >= 1 ? xb + L - k : 2 * L - 1;
-            for (int peer = 0; peer < pl.world; peer++) {
-                if (peer == me) continue;
-                int plo, phi;
-                if (k >= 1) { // the peer's finer level reads rows [cy0, cy1) of cum_k
-                    const LevelStrip pf = pl.level(k - 1, peer);
-                    plo = pf.cy0, phi = pf.cy1;
-                } else {
-                    pl.fb_rows(peer, &plo, &phi);
-                }
-                if (!overlap(s.y0, s.y1, plo, phi, &lo, &hi)) continue;
-                if (cnt < 2 && st->peer_arena[peer]) {
-                    const ArenaLayout &pa = st->peer_lay[peer];
-                    push[cnt].dst = reinterpret_cast<float *>(st->peer_arena[peer] + (k >= 1 ? peer_cum_in(peer, k - 1) : pa.fbh)) +
-                                    ((ptrdiff_t)s.eb0 - plo) * (ptrdiff_t)s.w * 2;
-                    push[cnt].row_lo = lo - s.eb0;
-                    push[cnt].row_hi = hi - s.eb0;
-                    push[cnt].flag = flag_ptr(st->peer_arena[peer], pa, pa.arrive(xn, me));
-                    push[cnt].done = flag_ptr(st->arena, st->lay, st->lay.done(peer));
-                    add_unique(st->done_from, peer);
-                }
-                cnt++;
+        if (peer_mode && st->fused && (k >= 1 || (bwd && checked)) && !st->send[xn].empty() && st->send[xn].size() <= 2) {
+            for (const HaloRows &e : st->send[xn]) {
+                const ArenaLayout &pa = st->peer_lay[e.peer];
+                push[npush].dst = reinterpret_cast<float *>(st->peer_arena[e.peer] + (k >= 1 ? peer_cum_in(e.peer, k - 1) : pa.fbh)) +
+                                  ((ptrdiff_t)s.eb0 - e.base) * (ptrdiff_t)s.w * 2;
+                push[npush].row_lo = e.lo - s.eb0;
+                push[npush].row_hi = e.hi - s.eb0;
+                push[npush].flag = flag_ptr(st->peer_arena[e.peer], pa, pa.arrive(xn, me));
+                push[npush].done = flag_ptr(st->arena, st->lay, st->lay.done(e.peer));
+                npush++;
             }
-            if (cnt >= 1 && cnt <= 2) {
-                npush = cnt;
-                pushed_by_kernel = true;
-            }
+            pushed_by_kernel = true;
         }
         if (k == 0 && bwd) *check_pushed = pushed_by_kernel;
         if (!on(pb + 2 * j + 1)) continue;
-        LkLevelArgs a{};
-        a.prev = bwd ? st->next[k] : st->prev[k];
-        a.next = bwd ? st->prev[k] : st->next[k];
-        a.pitch = st->pitch[k];
-        a.image_stride = a.pitch * (size_t)(s.eb1 - s.eb0);
-        a.w = s.w;
-        a.h_local = s.eb1 - s.eb0;
-        a.y_off = s.eb0;
-        a.h_global = s.h;
-        a.out_y0 = s.y0 - s.eb0;
-        a.out_y1 = s.y1 - s.eb0;
-        a.n_pairs = 1;
-        a.win = pl.win;
-        a.warp_mode = st->warp_mode;
-        a.flow_scale = st->flow_scale;
+        LkLevelArgs a = lk_args_strip(bwd ? st->next[k] : st->prev[k], bwd ? st->prev[k] : st->next[k], st->pitch[k], s.w, s.eb1 - s.eb0,
+                                      s.eb0, s.h, s.y0 - s.eb0, s.y1 - s.eb0, pl.win, st->warp_mode, st->flow_scale, flow[k],
+                                      ctx_sm_count(st->ctx), ctx_solve_fast(st->ctx));
         a.cum_in = k < L - 1 ? cum_in[k] : nullptr;
         a.cum_w = s.w >> 1;
         a.cum_h_global = s.h >> 1;
         a.cum_y_off = s.cy0;
         a.cum_h_local = std::max(s.cy1 - s.cy0, 1);
-        a.cum_pair_stride = 0;
-        a.flow_out = flow[k];
         // every level but the finest feeds the next one; level 0 writes the total flow (always in a checked pair)
         const bool want_cum = k > 0 || checked || (L > 1 && st->want_total);
         a.cum_out = want_cum ? cum_dst[k] : nullptr;
-        a.flow_pair_stride = 0;
         a.reach_overflow = st->overflow;
-        a.sm_count = ctx_sm_count(st->ctx);
-        a.solve_fast = ctx_solve_fast(st->ctx);
         if (npush > 0 && a.cum_out) {
             a.npush = npush;
             a.push[0] = push[0];
@@ -1026,9 +998,10 @@ int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream
             a.push_counter = flag_ptr(st->arena, st->lay, st->lay.fused(xn));
         }
         if (wait_in_kernel) {
-            a.nwait = nwait;
-            for (int d = 0; d < nwait; d++)
-                a.wait[d] = {flag_ptr(st->arena, st->lay, st->lay.arrive(xb + j, wait_src[d].peer)), wait_src[d].crow_lo, wait_src[d].crow_hi};
+            const std::vector<HaloRows> &rv = st->recv[x];
+            a.nwait = (int)rv.size();
+            for (int d = 0; d < a.nwait; d++)
+                a.wait[d] = {flag_ptr(st->arena, st->lay, st->lay.arrive(x, rv[d].peer)), rv[d].lo - s.cy0, rv[d].hi - s.cy0};
         }
         a.epoch_src = flag_ptr(st->arena, st->lay, st->lay.pairs());
         int rc = launch_lk_level(a, q, launches);
@@ -1092,7 +1065,6 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
         return OFB_ERR_INVALID;
     }
     unsigned long long *launches = ctx_launch_counter(st->ctx);
-    std::vector<int> all_sources = st->fb_sources; // every rank that pushes to me during a pair of either kind
     if (pitch < (size_t)pl.W) {
         set_error("strips_run: pitch %zu smaller than the width %d", pitch, pl.W);
         return OFB_ERR_INVALID;
@@ -1110,45 +1082,28 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
     }
     // (the error flag st->overflow is sticky: kernels OR into it, only ofb_strips_check clears it)
     // ONE image exchange, on level 0: the rows of my buffer that other ranks own (and vice versa), in place
+    const int eb0 = st->s[0].eb0;
+    const size_t P = st->pitch[0];
     if (n) {
-        const LevelStrip &s = st->s[0];
-        const size_t P = st->pitch[0];
         OFB_NCCL_TRY(n->GroupStart());
-        for (int peer = 0; peer < pl.world; peer++) {
-            if (peer == me) continue;
-            const LevelStrip &ps = st->peer0[peer];
-            int lo, hi;
-            if (overlap(s.y0, s.y1, ps.eb0, ps.eb1, &lo, &hi)) { // my rows the peer's buffer holds
-                OFB_NCCL_TRY(n->Send(st->prev[0] + (size_t)(lo - s.eb0) * P, (size_t)(hi - lo) * P, NCCL_UINT8, peer, st->comm, q));
-                OFB_NCCL_TRY(n->Send(st->next[0] + (size_t)(lo - s.eb0) * P, (size_t)(hi - lo) * P, NCCL_UINT8, peer, st->comm, q));
-            }
-            if (overlap(ps.y0, ps.y1, s.eb0, s.eb1, &lo, &hi)) { // the peer's rows my buffer holds
-                OFB_NCCL_TRY(n->Recv(st->prev[0] + (size_t)(lo - s.eb0) * P, (size_t)(hi - lo) * P, NCCL_UINT8, peer, st->comm, q));
-                OFB_NCCL_TRY(n->Recv(st->next[0] + (size_t)(lo - s.eb0) * P, (size_t)(hi - lo) * P, NCCL_UINT8, peer, st->comm, q));
-            }
+        for (const HaloRows &e : st->send[0]) {
+            OFB_NCCL_TRY(n->Send(st->prev[0] + (size_t)(e.lo - eb0) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
+            OFB_NCCL_TRY(n->Send(st->next[0] + (size_t)(e.lo - eb0) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
+        }
+        for (const HaloRows &e : st->recv[0]) {
+            OFB_NCCL_TRY(n->Recv(st->prev[0] + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
+            OFB_NCCL_TRY(n->Recv(st->next[0] + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
         }
         OFB_NCCL_TRY(n->GroupEnd());
     }
     if (peer_mode) {
-        const LevelStrip &s = st->s[0];
-        const size_t P = st->pitch[0];
         std::vector<PeerSend> sends;
-        std::vector<int> sources;
-        for (int peer = 0; peer < pl.world; peer++) {
-            if (peer == me) continue;
-            const LevelStrip &ps = st->peer0[peer];
-            int lo, hi;
-            if (overlap(s.y0, s.y1, ps.eb0, ps.eb1, &lo, &hi)) { // my rows the peer's buffer holds
-                const ArenaLayout &pa = st->peer_lay[peer];
-                sends.push_back({peer, st->prev[0] + (size_t)(lo - s.eb0) * P, pa.prev0 + (size_t)(lo - ps.eb0) * P, (size_t)(hi - lo) * P});
-                sends.push_back({peer, st->next[0] + (size_t)(lo - s.eb0) * P, pa.next0 + (size_t)(lo - ps.eb0) * P, (size_t)(hi - lo) * P});
-            }
-            if (overlap(ps.y0, ps.y1, s.eb0, s.eb1, &lo, &hi)) { // the peer's rows my buffer holds
-                sources.push_back(peer);
-                add_unique(all_sources, peer);
-            }
+        for (const HaloRows &e : st->send[0]) {
+            const ArenaLayout &pa = st->peer_lay[e.peer];
+            sends.push_back({e.peer, st->prev[0] + (size_t)(e.lo - eb0) * P, pa.prev0 + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P});
+            sends.push_back({e.peer, st->next[0] + (size_t)(e.lo - eb0) * P, pa.next0 + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P});
         }
-        int rc = peer_exchange(st, 0, sends, sources, q, launches, on(0), on(1));
+        int rc = peer_exchange(st, 0, sends, q, launches, on(0), on(1));
         if (rc) return rc;
     }
     // pyramid: every buffer row of level k+1 from the buffer rows of level k (halo rows are built locally)
@@ -1159,24 +1114,20 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
         if (rc) return rc;
     }
     bool check_pushed = false;
-    int rc = strips_levels(st, false, fb != nullptr, n, q, phase, all_sources, &check_pushed, launches);
+    int rc = strips_levels(st, false, fb != nullptr, n, q, phase, &check_pushed, launches);
     if (rc) return rc;
     if (fb) {
-        if ((rc = strips_levels(st, true, true, n, q, phase, all_sources, &check_pushed, launches))) return rc;
+        if ((rc = strips_levels(st, true, true, n, q, phase, &check_pushed, launches))) return rc;
         // exchange 2L-1: my own rows of the backward total that the neighbours' checks sample (unless level 0's kernel pushed
         // them), then the wait for the rows I sample
         if (peer_mode) {
             const LevelStrip &s = st->s[0];
             const size_t rowf = (size_t)s.w * 2;
             std::vector<PeerSend> sends;
-            for (int peer = 0; peer < pl.world; peer++) {
-                int plo, phi, lo, hi;
-                pl.fb_rows(peer, &plo, &phi);
-                if (peer != me && overlap(s.y0, s.y1, plo, phi, &lo, &hi))
-                    sends.push_back({peer, st->fbh + (size_t)(lo - st->hy0) * rowf, st->peer_lay[peer].fbh + (size_t)(lo - plo) * rowf * 4,
-                                     (size_t)(hi - lo) * rowf * 4});
-            }
-            if ((rc = peer_exchange(st, 2 * L - 1, sends, st->fb_sources, q, launches, on(4 * L - 1) && !check_pushed, on(4 * L))))
+            for (const HaloRows &e : st->send[2 * L - 1])
+                sends.push_back({e.peer, st->fbh + (size_t)(e.lo - st->hy0) * rowf, st->peer_lay[e.peer].fbh + (size_t)(e.lo - e.base) * rowf * 4,
+                                 (size_t)(e.hi - e.lo) * rowf * 4});
+            if ((rc = peer_exchange(st, 2 * L - 1, sends, q, launches, on(4 * L - 1) && !check_pushed, on(4 * L))))
                 return rc;
         }
         if (on(4 * L)) {
@@ -1189,7 +1140,7 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
     }
     if (peer_mode && on(nphase - 1)) { // the rows my neighbours pushed have been used: they may push the next pair's
         PeerDoneArgs d{};
-        for (int src : all_sources) {
+        for (int src : st->sources) {
             if (d.n == 2 * PEER_MAX_DST) {
                 set_error("strips: more than %d ranks push to this one", 2 * PEER_MAX_DST);
                 return OFB_ERR_UNSUPPORTED;

@@ -11,10 +11,11 @@ medians over the rounds are reported.
   host  `lean`: ofb_flow_pairs_host_ex, planar gray in, total flow out (8 B/px: bench.py's `e2e.lean`);
         `fb`:   ofb_flow_pairs_fb_host on the same pairs, planar gray in, forward total + status out (9 B/px).
   stream (ms per push of a 1080p BGR frame): `push` (ofb_stream_push_bgr_host with the total flow: the residual flow of
-        every level and the total come back, 18.5 B/px at 3 levels), `push_fb` (forward total + status back, 9 B/px) with the
+        every level and the total come back, 18.5 B/px at 3 levels), `push_no_total` (the same without the total, 10.5 B/px:
+        level 0 composes the cumulative flow on the fly, level 1 does not write its own), `push_fb` (forward total + status back, 9 B/px) with the
         backward level loop on the stream's second CUDA stream (the default) and with OFB_FB_SERIAL=1 (after the forward
         loop on the context stream).  The override is read once per process, so each mode runs in child processes of its
-        own, which alternate; `push` is timed in both, alternating with `push_fb`.  The children also hash their last
+        own, which alternate; `push` and `push_no_total` are timed in both, alternating with `push_fb`.  The children also hash their last
         outputs: the two modes must give the same bytes.  `push` downloads twice the bytes of `push_fb`, so the
         difference of the two is no cost of the check; the fork is judged by `push_fb` forked against serial.
 The card's name, power limit and maximum SM clock are read with nvidia-smi, the SM clock under load (and any throttle
@@ -76,6 +77,10 @@ def stream_child(mode, rounds, pushes):
         _lib.check(lib.ofb_stream_push_bgr_host(st._h, u8(frames[t[0] % 8]), fptrs, f32(total), C.byref(has)))
         t[0] += 1
 
+    def push_no_total():
+        _lib.check(lib.ofb_stream_push_bgr_host(st._h, u8(frames[t[0] % 8]), fptrs, None, C.byref(has)))
+        t[0] += 1
+
     def push_fb():
         _lib.check(lib.ofb_stream_push_bgr_host_fb(st._h, u8(frames[t[0] % 8]), ALPHA, BETA, None, f32(fwd), None, u8(status), None,
                                                    C.byref(has)))
@@ -87,14 +92,16 @@ def stream_child(mode, rounds, pushes):
             fn()
         return (time.perf_counter() - t0) / pushes * 1e3
 
-    for fn in (push, push_fb, push, push_fb):  # warm-up: kernels loaded, buffers and the second stream created
-        block(fn)
-    ms = {"push": [], "push_fb": []}
+    arms = {"push": push, "push_no_total": push_no_total, "push_fb": push_fb}
+    for _ in range(2):  # warm-up: kernels loaded, buffers and the second stream created
+        for fn in arms.values():
+            block(fn)
+    ms = {k: [] for k in arms}
     clocks = ClockSampler(0)
     clocks.start()
     for _ in range(rounds):
-        ms["push"].append(block(push))
-        ms["push_fb"].append(block(push_fb))
+        for k, fn in arms.items():
+            ms[k].append(block(fn))
     clk = clocks.stop()
     # the last push_fb's frames are fixed by the counter: identical inputs in every child
     digest = hashlib.sha256(fwd.tobytes() + status.tobytes()).hexdigest()
@@ -192,13 +199,13 @@ def main():
     kids = run_children(args.rounds, args.pushes, args.children)
     level_bytes = sum(8 / 4 ** k for k in range(LEVELS))  # residual flow of every level, per level-0 pixel
     stream = {"pushes_per_block": args.pushes, "rounds_per_child": args.rounds, "children_per_mode": args.children,
-              "d2h_bytes_per_px": {"push": level_bytes + 8, "push_fb": 9}, "h2d_bytes_per_px": 3}
+              "d2h_bytes_per_px": {"push": level_bytes + 8, "push_no_total": level_bytes, "push_fb": 9}, "h2d_bytes_per_px": 3}
     for mode in ("fork", "serial"):
-        push = [x for c in kids[mode] for x in c["ms"]["push"]]
-        pfb = [x for c in kids[mode] for x in c["ms"]["push_fb"]]
-        stream[mode] = {"push_ms_median": float(np.median(push)), "push_fb_ms_median": float(np.median(pfb)),
-                        "push_fb_ms_min": float(np.min(pfb)), "push_fb_ms_max": float(np.max(pfb)),
-                        "clocks_under_load_per_child": [c["clocks_under_load"] for c in kids[mode]]}
+        stream[mode] = {"clocks_under_load_per_child": [c["clocks_under_load"] for c in kids[mode]]}
+        for arm in ("push", "push_no_total", "push_fb"):
+            v = [x for c in kids[mode] for x in c["ms"][arm]]
+            stream[mode].update({f"{arm}_ms_median": float(np.median(v)), f"{arm}_ms_min": float(np.min(v)),
+                                 f"{arm}_ms_max": float(np.max(v))})
     digests = {c["last_push_fb_sha256"] for m in ("fork", "serial") for c in kids[m]}
     stream["fork_and_serial_same_bytes"] = len(digests) == 1
     stream["fork_saves_ms"] = stream["serial"]["push_fb_ms_median"] - stream["fork"]["push_fb_ms_median"]
