@@ -93,9 +93,8 @@ SIGNATURES = {
     "ofb_stream_push_bgr_host": (C.c_int, [_vp, u8p, C.POINTER(f32p), f32p, i32p]),
     "ofb_stream_destroy": (C.c_int, [_vp]),
     "ofb_strips_plan_query": (C.c_int, [C.c_int] * 8 + [i32p]),
-    "ofb_strips_nccl_unique_id": (C.c_int, [_vp]),
     "ofb_strips_create": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
-                                    _vp, C.POINTER(_vp)]),
+                                    C.POINTER(_vp)]),
     "ofb_strips_own_rows": (C.c_int, [_vp, C.c_int, i32p, i32p]),
     "ofb_strips_run_device": (C.c_int, [_vp, _vp, _vp, _sz, _vp]),
     "ofb_strips_run_phase_device": (C.c_int, [_vp, _vp, _vp, _sz, C.c_int, _vp]),
@@ -110,7 +109,7 @@ SIGNATURES = {
     "ofb_strips_peer_arena": (C.c_int, [_vp, C.POINTER(_vp)]),
     "ofb_strips_peer_connect_local": (C.c_int, [_vp, C.POINTER(_vp)]),
     "ofb_strips_create_fb": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
-                                       C.c_int, _vp, C.POINTER(_vp)]),
+                                       C.c_int, C.POINTER(_vp)]),
     "ofb_strips_run_fb_device": (C.c_int, [_vp, _vp, _vp, _sz, C.c_float, C.c_float, C.c_int, _vp]),
     "ofb_strips_run_fb_phase_device": (C.c_int, [_vp, _vp, _vp, _sz, C.c_float, C.c_float, C.c_int, C.c_int, _vp]),
     "ofb_strips_fb_result": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),

@@ -551,7 +551,7 @@ using namespace ofb;
 extern "C" {
 
 const char *ofb_last_error(void) { return g_err; }
-int ofb_version(void) { return 100; }
+int ofb_version(void) { return 101; }
 
 int ofb_ctx_create(int device, ofb_ctx **out)
 {

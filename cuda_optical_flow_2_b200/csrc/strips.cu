@@ -3,28 +3,21 @@
 // One process per GPU.  The strip schedule is the one of cuda_optical_flow_2_b200/dist.py (StripPlan: bounds fixed
 // on the coarsest level and doubled per finer level, image halo = window radius + stencil + warp reach, coarser
 // cumulative-flow halo), but here the whole pair -- own-row upload, per-level halo exchange, pyramid, fused level
-// kernels -- is enqueued on one CUDA stream from C++ with no host synchronisation, and the halo rows move by NCCL
-// send/recv (NVLink / NVSwitch) straight between the ranks' image and flow buffers: rows are contiguous, so there
-// is no staging copy.  Only level-0 image rows are exchanged (the coarser levels' halo rows are rebuilt locally), so a
-// pair of L levels costs L exchanges: one for the images, L-1 for the cumulative flow.  The Python StripRunner runs
-// the 2L-1-exchange form of the schedule through torch and is bound by ~100 us of host work per exchange.
+// kernels -- is enqueued on one CUDA stream from C++ with no host synchronisation.  Only level-0 image rows are
+// exchanged (the coarser levels' halo rows are rebuilt locally), so a pair of L levels costs L exchanges: one for the
+// images, L-1 for the cumulative flow.  The Python StripRunner runs the 2L-1-exchange form of the schedule through torch
+// and is bound by ~100 us of host work per exchange.
 //
-// Second transport, peer memory (ofb_strips_peer_*): every rank keeps the buffers its neighbours write into -- the
-// level-0 image rows and the coarser cumulative-flow rows -- in ONE device allocation (the arena) whose CUDA IPC
-// handle the application all-gathers once.  An exchange is then a copy kernel of the SENDER that stores the halo rows
-// straight into the receiver's arena over NVLink and raises an epoch flag there, and a one-block wait kernel on the
-// receiver's stream; no NCCL call, no host work beyond two launches (~5 us instead of ~30 us per exchange).
-//
-// NCCL is not a link-time dependency of the library: libnccl.so.2 is opened on first use (inside a torch process
-// that is the copy torch already loaded), and every symbol is resolved with dlsym.
+// The halo rows move through peer memory: every rank keeps the buffers its neighbours write into -- the level-0 image
+// rows and the coarser cumulative-flow rows -- in ONE device allocation (the arena) whose CUDA IPC handle the
+// application all-gathers once.  An exchange is then a store of the SENDER's kernels straight into the receiver's arena
+// over NVLink plus an epoch flag raised there, and a wait for that flag on the receiver's stream: no collective, no host
+// work beyond at most two launches per exchange.
 #include "ofb_common.cuh"
-
-#include <dlfcn.h>
 
 #include <algorithm>
 #include <cmath>
 #include <cstring>
-#include <mutex>
 #include <new>
 #include <vector>
 
@@ -35,58 +28,6 @@ int ctx_device(const ofb_ctx *c);
 int ctx_sm_count(const ofb_ctx *c);
 int ctx_solve_fast(const ofb_ctx *c);
 unsigned long long *ctx_launch_counter(ofb_ctx *c);
-
-// ---- NCCL through dlopen ------------------------------------------------------------------------------------
-typedef struct ncclComm *ncclComm_t;
-struct NcclUniqueId {
-    char internal[128];
-};
-enum { NCCL_SUCCESS = 0, NCCL_UINT8 = 1 };
-struct NcclApi {
-    int (*GetUniqueId)(NcclUniqueId *);
-    int (*CommInitRank)(ncclComm_t *, int, NcclUniqueId, int);
-    int (*CommDestroy)(ncclComm_t);
-    int (*Send)(const void *, size_t, int, int, ncclComm_t, cudaStream_t);
-    int (*Recv)(void *, size_t, int, int, ncclComm_t, cudaStream_t);
-    int (*GroupStart)();
-    int (*GroupEnd)();
-    const char *(*GetErrorString)(int);
-    bool ok = false;
-};
-static NcclApi *nccl()
-{
-    static NcclApi api;
-    static std::once_flag once;
-    std::call_once(once, [] {
-        void *h = dlopen("libnccl.so.2", RTLD_NOW | RTLD_GLOBAL);
-        if (!h) h = dlopen("libnccl.so", RTLD_NOW | RTLD_GLOBAL);
-        if (!h) return;
-        bool all = true;
-        auto sym = [&](const char *n) {
-            void *p = dlsym(h, n);
-            if (!p) all = false;
-            return p;
-        };
-        api.GetUniqueId = reinterpret_cast<decltype(api.GetUniqueId)>(sym("ncclGetUniqueId"));
-        api.CommInitRank = reinterpret_cast<decltype(api.CommInitRank)>(sym("ncclCommInitRank"));
-        api.CommDestroy = reinterpret_cast<decltype(api.CommDestroy)>(sym("ncclCommDestroy"));
-        api.Send = reinterpret_cast<decltype(api.Send)>(sym("ncclSend"));
-        api.Recv = reinterpret_cast<decltype(api.Recv)>(sym("ncclRecv"));
-        api.GroupStart = reinterpret_cast<decltype(api.GroupStart)>(sym("ncclGroupStart"));
-        api.GroupEnd = reinterpret_cast<decltype(api.GroupEnd)>(sym("ncclGroupEnd"));
-        api.GetErrorString = reinterpret_cast<decltype(api.GetErrorString)>(sym("ncclGetErrorString"));
-        api.ok = all;
-    });
-    return api.ok ? &api : nullptr;
-}
-#define OFB_NCCL_TRY(expr)                                                                                    \
-    do {                                                                                                      \
-        int _r = (expr);                                                                                      \
-        if (_r != NCCL_SUCCESS) {                                                                             \
-            ofb::set_error("%s:%d: %s failed: %s", __FILE__, __LINE__, #expr, ofb::nccl()->GetErrorString(_r)); \
-            return OFB_ERR_CUDA;                                                                              \
-        }                                                                                                     \
-    } while (0)
 
 // ---- the strip schedule (dist.py: StripPlan) ---------------------------------------------------------------------
 struct LevelStrip {
@@ -146,7 +87,7 @@ struct StripPlan {
     }
 };
 
-// ---- peer-memory transport ------------------------------------------------------------------------------------
+// ---- peer memory ------------------------------------------------------------------------------------------------
 // Arena of one rank: [prev level 0][next level 0][cum_in level 0 .. L-2][flags]; a handle that runs checked pairs also has
 // [cum_in_b level 0 .. L-2][fbh: held rows of the backward total flow] before the flags.  Every rank can compute every
 // other rank's layout from the plan, so a peer address is (peer arena base) + (offset computed here).
@@ -340,7 +281,6 @@ struct ofb_strips {
     StripPlan plan;
     int rank = 0, warp_mode = OFB_WARP_BILINEAR;
     float flow_scale = 1.0f;
-    ncclComm_t comm = nullptr;
     std::vector<LevelStrip> s;                 // this rank's strip per level
     // the halo-row table, per exchange x in [0, lay.nx) (numbering: ArenaLayout): rows this rank sends and receives
     std::vector<std::vector<HaloRows>> send, recv;
@@ -351,10 +291,10 @@ struct ofb_strips {
     std::vector<float *> cum_dst;              // where level k's kernel writes its cumulative flow (buffer-row indexing like
                                                // flow[k]): straight into cum_in[k-1], whose rows [cy0, cy1) contain the own rows
     int want_total = 1;                        // level 0 also writes its cumulative flow (the total flow of the pair)
-    int fused = 1;                             // peer-memory transport: cumulative-flow halo rows are pushed by the level kernels themselves
+    int fused = 1;                             // cumulative-flow halo rows are pushed by the level kernels themselves
     int *overflow = nullptr;
     std::vector<void *> allocs;
-    // peer-memory transport
+    // peer memory
     uint8_t *arena = nullptr;               // my arena (one cudaMalloc: prev[0], next[0], cum_in[], flags live in it)
     ArenaLayout lay;
     std::vector<uint8_t *> peer_arena;      // base of every rank's arena in this process's address space (nullptr: not mapped)
@@ -389,7 +329,7 @@ inline bool overlap(int own0, int own1, int b0, int b1, int *lo, int *hi)
     return *lo < *hi;
 }
 
-// ---- peer-memory transport: one exchange ------------------------------------------------------------------------------
+// ---- peer memory: one exchange ---------------------------------------------------------------------------------------
 struct PeerSend {
     int peer;
     const void *src;
@@ -490,37 +430,16 @@ int ofb_strips_plan_query(int w, int h, int levels, int win, int world, int rank
     return OFB_OK;
 }
 
-int ofb_strips_nccl_unique_id(void *id128)
-{
-    NcclApi *n = nccl();
-    if (!n) {
-        set_error("libnccl.so.2 could not be loaded");
-        return OFB_ERR_UNSUPPORTED;
-    }
-    if (!id128) {
-        set_error("NULL id buffer");
-        return OFB_ERR_INVALID;
-    }
-    NcclUniqueId id;
-    OFB_NCCL_TRY(n->GetUniqueId(&id));
-    memcpy(id128, &id, sizeof id);
-    return OFB_OK;
-}
-
 } // extern "C"
 
 // ofb_strips_create (fb_reach < 0) and ofb_strips_create_fb
 static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                              int reach, int fb_reach, const void *nccl_id128, ofb_strips **out)
+                              int reach, int fb_reach, ofb_strips **out)
 {
     if (!ctx || !out || w < 1 || h < 1 || levels < 1 || levels > OFB_MAX_LEVELS || (win & 1) == 0 || win < 3 ||
         win > OFB_MAX_WINDOW || world < 1 || rank < 0 || rank >= world || reach < 0) {
         set_error("strips_create: bad arguments");
         return OFB_ERR_INVALID;
-    }
-    if (fb_reach >= 0 && world > 1 && nccl_id128) {
-        set_error("strips_create_fb: checked pairs run on the peer-memory transport (nccl_id128 = NULL) or on one rank");
-        return OFB_ERR_UNSUPPORTED;
     }
     if (warp_mode == OFB_WARP_AS_WRITTEN && levels > 1) {
         set_error("OFB_WARP_AS_WRITTEN needs pixel (0,0) of every coarser level: not available on strips");
@@ -648,21 +567,6 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
         rc = dev_alloc(st, &p, sizeof(int));
         st->overflow = static_cast<int *>(p);
     }
-    if (rc == OFB_OK && world > 1 && nccl_id128) {
-        NcclApi *n = nccl();
-        if (!n) {
-            set_error("libnccl.so.2 could not be loaded");
-            rc = OFB_ERR_UNSUPPORTED;
-        } else {
-            NcclUniqueId id;
-            memcpy(&id, nccl_id128, sizeof id);
-            const int r = n->CommInitRank(&st->comm, world, id, rank);
-            if (r != NCCL_SUCCESS) {
-                set_error("ncclCommInitRank failed: %s", n->GetErrorString(r));
-                rc = OFB_ERR_CUDA;
-            }
-        }
-    }
     // every kernel a pair launches is loaded now: a lazily loaded kernel may synchronise the context at its first
     // launch, which must not happen behind a kernel that waits for a neighbour
     if (rc == OFB_OK) rc = preload_lk_level(win);
@@ -698,22 +602,22 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
 extern "C" {
 
 int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                      int reach, const void *nccl_id128, ofb_strips **out)
+                      int reach, ofb_strips **out)
 {
-    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, -1, nccl_id128, out);
+    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, -1, out);
 }
 
 int ofb_strips_create_fb(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                         int reach, int fb_reach, const void *nccl_id128, ofb_strips **out)
+                         int reach, int fb_reach, ofb_strips **out)
 {
     if (fb_reach < 0 || !(std::isfinite(flow_scale) && flow_scale > 0.0f)) {
         set_error("strips_create_fb: fb_reach %d must be >= 0 and flow_scale %g finite and > 0", fb_reach, (double)flow_scale);
         return OFB_ERR_INVALID;
     }
-    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, fb_reach, nccl_id128, out);
+    return strips_create_impl(ctx, w, h, levels, win, warp_mode, flow_scale, world, rank, reach, fb_reach, out);
 }
 
-// ---- peer-memory transport: set-up -------------------------------------------------------------------------------
+// ---- peer memory: set-up ----------------------------------------------------------------------------------------
 // The 128-byte blob a rank publishes: its arena's CUDA IPC handle and the arena's offset inside the allocation the
 // handle stands for (small cudaMalloc blocks share one).
 int ofb_strips_peer_handle(ofb_strips *st, void *blob128)
@@ -824,7 +728,7 @@ int ofb_strips_destroy(ofb_strips *st)
         DeviceGuard guard(ctx_device(st->ctx));
         if (guard.ok) {
             cudaDeviceSynchronize();
-            if (st->plan.world > 1 && st->peers_connected && !st->comm && !st->done_from.empty()) {
+            if (st->plan.world > 1 && st->peers_connected && !st->done_from.empty()) {
                 PeerDrainArgs d{};
                 for (int dst : st->done_from)
                     if (d.n < 2 * PEER_MAX_DST) d.flag[d.n++] = flag_ptr(st->arena, st->lay, st->lay.done(dst));
@@ -834,7 +738,6 @@ int ofb_strips_destroy(ofb_strips *st)
                 cudaDeviceSynchronize();
             }
             for (void *p : st->ipc_opened) cudaIpcCloseMemHandle(p);
-            if (st->comm && nccl()) nccl()->CommDestroy(st->comm);
             for (void *p : st->allocs) cudaFree(p);
         }
     }
@@ -895,7 +798,7 @@ int ofb_strips_set_total(ofb_strips *st, int on)
 }
 
 // Whether the cumulative-flow halo rows are pushed by the level kernels themselves (default) or by separate copy / wait
-// kernels (peer-memory transport; for comparison).
+// kernels (for comparison).
 int ofb_strips_set_fused(ofb_strips *st, int on)
 {
     if (!st) {
@@ -914,12 +817,12 @@ namespace {
 // neighbours' cumulative-flow rows arrive by exchange xb + L - 1 - k; the loop's phases start at pb (see
 // strips_run_impl).  In the backward loop of a checked pair level 0 writes the backward total into fbh, and -- fused
 // form, at most two targets -- its kernel also pushes the rows the neighbours' checks need (*check_pushed).
-int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream_t q, int phase, bool *check_pushed,
+int strips_levels(ofb_strips *st, bool bwd, bool checked, cudaStream_t q, int phase, bool *check_pushed,
                   unsigned long long *launches)
 {
     auto on = [phase](int ph) { return phase < 0 || phase == ph; };
     const StripPlan &pl = st->plan;
-    const bool peer_mode = pl.world > 1 && !st->comm;
+    const bool peer_mode = pl.world > 1;
     const int L = pl.levels, me = st->rank;
     const int pb = bwd ? 2 * L - 1 : 0, xb = bwd ? L - 1 : 0;
     const std::vector<float *> &flow = bwd ? st->flow_b : st->flow, &cum_in = bwd ? st->cum_in_b : st->cum_in;
@@ -936,15 +839,6 @@ int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream
             // level k+1 wrote its own rows of cum_{k+1} straight into cum_in[k] (cum_dst); the neighbours' rows follow
             const float *src = cum_dst[k + 1]; // buffer-row indexing of level k+1 (origin up.eb0)
             const size_t rowf = (size_t)up.w * 2;  // floats per row
-            if (n) {
-                OFB_NCCL_TRY(n->GroupStart());
-                for (const HaloRows &e : st->send[x])
-                    OFB_NCCL_TRY(n->Send(src + (size_t)(e.lo - up.eb0) * rowf, (size_t)(e.hi - e.lo) * rowf * 4, NCCL_UINT8, e.peer, st->comm, q));
-                for (const HaloRows &e : st->recv[x])
-                    OFB_NCCL_TRY(n->Recv(cum_in[k] + (size_t)(e.lo - e.base) * rowf, (size_t)(e.hi - e.lo) * rowf * 4, NCCL_UINT8, e.peer,
-                                         st->comm, q));
-                OFB_NCCL_TRY(n->GroupEnd());
-            }
             if (peer_mode) {
                 std::vector<PeerSend> sends;
                 for (const HaloRows &e : st->send[x])
@@ -1016,8 +910,8 @@ int strips_levels(ofb_strips *st, bool bwd, bool checked, NcclApi *n, cudaStream
 // fb != NULL: a checked pair (handles of ofb_strips_create_fb): the backward level loop on the same pyramid, the exchange
 // of the backward total rows the neighbours' checks sample, and the check of the own rows.
 //
-// `phase` < 0: the whole pair.  Otherwise one of its phases (peer-memory transport only), so that a host can interleave
-// the ranks of ONE process on ONE stream in an order in which no kernel ever waits for a later one:
+// `phase` < 0: the whole pair.  Otherwise one of its phases, so that a host can interleave the ranks of ONE process on ONE
+// stream in an order in which no kernel ever waits for a later one:
 //   phase 0      own-row upload, push of the level-0 image rows (exchange 0)
 //   phase 1      wait for exchange 0, pyramid, coarsest level L-1
 //   phase 2j     push of the cumulative-flow rows of level L-j (exchange j),            j = 1 .. L-1
@@ -1052,16 +946,15 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
     auto on = [phase](int ph) { return phase < 0 || phase == ph; };
     cudaStream_t q = static_cast<cudaStream_t>(stream);
     const StripPlan &pl = st->plan;
-    const bool peer_mode = pl.world > 1 && !st->comm;
+    const bool peer_mode = pl.world > 1;
     if (peer_mode && !st->peers_connected) {
-        set_error("strips_run: no transport (create with a NCCL id, or call ofb_strips_peer_connect first)");
+        set_error("strips_run: world > 1 and the peers are not connected (call ofb_strips_peer_connect first)");
         return OFB_ERR_INVALID;
     }
-    NcclApi *n = pl.world > 1 && !peer_mode ? nccl() : nullptr;
     const int L = pl.levels, me = st->rank;
     const int nphase = fb ? 4 * L + 1 : 2 * L;
-    if (phase >= 0 && (n || phase >= nphase)) {
-        set_error("strips_run_phase: phase %d of %d (phases exist for the peer-memory transport and one rank only)", phase, nphase);
+    if (phase >= nphase) {
+        set_error("strips_run_phase: phase %d of %d", phase, nphase);
         return OFB_ERR_INVALID;
     }
     unsigned long long *launches = ctx_launch_counter(st->ctx);
@@ -1084,18 +977,6 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
     // ONE image exchange, on level 0: the rows of my buffer that other ranks own (and vice versa), in place
     const int eb0 = st->s[0].eb0;
     const size_t P = st->pitch[0];
-    if (n) {
-        OFB_NCCL_TRY(n->GroupStart());
-        for (const HaloRows &e : st->send[0]) {
-            OFB_NCCL_TRY(n->Send(st->prev[0] + (size_t)(e.lo - eb0) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
-            OFB_NCCL_TRY(n->Send(st->next[0] + (size_t)(e.lo - eb0) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
-        }
-        for (const HaloRows &e : st->recv[0]) {
-            OFB_NCCL_TRY(n->Recv(st->prev[0] + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
-            OFB_NCCL_TRY(n->Recv(st->next[0] + (size_t)(e.lo - e.base) * P, (size_t)(e.hi - e.lo) * P, NCCL_UINT8, e.peer, st->comm, q));
-        }
-        OFB_NCCL_TRY(n->GroupEnd());
-    }
     if (peer_mode) {
         std::vector<PeerSend> sends;
         for (const HaloRows &e : st->send[0]) {
@@ -1114,10 +995,10 @@ static int strips_run_impl(ofb_strips *st, const uint8_t *prev_own_d, const uint
         if (rc) return rc;
     }
     bool check_pushed = false;
-    int rc = strips_levels(st, false, fb != nullptr, n, q, phase, &check_pushed, launches);
+    int rc = strips_levels(st, false, fb != nullptr, q, phase, &check_pushed, launches);
     if (rc) return rc;
     if (fb) {
-        if ((rc = strips_levels(st, true, true, n, q, phase, &check_pushed, launches))) return rc;
+        if ((rc = strips_levels(st, true, true, q, phase, &check_pushed, launches))) return rc;
         // exchange 2L-1: my own rows of the backward total that the neighbours' checks sample (unless level 0's kernel pushed
         // them), then the wait for the rows I sample
         if (peer_mode) {

@@ -376,50 +376,37 @@ class StripRunner:
 
 class NativeStrips:
     """The native row-strip runner (csrc/strips.cu): the same schedule as StripRunner, but a whole pair is enqueued
-    from C++ on one stream.  transport "nccl": the halo rows move by NCCL send/recv between the ranks' buffers;
-    "peer": by the sender's copy kernel straight into the receiver's memory over NVLink (CUDA IPC), epoch flags instead
-    of a collective; "local": peer memory between ranks living in this process (connect_local, tests).
-    `torch.distributed` is used once, to hand round the NCCL unique id or the IPC handles.
+    from C++ on one stream.  The halo rows move through peer memory: the sender's kernels store them straight into the
+    receiver's memory over NVLink and raise epoch flags there.  transport "peer": ranks in separate processes, connected
+    over CUDA IPC (`torch.distributed` is used once, to hand round the IPC handles); "local": ranks living in this process
+    (connect_local, tests).
 
     fb_reach (an int >= 0) makes a handle that can also run checked pairs (run_fb: the forward-backward consistency check
-    of Context.flow_pairs_fb_device on the strips; peer or local transport, or world 1): a rank's check may sample
-    backward rows up to fb_reach rows beyond its own."""
+    of Context.flow_pairs_fb_device on the strips): a rank's check may sample backward rows up to fb_reach rows beyond its
+    own."""
 
     def __init__(self, ctx, w: int, h: int, levels: int, win: int, world: int, rank: int, device, warp_mode: int = WARP_BILINEAR,
-                 flow_scale: float = 1.0, reach: int = 16, transport: str = "nccl", fb_reach: Optional[int] = None):
+                 flow_scale: float = 1.0, reach: int = 16, transport: str = "peer", fb_reach: Optional[int] = None):
         import ctypes as C
 
         import torch
 
         from . import _lib as L
 
-        if transport not in ("nccl", "peer", "local"):
-            raise ValueError(f"unknown strip transport {transport!r}")
+        if transport not in ("peer", "local"):
+            raise ValueError(f"strip transport must be 'peer' or 'local', not {transport!r}")
         self.torch, self.C, self.L, self.lib, self.ctx = torch, C, L, L.load(), ctx
         self.w, self.h, self.levels, self.dev, self.world, self.rank = w, h, levels, device, world, rank
         self.flow_scale = flow_scale
         self._transport = transport
-        idbuf = torch.zeros(128, dtype=torch.uint8)
-        use_nccl = world > 1 and transport == "nccl"
-        if use_nccl:
-            import torch.distributed as dist
-
-            if rank == 0:
-                raw = (C.c_ubyte * 128)()
-                L.check(self.lib.ofb_strips_nccl_unique_id(C.cast(raw, C.c_void_p)))
-                idbuf = torch.tensor(list(raw), dtype=torch.uint8)
-            idbuf = idbuf.to(device)
-            dist.broadcast(idbuf, 0)
-        raw = (C.c_ubyte * 128)(*idbuf.cpu().tolist())
         hnd = C.c_void_p()
-        nccl_id = C.cast(raw, C.c_void_p) if use_nccl else None
         self.fb_reach = fb_reach
         if fb_reach is None:
             L.check(self.lib.ofb_strips_create(ctx._h, w, h, levels, win, warp_mode, C.c_float(flow_scale), world, rank, reach,
-                                               nccl_id, C.byref(hnd)))
+                                               C.byref(hnd)))
         else:
             L.check(self.lib.ofb_strips_create_fb(ctx._h, w, h, levels, win, warp_mode, C.c_float(flow_scale), world, rank, reach,
-                                                  int(fb_reach), nccl_id, C.byref(hnd)))
+                                                  int(fb_reach), C.byref(hnd)))
         self._h = hnd
         if world > 1 and transport == "peer":
             import torch.distributed as dist

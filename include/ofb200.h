@@ -245,31 +245,24 @@ int ofb_stream_destroy(ofb_stream *s);
 /* ---- row strips of one large pair over several GPUs (BASELINE configs[4]); the reference is single-GPU ----------
  * One process per GPU, one handle per process.  The schedule (strip bounds fixed on the coarsest level and doubled
  * per finer level; per level the neighbours' image halo rows and the next-coarser cumulative-flow rows) is that of
- * cuda_optical_flow_2_b200/dist.py; here a whole pair is enqueued on one stream without host synchronisation and
- * the halo rows move by NCCL send/recv between the ranks' buffers (libnccl.so.2 is opened on first use; it is not
- * a link-time dependency).  The result is bit-identical to the whole-frame result unless ofb_strips_check reports
- * that a warp sample reached past the exchanged rows (`reach`, in rows of the level being warped).
- * Two transports for the halo rows:
- *   NCCL send/recv   : ofb_strips_create with rank 0's broadcast ofb_strips_nccl_unique_id;
- *   peer memory      : ofb_strips_create with nccl_id128 = NULL, then every rank publishes ofb_strips_peer_handle
- *                      (128 bytes: a CUDA IPC handle of the one allocation its neighbours write into), the
- *                      application all-gathers the blobs and hands them to ofb_strips_peer_connect.  An exchange is
- *                      then a copy kernel of the sender that stores the rows into the receiver's memory over NVLink
- *                      and raises an epoch flag there, plus a one-block wait kernel on the receiver's stream.
- *                      ofb_strips_peer_connect_local does the same for ranks living in one process.
+ * cuda_optical_flow_2_b200/dist.py; here a whole pair is enqueued on one stream without host synchronisation.
+ * The result is bit-identical to the whole-frame result unless ofb_strips_check reports that a warp sample reached
+ * past the exchanged rows (`reach`, in rows of the level being warped).
+ * The halo rows move through peer memory.  After ofb_strips_create (not a collective) every rank of a world > 1
+ * publishes ofb_strips_peer_handle (128 bytes: a CUDA IPC handle of the one allocation its neighbours write into), the
+ * application all-gathers the blobs and hands them to ofb_strips_peer_connect.  An exchange is then a store of the
+ * sender's kernels into the receiver's memory over NVLink plus an epoch flag raised there, and a wait for that flag on the
+ * receiver's stream.  ofb_strips_peer_connect_local does the same for ranks living in one process.
  *   ofb_strips_plan_query     : host only, no device: the rows {y0, y1, by0, by1, cy0, cy1, eb0, eb1} of a level on a rank
- *   ofb_strips_nccl_unique_id : rank 0 makes the 128-byte id, the application broadcasts it (any transport)
- *   ofb_strips_create         : collective over all ranks when a NCCL id is given (ncclCommInitRank)
  *   ofb_strips_check          : synchronises; *overflow bit 0 = a warp sample reached past the halo rows, bit 1 = a
- *                               neighbour's rows did not arrive within 4 s (peer-memory transport), bit 2 = a checked
- *                               pair's check needed a backward tap outside the rows the rank holds (OFB_FB_UNCHECKED
- *                               pixels: raise fb_reach).  The flag is sticky: it covers every pair since the previous
- *                               check, which clears it
- *   ofb_strips_run_phase_device: one of the 2 * levels phases of a pair (peer-memory transport): 0 = upload + push of the
- *                               level-0 image rows; 1 = wait, pyramid, coarsest level; 2j = push of the cumulative flow of
- *                               level L-j; 2j+1 = wait, level L-1-j (j = 1 .. L-1).  A host that runs several ranks in ONE
- *                               process on ONE stream (tests on a single GPU) enqueues phase p of every rank before phase
- *                               p+1 of any: no kernel then ever waits for a kernel enqueued after it
+ *                               neighbour's rows did not arrive within 4 s, bit 2 = a checked pair's check needed a
+ *                               backward tap outside the rows the rank holds (OFB_FB_UNCHECKED pixels: raise fb_reach).
+ *                               The flag is sticky: it covers every pair since the previous check, which clears it
+ *   ofb_strips_run_phase_device: one of the 2 * levels phases of a pair: 0 = upload + push of the level-0 image rows;
+ *                               1 = wait, pyramid, coarsest level; 2j = push of the cumulative flow of level L-j;
+ *                               2j+1 = wait, level L-1-j (j = 1 .. L-1).  A host that runs several ranks in ONE process
+ *                               on ONE stream (tests on a single GPU) enqueues phase p of every rank before phase p+1 of
+ *                               any: no kernel then ever waits for a kernel enqueued after it
  *   ofb_strips_destroy        : waits (bounded) until every neighbour has acknowledged this rank's last pair before its
  *                               arena is unmapped and freed; all ranks must have run the same number of pairs.  Across
  *                               processes also put a barrier between the last check and the destroy calls
@@ -280,9 +273,8 @@ int ofb_stream_destroy(ofb_stream *s);
  *   ofb_strips_set_total      : whether level 0 also writes the total flow of the pair (default on) */
 typedef struct ofb_strips ofb_strips;
 int ofb_strips_plan_query(int w, int h, int levels, int win, int world, int rank, int reach, int level, int *out8);
-int ofb_strips_nccl_unique_id(void *id128);
 int ofb_strips_create(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                      int reach, const void *nccl_id128, ofb_strips **out);
+                      int reach, ofb_strips **out);
 int ofb_strips_own_rows(const ofb_strips *s, int level, int *y0, int *y1);
 int ofb_strips_run_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, void *stream);
 int ofb_strips_run_phase_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, int phase,
@@ -308,8 +300,7 @@ int ofb_strips_peer_connect_local(ofb_strips *s, void *const *arenas_d);
  *                          rank's check may sample: it holds backward total rows [max(0, y0 - fb_reach), min(h, y1 +
  *                          fb_reach + 1)).  The arena also holds the backward direction's regions, so a handle that runs
  *                          checked pairs is created this way (before ofb_strips_peer_handle / _connect).  flow_scale > 0.
- *                          Peer-memory transport or world == 1 only: world > 1 with a NCCL id is OFB_ERR_UNSUPPORTED
- *                          (nothing allocated).  Plain pairs (ofb_strips_run_device) run on it unchanged, and plain and
+ *                          Plain pairs (ofb_strips_run_device) run on it unchanged, and plain and
  *                          checked pairs may alternate; all ranks must be created with the same fb_reach.
  *   ofb_strips_run_fb_device : one checked pair; alpha >= 0, beta >= 0 as in ofb_flow_pairs_fb_device; want_err2 = 0 leaves
  *                          the err2 buffer untouched.  Bad arguments are refused before anything is enqueued.
@@ -329,7 +320,7 @@ int ofb_strips_peer_connect_local(ofb_strips *s, void *const *arenas_d);
  * ofb_strips_check reports bit 0 or bit 2, every output is bit-identical to rows [y0, y1) of ofb_flow_pairs_fb_device on
  * the whole frame with the same parameters and solve mode. */
 int ofb_strips_create_fb(ofb_ctx *ctx, int w, int h, int levels, int win, int warp_mode, float flow_scale, int world, int rank,
-                         int reach, int fb_reach, const void *nccl_id128, ofb_strips **out);
+                         int reach, int fb_reach, ofb_strips **out);
 int ofb_strips_run_fb_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha,
                              float beta, int want_err2, void *stream);
 int ofb_strips_run_fb_phase_device(ofb_strips *s, const uint8_t *prev_own_d, const uint8_t *next_own_d, size_t pitch, float alpha,

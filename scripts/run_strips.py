@@ -1,8 +1,9 @@
 """Row-strip run of one large pair over N GPUs (torchrun), BASELINE.json configs[4]:
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         scripts/run_strips.py [--w 7680 --h 4320 --levels 4 --win 9 --reps 10 --check]
-Every rank generates the same synthetic frames, keeps only its own rows, exchanges halos over NCCL
-per pyramid level and solves its strip.  --check compares against the whole-frame result computed
+Every rank generates the same synthetic frames, keeps only its own rows, exchanges halos per pyramid
+level and solves its strip: the Python StripRunner over torch.distributed, or with --native the native
+runner over peer memory (CUDA IPC).  --check compares against the whole-frame result computed
 on rank 0's GPU (bit for bit).  Prints one JSON line on rank 0."""
 import argparse, json, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -18,8 +19,8 @@ ap.add_argument("--w", type=int, default=7680); ap.add_argument("--h", type=int,
 ap.add_argument("--levels", type=int, default=4); ap.add_argument("--win", type=int, default=9)
 ap.add_argument("--reps", type=int, default=10); ap.add_argument("--reach", type=int, default=16)
 ap.add_argument("--check", action="store_true")
-ap.add_argument("--transport", default="gather", choices=["gather", "p2p", "nccl", "peer"], help="Python runner: one all-gather per exchange (gather) or grouped send/recv (p2p); --native: NCCL send/recv (nccl, default) or the sender's copy kernel into the receiver's memory over NVLink with epoch flags (peer)")
-ap.add_argument("--native", action="store_true", help="the native runner (csrc/strips.cu: C++ host side, NCCL send/recv between the ranks' buffers)")
+ap.add_argument("--transport", default="gather", choices=["gather", "p2p"], help="Python runner only: one all-gather per exchange (gather) or grouped send/recv (p2p)")
+ap.add_argument("--native", action="store_true", help="the native runner (csrc/strips.cu: C++ host side; the sender's kernels store the halo rows into the receiver's memory over NVLink and raise epoch flags there)")
 ap.add_argument("--total", action="store_true", help="--native: level 0 also writes the total flow of the pair (8 more bytes per pixel)")
 ap.add_argument("--copy-in", action="store_true", help="--native: the own rows are copied into the runner every pair instead of living there (ofb_strips_input)")
 ap.add_argument("--graph", action="store_true", help="capture one pair in a CUDA graph and replay it (1 GPU: works, -8 %; with NCCL exchanges the capture hung on this stack, PyTorch 2.11 + NCCL 2.28: unresolved)")
@@ -38,14 +39,14 @@ class Solo(DistTransport):
 
 if world == 1:
     tp = type("T", (), {"exchange": lambda self, s, r: None})()
-elif a.transport in ("gather", "nccl", "peer"):
+elif a.transport == "gather":
     tp = GatherTransport(rank, world, dev)
 else:
     tp = Solo()
 rn = StripRunner(ctx, plan, rank, tp, dev, WARP_BILINEAR)
 s0 = rn.strips[0]
 pr, nr = prev[0, s0.y0:s0.y1, :a.w], nxt[0, s0.y0:s0.y1, :a.w]
-nat = NativeStrips(ctx, a.w, a.h, a.levels, a.win, world, rank, dev, WARP_BILINEAR, 1.0, a.reach, transport="peer" if a.transport == "peer" else "nccl") if a.native else None
+nat = NativeStrips(ctx, a.w, a.h, a.levels, a.win, world, rank, dev, WARP_BILINEAR, 1.0, a.reach, transport="peer") if a.native else None
 nin = (prev[0, s0.y0:s0.y1], nxt[0, s0.y0:s0.y1])
 if nat is not None:
     nat.set_total(a.total)
@@ -103,5 +104,5 @@ if rank == 0:
            sum((hi - lo) * (a.w >> (k + 1)) * 8 for k in range(a.levels) for _, lo, hi, _ in plan.cum_messages(k, 0))
     print(json.dumps({"mode": "row-strips", "w": a.w, "h": a.h, "levels": a.levels, "win": a.win, "n_gpus": world,
                       "ms_per_pair": t.item(), "mpx_pairs_per_s": a.w * a.h / 1e6 / (t.item() / 1e3),
-                      "bit_identical_to_whole_frame": ok, "cuda_graph": bool(a.graph), "native": bool(a.native), "transport": a.transport if world > 1 else None, "halo_bytes_sent_rank0_per_pair": halo}), flush=True)
+                      "bit_identical_to_whole_frame": ok, "cuda_graph": bool(a.graph), "native": bool(a.native), "transport": ("peer" if a.native else a.transport) if world > 1 else None, "halo_bytes_sent_rank0_per_pair": halo}), flush=True)
 if world > 1: dist.destroy_process_group()

@@ -19,7 +19,7 @@ def declared_symbols():
     return sorted(set(re.findall(r"\b(ofb_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_and_abi_version():
     from cuda_optical_flow_2_b200 import _lib
 
     lib = _lib.load()
@@ -28,7 +28,7 @@ def test_library_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), f"libofb200.so does not export {n}"
     assert sorted(_lib.SIGNATURES) == names, "Python binding and header disagree"
-    assert lib.ofb_version() == 100
+    assert lib.ofb_version() == 101
 
 
 @pytest.mark.parametrize("npix,threads", [(0, 1), (1, 1), (15, 2), (16, 1), (1000003, 3), (2 * 1920 * 1080, 4)])

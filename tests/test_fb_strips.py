@@ -364,7 +364,7 @@ def test_checked_pair_replays_as_cuda_graph(ctx, oracle):
 
 
 @pytest.mark.gpu
-def test_refusals_enqueue_nothing(ctx, oracle):
+def test_checked_strip_refusals_enqueue_nothing(ctx, oracle):
     import ctypes as C
 
     import torch
@@ -374,14 +374,11 @@ def test_refusals_enqueue_nothing(ctx, oracle):
 
     lib = _lib.load()
     h = C.c_void_p()
-    nid = (C.c_ubyte * 128)()
     W, H = 640, 480
-    assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 2, C.c_float(1.0), 2, 0, 16, 8, C.cast(nid, C.c_void_p), C.byref(h)) == \
-        _lib.OFB_ERR_UNSUPPORTED
     for scale in (0.0, -1.0, float("nan")):
-        assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 2, C.c_float(scale), 1, 0, 16, 8, None, C.byref(h)) == _lib.OFB_ERR_INVALID
-    assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 2, C.c_float(1.0), 1, 0, 16, -1, None, C.byref(h)) == _lib.OFB_ERR_INVALID
-    assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 0, C.c_float(1.0), 1, 0, 16, 8, None, C.byref(h)) == \
+        assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 2, C.c_float(scale), 1, 0, 16, 8, C.byref(h)) == _lib.OFB_ERR_INVALID
+    assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 2, C.c_float(1.0), 1, 0, 16, -1, C.byref(h)) == _lib.OFB_ERR_INVALID
+    assert lib.ofb_strips_create_fb(ctx._h, W, H, 3, 9, 0, C.c_float(1.0), 1, 0, 16, 8, C.byref(h)) == \
         _lib.OFB_ERR_UNSUPPORTED  # OFB_WARP_AS_WRITTEN, as ofb_strips_create
     ranks = _make_ranks(ctx, W, H, 3, 9, 2, 2, fb_reach=8)
     plain = _make_ranks(ctx, W, H, 3, 9, 2, 2, fb_reach=None)

@@ -1,5 +1,5 @@
 """Host orchestration shared by the entry points: the frame stream's plain push on the whole-frame level loop, and the
-native row-strip runner over its NCCL transport.
+native row-strip runner across processes.
 
 - A push without a total flow composes the cumulative flow at level 0 (at least 3 levels, even sizes, a per-pixel warp
   mode), like every other whole-frame entry point.  Its flow must equal a push with the total, bit for bit, and the
@@ -7,8 +7,8 @@ native row-strip runner over its NCCL transport.
 - A plain push launches grayscale, the optional bilateral filter (range table + filter), the pyramid and one kernel per
   level, with or without the total.
 - With profiling on, a push records one pyramid record and, from the second frame on, one record per level.
-- The native strip runner over NCCL send/recv (scripts/run_strips.py --native --transport nccl under torchrun) equals
-  the whole frame bit for bit on 2 and 3 processes.
+- The native strip runner over peer memory (scripts/run_strips.py --native under torchrun, CUDA IPC between the
+  processes) equals the whole frame bit for bit on 2 and 3 processes.
 """
 from __future__ import annotations
 
@@ -95,9 +95,10 @@ def test_stream_push_profile_records(ctx, oracle, levels):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("nproc", [2, 3])
-def test_native_strips_over_nccl(nproc):
-    """One process per GPU, halo rows by NCCL send/recv between the ranks' buffers (csrc/strips.cu), three levels of a
-    1080p pair; every rank's own rows of every level equal the whole frame.  Skipped with fewer GPUs than processes."""
+def test_native_strips_over_peer_memory(nproc):
+    """One process per GPU, halo rows stored by the sender's kernels into the receiver's memory over CUDA IPC
+    (csrc/strips.cu), three levels of a 1080p pair; every rank's own rows of every level equal the whole frame.  Skipped
+    with fewer GPUs than processes."""
     import torch
 
     if torch.cuda.device_count() < nproc:
@@ -106,10 +107,10 @@ def test_native_strips_over_nccl(nproc):
         sk.bind(("127.0.0.1", 0))
         port = sk.getsockname()[1]
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(nproc), "--master-addr", "127.0.0.1",
-           "--master-port", str(port), os.path.join(ROOT, "scripts", "run_strips.py"), "--native", "--transport", "nccl", "--check",
+           "--master-port", str(port), os.path.join(ROOT, "scripts", "run_strips.py"), "--native", "--check",
            "--w", "1920", "--h", "1080", "--levels", "3", "--reps", "4"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     rec = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
-    assert rec["n_gpus"] == nproc and rec["native"] is True and rec["transport"] == "nccl"
+    assert rec["n_gpus"] == nproc and rec["native"] is True and rec["transport"] == "peer"
     assert rec["bit_identical_to_whole_frame"] is True
