@@ -9,7 +9,8 @@ the C ABI in include/ofb200.h -- there is no CPU path here.
 The device-resident entry points (`flow_pairs_device`, `flow_pairs_fb_device`, `fb_check_device`, `lk_level_device`,
 `pyr_down_device`) take
 torch CUDA tensors only as owners of device memory; torch does none of the arithmetic.  The forward-backward check also
-runs on host batches (`flow_pairs_fb_host`) and on the frame stream (`FrameStream.push_fb`).
+runs on host batches (`flow_pairs_fb_host`) and on the frame stream (`FrameStream.push_fb`).  `track_points_device`
+follows a list of sub-pixel points through the pyramids (the KLT tracker).
 """
 from __future__ import annotations
 
@@ -139,11 +140,13 @@ class Context:
         L.check(self._lib.ofb_ctx_reserve_pairs_fb(self._h, C.byref(p)))
 
     def profile_enable(self, on: bool = True) -> None:
-        """CUDA-event timing around each fused-LK launch (tag = level), the pyramid build and the forward-backward check."""
+        """CUDA-event timing around each fused-LK launch (tag = level), the pyramid build, the forward-backward check and
+        the point tracker's kernel."""
         L.check(self._lib.ofb_ctx_profile_enable(self._h, 1 if on else 0))
 
     def profile_read(self, tag: int) -> tuple[float, int]:
-        """(summed milliseconds, number of records) for a tag: a pyramid level, PROFILE_PYRAMID or PROFILE_FB_CHECK."""
+        """(summed milliseconds, number of records) for a tag: a pyramid level, PROFILE_PYRAMID, PROFILE_FB_CHECK or
+        PROFILE_TRACK."""
         ms, n = C.c_double(), C.c_ulonglong()
         L.check(self._lib.ofb_ctx_profile_read(self._h, int(tag), C.byref(ms), C.byref(n)))
         return ms.value, n.value
@@ -408,6 +411,33 @@ class Context:
                                                    status.data_ptr(), err2.data_ptr() if err2 is not None else None,
                                                    C.c_void_p(stream)))
         return fwd, bwd, status, err2
+
+    def track_points_device(self, prev, next, w: int, levels: int, win: int, points, flow_scale: float = 1.0, iters: int = 30,
+                            eps: float = 0.01, min_eig: float = 0.0, stream: int = 0):
+        """Sparse pyramidal Lucas-Kanade (the KLT tracker): follow `points`, a float32 (n, m, 2) CUDA tensor of (x, y)
+        level-0 positions (m points per pair), from prev to next through `levels` pyramid levels with up to `iters`
+        Gauss-Newton iterations per level, stopping a level early once both components of an update are below `eps` px
+        (the defaults are OpenCV's).  prev/next as in flow_pairs_device.  Returns (flow (n, m, 2) float32 in flow units --
+        s * flow px with s = flow_scale --, status (n, m) uint8 PT_* codes).  min_eig > 0 marks points whose window's
+        smaller structure-tensor eigenvalue, divided by 2 win^2, is below it PT_LOW_TEXTURE (rule: include/ofb200.h)."""
+        import torch
+
+        if prev.dtype != torch.uint8 or prev.dim() != 3 or not prev.is_contiguous() or prev.shape != next.shape:
+            raise ValueError("prev/next must be contiguous uint8 (n, h, pitch) CUDA tensors of equal shape")
+        n, h, pitch = prev.shape
+        if not (prev.is_cuda and next.device == prev.device):
+            raise ValueError("prev/next must be CUDA tensors on one device")
+        if points.dtype != torch.float32 or points.dim() != 3 or points.shape[0] != n or points.shape[2] != 2 or \
+                not points.is_contiguous() or points.device != prev.device:
+            raise ValueError("points must be a contiguous float32 (n, m, 2) CUDA tensor on prev's device, one row per pair")
+        m = points.shape[1]
+        flow = torch.empty((n, m, 2), dtype=torch.float32, device=prev.device)
+        status = torch.empty((n, m), dtype=torch.uint8, device=prev.device)
+        p = OfbParams(w, h, levels, win, WARP_BILINEAR, flow_scale, n)
+        L.check(self._lib.ofb_track_points_device(self._h, C.byref(p), prev.data_ptr(), next.data_ptr(), pitch, pitch * h,
+                                                  points.data_ptr(), m, int(iters), C.c_float(eps), C.c_float(min_eig),
+                                                  flow.data_ptr(), status.data_ptr(), C.c_void_p(stream)))
+        return flow, status
 
     def pyr_down_device(self, src, sw: int, dst=None, stream: int = 0):
         """src: torch.uint8 (n, sh, pitch) -> dst (n, sh>>1, pitch_d)."""

@@ -870,6 +870,76 @@ int ofb_ctx_reserve_pairs_fb(ofb_ctx *c, const ofb_params *p)
     return ws_reserve(c, fp.bytes);
 }
 
+int ofb_track_points_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d, size_t pitch_bytes,
+                            size_t image_stride_bytes, const float *points_d, int n_points, int iters, float eps, float min_eig,
+                            float *flow_d, uint8_t *status_d, void *stream)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_params(p);
+    if (rc) return rc;
+    if (p->warp_mode != OFB_WARP_BILINEAR) {
+        set_error("track_points: warp mode %d (points are sampled bilinearly: OFB_WARP_BILINEAR only)", p->warp_mode);
+        return OFB_ERR_INVALID;
+    }
+    // s256 = flow_scale * 256 must be finite too: rint(d * s256) of an infinite s256 has no integer value
+    if (!(std::isfinite(p->flow_scale * 256.0f) && p->flow_scale > 0.0f)) {
+        set_error("flow_scale %g must be > 0 with flow_scale * 256 finite", (double)p->flow_scale);
+        return OFB_ERR_INVALID;
+    }
+    if ((rc = check_device_frames(p, prev_d && next_d && points_d && flow_d && status_d, "NULL frame, point, flow or status pointer",
+                                  pitch_bytes, image_stride_bytes)))
+        return rc;
+    if ((reinterpret_cast<uintptr_t>(points_d) | reinterpret_cast<uintptr_t>(flow_d)) & 7) {
+        set_error("points and flow must be 8-byte aligned");
+        return OFB_ERR_INVALID;
+    }
+    if (n_points < 1 || n_points > (1 << 24)) {
+        set_error("n_points %d outside 1..%d", n_points, 1 << 24);
+        return OFB_ERR_INVALID;
+    }
+    if (iters < 1 || iters > 64) {
+        set_error("iters %d outside 1..64", iters);
+        return OFB_ERR_INVALID;
+    }
+    if (!(std::isfinite(eps) && eps >= 0.0f && std::isfinite(min_eig) && min_eig >= 0.0f)) {
+        set_error("eps %g / min_eig %g must be finite and >= 0", (double)eps, (double)min_eig);
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    Carver cv;
+    PairPlan pl;
+    plan_pairs(p, &pl, &cv);
+    rc = ws_reserve(c, pl.bytes);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = ws_acquire(c, st))) return rc;
+    PairLevels lv;
+    if ((rc = build_pyramids(c, p, pl, c->ws, prev_d, next_d, pitch_bytes, image_stride_bytes, &lv, st))) return rc;
+    TrackArgs a = {};
+    for (int k = 0; k < p->levels; k++) {
+        a.prev[k] = lv.prev[k];
+        a.next[k] = lv.next[k];
+        a.pitch[k] = lv.pitch[k];
+        a.istr[k] = lv.istr[k];
+    }
+    a.w = p->w;
+    a.h = p->h;
+    a.levels = p->levels;
+    a.n_pairs = p->n_pairs;
+    a.n_points = n_points;
+    a.points = points_d;
+    a.flow = flow_d;
+    a.status = status_d;
+    a.iters = iters;
+    a.eps = eps;
+    a.min_eig = min_eig;
+    a.flow_scale = p->flow_scale;
+    if ((rc = prof_begin(c, OFB_PROFILE_TRACK, st))) return rc;
+    if ((rc = launch_track_points(a, p->win, st, &c->launches))) return rc;
+    if ((rc = prof_end(c, st))) return rc;
+    return ws_release(c, st);
+}
+
 int ofb_pyr_down_device(ofb_ctx *c, const uint8_t *src_d, size_t src_pitch, size_t src_image_stride, int sw, int sh,
                         uint8_t *dst_d, size_t dst_pitch, size_t dst_image_stride, int n_images, void *stream)
 {

@@ -171,6 +171,20 @@ int launch_fb_check_strip(const float *fwd, const float *bwd_rows, int w, int h,
                           unsigned long long *launches);
 int preload_fb_check_strip();
 
+// ---- sparse pyramidal LK, points tracked through the pyramid (track.cu) -------------------------------
+struct TrackArgs {
+    const uint8_t *prev[OFB_MAX_LEVELS], *next[OFB_MAX_LEVELS]; // level k of pair 0; pair i at + i * istr[k]
+    size_t pitch[OFB_MAX_LEVELS], istr[OFB_MAX_LEVELS];
+    int w, h, levels;          // level 0 size; level k is (w >> k) x (h >> k)
+    int n_pairs, n_points;     // points per pair
+    const float *points;       // float2 (x, y) in level-0 pixels, n_pairs * n_points
+    float *flow;               // float2, n_pairs * n_points
+    uint8_t *status;           // OFB_PT_*, n_pairs * n_points
+    int iters;
+    float eps, min_eig, flow_scale;
+};
+int launch_track_points(const TrackArgs &a, int win, cudaStream_t stream, unsigned long long *launches);
+
 int launch_grayscale(const uint8_t *src_c3, int w, int h, uint8_t *dst_c3, uint8_t *dst_planar, size_t dst_pitch,
                      cudaStream_t stream, unsigned long long *launches);
 int launch_bilateral(const uint8_t *src, const uint8_t *gray, size_t pitch, int channels, int w, int h, int ww, int wh,

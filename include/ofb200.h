@@ -417,6 +417,53 @@ int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, f
                                 float *const *flow_levels_h, float *fwd_total_h, float *bwd_total_h, uint8_t *status_h,
                                 float *err2_h, int *has_flow);
 
+/* ---- sparse pyramidal Lucas-Kanade: a list of points tracked through the pyramid; the reference has no counterpart ----
+ * The KLT tracker (OpenCV's calcOpticalFlowPyrLK): each point is followed coarse to fine with several Gauss-Newton
+ * iterations per level, on the pyramids of ofb_flow_pairs_device and with the dense path's derivative masks, bilinear rule
+ * and solve.  Point p = (x, y) of pair b is in level-0 pixels; its flow d is in flow units (displacement s*d px,
+ * s = p->flow_scale, as for the dense total flow).  Per point, in this order:
+ *   x or y not finite, or outside [0, w-1] x [0, h-1]                -> OFB_PT_OUTSIDE, flow NaN, not tracked
+ *   d = 0; for k = L-1 .. 0 (level k is (w>>k) x (h>>k)):
+ *     PX = rint(x * (256 >> k)), PY = rint(y * (256 >> k))  (the float product is exact; rint rounds half to even)
+ *     fields (exact integers, 0 outside the level): Ix = Dx (*) prev_k, Iy = Dy (*) prev_k, Sp = Dt (*) prev_k,
+ *       Sn = Dt (*) next_k -- the reference's masks as correlations with zero padding (OptFlowGpu.cu:1040-1090)
+ *     F@(X, Y), X, Y in 1/256 px: x0 = X >> 8, wx = X & 255 (arithmetic shift), likewise y0, wy; taps F00 = F(x0, y0),
+ *       F01 = F(x0+1, y0), F10 = F(x0, y0+1), F11 = F(x0+1, y0+1);
+ *       F@ = ((256-wy)*((256-wx)*F00 + wx*F01) + wy*((256-wx)*F10 + wx*F11) + 32768) >> 16   (the bilinear warp's rule)
+ *     over the win x win offsets o = (ox, oy), |ox|, |oy| <= win/2: gx = Ix@(P + 256 o), gy = Iy@(P + 256 o),
+ *       sp = Sp@(P + 256 o); a = sum gx*gx, dd = sum gy*gy, b = sum gx*gy (exact in int32: |gx|, |gy| <= 1020)
+ *     min_eig > 0: the smaller eigenvalue over 2 win^2, lam = ((a + dd) - sqrt(disc)) / (2 win^2), against min_eig,
+ *       undivided and squared (no square root, no division): in double, every operation rounded on its own, no fma,
+ *       t = a - dd, disc = t*t + 4*(b*b), T = (a + dd) - min_eig * (2 win^2) (the product is exact);
+ *       T < 0 or T*T < disc                                                                   -> OFB_PT_LOW_TEXTURE, stop
+ *     iterations i = 1 .. iters:
+ *       !(|s*d.u| < 32768 && |s*d.v| < 32768) (float products)                                  -> OFB_PT_OUTSIDE, stop
+ *       U = rint(d.u * s256), V = rint(d.v * s256), s256 = s * 256 (float; half to even)
+ *       It(o) = Sn@(P + (U, V) + 256 o) - sp(o); tx = sum gx*It, ty = sum gy*It (exact in int32: |It| <= 3825, win <= 19)
+ *       delta = the EXACT solve of (a, dd, b, tx, ty) (OFB_SOLVE_EXACT's operation order; the context's solve mode does
+ *         not apply); d += delta (float adds)
+ *       delta not finite (det == 0, Q3)                                                       -> OFB_PT_NONFINITE, stop
+ *       eps > 0 and |s*delta.u| < eps and |s*delta.v| < eps (float products): the level is done
+ *     d *= 2 unless k == 0
+ *   A point that stopped at level k reports 2^k * d.  A point that ran through level 0 is OFB_PT_TRACKED, or OFB_PT_OUTSIDE
+ *   with its flow kept when its final d fails the 32768 px test or its target (PX + U, PY + V) at level 0 lies outside
+ *   [0, (w-1)*256] x [0, (h-1)*256].
+ * With levels = 1, iters = 1, integer points and min_eig = 0 every sample is the field value itself and the solve is the
+ * dense path's: the flow of a point is that of ofb_flow_pairs_device's coarsest level at that pixel, bit for bit.
+ *   points_d: float2 (x, y), n_points per pair, pairs back to back (8-byte aligned); flow_d: the same shape (8-byte
+ *   aligned); status_d: one byte per point.  p->warp_mode must be OFB_WARP_BILINEAR, p->flow_scale > 0 with s256 finite;
+ *   1 <= n_points <= 2^24, 1 <= iters <= 64, eps and min_eig finite and >= 0; frames as in ofb_flow_pairs_device (at most
+ *   65535 pairs).  Bad arguments are refused before anything is enqueued.  The pyramids live in the context workspace:
+ *   ofb_ctx_reserve_pairs with the same parameters sizes it (CUDA graph capture).  With profiling on, the kernel gets an
+ *   OFB_PROFILE_TRACK record and the pyramid build its OFB_PROFILE_PYRAMID record. */
+#define OFB_PT_TRACKED 0
+#define OFB_PT_NONFINITE 1
+#define OFB_PT_LOW_TEXTURE 2
+#define OFB_PT_OUTSIDE 3
+int ofb_track_points_device(ofb_ctx *ctx, const ofb_params *p, const uint8_t *prev_d, const uint8_t *next_d,
+                            size_t pitch_bytes, size_t image_stride_bytes, const float *points_d, int n_points,
+                            int iters, float eps, float min_eig, float *flow_d, uint8_t *status_d, void *stream);
+
 /* Pinned host memory helpers for callers without a CUDA runtime of their own. */
 int ofb_host_alloc(void **ptr, size_t bytes);
 int ofb_host_free(void *ptr);
@@ -427,10 +474,12 @@ int ofb_ctx_launch_count(const ofb_ctx *ctx, unsigned long long *count);
 /* In-situ kernel timing for the roofline report.  While enabled, ofb_flow_pairs_device/_host put a
  * CUDA-event pair (on the stream the work is launched on) around every fused-LK launch, tagged with
  * its pyramid level, and around the pyramid build, tagged OFB_PROFILE_PYRAMID; the forward-backward entry points
- * also around the check kernel, tagged OFB_PROFILE_FB_CHECK.  _enable(on) also
+ * also around the check kernel, tagged OFB_PROFILE_FB_CHECK, and ofb_track_points_device around its kernel, tagged
+ * OFB_PROFILE_TRACK.  _enable(on) also
  * discards earlier records.  _read waits for the tagged events and returns their summed duration. */
 #define OFB_PROFILE_PYRAMID 100
 #define OFB_PROFILE_FB_CHECK 101
+#define OFB_PROFILE_TRACK 102
 int ofb_ctx_profile_enable(ofb_ctx *ctx, int on);
 int ofb_ctx_profile_read(ofb_ctx *ctx, int tag, double *ms_sum, unsigned long long *n_records);
 
