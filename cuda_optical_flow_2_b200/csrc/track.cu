@@ -78,7 +78,7 @@ __global__ void __launch_bounds__(TRK_WARPS * 32, 4) track_points_kernel(const T
         return;
     }
     const float fs = a.flow_scale, s256 = __fmul_rn(a.flow_scale, 256.0f);
-    const double win2 = (double)(2 * WIN * WIN);
+    const double win2 = (double)(WIN * WIN);
     float2 od = make_float2(0.0f, 0.0f); // the flow reported: od at level ok, status ost
     int ok = 0, ost = OFB_PT_TRACKED;
     float2 d = make_float2(0.0f, 0.0f);
@@ -133,14 +133,14 @@ __global__ void __launch_bounds__(TRK_WARPS * 32, 4) track_points_kernel(const T
         sxx = __reduce_add_sync(0xffffffffu, sxx);
         syy = __reduce_add_sync(0xffffffffu, syy);
         sxy = __reduce_add_sync(0xffffffffu, sxy);
-        // lam < min_eig, lam = ((A + D) - sqrt(disc)) / (2 WIN^2), as (A + D) - M < sqrt(disc) with M = 2 WIN^2 min_eig
-        // (exact in double), squared: no square root and no division, whose slow paths are subroutine calls that make
-        // ptxas spill around them
+        // lam < min_eig, lam = l1 / WIN^2 with l1 the smaller eigenvalue of [[A, B], [B, D]], as l1 < mu, mu = WIN^2 min_eig
+        // (exact in double): mu > S/2, or the characteristic polynomial at mu is negative, det < mu (S - mu), S = A + D,
+        // det = A D - B^2 exact in int64 (so det == 0, l1 == 0, is below every mu > 0).  No square root and no division,
+        // whose slow paths are subroutine calls that make ptxas spill around them
         if (a.min_eig > 0.0f) {
-            const double A = (double)sxx, D = (double)syy, B = (double)sxy, t = __dsub_rn(A, D);
-            const double disc = __dadd_rn(__dmul_rn(t, t), __dmul_rn(4.0, __dmul_rn(B, B)));
-            const double T = __dsub_rn(__dadd_rn(A, D), __dmul_rn((double)a.min_eig, win2));
-            if (T < 0.0 || __dmul_rn(T, T) < disc) {
+            const double S = __dadd_rn((double)sxx, (double)syy), mu = __dmul_rn((double)a.min_eig, win2);
+            const double det = __ll2double_rn((long long)sxx * syy - (long long)sxy * sxy);
+            if (mu > __dmul_rn(0.5, S) || det < __dmul_rn(mu, __dsub_rn(S, mu))) {
                 od = d, ok = k, ost = OFB_PT_LOW_TEXTURE;
                 break;
             }

@@ -432,10 +432,13 @@ int ofb_stream_push_bgr_host_fb(ofb_stream *s, const unsigned char *frame_bgr, f
  *       F@ = ((256-wy)*((256-wx)*F00 + wx*F01) + wy*((256-wx)*F10 + wx*F11) + 32768) >> 16   (the bilinear warp's rule)
  *     over the win x win offsets o = (ox, oy), |ox|, |oy| <= win/2: gx = Ix@(P + 256 o), gy = Iy@(P + 256 o),
  *       sp = Sp@(P + 256 o); a = sum gx*gx, dd = sum gy*gy, b = sum gx*gy (exact in int32: |gx|, |gy| <= 1020)
- *     min_eig > 0: the smaller eigenvalue over 2 win^2, lam = ((a + dd) - sqrt(disc)) / (2 win^2), against min_eig,
- *       undivided and squared (no square root, no division): in double, every operation rounded on its own, no fma,
- *       t = a - dd, disc = t*t + 4*(b*b), T = (a + dd) - min_eig * (2 win^2) (the product is exact);
- *       T < 0 or T*T < disc                                                                   -> OFB_PT_LOW_TEXTURE, stop
+ *     min_eig > 0: lam < min_eig, lam = l1 / win^2 with l1 the smaller eigenvalue of [[a, b], [b, dd]], decided on the
+ *       characteristic polynomial at mu = min_eig * win^2 (no square root, no division): in double, every operation
+ *       rounded on its own, no fma, S = a + dd, mu = min_eig * (win^2) (both exact), det = a*dd - b*b exact in int64,
+ *       then rounded to double; a window with det == 0 (lam = 0) is below every min_eig > 0.  Elsewhere the decision
+ *       is that of the exact lam < min_eig except for min_eig within a relative 1e-6 of lam (the bound is reached
+ *       only on near-isotropic windows, where the polynomial has a near-double root);
+ *       mu > 0.5*S or det < mu * (S - mu)                                                     -> OFB_PT_LOW_TEXTURE, stop
  *     iterations i = 1 .. iters:
  *       !(|s*d.u| < 32768 && |s*d.v| < 32768) (float products)                                  -> OFB_PT_OUTSIDE, stop
  *       U = rint(d.u * s256), V = rint(d.v * s256), s256 = s * 256 (float; half to even)

@@ -87,10 +87,9 @@ static uint8_t track_one(const Level *prev, const Level *next, int levels, int w
                 b += gx[i] * gy[i];
             }
         if (min_eig > 0.0f) {
-            const double A = a, D = dd, B = b, t = A - D;
-            const double disc = t * t + 4.0 * (B * B);
-            const double T = (A + D) - (double)min_eig * (double)(2 * win * win);
-            if (T < 0.0 || T * T < disc) {
+            const double S = (double)a + (double)dd, mu = (double)min_eig * (double)(win * win);
+            const double det = (double)((int64_t)a * dd - (int64_t)b * b);
+            if (mu > 0.5 * S || det < mu * (S - mu)) {
                 out[0] = du * (float)(1 << k);
                 out[1] = dv * (float)(1 << k);
                 return PT_LOW_TEXTURE;
