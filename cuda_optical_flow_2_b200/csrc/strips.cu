@@ -5,8 +5,7 @@
 // cumulative-flow halo), but here the whole pair -- own-row upload, per-level halo exchange, pyramid, fused level
 // kernels -- is enqueued on one CUDA stream from C++ with no host synchronisation.  Only level-0 image rows are
 // exchanged (the coarser levels' halo rows are rebuilt locally), so a pair of L levels costs L exchanges: one for the
-// images, L-1 for the cumulative flow.  The Python StripRunner runs the 2L-1-exchange form of the schedule through torch
-// and is bound by ~100 us of host work per exchange.
+// images, L-1 for the cumulative flow.
 //
 // The halo rows move through peer memory: every rank keeps the buffers its neighbours write into -- the level-0 image
 // rows and the coarser cumulative-flow rows -- in ONE device allocation (the arena) whose CUDA IPC handle the
@@ -40,7 +39,8 @@ struct LevelStrip {
 struct StripPlan {
     int W, H, levels, win, world, reach, r, img_halo;
     int fb_reach = -1; // >= 0: handle of ofb_strips_create_fb (checked pairs); level-0 backward rows beyond the own rows held
-    std::vector<int> coarse_bounds;
+    // first row of `rank`'s strip on the coarsest level; coarse_bound(world) is that level's height
+    int coarse_bound(int rank) const { return (int)(((long long)rank * (H >> (levels - 1))) / world); }
     // rows [lo, hi) of the level-0 backward total flow that `rank`'s check holds
     void fb_rows(int rank, int *lo, int *hi) const
     {
@@ -54,8 +54,8 @@ struct StripPlan {
         LevelStrip s;
         s.w = W >> k;
         s.h = H >> k;
-        s.y0 = coarse_bounds[rank] << sh;
-        s.y1 = rank == world - 1 ? s.h : coarse_bounds[rank + 1] << sh;
+        s.y0 = coarse_bound(rank) << sh;
+        s.y1 = rank == world - 1 ? s.h : coarse_bound(rank + 1) << sh;
         s.by0 = std::max(0, s.y0 - img_halo);
         s.by1 = std::min(s.h, s.y1 + img_halo);
         if (k < levels - 1) {
@@ -398,6 +398,22 @@ void add_unique(std::vector<int> &v, int x)
 {
     if (std::find(v.begin(), v.end(), x) == v.end()) v.push_back(x);
 }
+// The schedule of a w x h pair of `levels` levels cut into `world` strips (arguments checked by the caller); refuses a
+// coarsest level with fewer rows than strips.
+int make_plan(int w, int h, int levels, int win, int world, int reach, int fb_reach, StripPlan *pl)
+{
+    const int hc = h >> (levels - 1);
+    if (hc < world || (w >> (levels - 1)) < 1) {
+        set_error("coarsest level has %d rows, cannot cut it into %d strips", hc, world);
+        return OFB_ERR_INVALID;
+    }
+    pl->W = w, pl->H = h, pl->levels = levels, pl->win = win, pl->world = world, pl->reach = reach;
+    pl->fb_reach = fb_reach;
+    pl->r = win / 2;
+    // image halo: 3x3 stencil + window radius + one row of even-row alignment + warp reach + bilinear tap
+    pl->img_halo = pl->r + 2 + reach + 2;
+    return OFB_OK;
+}
 } // namespace
 
 extern "C" {
@@ -413,17 +429,8 @@ int ofb_strips_plan_query(int w, int h, int levels, int win, int world, int rank
         set_error("strips_plan_query: bad arguments");
         return OFB_ERR_INVALID;
     }
-    const int hc = h >> (levels - 1);
-    if (hc < world || (w >> (levels - 1)) < 1) {
-        set_error("coarsest level has %d rows, cannot cut it into %d strips", hc, world);
-        return OFB_ERR_INVALID;
-    }
     StripPlan pl;
-    pl.W = w, pl.H = h, pl.levels = levels, pl.win = win, pl.world = world, pl.reach = reach;
-    pl.r = win / 2;
-    pl.img_halo = pl.r + 2 + reach + 2;
-    for (int rk = 0; rk < world; rk++) pl.coarse_bounds.push_back((int)(((long long)rk * hc) / world));
-    pl.coarse_bounds.push_back(hc);
+    if (int rc = make_plan(w, h, levels, win, world, reach, -1, &pl)) return rc;
     const LevelStrip s = pl.strips(rank)[level];
     const int v[8] = {s.y0, s.y1, s.by0, s.by1, s.cy0, s.cy1, s.eb0, s.eb1};
     memcpy(out8, v, sizeof v);
@@ -445,11 +452,8 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
         set_error("OFB_WARP_AS_WRITTEN needs pixel (0,0) of every coarser level: not available on strips");
         return OFB_ERR_UNSUPPORTED;
     }
-    const int hc = h >> (levels - 1);
-    if (hc < world || (w >> (levels - 1)) < 1) {
-        set_error("coarsest level has %d rows, cannot cut it into %d strips", hc, world);
-        return OFB_ERR_INVALID;
-    }
+    StripPlan pl;
+    if (int rc = make_plan(w, h, levels, win, world, reach, fb_reach, &pl)) return rc;
     DeviceGuard guard(ctx_device(ctx));
     if (!guard.ok) return OFB_ERR_CUDA;
     ofb_strips *st = new (std::nothrow) ofb_strips;
@@ -462,14 +466,7 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
     st->rank = rank;
     st->warp_mode = warp_mode;
     st->flow_scale = flow_scale;
-    StripPlan &pl = st->plan;
-    pl.W = w, pl.H = h, pl.levels = levels, pl.win = win, pl.world = world, pl.reach = reach;
-    pl.fb_reach = fb_reach;
-    pl.r = win / 2;
-    // image halo: 3x3 stencil + window radius + one row of even-row alignment + warp reach + bilinear tap
-    pl.img_halo = pl.r + 2 + reach + 2;
-    for (int rk = 0; rk < world; rk++) pl.coarse_bounds.push_back((int)(((long long)rk * hc) / world));
-    pl.coarse_bounds.push_back(hc);
+    st->plan = pl;
     int rc = OFB_OK;
     st->s = pl.strips(rank);
     // what neighbours write into (level-0 image rows, coarser cumulative-flow rows, flags): one allocation, the arena

@@ -8,21 +8,22 @@ The reference is single-GPU (SURVEY.md 2.1: no streams, no NCCL, no threads); bo
 * row strips -- one very large pair is cut into horizontal strips.  Strips nest across pyramid
   levels (bounds are fixed on the coarsest level and doubled per finer level), every level needs
   its neighbours' image rows (stencil halo + warp reach) and the next-coarser level's cumulative
-  flow rows, exchanged with the rank above and below once per level: `dist.batch_isend_irecv`
-  (NCCL over NVLink on GPUs, gloo in the CPU tests).  The result is bit-identical to the 1-GPU
-  result as long as no warp sample reaches past the exchanged rows; the kernel raises a flag
-  otherwise and `StripRunner` turns it into an error instead of returning different numbers.
+  flow rows.  `NativeStrips` runs a whole pair from the library (csrc/strips.cu): the sender's
+  kernels store the halo rows straight into the receiver's memory over NVLink, one exchange per
+  pyramid level.  The result is bit-identical to the 1-GPU result as long as no warp sample
+  reaches past the rows held; the kernel raises a flag otherwise and `NativeStrips.check()` turns
+  it into an error instead of returning different numbers.
 
 torch is used for device memory, streams and the process group only; all arithmetic is in the
-C-ABI library.  The strip schedule itself (`StripPlan`) is plain Python and unit-tested on CPU.
+C-ABI library.  `StripPlan` restates the strip schedule in plain Python: it is unit-tested on CPU
+and is the reference the library's schedule is tested against.
 """
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Optional, Sequence, Tuple
+from typing import List, Optional, Tuple
 
-from ._lib import WARP_AS_WRITTEN, WARP_BILINEAR
-from .api import align_up
+from ._lib import WARP_BILINEAR
 
 
 # ------------------------------------------------------------------------------------------ frame batch
@@ -150,234 +151,10 @@ class StripPlan:
                 raise AssertionError(f"level {k}: strips do not cover the image")
 
 
-class Transport:
-    """Moves halo rows between ranks.  `exchange(sends, recvs)`: sends = [(peer, tensor)], recvs =
-    [(peer, tensor)] filled in place; both lists are ordered by peer on every rank."""
-
-    def exchange(self, sends, recvs) -> None:  # pragma: no cover - interface
-        raise NotImplementedError
-
-
-class DistTransport(Transport):
-    """torch.distributed point-to-point (NCCL on GPUs: NVLink/NVSwitch peer copies; gloo on CPU)."""
-
-    def __init__(self, group=None):
-        import torch.distributed as dist
-
-        self.dist, self.group = dist, group
-
-    def exchange(self, sends, recvs) -> None:
-        dist = self.dist
-        ops = [dist.P2POp(dist.irecv, t, peer, group=self.group) for peer, t in recvs]
-        ops += [dist.P2POp(dist.isend, t, peer, group=self.group) for peer, t in sends]
-        if ops:
-            for req in dist.batch_isend_irecv(ops):
-                req.wait()
-
-
-class GatherTransport(Transport):
-    """Halo exchange as ONE all-gather per exchange: every rank contributes two fixed-size slots (its message to
-    the rank below, its message to the rank above) and reads its neighbours' slots.  More bytes than point-to-point
-    (world x 2 slots, still a few MB over NVSwitch) but a single collective of constant shape per exchange, which
-    -- unlike grouped send/recv -- captures cleanly in a CUDA graph, so a whole pair (kernels + exchanges) replays
-    without host work.  Only adjacent ranks may talk (halo smaller than a strip).  Slot sizes are agreed on with an
-    all-reduce the first time each exchange of a step is seen; `begin_step()` restarts the numbering."""
-
-    def __init__(self, rank: int, world: int, device, group=None):
-        import torch
-        import torch.distributed as dist
-
-        self.torch, self.dist, self.group = torch, dist, group
-        self.rank, self.world, self.dev = rank, world, device
-        self._idx, self._bufs = 0, []
-
-    def begin_step(self) -> None:
-        self._idx = 0
-
-    def exchange(self, sends, recvs) -> None:
-        torch, dist = self.torch, self.dist
-        i = self._idx
-        self._idx += 1
-        if i >= len(self._bufs):  # first step only (never under graph capture): agree on the slot size
-            n = max([t.numel() * t.element_size() for _, t in list(sends) + list(recvs)] + [16])
-            tt = torch.tensor([n], dtype=torch.int64, device=self.dev)
-            dist.all_reduce(tt, op=dist.ReduceOp.MAX, group=self.group)
-            n = (int(tt.item()) + 15) // 16 * 16
-            self._bufs.append((torch.zeros((2, n), dtype=torch.uint8, device=self.dev),
-                               torch.zeros((self.world, 2, n), dtype=torch.uint8, device=self.dev)))
-        out, inn = self._bufs[i]
-        for peer, t in sends:
-            if abs(peer - self.rank) != 1:
-                raise ValueError("GatherTransport: only adjacent ranks exchange halos")
-            b = t.reshape(-1).view(torch.uint8)
-            out[0 if peer < self.rank else 1, : b.numel()].copy_(b)
-        dist.all_gather_into_tensor(inn.view(-1), out.view(-1), group=self.group)
-        for peer, t in recvs:
-            if abs(peer - self.rank) != 1:
-                raise ValueError("GatherTransport: only adjacent ranks exchange halos")
-            nb = t.numel() * t.element_size()
-            t.copy_(inn[peer, 1 if peer < self.rank else 0, :nb].view(t.dtype).view(t.shape))
-
-
-class StripRunner:
-    """One rank's share of a row-strip solve.  All tensors are torch tensors on this rank's device."""
-
-    def __init__(self, ctx, plan: StripPlan, rank: int, transport: Transport, device, warp_mode: int = WARP_BILINEAR,
-                 flow_scale: float = 1.0):
-        import torch
-
-        if warp_mode == WARP_AS_WRITTEN and plan.levels > 1:
-            raise ValueError("OFB_WARP_AS_WRITTEN needs pixel (0,0) of every coarser level: not available on strips")
-        self.torch, self.ctx, self.plan, self.rank, self.tp, self.dev = torch, ctx, plan, rank, transport, device
-        self.warp_mode, self.flow_scale = warp_mode, flow_scale
-        # CUDA stream handle the kernels are enqueued on (0 = the default stream).  `use_current_stream()`
-        # re-reads torch's current stream, which is what CUDA-graph capture of `step()` needs.
-        self.stream = 0
-        self.strips = [plan.level(k, rank) for k in range(plan.levels)]
-        self.pitch = [align_up(s.w, 64) for s in self.strips]
-        z = lambda rows, cols, dt: torch.zeros((rows, cols), dtype=dt, device=device)
-        self.prev = [z(s.buf_rows, p, torch.uint8) for s, p in zip(self.strips, self.pitch)]
-        self.next = [z(s.buf_rows, p, torch.uint8) for s, p in zip(self.strips, self.pitch)]
-        # flow / cumulative flow: rows of the image buffer (same origin by0), only own rows are written
-        self.flow = [torch.zeros((s.buf_rows, s.w, 2), dtype=torch.float32, device=device) for s in self.strips]
-        self.cum = [torch.zeros((s.buf_rows, s.w, 2), dtype=torch.float32, device=device) for s in self.strips]
-        # coarser cumulative flow as the level-k kernel wants it: rows [cy0, cy1) of level k+1
-        self.cum_in = [torch.zeros((max(s.cy1 - s.cy0, 1), s.w >> 1, 2), dtype=torch.float32, device=device)
-                       for s in self.strips]
-        self.overflow = torch.zeros(1, dtype=torch.int32, device=device)
-
-    def use_current_stream(self) -> None:
-        self.stream = self.torch.cuda.current_stream(self.dev).cuda_stream
-
-    def step(self, prev_rows, next_rows) -> None:
-        """One pair, everything asynchronous on the stream (no host synchronisation): capturable in a CUDA
-        graph together with its NCCL halo exchanges.  Call check_overflow() afterwards (it synchronises)."""
-        if hasattr(self.tp, "begin_step"):
-            self.tp.begin_step()
-        self.load_level0(prev_rows, next_rows)
-        self.build_pyramid()
-        self.solve(check=False)
-
-    # -- data in ---------------------------------------------------------------------------------
-    def load_level0(self, prev_rows, next_rows) -> None:
-        """prev_rows/next_rows: (own_rows, w) uint8 tensors with this rank's OWN rows of the two frames."""
-        s = self.strips[0]
-        a = s.y0 - s.by0
-        self.prev[0][a:a + s.own_rows, :s.w] = prev_rows
-        self.next[0][a:a + s.own_rows, :s.w] = next_rows
-
-    # -- exchanges -------------------------------------------------------------------------------
-    # Each exchange is described as (sends, recvs, finish): tensors to send per peer, buffers to
-    # receive into per peer, and a closure that files the received rows.  `_run` hands them to the
-    # transport; the single-process emulation matches sends to recvs itself.
-    def image_exchange(self, k: int):
-        plan, s, torch = self.plan, self.strips[k], self.torch
-        sends, recvs, stage = [], [], []
-        for peer, lo, hi, _ in plan.halo_messages(k, self.rank):
-            sends.append((peer, torch.stack([self.prev[k][lo - s.by0:hi - s.by0],
-                                             self.next[k][lo - s.by0:hi - s.by0]]).contiguous()))
-        for peer in range(plan.world):
-            if peer == self.rank:
-                continue
-            pl = plan.level(k, peer)
-            lo, hi = max(pl.y0, s.by0), min(pl.y1, s.by1)
-            if lo < hi:
-                buf = torch.empty((2, hi - lo, self.pitch[k]), dtype=torch.uint8, device=self.dev)
-                recvs.append((peer, buf))
-                stage.append((lo, hi, buf))
-
-        def finish():
-            for lo, hi, buf in stage:
-                self.prev[k][lo - s.by0:hi - s.by0] = buf[0]
-                self.next[k][lo - s.by0:hi - s.by0] = buf[1]
-
-        return sends, recvs, finish
-
-    def cum_exchange(self, k: int):
-        """Rows [cy0, cy1) of cum_{k+1} into cum_in[k]: own rows copied here, the rest from neighbours."""
-        plan, s, torch = self.plan, self.strips[k], self.torch
-        up = self.strips[k + 1]
-        src = self.cum[k + 1] if k + 1 < plan.levels - 1 else self.flow[k + 1]  # cum of the coarsest level is its flow
-        lo, hi = max(up.y0, s.cy0), min(up.y1, s.cy1)
-        if lo < hi:
-            self.cum_in[k][lo - s.cy0:hi - s.cy0] = src[lo - up.by0:hi - up.by0]
-        sends, recvs, stage = [], [], []
-        for peer, lo, hi, _ in plan.cum_messages(k, self.rank):
-            sends.append((peer, src[lo - up.by0:hi - up.by0].contiguous()))
-        for peer in range(plan.world):
-            if peer == self.rank:
-                continue
-            pu = plan.level(k + 1, peer)
-            lo, hi = max(pu.y0, s.cy0), min(pu.y1, s.cy1)
-            if lo < hi:
-                buf = torch.empty((hi - lo, up.w, 2), dtype=torch.float32, device=self.dev)
-                recvs.append((peer, buf))
-                stage.append((lo, hi, buf))
-
-        def finish():
-            for lo, hi, buf in stage:
-                self.cum_in[k][lo - s.cy0:hi - s.cy0] = buf
-
-        return sends, recvs, finish
-
-    def _run(self, ex) -> None:
-        sends, recvs, finish = ex
-        self.tp.exchange(sends, recvs)
-        finish()
-
-    # -- compute ---------------------------------------------------------------------------------
-    def build_pyramid(self) -> None:
-        """Level k+1 own rows from level k own rows +-1 (after the level-k halo exchange), for both frames."""
-        plan = self.plan
-        for k in range(plan.levels):
-            self._run(self.image_exchange(k))
-            if k + 1 < plan.levels:
-                self.pyr_down_own(k)
-
-    def pyr_down_own(self, k: int) -> None:
-        s, d = self.strips[k], self.strips[k + 1]
-        for buf in (self.prev, self.next):
-            self.ctx.pyr_down_strip_device(buf[k], s.w, s.by0, buf[k + 1][d.y0 - d.by0:d.y1 - d.by0], d.y0, d.y1,
-                                           stream=self.stream)
-
-    def lk_level_own(self, k: int) -> None:
-        plan, s = self.plan, self.strips[k]
-        want_cum = (0 < k < plan.levels - 1) or (k == 0 and plan.levels > 1)
-        self.ctx.lk_level_strip_device(self.prev[k], self.next[k], s.w, s.by0, s.h, s.y0 - s.by0, s.y1 - s.by0, plan.win,
-                                       self.warp_mode, self.flow_scale, self.cum_in[k] if k < plan.levels - 1 else None,
-                                       s.cy0, self.flow[k], cum_out=self.cum[k] if want_cum else None,
-                                       overflow_flag=self.overflow, stream=self.stream)
-
-    def check_overflow(self) -> None:
-        if int(self.overflow.item()) != 0:
-            raise RuntimeError(f"rank {self.rank}: a warp sample reached past the exchanged halo rows: raise "
-                               f"StripPlan.reach (currently {self.plan.reach} rows)")
-
-    def solve(self, check: bool = True) -> None:
-        """Coarse to fine: exchange cum_{k+1} halo rows, run the fused strip kernel on own rows."""
-        plan = self.plan
-        self.overflow.zero_()
-        for k in range(plan.levels - 1, -1, -1):
-            if k < plan.levels - 1:
-                self._run(self.cum_exchange(k))
-            self.lk_level_own(k)
-        if check:
-            self.check_overflow()
-
-    def own_flow(self, k: int):
-        s = self.strips[k]
-        return self.flow[k][s.y0 - s.by0:s.y1 - s.by0]
-
-    def own_total_flow(self):
-        s = self.strips[0]
-        src = self.cum[0] if self.plan.levels > 1 else self.flow[0]
-        return src[s.y0 - s.by0:s.y1 - s.by0]
-
-
 class NativeStrips:
-    """The native row-strip runner (csrc/strips.cu): the same schedule as StripRunner, but a whole pair is enqueued
-    from C++ on one stream.  The halo rows move through peer memory: the sender's kernels store them straight into the
-    receiver's memory over NVLink and raise epoch flags there.  transport "peer": ranks in separate processes, connected
+    """The row-strip runner (csrc/strips.cu): the schedule of StripPlan, a whole pair enqueued from C++ on one stream.
+    The halo rows move through peer memory: the sender's kernels store them straight into the receiver's memory over
+    NVLink and raise epoch flags there.  transport "peer": ranks in separate processes, connected
     over CUDA IPC (`torch.distributed` is used once, to hand round the IPC handles); "local": ranks living in this process
     (connect_local, tests).
 
@@ -577,53 +354,3 @@ def _device_view(torch, ptr: int, shape, device):
         __cuda_array_interface__ = {"shape": (n,), "typestr": "<f4", "data": (ptr, False), "version": 3}
 
     return torch.as_tensor(_Holder(), device=device).view(*shape)
-
-
-def run_strips_local(ctx, prev0, next0, levels: int, win: int, world: int, warp_mode: int = WARP_BILINEAR,
-                     flow_scale: float = 1.0, reach: int = 16):
-    """Emulate `world` ranks on ONE device: the same StripRunner code, with every halo exchange done
-    as local copies between the rank objects.  prev0/next0: (H, >=W) uint8 tensors holding the whole
-    frames.  Returns (plan, runners).  Used to check that strips + halos reproduce the whole-frame
-    result bit for bit without needing several GPUs."""
-    return _run_strips_local(ctx, prev0, next0, levels, win, world, warp_mode, flow_scale, reach, None)
-
-
-def run_strips_local_w(ctx, prev0, next0, w: int, levels: int, win: int, world: int, warp_mode: int = WARP_BILINEAR,
-                       flow_scale: float = 1.0, reach: int = 16):
-    """As run_strips_local for pitched frames: only the first w columns of each row are image."""
-    return _run_strips_local(ctx, prev0, next0, levels, win, world, warp_mode, flow_scale, reach, w)
-
-
-def _run_strips_local(ctx, prev0, next0, levels, win, world, warp_mode, flow_scale, reach, width: Optional[int]):
-    H = prev0.shape[0]
-    W = width if width is not None else prev0.shape[1]
-    plan = StripPlan(W, H, levels, win, world, reach)
-    plan.validate()
-    runners = [StripRunner(ctx, plan, rk, Transport(), prev0.device, warp_mode, flow_scale) for rk in range(world)]
-    for rn in runners:
-        s = rn.strips[0]
-        rn.load_level0(prev0[s.y0:s.y1, :W], next0[s.y0:s.y1, :W])
-
-    def lockstep(make):
-        posts = [(rn, make(rn)) for rn in runners]
-        outbox = {(rn.rank, dst): t for rn, (sends, _, _) in posts for dst, t in sends}
-        for rn, (_, recvs, finish) in posts:
-            for src, t in recvs:
-                t.copy_(outbox[(src, rn.rank)])
-            finish()
-
-    for k in range(levels):
-        lockstep(lambda rn: rn.image_exchange(k))
-        if k + 1 < levels:
-            for rn in runners:
-                rn.pyr_down_own(k)
-    for rn in runners:
-        rn.overflow.zero_()
-    for k in range(levels - 1, -1, -1):
-        if k < levels - 1:
-            lockstep(lambda rn: rn.cum_exchange(k))
-        for rn in runners:
-            rn.lk_level_own(k)
-    for rn in runners:
-        rn.check_overflow()
-    return plan, runners

@@ -1,13 +1,12 @@
-"""Multi-GPU host logic.  CPU: strip schedule invariants and a world_size-2 gloo run of the halo
-exchange.  GPU: N emulated ranks on one device must reproduce the whole-frame flow bit for bit."""
+"""Multi-GPU host logic.  CPU: batch sharding, the strip schedule's invariants, and the native runner's schedule against
+StripPlan.  GPU: the native strip runner, N ranks on one device (or one per GPU), must reproduce the whole-frame flow bit
+for bit, and must report a warp that reaches past the rows it holds."""
 import os
-import socket
-import sys
 
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+BIL, NEAR = 2, 1  # OFB_WARP_BILINEAR, _NEAREST
 
 
 def test_shard_range_partitions_the_batch():
@@ -53,147 +52,13 @@ def test_strip_plan_invariants(W, H, levels, win, world):
             assert (got[s.by0:s.by1] == 1).all() and got.sum() == s.buf_rows
 
 
-def _free_port():
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        return s.getsockname()[1]
-
-
-def _gloo_worker(rank, world, port, q, transport="p2p"):
-    """Each rank fills its own rows with a global-row pattern; after the exchange its buffer (own rows
-    + halo) must equal the pattern of the whole image, for images and for the coarser flow."""
-    sys.path.insert(0, ROOT)
-    import torch
-    import torch.distributed as dist
-
-    from cuda_optical_flow_2_b200.dist import DistTransport, GatherTransport, StripPlan, StripRunner
-
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        W, H, levels, win = 96, 160, 3, 5
-        plan = StripPlan(W, H, levels, win, world, reach=4)
-        tp = GatherTransport(rank, world, torch.device("cpu")) if transport == "gather" else DistTransport()
-        rn = StripRunner(None, plan, rank, tp, torch.device("cpu"))
-        ok = True
-        for k in range(levels):
-            s = rn.strips[k]
-            rows = torch.arange(s.by0, s.by1)
-            own = (rows >= s.y0) & (rows < s.y1)
-            pat_p = ((rows[:, None] * 7 + torch.arange(rn.pitch[k])[None, :] * 3 + k) % 251).to(torch.uint8)
-            pat_n = ((rows[:, None] * 5 + torch.arange(rn.pitch[k])[None, :] * 11 + k) % 241).to(torch.uint8)
-            rn.prev[k][own] = pat_p[own]
-            rn.next[k][own] = pat_n[own]
-            rn._run(rn.image_exchange(k))
-            ok &= bool(torch.equal(rn.prev[k], pat_p) and torch.equal(rn.next[k], pat_n))
-        for k in range(levels - 2, -1, -1):
-            s, up = rn.strips[k], rn.strips[k + 1]
-            src = rn.cum[k + 1] if k + 1 < levels - 1 else rn.flow[k + 1]
-            rows = torch.arange(up.by0, up.by1, dtype=torch.float32)
-            own = (rows >= up.y0) & (rows < up.y1)
-            pat = rows[:, None, None] * 1000 + torch.arange(up.w, dtype=torch.float32)[None, :, None] + \
-                torch.tensor([0.25, 0.5])[None, None, :]
-            src[own] = pat[own]
-            rn._run(rn.cum_exchange(k))
-            crow = torch.arange(s.cy0, s.cy1, dtype=torch.float32)
-            exp = crow[:, None, None] * 1000 + torch.arange(up.w, dtype=torch.float32)[None, :, None] + \
-                torch.tensor([0.25, 0.5])[None, None, :]
-            ok &= bool(torch.equal(rn.cum_in[k][: s.cy1 - s.cy0], exp))
-        q.put((rank, ok))
-    finally:
-        dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("world,transport", [(2, "p2p"), (3, "p2p"), (2, "gather"), (3, "gather")])
-def test_halo_exchange_over_gloo(world, transport):
-    """Grouped send/recv, and the one-all-gather-per-exchange transport that CUDA graphs can capture."""
-    import torch.multiprocessing as mp
-
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_gloo_worker, args=(r, world, port, q, transport)) for r in range(world)]
-    for p in procs:
-        p.start()
-    results = [q.get(timeout=120) for _ in range(world)]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    assert sorted(results) == [(r, True) for r in range(world)]
-
-
 # ------------------------------------------------------------------------------------------------- GPU
-@pytest.mark.gpu
-@pytest.mark.parametrize("W,H,levels,win,world,mode", [(640, 480, 3, 9, 2, 2), (640, 480, 3, 9, 4, 2), (322, 406, 2, 5, 3, 2),
-                                                       (640, 480, 3, 9, 3, 1), (1920, 1080, 3, 9, 8, 2),
-                                                       (512, 384, 1, 9, 4, 2)])
-def test_strips_reproduce_whole_frame_bit_for_bit(ctx, oracle, W, H, levels, win, world, mode):
-    import torch
-
-    from cuda_optical_flow_2_b200 import planar_to_device
-    from cuda_optical_flow_2_b200.dist import run_strips_local_w
-
-    prev = oracle.make_frame(W, H, 0, 0, 8, 77)
-    nxt = oracle.make_frame(W, H, 2.0, -1.5, 8, 77)
-    dp, dn = planar_to_device(prev[None]), planar_to_device(nxt[None])
-    total = torch.empty((1, H, W, 2), dtype=torch.float32, device="cuda")
-    whole = ctx.flow_pairs_device(dp, dn, W, levels, win, warp_mode=mode, total_flow=total)
-    plan, runners = run_strips_local_w(ctx, dp[0], dn[0], W, levels, win, world, warp_mode=mode, reach=16)
-    torch.cuda.synchronize()
-    for k in range(levels):
-        got = torch.cat([rn.own_flow(k) for rn in runners]).cpu().numpy()
-        ref = whole[k][0].cpu().numpy()
-        assert got.shape == ref.shape
-        assert np.array_equal(np.isnan(got), np.isnan(ref)), f"level {k}"
-        m = ~np.isnan(ref)
-        assert np.array_equal(got[m], ref[m]), f"level {k}: strips differ from the whole-frame result"
-    got = torch.cat([rn.own_total_flow() for rn in runners]).cpu().numpy()
-    ref = total[0].cpu().numpy()
-    m = ~np.isnan(ref)
-    assert np.array_equal(got[m], ref[m]), "total flow"
-
-
-@pytest.mark.gpu
-def test_strip_reach_overflow_is_reported(ctx, oracle):
-    """A warp that reaches past the exchanged rows must raise, not silently change the numbers."""
-    from cuda_optical_flow_2_b200 import planar_to_device
-    from cuda_optical_flow_2_b200.dist import run_strips_local_w
-
-    W, H = 320, 480
-    prev = oracle.make_frame(W, H, 0, 0, 8, 5)
-    nxt = oracle.make_frame(W, H, 0.0, 14.0, 8, 5)  # large vertical motion
-    with pytest.raises(RuntimeError, match="reach"):
-        run_strips_local_w(ctx, planar_to_device(prev[None])[0], planar_to_device(nxt[None])[0], W, 3, 9, 4, reach=1)
-
-
-@pytest.mark.gpu
-def test_config4_8k_strips_equal_whole_frame(ctx, oracle):
-    """configs[4]: 7680x4320 pair cut into 8 row strips (emulated ranks on one GPU)."""
-    import torch
-
-    from cuda_optical_flow_2_b200 import planar_to_device
-    from cuda_optical_flow_2_b200.dist import run_strips_local_w
-
-    W, H, levels, win = 7680, 4320, 4, 9
-    prev = oracle.make_frame(W, H, 0, 0, 16, 3)
-    nxt = oracle.make_frame(W, H, 6.0, 4.0, 16, 3)
-    dp, dn = planar_to_device(prev[None]), planar_to_device(nxt[None])
-    whole = ctx.flow_pairs_device(dp, dn, W, levels, win)
-    plan, runners = run_strips_local_w(ctx, dp[0], dn[0], W, levels, win, 8, reach=16)
-    torch.cuda.synchronize()
-    for k in range(levels):
-        got = torch.cat([rn.own_flow(k) for rn in runners])
-        ref = whole[k][0]
-        m = ~torch.isnan(ref)
-        assert torch.equal(torch.isnan(got), torch.isnan(ref)) and torch.equal(got[m], ref[m]), f"level {k}"
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("W,H,levels,win", [(640, 480, 3, 9), (322, 406, 2, 5), (1920, 1080, 4, 15)])
 def test_native_strip_runner_world_one_equals_whole_frame(ctx, oracle, W, H, levels, win):
     """csrc/strips.cu on a single rank (no exchange): own-row upload, locally built pyramid, strip variants of the
-    kernels -- bit for bit the whole-frame result.  (The multi-rank exchange is exercised by scripts/run_strips.py
-    --native under torchrun; its schedule is the one the gloo tests above check.)"""
+    kernels -- bit for bit the whole-frame result.  (The multi-rank exchange is exercised by the peer-memory tests
+    below; its schedule is the one test_strip_plan_invariants checks.)"""
     import torch
 
     from cuda_optical_flow_2_b200 import WARP_BILINEAR, planar_to_device
@@ -218,23 +83,27 @@ def test_native_strip_runner_world_one_equals_whole_frame(ctx, oracle, W, H, lev
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("W,H,levels,win,world", [(640, 480, 3, 9, 2), (322, 406, 2, 5, 3), (1920, 1080, 4, 15, 4),
-                                                   (7680, 4320, 4, 9, 8)])
-def test_native_strips_peer_memory_transport_equals_whole_frame(ctx, oracle, W, H, levels, win, world):
+@pytest.mark.parametrize("W,H,levels,win,world,mode", [(640, 480, 3, 9, 2, BIL), (640, 480, 3, 9, 3, NEAR), (640, 480, 3, 9, 4, BIL),
+                                                       (322, 406, 2, 5, 3, BIL), (322, 406, 2, 5, 3, NEAR),
+                                                       (1920, 1080, 3, 9, 8, BIL), (1920, 1080, 4, 15, 4, BIL),
+                                                       (1920, 1080, 4, 15, 4, NEAR), (512, 384, 1, 9, 4, BIL),
+                                                       (7680, 4320, 4, 9, 8, BIL)])
+def test_native_strips_peer_memory_transport_equals_whole_frame(ctx, oracle, W, H, levels, win, world, mode):
     """csrc/strips.cu with the peer-memory transport: `world` ranks live in this process on one GPU; the sender's copy
     kernel stores halo rows straight into the receiver's arena and raises an epoch flag, the receiver's wait kernel
     checks it.  All ranks share ONE stream and their pairs are enqueued phase by phase (run_local_sequenced), so every
     flag is raised by a kernel ahead of its waiter: kernels of different ranks never have to be co-scheduled on the one
     GPU.  Three pairs back to back (flags, epochs and the done handshake are re-used), each bit for bit the whole-frame
-    result.  Across processes the same kernels run on CUDA IPC mappings, each rank enqueuing its whole pair at once
+    result at every level and in the total flow (at one level the residual flow), in both per-pixel warp modes.  Across
+    processes the same kernels run on CUDA IPC mappings, each rank enqueuing its whole pair at once
     (test_native_strips_two_processes_over_cuda_ipc, bench.py under torchrun)."""
     import torch
 
-    from cuda_optical_flow_2_b200 import WARP_BILINEAR, planar_to_device
+    from cuda_optical_flow_2_b200 import planar_to_device
     from cuda_optical_flow_2_b200.dist import NativeStrips
 
     dev = torch.device("cuda", 0)
-    ranks = [NativeStrips(ctx, W, H, levels, win, world, rk, dev, WARP_BILINEAR, 1.0, 16, transport="local") for rk in range(world)]
+    ranks = [NativeStrips(ctx, W, H, levels, win, world, rk, dev, mode, 1.0, 16, transport="local") for rk in range(world)]
     streams = [torch.cuda.Stream(dev) for _ in range(world)]
     try:
         NativeStrips.connect_local(ranks)
@@ -243,7 +112,7 @@ def test_native_strips_peer_memory_transport_equals_whole_frame(ctx, oracle, W, 
             nxt = oracle.make_frame(W, H, dx, dy, 8, 900 + trial)
             dp, dn = planar_to_device(prev[None]), planar_to_device(nxt[None])
             total = torch.empty((1, H, W, 2), dtype=torch.float32, device=dev)
-            whole = ctx.flow_pairs_device(dp, dn, W, levels, win, warp_mode=WARP_BILINEAR, total_flow=total)
+            whole = ctx.flow_pairs_device(dp, dn, W, levels, win, warp_mode=mode, total_flow=total)
             torch.cuda.synchronize()
             inputs = []
             for ns in ranks:
@@ -275,6 +144,68 @@ def test_native_strips_peer_memory_transport_equals_whole_frame(ctx, oracle, W, 
         torch.cuda.synchronize()
         for ns in ranks:
             ns.close()
+
+
+@pytest.mark.gpu
+def test_native_strip_reach_overflow_is_reported(ctx, oracle):
+    """A warp that reaches past the rows a rank holds must raise, not silently change the numbers.  With reach=1 a middle
+    rank of this 320x480 pair (3 levels, window 9, 4 ranks) holds its own rows plus 39 above and 36 below at level 0, 19
+    and 18 at level 1: the halo and the rows the coarser levels' halo rows are rebuilt from.  On these frames the flow of
+    the coarsest level, which the strips compute exactly, makes rank 1's level-1 warp ask for rows past those (the rule of
+    test_row_split.requested_rows), so its flag is certain.  With the default reach=16 no rank asks for a row it does not
+    hold, and the strips equal the whole frame bit for bit."""
+    import ctypes as C
+
+    import torch
+    from test_row_split import reach_flag, requested_rows
+
+    from cuda_optical_flow_2_b200 import _lib, planar_to_device
+    from cuda_optical_flow_2_b200.dist import NativeStrips
+
+    W, H, levels, win, world = 320, 480, 3, 9, 4
+    prev = oracle.make_frame(W, H, 0, 0, 16, 5)
+    nxt = oracle.make_frame(W, H, 0.0, 20.0, 16, 5)  # large vertical motion
+    _, cums = oracle.flow_pair(prev, nxt, levels, win, BIL, oracle.SUMS_EXACT, want_cum=True)
+    lib, out = _lib.load(), (C.c_int * 8)()
+
+    def flagged(reach):
+        """(rank, level) whose warp, on the whole frame's coarser flow, asks for a row outside the rows the rank holds."""
+        got = []
+        for rk in range(world):
+            for k in range(levels - 1):
+                _lib.check(lib.ofb_strips_plan_query(W, H, levels, win, world, rk, reach, k, out))
+                y0, y1, _, _, cy0, cy1, eb0, eb1 = list(out)
+                if reach_flag(requested_rows(cums[k + 1], W >> k, H >> k, BIL, y0, y1, win), eb0, eb1 - eb0, cy0, cy1 - cy0):
+                    got.append((rk, k))
+        return got
+
+    assert (1, 1) in flagged(1) and flagged(16) == []
+    dev = torch.device("cuda", 0)
+    dp, dn = planar_to_device(prev[None]), planar_to_device(nxt[None])
+    whole = ctx.flow_pairs_device(dp, dn, W, levels, win, warp_mode=BIL)
+    torch.cuda.synchronize()
+    for reach in (1, 16):
+        ranks = [NativeStrips(ctx, W, H, levels, win, world, rk, dev, BIL, 1.0, reach, transport="local") for rk in range(world)]
+        try:
+            NativeStrips.connect_local(ranks)
+            st = torch.cuda.current_stream().cuda_stream
+            inputs = [(dp[0, y0:y1], dn[0, y0:y1]) for y0, y1 in (ns.own_rows(0) for ns in ranks)]
+            NativeStrips.run_local_sequenced(ranks, inputs, st)
+            if reach == 1:
+                with pytest.raises(RuntimeError, match="raise `reach`"):
+                    ranks[1].check(st)
+                continue
+            for ns in ranks:
+                ns.check(st)
+                for k in range(levels):
+                    y0, y1 = ns.own_rows(k)
+                    ref, got = whole[k][0, y0:y1], ns.own_flow(k)
+                    m = ~torch.isnan(ref)
+                    assert torch.equal(torch.isnan(ref), torch.isnan(got)) and torch.equal(ref[m], got[m]), f"rank {ns.rank} level {k}"
+        finally:
+            torch.cuda.synchronize()
+            for ns in ranks:
+                ns.close()
 
 
 @pytest.mark.gpu
@@ -363,9 +294,10 @@ def test_native_strips_two_processes_over_cuda_ipc():
 
 
 def test_native_strip_plan_matches_python_plan():
-    """The schedule exists twice -- StripPlan here (Python runner, gloo tests) and in csrc/strips.cu (native runner):
-    own rows, kernel rows and coarse-flow rows must agree for every rank and level; the native image buffers may
-    only be larger (they also hold the rows from which the coarser levels' halo rows are rebuilt locally)."""
+    """The schedule exists twice -- StripPlan here (the Python restatement, checked by test_strip_plan_invariants) and in
+    csrc/strips.cu (the runner): own rows, kernel rows and coarse-flow rows must agree for every rank and level; the
+    native image buffers may only be larger (they also hold the rows from which the coarser levels' halo rows are
+    rebuilt locally)."""
     import ctypes as C
 
     from cuda_optical_flow_2_b200 import _lib

@@ -7,8 +7,8 @@ native row-strip runner across processes.
 - A plain push launches grayscale, the optional bilateral filter (range table + filter), the pyramid and one kernel per
   level, with or without the total.
 - With profiling on, a push records one pyramid record and, from the second frame on, one record per level.
-- The native strip runner over peer memory (scripts/run_strips.py --native under torchrun, CUDA IPC between the
-  processes) equals the whole frame bit for bit on 2 and 3 processes.
+- The native strip runner over peer memory (scripts/run_strips.py under torchrun, CUDA IPC between the processes)
+  equals the whole frame bit for bit on 2 and 3 processes.
 """
 from __future__ import annotations
 
@@ -107,10 +107,10 @@ def test_native_strips_over_peer_memory(nproc):
         sk.bind(("127.0.0.1", 0))
         port = sk.getsockname()[1]
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(nproc), "--master-addr", "127.0.0.1",
-           "--master-port", str(port), os.path.join(ROOT, "scripts", "run_strips.py"), "--native", "--check",
+           "--master-port", str(port), os.path.join(ROOT, "scripts", "run_strips.py"), "--check",
            "--w", "1920", "--h", "1080", "--levels", "3", "--reps", "4"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     rec = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
-    assert rec["n_gpus"] == nproc and rec["native"] is True and rec["transport"] == "peer"
+    assert rec["n_gpus"] == nproc and rec["transport"] == "peer"
     assert rec["bit_identical_to_whole_frame"] is True
