@@ -10,7 +10,8 @@ The device-resident entry points (`flow_pairs_device`, `flow_pairs_fb_device`, `
 `pyr_down_device`) take
 torch CUDA tensors only as owners of device memory; torch does none of the arithmetic.  The forward-backward check also
 runs on host batches (`flow_pairs_fb_host`) and on the frame stream (`FrameStream.push_fb`).  `track_points_device`
-follows a list of sub-pixel points through the pyramids (the KLT tracker).
+follows a list of sub-pixel points through the pyramids (the KLT tracker), and `detect_corners_device` finds points for it
+to start from (Shi-Tomasi corners on the tracker's own texture measure).
 """
 from __future__ import annotations
 
@@ -141,12 +142,12 @@ class Context:
 
     def profile_enable(self, on: bool = True) -> None:
         """CUDA-event timing around each fused-LK launch (tag = level), the pyramid build, the forward-backward check and
-        the point tracker's kernel."""
+        the point tracker's kernel and the corner detector's kernels."""
         L.check(self._lib.ofb_ctx_profile_enable(self._h, 1 if on else 0))
 
     def profile_read(self, tag: int) -> tuple[float, int]:
-        """(summed milliseconds, number of records) for a tag: a pyramid level, PROFILE_PYRAMID, PROFILE_FB_CHECK or
-        PROFILE_TRACK."""
+        """(summed milliseconds, number of records) for a tag: a pyramid level, PROFILE_PYRAMID, PROFILE_FB_CHECK,
+        PROFILE_TRACK or PROFILE_CORNERS."""
         ms, n = C.c_double(), C.c_ulonglong()
         L.check(self._lib.ofb_ctx_profile_read(self._h, int(tag), C.byref(ms), C.byref(n)))
         return ms.value, n.value
@@ -419,7 +420,8 @@ class Context:
         Gauss-Newton iterations per level, stopping a level early once both components of an update are below `eps` px
         (the defaults are OpenCV's).  prev/next as in flow_pairs_device.  Returns (flow (n, m, 2) float32 in flow units --
         s * flow px with s = flow_scale --, status (n, m) uint8 PT_* codes).  min_eig > 0 marks points whose window's
-        smaller structure-tensor eigenvalue, divided by 2 win^2, is below it PT_LOW_TEXTURE (rule: include/ofb200.h)."""
+        smaller structure-tensor eigenvalue, divided by win^2, is below it PT_LOW_TEXTURE (rule: include/ofb200.h); that
+        value is the score of min_eig_map_device."""
         import torch
 
         if prev.dtype != torch.uint8 or prev.dim() != 3 or not prev.is_contiguous() or prev.shape != next.shape:
@@ -438,6 +440,55 @@ class Context:
                                                   points.data_ptr(), m, int(iters), C.c_float(eps), C.c_float(min_eig),
                                                   flow.data_ptr(), status.data_ptr(), C.c_void_p(stream)))
         return flow, status
+
+    @staticmethod
+    def _corner_images(imgs, w: int):
+        import torch
+
+        if not isinstance(imgs, torch.Tensor) or imgs.dtype != torch.uint8 or imgs.dim() != 3 or not imgs.is_contiguous() \
+                or not imgs.is_cuda:
+            raise ValueError("imgs must be a contiguous uint8 (n, h, pitch) CUDA tensor")
+        n, h, pitch = imgs.shape
+        if not 1 <= w <= pitch:
+            raise ValueError(f"w {w} outside 1..pitch {pitch}")
+        return n, h, pitch
+
+    def min_eig_map_device(self, imgs, w: int, win: int, stream: int = 0):
+        """The Shi-Tomasi score of every pixel of the (n, h, pitch) uint8 images (the layout track_points_device takes):
+        the smaller eigenvalue of the window's structure tensor of the tracker's Sobel fields, over win^2 -- the value the
+        tracker compares with min_eig (rule: include/ofb200.h).  Returns (n, h, w) float32."""
+        import torch
+
+        n, h, pitch = self._corner_images(imgs, w)
+        out = torch.empty((n, h, w), dtype=torch.float32, device=imgs.device)
+        L.check(self._lib.ofb_min_eig_map_device(self._h, imgs.data_ptr(), pitch, pitch * h, w, h, n, win, out.data_ptr(),
+                                                 C.c_void_p(stream)))
+        return out
+
+    def detect_corners_device(self, imgs, w: int, win: int, max_corners: int, quality_level: float = 0.01,
+                              min_distance: float = 10.0, min_score: float = 0.0, stream: int = 0):
+        """Shi-Tomasi corners (goodFeaturesToTrack) of each of the (n, h, pitch) uint8 images: interior strict local maxima
+        of the score above max(quality_level * the image's largest score, min_score), strongest first, at least
+        min_distance px apart, at most max_corners per image (rule: include/ofb200.h).  Returns (corners (n, max_corners, 2)
+        float32 integer (x, y), scores (n, max_corners) float32, counts (n,) int32); the slots past an image's count are NaN,
+        so `corners` can go straight to track_points_device as its points.  Nothing waits on the host."""
+        import torch
+
+        n, h, pitch = self._corner_images(imgs, w)
+        dev = imgs.device
+        corners = torch.empty((n, max_corners, 2), dtype=torch.float32, device=dev) if max_corners >= 1 else None
+        scores = torch.empty((n, max_corners), dtype=torch.float32, device=dev) if max_corners >= 1 else None
+        counts = torch.empty((n,), dtype=torch.int32, device=dev)
+        L.check(self._lib.ofb_detect_corners_device(self._h, imgs.data_ptr(), pitch, pitch * h, w, h, n, win, int(max_corners),
+                                                    C.c_float(quality_level), C.c_float(min_distance), C.c_float(min_score),
+                                                    corners.data_ptr() if corners is not None else None,
+                                                    scores.data_ptr() if scores is not None else None, counts.data_ptr(),
+                                                    C.c_void_p(stream)))
+        return corners, scores, counts
+
+    def reserve_corners(self, w: int, h: int, n_images: int, win: int, max_corners: int) -> None:
+        """Size the context workspace for detect_corners_device calls of this shape now (CUDA graph capture)."""
+        L.check(self._lib.ofb_ctx_reserve_corners(self._h, w, h, n_images, win, max_corners))
 
     def pyr_down_device(self, src, sw: int, dst=None, stream: int = 0):
         """src: torch.uint8 (n, sh, pitch) -> dst (n, sh>>1, pitch_d)."""

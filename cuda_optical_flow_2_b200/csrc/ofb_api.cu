@@ -940,6 +940,165 @@ int ofb_track_points_device(ofb_ctx *c, const ofb_params *p, const uint8_t *prev
     return ws_release(c, st);
 }
 
+// ---- Shi-Tomasi corners: the frame and size limits both entry points share, and the detector's workspace ----------------
+static int check_corner_sizes(int w, int h, int n_images, int win)
+{
+    if (n_images < 1 || n_images > 65535) {
+        set_error("corners: n_images %d outside 1..65535", n_images);
+        return OFB_ERR_INVALID;
+    }
+    if (w < 1 || h < 1 || (long long)w * h >= (1ll << 31)) {
+        set_error("corners: image %dx%d (w, h >= 1 and w * h < 2^31)", w, h);
+        return OFB_ERR_INVALID;
+    }
+    if (win < 3 || win > OFB_MAX_WINDOW || !(win & 1)) {
+        set_error("corners: window %d not supported (odd 3..%d)", win, OFB_MAX_WINDOW);
+        return OFB_ERR_UNSUPPORTED;
+    }
+    return OFB_OK;
+}
+static int check_corner_frames(const uint8_t *img_d, size_t pitch_bytes, size_t image_stride_bytes, int w, int h, int n_images,
+                               int win)
+{
+    const int rc = check_corner_sizes(w, h, n_images, win);
+    if (rc) return rc;
+    ofb_params p = {w, h, 1, win, OFB_WARP_BILINEAR, 1.0f, n_images};
+    return check_device_frames(&p, img_d != nullptr, "corners: NULL image pointer", pitch_bytes, image_stride_bytes);
+}
+
+struct CornerWs {
+    CornerPlan cp;
+    size_t off_map, off_max, off_beg, off_end, off_kin, off_kout, off_grid, off_sort, sort_bytes, bytes;
+};
+
+static int plan_corner_ws(int w, int h, int n, int win, CornerWs *p)
+{
+    plan_corners(w, h, n, win, &p->cp);
+    if (p->cp.total >= (1ll << 31)) {
+        set_error("corners: %d images of %dx%d hold %lld candidate slots (the per-image sort takes < 2^31)", n, w, h, p->cp.total);
+        return OFB_ERR_UNSUPPORTED;
+    }
+    int rc = corner_sort_bytes(p->cp.total, n, &p->sort_bytes);
+    if (rc) return rc;
+    Carver cv;
+    p->off_map = cv.take((size_t)w * h * n * sizeof(float));
+    p->off_max = cv.take((size_t)n * sizeof(unsigned));
+    p->off_beg = cv.take((size_t)n * sizeof(int));
+    p->off_end = cv.take((size_t)n * sizeof(int));
+    p->off_kin = cv.take((size_t)p->cp.total * 8);
+    p->off_kout = cv.take((size_t)p->cp.total * 8);
+    p->off_grid = cv.take((size_t)p->cp.iw * p->cp.ih * n * sizeof(int));
+    p->off_sort = cv.take(p->sort_bytes);
+    p->bytes = cv.off;
+    return OFB_OK;
+}
+
+int ofb_min_eig_map_device(ofb_ctx *c, const uint8_t *img_d, size_t pitch_bytes, size_t image_stride_bytes, int w, int h,
+                           int n_images, int win, float *score_d, void *stream)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_corner_frames(img_d, pitch_bytes, image_stride_bytes, w, h, n_images, win);
+    if (rc) return rc;
+    if (!score_d || (reinterpret_cast<uintptr_t>(score_d) & 3)) {
+        set_error("corners: score map NULL or not 4-byte aligned");
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CornerArgs a = {};
+    a.img = img_d;
+    a.pitch = pitch_bytes;
+    a.istr = image_stride_bytes;
+    a.w = w;
+    a.h = h;
+    a.n = n_images;
+    a.m = win / 2 + 1;
+    a.map = score_d;
+    a.map_stride = (size_t)w * h;
+    if ((rc = prof_begin(c, OFB_PROFILE_CORNERS, st))) return rc;
+    if ((rc = launch_corner_score(a, win, st, &c->launches))) return rc;
+    return prof_end(c, st);
+}
+
+int ofb_detect_corners_device(ofb_ctx *c, const uint8_t *img_d, size_t pitch_bytes, size_t image_stride_bytes, int w, int h,
+                              int n_images, int win, int max_corners, float quality_level, float min_distance, float min_score,
+                              float *corners_d, float *scores_d, int *counts_d, void *stream)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_corner_frames(img_d, pitch_bytes, image_stride_bytes, w, h, n_images, win);
+    if (rc) return rc;
+    if (max_corners < 1 || max_corners > (1 << 20)) {
+        set_error("corners: max_corners %d outside 1..%d", max_corners, 1 << 20);
+        return OFB_ERR_INVALID;
+    }
+    if (!(std::isfinite(quality_level) && quality_level >= 0.0f && quality_level <= 1.0f)) {
+        set_error("corners: quality_level %g must be finite and in [0, 1]", (double)quality_level);
+        return OFB_ERR_INVALID;
+    }
+    if (!(std::isfinite(min_distance) && min_distance >= 0.0f && std::isfinite(min_score) && min_score >= 0.0f)) {
+        set_error("corners: min_distance %g / min_score %g must be finite and >= 0", (double)min_distance, (double)min_score);
+        return OFB_ERR_INVALID;
+    }
+    if (!corners_d || !counts_d) {
+        set_error("corners: NULL corner or count pointer");
+        return OFB_ERR_INVALID;
+    }
+    if ((reinterpret_cast<uintptr_t>(corners_d) & 7) || (reinterpret_cast<uintptr_t>(scores_d) & 3) ||
+        (reinterpret_cast<uintptr_t>(counts_d) & 3)) {
+        set_error("corners: corners must be 8-byte aligned, scores and counts 4-byte aligned");
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    CornerWs ws;
+    if ((rc = plan_corner_ws(w, h, n_images, win, &ws))) return rc;
+    if ((rc = ws_reserve(c, ws.bytes))) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = ws_acquire(c, st))) return rc;
+    DetectArgs d = {};
+    d.plan = ws.cp;
+    d.img = img_d;
+    d.pitch = pitch_bytes;
+    d.istr = image_stride_bytes;
+    d.w = w;
+    d.h = h;
+    d.n = n_images;
+    d.max_corners = max_corners;
+    d.quality_level = quality_level;
+    d.min_distance = min_distance;
+    d.min_score = min_score;
+    d.map = reinterpret_cast<float *>(c->ws + ws.off_map);
+    d.max_bits = reinterpret_cast<unsigned *>(c->ws + ws.off_max);
+    d.seg_begin = reinterpret_cast<int *>(c->ws + ws.off_beg);
+    d.seg_end = reinterpret_cast<int *>(c->ws + ws.off_end);
+    d.keys_in = reinterpret_cast<unsigned long long *>(c->ws + ws.off_kin);
+    d.keys_out = reinterpret_cast<unsigned long long *>(c->ws + ws.off_kout);
+    d.grid = reinterpret_cast<int *>(c->ws + ws.off_grid);
+    d.sort_tmp = c->ws + ws.off_sort;
+    d.sort_bytes = ws.sort_bytes;
+    d.corners = corners_d;
+    d.scores = scores_d;
+    d.counts = counts_d;
+    if ((rc = prof_begin(c, OFB_PROFILE_CORNERS, st))) return rc;
+    if ((rc = launch_detect_corners(d, win, st, &c->launches))) return rc;
+    if ((rc = prof_end(c, st))) return rc;
+    return ws_release(c, st);
+}
+
+int ofb_ctx_reserve_corners(ofb_ctx *c, int w, int h, int n_images, int win, int max_corners)
+{
+    OFB_CHECK_CTX(c);
+    int rc = check_corner_sizes(w, h, n_images, win);
+    if (rc) return rc;
+    if (max_corners < 1 || max_corners > (1 << 20)) {
+        set_error("corners: max_corners %d outside 1..%d", max_corners, 1 << 20);
+        return OFB_ERR_INVALID;
+    }
+    OFB_GUARD(c);
+    CornerWs ws;
+    if ((rc = plan_corner_ws(w, h, n_images, win, &ws))) return rc;
+    return ws_reserve(c, ws.bytes);
+}
+
 int ofb_pyr_down_device(ofb_ctx *c, const uint8_t *src_d, size_t src_pitch, size_t src_image_stride, int sw, int sh,
                         uint8_t *dst_d, size_t dst_pitch, size_t dst_image_stride, int n_images, void *stream)
 {

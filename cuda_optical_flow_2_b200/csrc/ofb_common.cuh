@@ -185,6 +185,44 @@ struct TrackArgs {
 };
 int launch_track_points(const TrackArgs &a, int win, cudaStream_t stream, unsigned long long *launches);
 
+// ---- Shi-Tomasi corners for the tracker (corners.cu) ---------------------------------------------------------------
+struct CornerArgs {
+    const uint8_t *img;  // image i at img + i * istr
+    size_t pitch, istr;
+    int w, h, n;
+    int m;               // interior margin win/2 + 1
+    float *map;          // score of image i at map + i * map_stride, rows of w floats
+    size_t map_stride;
+    unsigned *max_bits;  // optional: per image, the float bits of the interior maximum (zeroed before the launch)
+};
+int launch_corner_score(const CornerArgs &a, int win, cudaStream_t stream, unsigned long long *launches);
+struct CornerPlan {
+    int m, iw, ih;       // interior margin and size (0 when the image has no interior)
+    long long cap;       // candidate slots per image: ceil(iw/2) * ceil(ih/2)
+    long long total;     // cap * n
+};
+void plan_corners(int w, int h, int n, int win, CornerPlan *p);
+int corner_sort_bytes(long long total, int n, size_t *bytes); // temporary storage of the per-image sort
+struct DetectArgs {
+    CornerPlan plan;
+    const uint8_t *img;
+    size_t pitch, istr;
+    int w, h, n, max_corners;
+    float quality_level, min_distance, min_score;
+    // workspace
+    float *map;                              // n * h * w
+    unsigned *max_bits;                      // n
+    int *seg_begin, *seg_end;                // n each
+    unsigned long long *keys_in, *keys_out;  // plan.total each
+    int *grid;                               // n * iw * ih (the finest cell grid)
+    void *sort_tmp;
+    size_t sort_bytes;
+    // outputs
+    float *corners, *scores;
+    int *counts;
+};
+int launch_detect_corners(const DetectArgs &d, int win, cudaStream_t stream, unsigned long long *launches);
+
 int launch_grayscale(const uint8_t *src_c3, int w, int h, uint8_t *dst_c3, uint8_t *dst_planar, size_t dst_pitch,
                      cudaStream_t stream, unsigned long long *launches);
 int launch_bilateral(const uint8_t *src, const uint8_t *gray, size_t pitch, int channels, int w, int h, int ww, int wh,

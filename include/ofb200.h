@@ -467,6 +467,49 @@ int ofb_track_points_device(ofb_ctx *ctx, const ofb_params *p, const uint8_t *pr
                             size_t pitch_bytes, size_t image_stride_bytes, const float *points_d, int n_points,
                             int iters, float eps, float min_eig, float *flow_d, uint8_t *status_d, void *stream);
 
+/* ---- Shi-Tomasi corners for the tracker: points to start from, found on the device; the reference has no counterpart ----
+ * goodFeaturesToTrack's role with the tracker's own texture measure, so that a detected point is one the tracker accepts.
+ * Images are planar u8 with the layout of ofb_flow_pairs_device (image i at img_d + i*image_stride_bytes), w x h each,
+ * 1 <= n_images <= 65535, w * h < 2^31, odd win 3..19.
+ * Score of pixel (x, y) (every pixel; ofb_min_eig_map_device writes it, n_images*h*w floats, tightly packed):
+ *   gx = Dx (*) img, gy = Dy (*) img: the tracker's Ix, Iy at level 0 (Sobel correlations, 0 outside the frame; |g| <= 1020)
+ *   over the win x win window centred on the pixel (field positions outside the frame contribute 0), exact in int32:
+ *     A = sum gx^2, D = sum gy^2, B = sum gx*gy
+ *   det = A*D - B*B, T = A - D, disc = T*T + 4*B*B exact in int64; S = A + D
+ *   l1 = 0 if S == 0, else in double, every operation rounded to nearest on its own, no fma:
+ *     l1 = (2.0 * (double)det) / ((double)S + sqrt((double)disc))     (the stable form of (S - sqrt(disc)) / 2)
+ *   score = (float)(l1 / (double)(win*win))
+ * This is the lam that ofb_track_points_device compares with min_eig: at an integer point with levels = 1 its a, dd, b are
+ * A, D, B.
+ * Detection, per image:
+ *   interior: m <= x <= w-1-m and m <= y <= h-1-m, m = win/2 + 1 (every Sobel tap of the window lies inside the frame, so
+ *     the zero padding cannot make corners); an image smaller than 2m+1 in either direction yields 0 corners
+ *   thr = max(quality_level * max_score, min_score) (a float product), max_score the largest interior score; a pixel
+ *     qualifies if score > thr (so a score of 0 never does)
+ *   key order: p precedes q if score(p) > score(q), or the scores are equal and y_p*w + x_p < y_q*w + x_q
+ *   candidates: qualifying interior pixels that precede each of their interior 8-neighbours (a strict local maximum in key
+ *     order: a plateau yields one candidate per 3x3 neighbourhood, unlike OpenCV's score == dilate(score)); no two are
+ *     8-adjacent, so an image has at most ceil(iw/2) * ceil(ih/2) of them (iw x ih the interior)
+ *   selection: the candidates in key order; one is accepted unless an accepted corner lies at
+ *     (double)(dx*dx + dy*dy) < (double)min_distance * (double)min_distance (dx, dy integer pixel differences, the sum
+ *     exact in int64); stop after max_corners.  (OpenCV's sequential greedy; min_distance <= 1 suppresses nothing.)
+ *   output: corners_d[i*max_corners + k] = (x, y) of the k-th accepted corner as floats, strongest first; scores_d
+ *     (optional) its score; counts_d[i] the number accepted; the slots after it hold NaN (corners and scores), which the
+ *     tracker reports OFB_PT_OUTSIDE: corners_d can be passed to ofb_track_points_device as its points.
+ * Both calls are asynchronous on `stream` and never wait on the host (the counts stay on the device), so detection followed
+ * by tracking can be captured as one CUDA graph after ofb_ctx_reserve_corners (and ofb_ctx_reserve_pairs) have sized the
+ * workspace.  Limits: 1 <= max_corners <= 2^20, quality_level finite in [0, 1], min_distance and min_score finite and >= 0,
+ * frames as in ofb_flow_pairs_device, corners_d 8-byte aligned, score_d / scores_d / counts_d 4-byte aligned; the
+ * candidate slots n_images * ceil(iw/2) * ceil(ih/2) below 2^31 (OFB_ERR_UNSUPPORTED otherwise).  Bad arguments are
+ * refused before anything is enqueued, the outputs untouched.  The detector's score map, candidates and cell grid live in
+ * the context workspace.  With profiling on, each call gets one OFB_PROFILE_CORNERS record around its kernels. */
+int ofb_min_eig_map_device(ofb_ctx *ctx, const uint8_t *img_d, size_t pitch_bytes, size_t image_stride_bytes, int w, int h,
+                           int n_images, int win, float *score_d, void *stream);
+int ofb_detect_corners_device(ofb_ctx *ctx, const uint8_t *img_d, size_t pitch_bytes, size_t image_stride_bytes, int w,
+                              int h, int n_images, int win, int max_corners, float quality_level, float min_distance,
+                              float min_score, float *corners_d, float *scores_d, int *counts_d, void *stream);
+int ofb_ctx_reserve_corners(ofb_ctx *ctx, int w, int h, int n_images, int win, int max_corners);
+
 /* Pinned host memory helpers for callers without a CUDA runtime of their own. */
 int ofb_host_alloc(void **ptr, size_t bytes);
 int ofb_host_free(void *ptr);
@@ -478,11 +521,12 @@ int ofb_ctx_launch_count(const ofb_ctx *ctx, unsigned long long *count);
  * CUDA-event pair (on the stream the work is launched on) around every fused-LK launch, tagged with
  * its pyramid level, and around the pyramid build, tagged OFB_PROFILE_PYRAMID; the forward-backward entry points
  * also around the check kernel, tagged OFB_PROFILE_FB_CHECK, and ofb_track_points_device around its kernel, tagged
- * OFB_PROFILE_TRACK.  _enable(on) also
+ * OFB_PROFILE_TRACK, and the corner entry points around their kernels, tagged OFB_PROFILE_CORNERS.  _enable(on) also
  * discards earlier records.  _read waits for the tagged events and returns their summed duration. */
 #define OFB_PROFILE_PYRAMID 100
 #define OFB_PROFILE_FB_CHECK 101
 #define OFB_PROFILE_TRACK 102
+#define OFB_PROFILE_CORNERS 103
 int ofb_ctx_profile_enable(ofb_ctx *ctx, int on);
 int ofb_ctx_profile_read(ofb_ctx *ctx, int tag, double *ms_sum, unsigned long long *n_records);
 
