@@ -56,7 +56,8 @@ __global__ void __launch_bounds__(CRN_THREADS) corner_score_kernel(const CornerA
     __shared__ int s_ca[CRN_TH * CS], s_cd[CRN_TH * CS], s_cb[CRN_TH * CS];
     const int t = threadIdx.x, z = blockIdx.z;
     const uint8_t *img = a.img + (size_t)z * a.istr;
-    for (int ty = blockIdx.y; ty * CRN_TH < a.h; ty += gridDim.y) { // (grid.y is capped at 65535)
+    // (grid.y is capped at 65535; ty * CRN_TH would overflow int past the last tile of a frame taller than 2^31 - 2^21)
+    for (int ty = blockIdx.y; ty <= (a.h - 1) / CRN_TH; ty += gridDim.y) {
         const int x0 = blockIdx.x * CRN_TW, y0 = ty * CRN_TH; // the tile's first output pixel
         // bytes of (x0 - R - 1, y0 - R - 1) .. + (BW, BH); 0 outside the frame
         for (int i = t; i < BH * BW; i += CRN_THREADS) {
@@ -142,7 +143,7 @@ __global__ void __launch_bounds__(CRN_THREADS) corner_score_kernel(const CornerA
 
 int launch_corner_score(const CornerArgs &a, int win, cudaStream_t stream, unsigned long long *launches)
 {
-    const dim3 grid((unsigned)((a.w + CRN_TW - 1) / CRN_TW), (unsigned)min((a.h + CRN_TH - 1) / CRN_TH, 65535), (unsigned)a.n);
+    const dim3 grid((unsigned)((a.w - 1) / CRN_TW + 1), (unsigned)min((a.h - 1) / CRN_TH + 1, 65535), (unsigned)a.n);
     switch (win) {
 #define OFB_CRN_CASE(W)                                                                   \
     case W: corner_score_kernel<W><<<grid, CRN_THREADS, 0, stream>>>(a); break;
@@ -252,18 +253,19 @@ __global__ void __launch_bounds__(SEL_CHUNK) corner_select_kernel(const SelArgs 
     __shared__ unsigned s_acc[SEL_WORDS], s_und[SEL_WORDS];
     __shared__ int s_total;
     const int t = threadIdx.x, z = blockIdx.x, lane = t & 31, wid = t >> 5;
-    const int end = a.seg_end[z];
+    // the chunk loop steps an offset inside the segment: a segment is at most one image's cap (< 2^29 keys), but it may end
+    // anywhere below 2^31, where base + SEL_CHUNK would wrap
+    const int begin = a.seg_begin[z], len = a.seg_end[z] - begin;
     int *grid = a.grid + (size_t)z * a.gw * a.gh;
     float2 *corners = reinterpret_cast<float2 *>(a.corners) + (size_t)z * a.max_corners;
     float *scores = a.scores ? a.scores + (size_t)z * a.max_corners : nullptr;
     int count = 0;
-    for (int base = a.seg_begin[z]; base < end && count < a.max_corners; base += SEL_CHUNK) {
-        const int j = base + t;
-        bool alive = j < end;
+    for (int off = 0; off < len && count < a.max_corners; off += SEL_CHUNK) {
+        bool alive = t < len - off;
         unsigned long long key = 0;
         int x = 0, y = 0;
         if (alive) {
-            key = a.keys[j];
+            key = a.keys[begin + off + t];
             const int idx = (int)(unsigned)key;
             y = idx / a.w;
             x = idx - y * a.w;
