@@ -11,27 +11,15 @@ GPU tests: every other item; each output is allocated with guard bands that must
 """
 import decimal
 import math
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-from test_corners import CornerOracle, assert_same_bits, content, exact_sums, plain_greedy
+from support import F32, assert_same_bits, content, cro, device_frames, exact_sums, plain_greedy  # noqa: F401 (cro is a fixture)
 
-F32 = np.float32
 WINS = list(range(3, 20, 2))
 FLT_MAX = float(np.finfo(F32).max)
 G = 64  # guard elements before and after every output buffer
-
-
-@pytest.fixture(scope="session")
-def crl(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("corner_oracle_limits") / "libcorneroracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "corner_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return CornerOracle(so)
 
 
 def f32_next(x, toward):
@@ -105,18 +93,6 @@ def _guards_intact(buf, fill):
     return bool((buf[:G] == fill).all()) and bool((buf[-G:] == fill).all())
 
 
-def _frames(imgs, pitch=None, stride=None, pad=0):
-    """(n, h, w) uint8 -> a flat CUDA buffer holding image i at byte i * stride with row pitch `pitch`, `pad` elsewhere."""
-    import torch
-
-    n, h, w = imgs.shape
-    pitch = pitch or w
-    stride = pitch * h if stride is None else stride
-    buf = np.full(stride * (n - 1) + pitch * (h - 1) + w, pad, np.uint8)
-    np.lib.stride_tricks.as_strided(buf, (n, h, w), (stride, pitch, 1))[...] = imgs
-    return torch.from_numpy(buf).cuda(), pitch, stride
-
-
 def _map_g(ctx, dev, pitch, stride, w, h, n, win, stream=None):
     import torch
 
@@ -154,10 +130,10 @@ def _detect_g(ctx, dev, pitch, stride, w, h, n, win, mc, ql=0.01, md=10.0, ms=0.
             counts.cpu().numpy())
 
 
-def _assert_detect(crl, imgs, got, win, mc, ql=0.01, md=10.0, ms=0.0, refs=None):
+def _assert_detect(cro, imgs, got, win, mc, ql=0.01, md=10.0, ms=0.0, refs=None):
     corners, scores, counts = got
     for i, img in enumerate(imgs):
-        rc, rs, rn = refs[i] if refs is not None else crl.detect(img, win, mc, quality_level=ql, min_distance=md,
+        rc, rs, rn = refs[i] if refs is not None else cro.detect(img, win, mc, quality_level=ql, min_distance=md,
                                                                  min_score=ms)
         assert counts[i] == rn, (i, counts[i], rn)
         assert_same_bits(corners[i], rc, f"image {i} corners")
@@ -169,11 +145,11 @@ def _assert_detect(crl, imgs, got, win, mc, ql=0.01, md=10.0, ms=0.0, refs=None)
 # ==================================================================================== 1. worst-case content
 @pytest.mark.parametrize("win", WINS)
 @pytest.mark.parametrize("kind", WORST)
-def test_worst_case_score_within_one_ulp(crl, kind, win):
+def test_worst_case_score_within_one_ulp(cro, kind, win):
     """The restatement stays within one float ulp of a 50-digit evaluation of l1 / win^2 where det and disc pass 2^53."""
     img = worst(kind, seed=win)
     h, w = img.shape
-    got = crl.score(img, win)
+    got = cro.score(img, win)
     A, D, B = exact_sums(img, win)
     assert (A + D).max() < 2 ** 31  # the kernel forms S = A + D in int32
     decimal.getcontext().prec = 50
@@ -208,15 +184,15 @@ def test_worst_case_content_reaches_past_2_53():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("win", WINS)
-def test_worst_case_content_kernel(ctx, crl, win):
+def test_worst_case_content_kernel(ctx, cro, win):
     imgs = np.stack([worst(k, seed=win) for k in WORST])
     n, h, w = imgs.shape
-    dev, pitch, stride = _frames(imgs)
+    dev, pitch, stride = device_frames(imgs)
     got = _map_g(ctx, dev, pitch, stride, w, h, n, win).cpu().numpy()
     for i, k in enumerate(WORST):
-        assert_same_bits(got[i], crl.score(imgs[i], win), f"{k} map")
+        assert_same_bits(got[i], cro.score(imgs[i], win), f"{k} map")
     for kw in (dict(ql=0.0, md=0.0), dict(ql=0.01, md=3.0)):
-        _assert_detect(crl, imgs, _detect_g(ctx, dev, pitch, stride, w, h, n, win, 200, **kw), win, 200, **kw)
+        _assert_detect(cro, imgs, _detect_g(ctx, dev, pitch, stride, w, h, n, win, 200, **kw), win, 200, **kw)
 
 
 # ==================================================================================== 2. tall frames
@@ -242,32 +218,32 @@ def test_tall_frames_step_every_grid_stride_loop():
 _tall_cache = {}
 
 
-def _tall(crl, kind, w, h, win, seed):
+def _tall(cro, kind, w, h, win, seed):
     """The frame, its restated map and the restated detections (md 0 and 3, max_corners 2^20), computed once."""
     key = (kind, w, h, win, seed)
     if key not in _tall_cache:
         img = np.random.default_rng(seed).integers(0, 256, (h, w), dtype=np.uint8) if kind == "noise" else \
             np.tile(worst("bnoise2", w, 4096, seed), (h // 4096 + 1, 1))[:h]
-        smap = crl.score(img, win)
-        sel = {md: crl.select(smap, win, 1 << 20, quality_level=0.0, min_distance=md) for md in (0.0, 3.0)}
+        smap = cro.score(img, win)
+        sel = {md: cro.select(smap, win, 1 << 20, quality_level=0.0, min_distance=md) for md in (0.0, 3.0)}
         _tall_cache[key] = img, smap, sel
     return _tall_cache[key]
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("n,win", [(1, 3), (2, 3), (1, 19)])
-def test_tall_frames(ctx, crl, n, win):
+def test_tall_frames(ctx, cro, n, win):
     """The whole map and the detections (2^20 corners reached) on frames taller than the grids' caps."""
     w, h = (TALL_W, TALL_H) if win == 3 else (TALL19_W, TALL19_H)
-    frames = [_tall(crl, k, w, h, win, s) for k, s in (("noise", 1), ("bnoise2", 2))[:n]]
+    frames = [_tall(cro, k, w, h, win, s) for k, s in (("noise", 1), ("bnoise2", 2))[:n]]
     imgs = np.stack([f[0] for f in frames])
-    dev, pitch, stride = _frames(imgs)
+    dev, pitch, stride = device_frames(imgs)
     got = _map_g(ctx, dev, pitch, stride, w, h, n, win).cpu().numpy()
     for i in range(n):
         assert_same_bits(got[i], frames[i][1], f"image {i} map")
     del got
     for md in (0.0, 3.0):
-        counts = _assert_detect(crl, imgs, _detect_g(ctx, dev, pitch, stride, w, h, n, win, 1 << 20, ql=0.0, md=md), win,
+        counts = _assert_detect(cro, imgs, _detect_g(ctx, dev, pitch, stride, w, h, n, win, 1 << 20, ql=0.0, md=md), win,
                                 1 << 20, ql=0.0, md=md, refs=[f[2][md] for f in frames])
         if win == 3:
             assert (counts == 1 << 20).all()
@@ -357,25 +333,25 @@ def crop_content(seed):
 
 
 @pytest.mark.parametrize("md,mc", [(0.0, 10_000), (3.0, 10_000), (10.0, 37)])
-def test_sparse_reference_equals_plain_greedy(crl, md, mc):
+def test_sparse_reference_equals_plain_greedy(cro, md, mc):
     """The sparse reference of the largest-frame test equals plain_greedy and the restatement on a whole small frame."""
     W, H, win = 400, 300, 3
     frame = np.zeros((H, W), np.uint8)
     pieces = []
     for i, (x0, y0) in enumerate(crop_layout(W, H, 9, 4)):
         frame[y0:y0 + 48, x0:x0 + 48] = crop_content(i)
-        pieces.append((x0, y0, crl.score(frame[y0:y0 + 48, x0:x0 + 48], win)))
-    smap = crl.score(frame, win)
+        pieces.append((x0, y0, cro.score(frame[y0:y0 + 48, x0:x0 + 48], win)))
+    smap = cro.score(frame, win)
     for x0, y0, s in pieces:
         assert_same_bits(smap[y0:y0 + 48, x0:x0 + 48], s, "crop map")
     acc = greedy(sparse_candidates(pieces, W, H, win, 0.01, 0.0), mc, md)
     assert acc == plain_greedy(smap, win, mc, 0.01, md, 0.0)
-    c, s, n = crl.select(smap, win, mc, quality_level=0.01, min_distance=md)
+    c, s, n = cro.select(smap, win, mc, quality_level=0.01, min_distance=md)
     assert n == len(acc) and np.array_equal(c[:n], np.array([(x, y) for x, y, _ in acc], F32))
 
 
 @pytest.mark.gpu
-def test_largest_frame(crl):
+def test_largest_frame(cro):
     """65535 x 32768 = 2^31 - 32768 pixels (the map's last raster index is within 2^16 of 2^31), zeros except 40 crops of
     content, some in the last rows and columns (candidate raster indices above 2^30, columns above 65400).  The map equals
     the restatement of each crop and is 0 elsewhere; the detections equal the sparse reference.  Device memory measured on
@@ -386,10 +362,10 @@ def test_largest_frame(crl):
     W, H, win = 65535, 32768, 3
     assert W * H == 2 ** 31 - 32768
     with Context(0) as ctx:  # its own workspace, measured here and freed at the end
-        _largest_frame(ctx, crl, W, H, win)
+        _largest_frame(ctx, cro, W, H, win)
 
 
-def _largest_frame(ctx, crl, W, H, win):
+def _largest_frame(ctx, cro, W, H, win):
     import torch
 
     torch.cuda.synchronize()
@@ -400,7 +376,7 @@ def _largest_frame(ctx, crl, W, H, win):
     for i, (x0, y0) in enumerate(crop_layout(W, H, 40, 11)):
         c = crop_content(i)
         img[y0:y0 + 48, x0:x0 + 48] = torch.from_numpy(c).cuda()
-        pieces.append((x0, y0, crl.score(c, win)))
+        pieces.append((x0, y0, cro.score(c, win)))
     dev = img.view(-1)
     smap = _map_g(ctx, dev, W, W * H, W, H, 1, win)[0]
     peak_map = free0 - torch.cuda.mem_get_info()[0]
@@ -455,12 +431,12 @@ LATTICES = {511: (73, 7), 512: (32, 16), 513: (27, 19), 1024: (32, 32), 1025: (4
 
 @pytest.mark.parametrize("count", sorted(LATTICES))
 @pytest.mark.parametrize("win", [3, 5, 9])
-def test_lattice_candidate_counts(crl, count, win):
+def test_lattice_candidate_counts(cro, count, win):
     """Each impulse of the lattice is exactly one candidate: the candidate counts straddle the 512-key chunks."""
     nx, ny = LATTICES[count]
     s = win + 3
     img = lattice(nx, ny, s, s, win, checker_bright)
-    _, _, n = crl.detect(img, win, 1 << 20, quality_level=0.0, min_distance=0.0)
+    _, _, n = cro.detect(img, win, 1 << 20, quality_level=0.0, min_distance=0.0)
     assert n == count
 
 
@@ -496,7 +472,7 @@ def test_selection_grid_restated():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("count", sorted(LATTICES))
-def test_chunk_boundaries(ctx, crl, count):
+def test_chunk_boundaries(ctx, cro, count):
     """Lattices of 511 .. 1537 candidates at windows 3 and 9: max_corners running out at count - 1, 512, 1024 and in the
     middle of a chunk; min_distance just above the spacing (each dim impulse's conflicts are bright ones, which fill the
     earlier chunks: the grid lookup), at the spacing, and the sweep."""
@@ -505,39 +481,39 @@ def test_chunk_boundaries(ctx, crl, count):
         s = win + 3
         img = lattice(nx, ny, s, s, win, checker_bright)[None]
         h, w = img.shape[1:]
-        dev, pitch, stride = _frames(img)
+        dev, pitch, stride = device_frames(img)
         mcs = sorted({count - 1, 512, 1024, 300, count + 3, 1 << 20} - {0})
         for md in [f32_next(s, s + 1), float(s), 0.0] + MD_SWEEP:
             for mc in (mcs if md in (f32_next(s, s + 1), 0.0) else [count + 3]):
-                _assert_detect(crl, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, win, mc, ql=0.0, md=md), win, mc, ql=0.0,
+                _assert_detect(cro, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, win, mc, ql=0.0, md=md), win, mc, ql=0.0,
                                md=md)
 
 
 @pytest.mark.gpu
-def test_exact_distance_lattice(ctx, crl):
+def test_exact_distance_lattice(ctx, cro):
     """Impulses on a 6 x 8 lattice: horizontal neighbours 6 apart, vertical 8, diagonal exactly 10 (6-8-10).  md 10 keeps
     the diagonal pairs, nextafter(10, 11) separates them; 1537 candidates, three chunks."""
     img = lattice(53, 29, 6, 8, 3, lambda i, j: 60 + (i * 7 + j * 13) % 190)[None]
     h, w = img.shape[1:]
-    dev, pitch, stride = _frames(img)
+    dev, pitch, stride = device_frames(img)
     got = {}
     for md in (6.0, f32_next(6, 7), 8.0, f32_next(8, 9), 10.0, f32_next(10, 11), f32_next(10, 0)):
-        got[md] = _assert_detect(crl, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, 3, 2000, ql=0.0, md=md), 3, 2000, ql=0.0,
+        got[md] = _assert_detect(cro, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, 3, 2000, ql=0.0, md=md), 3, 2000, ql=0.0,
                                  md=md)[0]
     assert got[10.0] > got[f32_next(10, 11)] and got[6.0] > got[f32_next(6, 7)]
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["noise", "natural"])
-def test_min_distance_sweep_4k(ctx, crl, kind):
+def test_min_distance_sweep_4k(ctx, cro, kind):
     w, h, win = 3840, 2160, 3
     img = content(kind, w, h, 21)[None] if kind == "noise" else \
         np.tile(content("natural", 480, 270, 21), (8, 8))[None]
-    dev, pitch, stride = _frames(img)
-    smap = crl.score(img[0], win)
+    dev, pitch, stride = device_frames(img)
+    smap = cro.score(img[0], win)
     for md in [0.0] + MD_SWEEP:
-        ref = crl.select(smap, win, 1 << 20, quality_level=0.0, min_distance=md)
-        _assert_detect(crl, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 1 << 20, ql=0.0, md=md), win, 1 << 20,
+        ref = cro.select(smap, win, 1 << 20, quality_level=0.0, min_distance=md)
+        _assert_detect(cro, img, _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 1 << 20, ql=0.0, md=md), win, 1 << 20,
                        ql=0.0, md=md, refs=[ref])
 
 
@@ -553,7 +529,7 @@ def mirrored(w, h, ax, ay, seed):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("win", [3, 9, 19])
-def test_ties_across_seams(ctx, crl, win):
+def test_ties_across_seams(ctx, cro, win):
     """Mirror axes on the score kernel's 32-column and 32-row tile seams, on the candidate kernel's warp seam (interior
     column x - m a multiple of 32) and its 8-row block seam; periodic content (a 7 x 5 tile) with md just above and below
     the periods."""
@@ -561,17 +537,17 @@ def test_ties_across_seams(ctx, crl, win):
     w, h = 203, 157
     imgs = np.stack([mirrored(w, h, 0, 0, 1), mirrored(w, h, m, m, 2), mirrored(w, h, m, m + 8, 3),
                      np.tile(np.random.default_rng(4).integers(0, 256, (5, 7), dtype=np.uint8), (h // 5 + 1, w // 7 + 1))[:h, :w]])
-    s0 = crl.score(imgs[0], win)
+    s0 = cro.score(imgs[0], win)
     x = 64 + 32
     assert (s0[40:110, x - 1] == s0[40:110, x]).all() and (s0[x - 1, 40:110] == s0[x, 40:110]).all()
-    s1 = crl.score(imgs[1], win)
+    s1 = cro.score(imgs[1], win)
     assert (s1[40:110, m + 63] == s1[40:110, m + 64]).all()
-    dev, pitch, stride = _frames(imgs)
+    dev, pitch, stride = device_frames(imgs)
     got = _map_g(ctx, dev, pitch, stride, w, h, len(imgs), win).cpu().numpy()
     for i in range(len(imgs)):
-        assert_same_bits(got[i], crl.score(imgs[i], win), f"image {i} map")
+        assert_same_bits(got[i], cro.score(imgs[i], win), f"image {i} map")
     for md in (0.0, 2.5, 4.9, 5.0, f32_next(5, 6), 6.9, 7.0, f32_next(7, 8)):
-        _assert_detect(crl, imgs, _detect_g(ctx, dev, pitch, stride, w, h, len(imgs), win, 3000, ql=0.0, md=md), win, 3000,
+        _assert_detect(cro, imgs, _detect_g(ctx, dev, pitch, stride, w, h, len(imgs), win, 3000, ql=0.0, md=md), win, 3000,
                        ql=0.0, md=md)
 
 
@@ -584,23 +560,23 @@ def bright_frame(w, h, seed):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("win", [3, 9])
-def test_threshold(ctx, crl, win):
+def test_threshold(ctx, cro, win):
     w, h = 120, 90
     m = win // 2 + 1
     img = bright_frame(w, h, win)
-    smap = crl.score(img, win)
+    smap = cro.score(img, win)
     inter = smap[m:h - m, m:w - m]
     assert smap.max() > 4 * inter.max() > 0  # over the whole frame, quality_level 0.5 would leave nothing
-    dev, pitch, stride = _frames(img[None])
-    n = _assert_detect(crl, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=0.5, md=0.0), win, 5000,
+    dev, pitch, stride = device_frames(img[None])
+    n = _assert_detect(cro, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=0.5, md=0.0), win, 5000,
                        ql=0.5, md=0.0)[0]
     assert n > 0
     # min_score at a candidate's exact score (excluded) and one ulp below (included)
-    _, rs, rn = crl.detect(img, win, 5000, quality_level=0.0, min_distance=0.0)
+    _, rs, rn = cro.detect(img, win, 5000, quality_level=0.0, min_distance=0.0)
     s = F32(rs[rn // 3])
     counts = []
     for ms in (float(s), f32_next(s, 0)):
-        counts.append(_assert_detect(crl, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=0.0, md=0.0,
+        counts.append(_assert_detect(cro, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=0.0, md=0.0,
                                                                ms=ms), win, 5000, ql=0.0, md=0.0, ms=ms)[0])
     assert counts[1] > counts[0]
     # quality_level * max equal to a candidate's score
@@ -615,7 +591,7 @@ def test_threshold(ctx, crl, win):
         if hit is not None:
             break
     assert hit is not None
-    n_eq = _assert_detect(crl, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=hit, md=0.0), win, 5000,
+    n_eq = _assert_detect(cro, img[None], _detect_g(ctx, dev, pitch, stride, w, h, 1, win, 5000, ql=hit, md=0.0), win, 5000,
                           ql=hit, md=0.0)[0]
     assert 0 < n_eq < rn
 
@@ -623,25 +599,25 @@ def test_threshold(ctx, crl, win):
 # ==================================================================================== 7. caller buffers and streams
 @pytest.mark.gpu
 @pytest.mark.parametrize("mc", [1, 7, 513])
-def test_caller_buffers(ctx, crl, mc):
+def test_caller_buffers(ctx, cro, mc):
     """Guarded outputs with odd max_corners (per-image slices at 8- but not 16-byte offsets), scores NULL, pitch = w with
     odd w, an odd image stride that is not a multiple of the pitch, and stride 0 with one image."""
     w, h, win = 67, 45, 5
     imgs = np.stack([content(k, w, h, i) for i, k in enumerate(["natural", "noise", "textured"])])
     for pitch, stride in ((w, w * h), (w, w * h + 13), (80, 80 * h + 7)):
-        dev, pitch, stride = _frames(imgs, pitch, stride, pad=0xFF)
+        dev, pitch, stride = device_frames(imgs, pitch, stride, 0xFF)
         assert_same_bits(_map_g(ctx, dev, pitch, stride, w, h, 3, win).cpu().numpy(),
-                         np.stack([crl.score(i, win) for i in imgs]), f"map, pitch {pitch} stride {stride}")
+                         np.stack([cro.score(i, win) for i in imgs]), f"map, pitch {pitch} stride {stride}")
         for sc in (True, False):
-            _assert_detect(crl, imgs, _detect_g(ctx, dev, pitch, stride, w, h, 3, win, mc, ql=0.0, md=3.0, with_scores=sc),
+            _assert_detect(cro, imgs, _detect_g(ctx, dev, pitch, stride, w, h, 3, win, mc, ql=0.0, md=3.0, with_scores=sc),
                            win, mc, ql=0.0, md=3.0)
-    dev, pitch, _ = _frames(imgs[:1], w)
-    assert_same_bits(_map_g(ctx, dev, pitch, 0, w, h, 1, win).cpu().numpy()[0], crl.score(imgs[0], win), "stride 0")
-    _assert_detect(crl, imgs[:1], _detect_g(ctx, dev, pitch, 0, w, h, 1, win, mc, ql=0.0, md=3.0), win, mc, ql=0.0, md=3.0)
+    dev, pitch, _ = device_frames(imgs[:1], w)
+    assert_same_bits(_map_g(ctx, dev, pitch, 0, w, h, 1, win).cpu().numpy()[0], cro.score(imgs[0], win), "stride 0")
+    _assert_detect(cro, imgs[:1], _detect_g(ctx, dev, pitch, 0, w, h, 1, win, mc, ql=0.0, md=3.0), win, mc, ql=0.0, md=3.0)
 
 
 @pytest.mark.gpu
-def test_stream_with_work_queued_ahead(ctx, crl):
+def test_stream_with_work_queued_ahead(ctx, cro):
     """The frames are written on a side stream behind a long spin kernel; detection on that stream must see them."""
     import torch
 
@@ -656,9 +632,9 @@ def test_stream_with_work_queued_ahead(ctx, crl):
         dev.copy_(src)
         got = _detect_g(ctx, dev, w, w * h, w, h, n, win, mc, ql=0.0, md=4.0, stream=side.cuda_stream)
         smap = _map_g(ctx, dev, w, w * h, w, h, n, win, stream=side.cuda_stream).cpu().numpy()
-    _assert_detect(crl, imgs, got, win, mc, ql=0.0, md=4.0)
+    _assert_detect(cro, imgs, got, win, mc, ql=0.0, md=4.0)
     for i in range(n):
-        assert_same_bits(smap[i], crl.score(imgs[i], win), f"image {i} map")
+        assert_same_bits(smap[i], cro.score(imgs[i], win), f"image {i} map")
 
 
 @pytest.mark.gpu
@@ -729,7 +705,7 @@ def reuse_sequence():
     return seq
 
 
-def _run_call(ctx, crl, oracle, call):
+def _run_call(ctx, cro, oracle, call):
     import torch
 
     w, h, n, win = call["w"], call["h"], call["n"], call["win"]
@@ -747,19 +723,19 @@ def _run_call(ctx, crl, oracle, call):
         torch.cuda.synchronize()
         return [flow.cpu().numpy(), st.cpu().numpy()]
     imgs = np.stack([content(("natural", "noise")[i % 2], w, h, call["seed"] * 10 + i) for i in range(n)])
-    dev, pitch, stride = _frames(imgs)
+    dev, pitch, stride = device_frames(imgs)
     if call["op"] == "map":
         got = _map_g(ctx, dev, pitch, stride, w, h, n, win).cpu().numpy()
         for i in range(n):
-            assert_same_bits(got[i], crl.score(imgs[i], win), f"{call} map {i}")
+            assert_same_bits(got[i], cro.score(imgs[i], win), f"{call} map {i}")
         return [got]
     got = _detect_g(ctx, dev, pitch, stride, w, h, n, win, call["mc"], ql=call["ql"], md=call["md"])
-    _assert_detect(crl, imgs, got, win, call["mc"], ql=call["ql"], md=call["md"])
+    _assert_detect(cro, imgs, got, win, call["mc"], ql=call["ql"], md=call["md"])
     return list(got)
 
 
 @pytest.mark.gpu
-def test_workspace_reuse(crl, oracle):
+def test_workspace_reuse(cro, oracle):
     """One fresh context runs the sequence; every result equals the restatement and the same call on a fresh context."""
     import torch
 
@@ -771,11 +747,11 @@ def test_workspace_reuse(crl, oracle):
     assert {c["op"] for c in seq} == {"map", "detect", "track", "reserve"}
     with Context(0) as a:
         for call in seq:
-            got = _run_call(a, crl, oracle, call)
+            got = _run_call(a, cro, oracle, call)
             if got is None:
                 continue
             with Context(0) as b:
-                ref = _run_call(b, crl, oracle, call)
+                ref = _run_call(b, cro, oracle, call)
             for g, r in zip(got, ref):
                 assert np.array_equal(np.asarray(g).view(np.uint8), np.asarray(r).view(np.uint8)), call
 

@@ -11,102 +11,17 @@ LOW_TEXTURE decision (tests/track_oracle.c).
 GPU tests: the kernels against the restatement over windows, sizes, layouts, batches, content and parameters; CUDA graph
 capture of detection followed by tracking; detect-then-track end to end; argument refusals; the profile record.
 """
-import ctypes as C
 import decimal
 import math
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-F32 = np.float32
-S815 = 8 / 15  # px per flow unit of the reference's masks (Sobel gain 8, Dt gain 15)
+from cuda_optical_flow_2_b200 import align_up
+from support import (F32, PT_LOW_TEXTURE, PT_OUTSIDE, PT_TRACKED, S815, assert_same_bits, content, cro, device_frames,  # noqa: F401
+                     exact_sums, plain_greedy, tro)
+
 WINS = list(range(3, 20, 2))
-PT_TRACKED, PT_LOW_TEXTURE, PT_OUTSIDE = 0, 2, 3
-
-
-class CornerOracle:
-    """tests/corner_oracle.c through ctypes."""
-
-    def __init__(self, so_path):
-        self._lib = C.CDLL(so_path)
-        self._lib.orc_min_eig_map.restype = None
-        self._lib.orc_min_eig_map.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_void_p]
-        self._lib.orc_detect_corners.restype = C.c_int
-        self._lib.orc_detect_corners.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float,
-                                                 C.c_void_p, C.c_void_p]
-
-    def score(self, img, win):
-        img = np.ascontiguousarray(img, np.uint8)
-        h, w = img.shape
-        out = np.empty((h, w), F32)
-        self._lib.orc_min_eig_map(img.ctypes.data, w, w, h, win, out.ctypes.data)
-        return out
-
-    def select(self, score, win, max_corners, quality_level=0.01, min_distance=10.0, min_score=0.0):
-        score = np.ascontiguousarray(score, F32)
-        h, w = score.shape
-        corners = np.empty((max_corners, 2), F32)
-        scores = np.empty(max_corners, F32)
-        n = self._lib.orc_detect_corners(score.ctypes.data, w, h, win, max_corners, quality_level, min_distance, min_score,
-                                         corners.ctypes.data, scores.ctypes.data)
-        return corners, scores, n
-
-    def detect(self, img, win, max_corners, **kw):
-        return self.select(self.score(img, win), win, max_corners, **kw)
-
-
-@pytest.fixture(scope="session")
-def cro(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("corner_oracle") / "libcorneroracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "corner_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return CornerOracle(so)
-
-
-# ------------------------------------------------------------------------------------ content
-def content(kind, w, h, seed=0):
-    rng = np.random.default_rng(seed)
-    yy, xx = np.mgrid[0:h, 0:w]
-    if kind == "zeros":
-        return np.zeros((h, w), np.uint8)
-    if kind == "full":
-        return np.full((h, w), 255, np.uint8)
-    if kind == "checker":
-        return (((xx + yy) & 1) * 255).astype(np.uint8)
-    if kind == "stripes":  # vertical period-4 stripes: gy = 0 everywhere, det = 0
-        return (((xx >> 1) & 1) * 255).astype(np.uint8)
-    if kind == "noise":
-        return rng.integers(0, 256, (h, w), dtype=np.uint8)
-    if kind == "isotropic":  # a radial pattern: near-isotropic windows (disc close to 0)
-        r = np.hypot(xx - w / 2 + 0.3, yy - h / 2 + 0.7)
-        return (127.5 + 127.5 * np.cos(r * 0.9)).astype(np.uint8)
-    if kind == "textured":
-        from oracle import oracle as O
-
-        return O.make_frame(w, h, 0.0, 0.0, 4, 1000 + seed)
-    if kind == "natural":  # smooth blobs plus a little noise
-        f = np.zeros((h, w))
-        for _ in range(12):
-            cx, cy, s, a = rng.uniform(0, w), rng.uniform(0, h), rng.uniform(2, 9), rng.uniform(-90, 90)
-            f += a * np.exp(-((xx - cx) ** 2 + (yy - cy) ** 2) / (2 * s * s))
-        return np.clip(128 + f + rng.normal(0, 3, (h, w)), 0, 255).astype(np.uint8)
-    raise ValueError(kind)
-
-
-def exact_sums(img, win):
-    """A, D, B by scipy correlations in int64 (zero mode): Sobel fields, then the window sums."""
-    from scipy.ndimage import correlate
-
-    i = img.astype(np.int64)
-    dx = np.array([[-1, 0, 1], [-2, 0, 2], [-1, 0, 1]], np.int64)
-    gx = correlate(i, dx, mode="constant", cval=0)
-    gy = correlate(i, dx.T, mode="constant", cval=0)
-    box = np.ones((win, win), np.int64)
-    return (correlate(gx * gx, box, mode="constant", cval=0), correlate(gy * gy, box, mode="constant", cval=0),
-            correlate(gx * gy, box, mode="constant", cval=0))
 
 
 # ------------------------------------------------------------------------------------ CPU: score vs exact arithmetic
@@ -139,42 +54,6 @@ def test_score_is_l1_over_win2_within_one_ulp(cro, win, kind):
 
 
 # ------------------------------------------------------------------------------------ CPU: selection vs a plain greedy
-def plain_greedy(score, win, max_corners, quality_level, min_distance, min_score):
-    """The rule of include/ofb200.h, written the slow, obvious way."""
-    h, w = score.shape
-    m = win // 2 + 1
-    if w < 2 * m + 1 or h < 2 * m + 1:
-        return []
-    inter = score[m:h - m, m:w - m]
-    thr = max(F32(quality_level) * F32(inter.max()), F32(min_score))
-    cands = []
-    for y in range(m, h - m):
-        for x in range(m, w - m):
-            s = score[y, x]
-            if not s > thr:
-                continue
-            ok = True
-            for dy in (-1, 0, 1):
-                for dx in (-1, 0, 1):
-                    nx, ny = x + dx, y + dy
-                    if (dx, dy) == (0, 0) or not (m <= nx <= w - 1 - m and m <= ny <= h - 1 - m):
-                        continue
-                    t = score[ny, nx]
-                    if not (s > t or (s == t and y * w + x < ny * w + nx)):
-                        ok = False
-            if ok:
-                cands.append((-float(s), y * w + x, x, y, s))
-    cands.sort()
-    md2 = float(min_distance) * float(min_distance)
-    acc = []
-    for _, _, x, y, s in cands:
-        if len(acc) == max_corners:
-            break
-        if all(float((x - ax) ** 2 + (y - ay) ** 2) >= md2 for ax, ay, _ in acc):
-            acc.append((x, y, s))
-    return acc
-
-
 def assert_selection(got, acc, max_corners):
     corners, scores, n = got
     assert n == len(acc)
@@ -261,17 +140,6 @@ def test_rectangle_corners_are_found_and_nothing_else(cro, win, tol):
 
 
 # ------------------------------------------------------------------------------------ CPU: the tie to the tracker
-@pytest.fixture(scope="session")
-def tro(oracle, tmp_path_factory):
-    from test_track_points import TrackOracle
-
-    so = str(tmp_path_factory.mktemp("track_oracle_c") / "libtrackoracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "track_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return TrackOracle(so, oracle)
-
-
 @pytest.mark.parametrize("win", [3, 9, 19])
 def test_score_is_the_trackers_low_texture_threshold(cro, tro, oracle, win):
     """levels = 1, iters = 1, integer points at every interior pixel with score > 0: min_eig = score * (1 - 1e-5) never
@@ -308,51 +176,30 @@ def test_null_context_is_rejected():
 
 
 # ------------------------------------------------------------------------------------ GPU
-def _to_device(imgs, pitch=None, stride_rows=None, pad=0):
-    """(n, h, w) uint8 -> a (n, stride_rows, pitch) CUDA tensor holding them, `pad` in every byte around."""
-    import torch
-
-    n, h, w = imgs.shape
-    pitch = pitch or (w + 15) // 16 * 16
-    stride_rows = stride_rows or h
-    buf = np.full((n, stride_rows, pitch), pad, np.uint8)
-    buf[:, :h, :w] = imgs
-    return torch.from_numpy(buf).cuda()
-
-
-def _map(ctx, dev, w, h, win):
+def _map(ctx, frames, imgs, win):
     import torch
 
     from cuda_optical_flow_2_b200 import _lib
 
-    n, rows, pitch = dev.shape
+    (dev, pitch, stride), (n, h, w) = frames, imgs.shape
     out = torch.empty((n, h, w), dtype=torch.float32, device=dev.device)
-    _lib.check(_lib.load().ofb_min_eig_map_device(ctx._h, dev.data_ptr(), pitch, pitch * rows, w, h, n, win, out.data_ptr(), None))
+    _lib.check(_lib.load().ofb_min_eig_map_device(ctx._h, dev.data_ptr(), pitch, stride, w, h, n, win, out.data_ptr(), None))
     return out.cpu().numpy()
 
 
-def _detect(ctx, dev, w, h, win, max_corners, quality_level=0.01, min_distance=10.0, min_score=0.0):
+def _detect(ctx, frames, imgs, win, max_corners, quality_level=0.01, min_distance=10.0, min_score=0.0):
     import torch
 
     from cuda_optical_flow_2_b200 import _lib
 
-    n, rows, pitch = dev.shape
+    (dev, pitch, stride), (n, h, w) = frames, imgs.shape
     corners = torch.empty((n, max_corners, 2), dtype=torch.float32, device=dev.device)
     scores = torch.empty((n, max_corners), dtype=torch.float32, device=dev.device)
     counts = torch.empty((n,), dtype=torch.int32, device=dev.device)
-    _lib.check(_lib.load().ofb_detect_corners_device(ctx._h, dev.data_ptr(), pitch, pitch * rows, w, h, n, win, max_corners,
+    _lib.check(_lib.load().ofb_detect_corners_device(ctx._h, dev.data_ptr(), pitch, stride, w, h, n, win, max_corners,
                                                      quality_level, min_distance, min_score, corners.data_ptr(),
                                                      scores.data_ptr(), counts.data_ptr(), None))
     return corners.cpu().numpy(), scores.cpu().numpy(), counts.cpu().numpy()
-
-
-def assert_same_bits(got, ref, what=""):
-    got, ref = np.asarray(got, F32), np.asarray(ref, F32)
-    assert got.shape == ref.shape, what
-    ng, nr = np.isnan(got), np.isnan(ref)
-    assert np.array_equal(ng, nr), f"{what}: NaN positions differ"
-    bad = got.view(np.uint32)[~ng] != ref.view(np.uint32)[~nr]
-    assert not bad.any(), f"{what}: {bad.sum()} values differ, first {np.argwhere(bad)[:3].tolist()}"
 
 
 def _check_detect(cro, imgs, got, win, max_corners, **kw):
@@ -374,13 +221,13 @@ def test_kernel_equals_restatement_windows_and_content(ctx, cro, win):
     around every image."""
     w, h = 67, 45
     imgs = np.stack([content(k, w, h, i) for i, k in enumerate(KINDS)])
-    dev = _to_device(imgs, pitch=96, stride_rows=h + 3, pad=0xFF)
-    got = _map(ctx, dev, w, h, win)
+    dev = device_frames(imgs, 96, 96 * (h + 3), 0xFF)
+    got = _map(ctx, dev, imgs, win)
     for i in range(len(imgs)):
         assert_same_bits(got[i], cro.score(imgs[i], win), f"{KINDS[i]} map")
     for kw in (dict(quality_level=0.01, min_distance=10.0), dict(quality_level=0.0, min_distance=0.0),
                dict(quality_level=0.0, min_distance=1.5)):
-        _check_detect(cro, imgs, _detect(ctx, dev, w, h, win, 300, **kw), win, 300, **kw)
+        _check_detect(cro, imgs, _detect(ctx, dev, imgs, win, 300, **kw), win, 300, **kw)
 
 
 @pytest.mark.gpu
@@ -389,11 +236,11 @@ def test_kernel_equals_restatement_sizes(ctx, cro, w, h):
     """Sizes around the 32 x 32 tile and the interior limit 2m+1, windows 3 and 9 (the large one at window 3 only)."""
     for win in ([3, 9] if w * h < 100_000 else [3]):
         imgs = np.stack([content("natural", w, h, 3), content("noise", w, h, 4)])
-        dev = _to_device(imgs)
-        got = _map(ctx, dev, w, h, win)
+        dev = device_frames(imgs, align_up(w, 16))
+        got = _map(ctx, dev, imgs, win)
         for i in range(2):
             assert_same_bits(got[i], cro.score(imgs[i], win), f"{w}x{h} win {win} map")
-        _check_detect(cro, imgs, _detect(ctx, dev, w, h, win, 500, quality_level=0.0, min_distance=3.0), win, 500,
+        _check_detect(cro, imgs, _detect(ctx, dev, imgs, win, 500, quality_level=0.0, min_distance=3.0), win, 500,
                       quality_level=0.0, min_distance=3.0)
 
 
@@ -401,10 +248,10 @@ def test_kernel_equals_restatement_sizes(ctx, cro, w, h):
 def test_kernel_equals_restatement_4k(ctx, cro):
     w, h, win = 3840, 2160, 3
     img = content("textured", w, h, 7)[None]
-    dev = _to_device(img)
-    assert_same_bits(_map(ctx, dev, w, h, win)[0], cro.score(img[0], win), "4K map")
+    dev = device_frames(img, align_up(w, 16))
+    assert_same_bits(_map(ctx, dev, img, win)[0], cro.score(img[0], win), "4K map")
     for kw in (dict(quality_level=0.01, min_distance=10.0), dict(quality_level=0.0, min_distance=0.0)):
-        _check_detect(cro, img, _detect(ctx, dev, w, h, win, 16384, **kw), win, 16384, **kw)
+        _check_detect(cro, img, _detect(ctx, dev, img, win, 16384, **kw), win, 16384, **kw)
 
 
 @pytest.mark.gpu
@@ -413,10 +260,10 @@ def test_kernel_equals_restatement_batches(ctx, cro, n):
     w, h, win = 24, 19, 5
     base = np.stack([content(k, w, h, i) for i, k in enumerate(KINDS)])
     imgs = np.stack([np.roll(base[i % len(base)], i // len(base), 1) for i in range(n)])
-    dev = _to_device(imgs)
+    dev = device_frames(imgs, align_up(w, 16))
     check = sorted(set([0, n // 2, n - 1] + list(range(min(n, 16)))))
-    got_map = _map(ctx, dev, w, h, win)
-    got = _detect(ctx, dev, w, h, win, 40, quality_level=0.0, min_distance=2.0)
+    got_map = _map(ctx, dev, imgs, win)
+    got = _detect(ctx, dev, imgs, win, 40, quality_level=0.0, min_distance=2.0)
     for i in check:
         assert_same_bits(got_map[i], cro.score(imgs[i], win), f"image {i} map")
     _check_detect(cro, imgs[check], tuple(g[check] for g in got), win, 40, quality_level=0.0, min_distance=2.0)
@@ -431,8 +278,8 @@ def test_kernel_equals_restatement_parameters(ctx, cro, case):
     w, h = 90, 70
     imgs = np.stack([content("checker", w, h), content("natural", w, h, 1), content("textured", w, h, 2),
                      content("noise", w, h, 3)])
-    dev = _to_device(imgs)
-    _check_detect(cro, imgs, _detect(ctx, dev, w, h, 3, mc, **kw), 3, mc, **kw)
+    dev = device_frames(imgs, align_up(w, 16))
+    _check_detect(cro, imgs, _detect(ctx, dev, imgs, 3, mc, **kw), 3, mc, **kw)
 
 
 @pytest.mark.gpu
@@ -444,8 +291,8 @@ def test_conflict_chains(ctx, cro):
     w, h, win = 1200, 12, 3
     img = np.zeros((h, w), np.uint8)
     img[6, 4:w - 4:2] = 255  # isolated bright pixels along a row
-    dev = _to_device(img[None])
-    got = _detect(ctx, dev, w, h, win, 4000, quality_level=0.0, min_distance=2.5)
+    dev = device_frames(img[None], align_up(w, 16))
+    got = _detect(ctx, dev, img[None], win, 4000, quality_level=0.0, min_distance=2.5)
     _check_detect(cro, img[None], got, win, 4000, quality_level=0.0, min_distance=2.5)
     torch.cuda.synchronize()
 

@@ -19,7 +19,7 @@ import functools
 import numpy as np
 import pytest
 
-from test_gpu_parity import assert_flow_identical, assert_flow_within_tolerance
+from support import assert_flow_within_tolerance, assert_values_equal, c_for, noise_pair, oracle_warp, solve, u_of
 
 FLOW_SCALES = [1.0, 8.0 / 15.0, 3.0]
 WINDOWS = [3, 9, 11, 19]
@@ -29,33 +29,6 @@ BELOW_32768 = np.nextafter(np.float32(32768), np.float32(0))
 
 
 # ------------------------------------------------------------------------------------ helpers
-def _f32(x):
-    return np.asarray(x, np.float32)
-
-
-def u_of(c, s):
-    """The displacement in px the oracle takes from a coarser vector component c at flow_scale s: (2 c) s in float32."""
-    with np.errstate(over="ignore", invalid="ignore"):
-        return (np.float32(2) * _f32(c)) * np.float32(s)
-
-
-def c_for(u_target, s):
-    """A float32 coarser component whose displacement u_of(c, s) is exactly u_target where one exists within a few ulps
-    of u_target / 2s, else the nearest float32 to u_target / 2s."""
-    u_target = _f32(u_target)
-    c0 = _f32(u_target.astype(np.float64) / (2.0 * float(np.float32(s))))
-    best = c0.copy()
-    hit = u_of(c0, s) == u_target
-    lo, hi = c0.copy(), c0.copy()
-    for _ in range(6):
-        lo, hi = np.nextafter(lo, np.float32(-np.inf)), np.nextafter(hi, np.float32(np.inf))
-        for cand in (lo, hi):
-            take = ~hit & (u_of(cand, s) == u_target)
-            best = np.where(take, cand, best)
-            hit |= take
-    return best
-
-
 def _coarse_index(w, h):
     """Per pixel of a level, the coarser pixel its vector comes from (indices clamped for odd sizes)."""
     cw, ch = w >> 1, h >> 1
@@ -294,19 +267,6 @@ def make_field(name, w, h, s, seed=0):
     return _field(name, w, h, float(s), seed).copy()
 
 
-def noise_pair(w, h, seed):
-    """Uniform-noise frames: every byte of the warped frame enters some window sum with a nonzero weight."""
-    rng = np.random.default_rng(seed)
-    prev = rng.integers(0, 256, (h, w), dtype=np.uint8)
-    nxt = np.ascontiguousarray(np.roll(prev, (1, -2), (0, 1)) ^ rng.integers(0, 16, (h, w), dtype=np.uint8))
-    return prev, nxt
-
-
-def oracle_warp(oracle, nxt, cum, mode, s):
-    h, w = nxt.shape
-    return oracle.warp(nxt, w, h, 0, 2, [np.zeros((h, w, 2), np.float32), cum], mode, np.float32(s))
-
-
 def expected_cum_out(cum, flow):
     h, w = flow.shape[:2]
     ti, tj = _coarse_index(w, h)
@@ -435,16 +395,11 @@ def test_probe_example_from_the_rule():
 
 
 # ------------------------------------------------------------------------------------ GPU: one warped level
-def _torch():
-    import torch
-
-    return torch
-
-
 def _run_level(ctx, oracle, fields, w, h, win, mode, s, want_cum, seed=0):
     """One warped level on a batch of pairs (one crafted field each) through lk_level_device; returns the device
     outputs and the oracle's (warped next -> lk_level) per pair."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     prevs, nexts, cums = [], [], []
@@ -485,9 +440,9 @@ def test_warped_level_on_crafted_flow(ctx, oracle, name, mode, s):
         flow, cum_out, refs, cums = _run_level(ctx, oracle, fields, w, h, win, mode, s, want_cum, seed=idx)
         for p in range(len(fields)):
             what = f"{fields[p]} (pair {p}) {w}x{h} win {win} mode {mode} s {s:.4f}"
-            assert_flow_identical(flow[p], refs[p], what)
+            assert_values_equal(flow[p], refs[p], what)
             if want_cum:
-                assert_flow_identical(cum_out[p], expected_cum_out(cums[p], refs[p]), what + " cum_out")
+                assert_values_equal(cum_out[p], expected_cum_out(cums[p], refs[p]), what + " cum_out")
 
 
 @pytest.mark.gpu
@@ -495,11 +450,10 @@ def test_warped_level_on_crafted_flow(ctx, oracle, name, mode, s):
 def test_warped_level_on_crafted_flow_fast_solve(ctx, oracle, name):
     """The same fields once through the tolerance-mode kernels (separate instantiations of the same gather): within the
     stated bar of the oracle on the oracle's warped frame, non-finite values on the same pixels."""
-    from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST
+    from cuda_optical_flow_2_b200 import SOLVE_FAST
 
     idx = sorted(FIELDS).index(name)
-    ctx.solve = SOLVE_FAST
-    try:
+    with solve(ctx, SOLVE_FAST):
         for mode in (0, 1, 2):
             for k, (w, h) in enumerate(SHAPES[1:3]):
                 win = WINDOWS[(idx + mode + 2 * k) % len(WINDOWS)]
@@ -511,8 +465,6 @@ def test_warped_level_on_crafted_flow_fast_solve(ctx, oracle, name):
                     assert_flow_within_tolerance(flow[p], refs[p], what)
                     if k == 1:
                         assert_flow_within_tolerance(cum_out[p], expected_cum_out(cums[p], refs[p]), what + " cum_out", ulps=False)
-    finally:
-        ctx.solve = SOLVE_EXACT
 
 
 @pytest.mark.gpu
@@ -520,7 +472,8 @@ def test_warped_level_on_crafted_flow_fast_solve(ctx, oracle, name):
 def test_as_written_one_vector_per_pair(ctx, oracle, s):
     """Warp as written: the coarser vector at (0, 0) moves the whole frame.  A batch in which every pair has a different
     special value there -- the single vector is per pair."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     vals = special_values(s) + [(np.float32(c_for(-0.5, s)), np.float32(c_for(-0.25, s))),
@@ -541,8 +494,8 @@ def test_as_written_one_vector_per_pair(ctx, oracle, s):
         flow, cum_out = flow.cpu().numpy(), cum_out.cpu().numpy()
         for k in range(len(vals)):
             ref = oracle.lk_level(prevs[k], oracle_warp(oracle, nexts[k], cums[k], 0, s), win, oracle.SUMS_EXACT)
-            assert_flow_identical(flow[k], ref, f"pair {k} value {vals[k]} {w}x{h}")
-            assert_flow_identical(cum_out[k], expected_cum_out(cums[k], ref), f"pair {k} cum_out")
+            assert_values_equal(flow[k], ref, f"pair {k} value {vals[k]} {w}x{h}")
+            assert_values_equal(cum_out[k], expected_cum_out(cums[k], ref), f"pair {k} cum_out")
 
 
 # ------------------------------------------------------------------------------------ GPU: the drop-in entry point
@@ -577,7 +530,7 @@ def test_drop_in_entry_on_crafted_residual_pyramid(ctx, oracle, mode, at_origin)
         warped = oracle.warp(nxt, w, h, 0, levels, flows, mode, np.float32(s))
         if mode == 2 and not at_origin:
             assert (warp_model_pyr_nan_mix(flows, w, h, s)).any(), "no one-NaN-component target"
-        assert_flow_identical(got[0], oracle.lk_level(prev, warped, win, oracle.SUMS_EXACT), f"mode {mode} s {s:.4f}")
+        assert_values_equal(got[0], oracle.lk_level(prev, warped, win, oracle.SUMS_EXACT), f"mode {mode} s {s:.4f}")
         for k in (1, 2):
             assert np.array_equal(got[k].view(np.uint32), flows[k].view(np.uint32)), "coarser levels must stay untouched"
 
@@ -612,7 +565,8 @@ def _tiled(imgs, n):
 def _check_copies(t, n, what, chunk=8192):
     """Every pair of the (n, ...) tensor equals its prototype bit for bit, on the device; returns the prototypes taken from
     the last PERIOD pairs (the batch's tail) as numpy, in prototype order."""
-    torch = _torch()
+    import torch
+
     v = t.view(n, -1).view(torch.int32)
     last = torch.arange(n - PERIOD, n, device=t.device)
     proto = torch.empty((PERIOD, v.shape[1]), dtype=torch.int32, device=t.device)
@@ -628,7 +582,8 @@ def _check_copies(t, n, what, chunk=8192):
 
 
 def _free():
-    torch = _torch()
+    import torch
+
     torch.cuda.synchronize()
     torch.cuda.empty_cache()
 
@@ -648,7 +603,7 @@ def test_flow_pairs_device_around_the_per_frame_pyramid_split(ctx, oracle, n, le
             got = _check_copies(flows[k], n, f"n {n} level {k}")
             for i in range(PERIOD):
                 ref = oracle.flow_pair(prevs[i], nexts[i], levels, win, 2, oracle.SUMS_EXACT)
-                assert_flow_identical(got[i], ref[k], f"n {n} prototype {i} level {k}")
+                assert_values_equal(got[i], ref[k], f"n {n} prototype {i} level {k}")
     finally:
         del dp, dn
         flows = None
@@ -661,7 +616,8 @@ def test_tail_split_at_the_grid_limit(ctx, oracle, monkeypatch, n, w, h):
     """One column strip, at least 128 rows: the level-0 kernel cuts the batch's last wave of pairs into 4 row blocks
     each (csrc/lk_win.cu), and its grid z (pairs plus 3 per tail pair) must stay within 65535.  Every copy equals its
     prototype, the prototypes equal the oracle, and the result equals the launch with the tail switched off."""
-    torch = _torch()
+    import torch
+
     levels, win = 2, 9
     prevs, nexts = _prototypes(oracle, w, h)
     dp, dn = _tiled(prevs, n), _tiled(nexts, n)
@@ -671,7 +627,7 @@ def test_tail_split_at_the_grid_limit(ctx, oracle, monkeypatch, n, w, h):
             got = _check_copies(flows[k], n, f"level {k}")
             for i in range(PERIOD):
                 ref = oracle.flow_pair(prevs[i], nexts[i], levels, win, 2, oracle.SUMS_EXACT)
-                assert_flow_identical(got[i], ref[k], f"prototype {i} level {k}")
+                assert_values_equal(got[i], ref[k], f"prototype {i} level {k}")
         monkeypatch.setenv("OFB_LK_TAIL", "0")
         plain = ctx.flow_pairs_device(dp, dn, w, levels, win)
         torch.cuda.synchronize()
@@ -687,7 +643,8 @@ def test_tail_split_at_the_grid_limit(ctx, oracle, monkeypatch, n, w, h):
 def test_fb_entry_at_the_grid_limit(ctx, oracle):
     """flow_pairs_fb_device at 65535 pairs: the totals equal two flow_pairs_device calls bit for bit, the status equals
     fb_check_device on those totals, and the forward prototypes equal the oracle."""
-    torch = _torch()
+    import torch
+
     n, w, h, levels, win = 65535, 24, 128, 2, 9
     prevs, nexts = _prototypes(oracle, w, h)
     dp, dn = _tiled(prevs, n), _tiled(nexts, n)
@@ -706,7 +663,7 @@ def test_fb_entry_at_the_grid_limit(ctx, oracle):
         got = _check_copies(fwd, n, "forward total")
         for i in range(PERIOD):
             _, cums = oracle.flow_pair(prevs[i], nexts[i], levels, win, 2, oracle.SUMS_EXACT, 1.0, want_cum=True)
-            assert_flow_identical(got[i], cums[0], f"prototype {i} forward total")
+            assert_values_equal(got[i], cums[0], f"prototype {i} forward total")
     finally:
         del dp, dn
         fwd = bwd = status = None
@@ -715,7 +672,8 @@ def test_fb_entry_at_the_grid_limit(ctx, oracle):
 
 @pytest.mark.gpu
 def test_65536_pairs_are_rejected(ctx):
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import OfbError
 
     n, w, h = 65536, 16, 16

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-BIL, NEAR = 2, 1  # OFB_WARP_BILINEAR, _NEAREST
+from support import BIL, NEAR, reach_flag, requested_rows
 
 
 def test_shard_range_partitions_the_batch():
@@ -152,12 +152,11 @@ def test_native_strip_reach_overflow_is_reported(ctx, oracle):
     rank of this 320x480 pair (3 levels, window 9, 4 ranks) holds its own rows plus 39 above and 36 below at level 0, 19
     and 18 at level 1: the halo and the rows the coarser levels' halo rows are rebuilt from.  On these frames the flow of
     the coarsest level, which the strips compute exactly, makes rank 1's level-1 warp ask for rows past those (the rule of
-    test_row_split.requested_rows), so its flag is certain.  With the default reach=16 no rank asks for a row it does not
+    support.requested_rows), so its flag is certain.  With the default reach=16 no rank asks for a row it does not
     hold, and the strips equal the whole frame bit for bit."""
     import ctypes as C
 
     import torch
-    from test_row_split import reach_flag, requested_rows
 
     from cuda_optical_flow_2_b200 import _lib, planar_to_device
     from cuda_optical_flow_2_b200.dist import NativeStrips

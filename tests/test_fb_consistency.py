@@ -2,8 +2,8 @@
 
 The check's arithmetic is pinned (include/ofb200.h): every multiply and add rounded on its own, no fma, the displacement
 rounded to 1/256 px as the bilinear warp does.  So three implementations must agree bit for bit: the CUDA kernel
-(csrc/fb_check.cu), the C restatement in tests/fb_oracle.c (compiled here into a temporary directory) and the numpy
-float32 restatement below.  The flow both directions are checked on comes from the pinned oracle's oracle.flow_pair.
+(csrc/fb_check.cu), the C restatement in tests/fb_oracle.c (compiled into a temporary directory) and the numpy
+float32 restatement support.np_fb_check.  The flow both directions are checked on comes from the pinned oracle's oracle.flow_pair.
 
 CPU tests (no mark): the oracle against numpy on inputs that reach every branch, the check's semantics on the oracle's
 flow (the GPU path is pinned to the oracle, so the thresholds are set here), and the ABI's NULL-context checks.
@@ -11,116 +11,12 @@ GPU tests: the kernel and the two-direction entry point against the oracle, the 
 ofb_flow_pairs_device calls, symmetry, adversarial content, CUDA graph replay and argument checks.
 """
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-FB_CONSISTENT, FB_INCONSISTENT, FB_OUTSIDE, FB_FWD_NONFINITE, FB_BWD_NONFINITE = 0, 1, 2, 3, 4
-F32 = np.float32
-S815 = 8 / 15  # a flow_scale whose products are not exact
-
-
-# ------------------------------------------------------------------------------------ numpy restatement
-def np_fb_check(fwd, bwd, s, alpha=0.01, beta=0.5):
-    """The header's rule on one (h, w, 2) pair, float32 throughout (numpy rounds every operation on its own)."""
-    s, alpha, beta = F32(s), F32(alpha), F32(beta)
-    h, w = fwd.shape[:2]
-    u, v = fwd[..., 0], fwd[..., 1]
-    ii, jj = np.meshgrid(np.arange(h, dtype=np.int64), np.arange(w, dtype=np.int64), indexing="ij")
-    with np.errstate(all="ignore"):
-        fin = np.isfinite(u) & np.isfinite(v)
-        du, dv = s * u, s * v
-        ranged = fin & (np.abs(du) < F32(32768)) & (np.abs(dv) < F32(32768))
-        X = jj * 256 + np.where(ranged, np.rint(du * F32(256)), F32(0)).astype(np.int64)
-        Y = ii * 256 + np.where(ranged, np.rint(dv * F32(256)), F32(0)).astype(np.int64)
-        inside = ranged & (X >= 0) & (X <= (w - 1) * 256) & (Y >= 0) & (Y <= (h - 1) * 256)
-        X, Y = np.where(inside, X, 0), np.where(inside, Y, 0)
-        x0, y0, wx, wy = X >> 8, Y >> 8, X & 255, Y & 255
-        x1, y1 = np.where(wx > 0, x0 + 1, x0), np.where(wy > 0, y0 + 1, y0)
-        b00, b01, b10, b11 = bwd[y0, x0], bwd[y0, x1], bwd[y1, x0], bwd[y1, x1]
-        bfin = np.isfinite(b00).all(-1) & np.isfinite(b01).all(-1) & np.isfinite(b10).all(-1) & np.isfinite(b11).all(-1)
-        fx = (wx.astype(F32) * F32(1 / 256))[..., None]
-        fy = (wy.astype(F32) * F32(1 / 256))[..., None]
-        top = b00 + fx * (b01 - b00)
-        bot = b10 + fx * (b11 - b10)
-        b = top + fy * (bot - top)
-        bu, bv = b[..., 0], b[..., 1]
-        eu, ev = s * (u + bu), s * (v + bv)
-        e2 = eu * eu + ev * ev
-        sbu, sbv = s * bu, s * bv
-        mag2 = (du * du + dv * dv) + (sbu * sbu + sbv * sbv)
-        cons = np.isfinite(e2) & (e2 <= alpha * mag2 + beta)
-    ok = inside & bfin
-    status = np.full((h, w), FB_OUTSIDE, np.uint8)
-    status[~fin] = FB_FWD_NONFINITE
-    status[inside & ~bfin] = FB_BWD_NONFINITE
-    status[ok & cons] = FB_CONSISTENT
-    status[ok & ~cons] = FB_INCONSISTENT
-    err2 = np.where(ok, e2, F32(np.nan)).astype(F32)
-    return status, err2
-
-
-def assert_same_bits(got, ref, what=""):
-    """Equal NaN positions, and every other value bit for bit (signed zeros and infinities included)."""
-    got, ref = np.asarray(got, F32), np.asarray(ref, F32)
-    assert got.shape == ref.shape, what
-    ng, nr = np.isnan(got), np.isnan(ref)
-    assert np.array_equal(ng, nr), f"{what}: NaN positions differ at {np.argwhere(ng != nr)[:5].tolist()}"
-    bad = got.view(np.uint32)[~ng] != ref.view(np.uint32)[~nr]
-    assert not bad.any(), f"{what}: {bad.sum()} values differ: got {got[~ng][bad][:4]} ref {ref[~nr][bad][:4]}"
-
-
-def assert_status_equal(got, ref, what=""):
-    assert got.shape == ref.shape, what
-    bad = got != ref
-    assert not bad.any(), f"{what}: {bad.sum()} statuses differ, first at {np.argwhere(bad)[:3].tolist()}: " \
-                          f"got {got[bad][:3]} ref {ref[bad][:3]}"
-
-
-# ------------------------------------------------------------------------------------ the C restatement
-class FbOracle:
-    """tests/fb_oracle.c (orc_fb_check) through ctypes, plus the pinned oracle's flow in both directions."""
-
-    def __init__(self, so_path, oracle):
-        self._lib = C.CDLL(so_path)
-        self._lib.orc_fb_check.restype = None
-        self._lib.orc_fb_check.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float,
-                                           C.c_void_p, C.c_void_p]
-        self.O = oracle
-
-    def fb_check(self, fwd, bwd, flow_scale=1.0, alpha=0.01, beta=0.5):
-        """(h, w, 2) or (n, h, w, 2) float32 totals -> (status uint8, err2 float32), shaped like the flow without its last
-        axis."""
-        fwd = np.ascontiguousarray(fwd, F32)
-        bwd = np.ascontiguousarray(bwd, F32)
-        assert fwd.shape == bwd.shape and fwd.shape[-1] == 2 and fwd.ndim in (3, 4)
-        h, w = fwd.shape[-3:-1]
-        f3, b3 = fwd.reshape(-1, h, w, 2), bwd.reshape(-1, h, w, 2)
-        status = np.empty(f3.shape[:3], np.uint8)
-        err2 = np.empty(f3.shape[:3], F32)
-        for i in range(f3.shape[0]):
-            self._lib.orc_fb_check(f3[i].ctypes.data, b3[i].ctypes.data, w, h, flow_scale, alpha, beta, err2[i].ctypes.data,
-                                   status[i].ctypes.data)
-        return status.reshape(fwd.shape[:-1]), err2.reshape(fwd.shape[:-1])
-
-    def fb_pair(self, prev, nxt, levels, win, warp_mode, flow_scale=1.0, alpha=0.01, beta=0.5):
-        """(fwd_total, bwd_total, status, err2): the level-0 compositions of oracle.flow_pair(prev, next) and
-        oracle.flow_pair(next, prev) with exact window sums, and their check."""
-        O = self.O
-        fwd = O.flow_pair(prev, nxt, levels, win, warp_mode, O.SUMS_EXACT, flow_scale, want_cum=True)[1][0]
-        bwd = O.flow_pair(nxt, prev, levels, win, warp_mode, O.SUMS_EXACT, flow_scale, want_cum=True)[1][0]
-        return (fwd, bwd) + self.fb_check(fwd, bwd, flow_scale, alpha, beta)
-
-
-@pytest.fixture(scope="session")
-def fbo(oracle, tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("fb_oracle") / "libfboracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "fb_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return FbOracle(so, oracle)
+from support import (F32, FB_BWD_NONFINITE, FB_CONSISTENT, FB_FWD_NONFINITE, FB_INCONSISTENT, FB_OUTSIDE, PAIRS, S815,
+                     assert_same_bits, assert_status_equal, assert_values_equal, fbo, np_fb_check, solve, to_device)  # noqa: F401
 
 
 # ------------------------------------------------------------------------------------ the pin's inputs
@@ -321,18 +217,12 @@ def test_null_context_is_rejected_by_the_fb_entry_points():
 
 
 # ------------------------------------------------------------------------------------ GPU
-def _dev(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
 @pytest.fixture
 def exact_ctx(ctx):
     from cuda_optical_flow_2_b200 import SOLVE_EXACT
 
-    assert ctx.solve == SOLVE_EXACT
-    return ctx
+    with solve(ctx, SOLVE_EXACT):
+        yield ctx
 
 
 @pytest.mark.gpu
@@ -340,7 +230,7 @@ def exact_ctx(ctx):
 @pytest.mark.parametrize("case", CASES, ids=CASE_IDS)
 def test_fb_check_device_equals_oracle(ctx, fbo, case, want_err2):
     _, fwd, bwd, s, alpha, beta = case
-    st, e2 = ctx.fb_check_device(_dev(fwd[None]), _dev(bwd[None]), s, alpha, beta, want_err2=want_err2)
+    st, e2 = ctx.fb_check_device(to_device(fwd[None]), to_device(bwd[None]), s, alpha, beta, want_err2=want_err2)
     rst, re2 = fbo.fb_check(fwd, bwd, s, alpha, beta)
     assert_status_equal(st[0].cpu().numpy(), rst)
     if want_err2:
@@ -360,7 +250,7 @@ def test_fb_check_device_batch(ctx, fbo, w, h, n, want_err2):
     bwd = np.stack([p[1] for p in pairs])
     fwd[1, 0, :3] = np.nan
     bwd[-1, 1:3, 2:5] = np.inf
-    st, e2 = ctx.fb_check_device(_dev(fwd), _dev(bwd), S815, want_err2=want_err2)
+    st, e2 = ctx.fb_check_device(to_device(fwd), to_device(bwd), S815, want_err2=want_err2)
     rst, re2 = fbo.fb_check(fwd, bwd, S815)
     assert_status_equal(st.cpu().numpy(), rst)
     if want_err2:
@@ -383,7 +273,6 @@ def _frames(oracle, w, h, n, seed=1234, dx=1.5, dy=-0.75):
 ])
 def test_flow_pairs_fb_device_equals_oracle(exact_ctx, oracle, fbo, mode, w, h, levels, win, n, flow_scale):
     from cuda_optical_flow_2_b200 import planar_to_device
-    from test_gpu_parity import assert_flow_identical
 
     prevs, nexts = _frames(oracle, w, h, n)
     fwd, bwd, st, e2 = exact_ctx.flow_pairs_fb_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win,
@@ -391,37 +280,33 @@ def test_flow_pairs_fb_device_equals_oracle(exact_ctx, oracle, fbo, mode, w, h, 
     fwd, bwd, st, e2 = (t.cpu().numpy() for t in (fwd, bwd, st, e2))
     for i in range(n):
         rf, rb, rst, re2 = fbo.fb_pair(prevs[i], nexts[i], levels, win, mode, flow_scale, 0.01, 0.5)
-        assert_flow_identical(fwd[i], rf, f"pair {i} forward total")
-        assert_flow_identical(bwd[i], rb, f"pair {i} backward total")
+        assert_values_equal(fwd[i], rf, f"pair {i} forward total")
+        assert_values_equal(bwd[i], rb, f"pair {i} backward total")
         assert_status_equal(st[i], rst, f"pair {i}")
         assert_same_bits(e2[i], re2, f"pair {i} err2")
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("solve", ["exact", "fast"])
+@pytest.mark.parametrize("kind", ["exact", "fast"])
 @pytest.mark.parametrize("w,h,levels,win,n", [(160, 120, 3, 9, 3), (203, 117, 4, 15, 2), (96, 64, 1, 5, 2)])
-def test_shared_pyramids_change_nothing(ctx, oracle, fbo, solve, w, h, levels, win, n):
+def test_shared_pyramids_change_nothing(ctx, oracle, fbo, kind, w, h, levels, win, n):
     """Both totals are bit-identical to two ofb_flow_pairs_device calls (prev, next) and (next, prev), in both solve
     modes (SOLVE_FAST has no bit-exact oracle across levels); the status is the oracle's check of those totals."""
     import torch
 
     from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST, planar_to_device
-    from test_gpu_parity import assert_flow_identical
 
     prevs, nexts = _frames(oracle, w, h, n, seed=77)
     p, q = planar_to_device(prevs), planar_to_device(nexts)
-    ctx.solve = SOLVE_FAST if solve == "fast" else SOLVE_EXACT
-    try:
+    with solve(ctx, SOLVE_FAST if kind == "fast" else SOLVE_EXACT):
         fwd, bwd, st, _ = ctx.flow_pairs_fb_device(p, q, w, levels, win, flow_scale=S815)
         ref_f = torch.empty((n, h, w, 2), dtype=torch.float32, device="cuda")
         ref_b = torch.empty_like(ref_f)
         ctx.flow_pairs_device(p, q, w, levels, win, flow_scale=S815, total_flow=ref_f)
         ctx.flow_pairs_device(q, p, w, levels, win, flow_scale=S815, total_flow=ref_b)
-    finally:
-        ctx.solve = SOLVE_EXACT
     ref_f, ref_b = ref_f.cpu().numpy(), ref_b.cpu().numpy()
-    assert_flow_identical(fwd.cpu().numpy(), ref_f, "forward total")
-    assert_flow_identical(bwd.cpu().numpy(), ref_b, "backward total")
+    assert_values_equal(fwd.cpu().numpy(), ref_f, "forward total")
+    assert_values_equal(bwd.cpu().numpy(), ref_b, "backward total")
     assert_status_equal(st.cpu().numpy(), fbo.fb_check(ref_f, ref_b, S815)[0])
 
 
@@ -444,7 +329,6 @@ def test_swapping_the_frames_swaps_the_totals(exact_ctx, oracle):
 def test_adversarial_content_status(exact_ctx, oracle, fbo, name, w, h, levels, win):
     """The pair 0 -> 255 and flat frames (det == 0 everywhere: every total flow NaN) give the oracle's status."""
     from cuda_optical_flow_2_b200 import planar_to_device
-    from test_adversarial_content import PAIRS
 
     prev, nxt = PAIRS[name](w, h)
     fwd, bwd, st, e2 = exact_ctx.flow_pairs_fb_device(planar_to_device(prev[None]), planar_to_device(nxt[None]), w, levels,
@@ -495,7 +379,7 @@ def test_profile_record_around_the_check(ctx):
     fwd, bwd = _random(64, 32, 3)
     ctx.profile_enable(True)
     try:
-        ctx.fb_check_device(_dev(fwd[None]), _dev(bwd[None]))
+        ctx.fb_check_device(to_device(fwd[None]), to_device(bwd[None]))
         ms, n = ctx.profile_read(PROFILE_FB_CHECK)
     finally:
         ctx.profile_enable(False)

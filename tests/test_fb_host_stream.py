@@ -8,6 +8,7 @@ also checked against the C restatement of the check (tests/fb_oracle.c, compiled
 returned totals.  The refactored upload of ofb_flow_pairs_host / _ex is checked for unchanged bytes and an unchanged
 number of launches, counted from the sub-batch plan.
 """
+import contextlib
 import ctypes as C
 import os
 import subprocess
@@ -16,25 +17,9 @@ import sys
 import numpy as np
 import pytest
 
-from test_fb_consistency import S815, FbOracle
+from support import ASW, BIL, NEAR, S815, assert_same_bytes, bgr_sequence, fbo, pyramid_launches, solve  # noqa: F401 (fbo: a fixture)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIL, NEAR, ASW = 2, 1, 0  # OFB_WARP_BILINEAR, _NEAREST, _AS_WRITTEN
-
-
-@pytest.fixture(scope="module")
-def fb_oracle(oracle, tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("fb_oracle_hs") / "libfboracle.so")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, os.path.join(ROOT, "tests", "fb_oracle.c"), "-lm"])
-    return FbOracle(so, oracle)
-
-
-def same_bits(got, ref, what=""):
-    got, ref = np.ascontiguousarray(got), np.ascontiguousarray(ref)
-    assert got.shape == ref.shape and got.dtype == ref.dtype, what
-    eq = got.view(np.uint8) == ref.view(np.uint8)
-    assert eq.all(), f"{what}: {(~eq).sum()} bytes differ"
 
 
 # ------------------------------------------------------------------------------------ launches counted from the plan
@@ -42,10 +27,6 @@ def n_sub_batches(n, lanes=3):
     """Sub-batches of the host pipeline (csrc/ofb_api.cu host_pipeline, default lanes)."""
     sub = min(max(n // (8 * lanes), 1), 8)
     return -(-n // sub)
-
-
-def pyramid_launches(levels):
-    return levels // 2  # two pyramid steps per launch where two are left: ceil((levels - 1) / 2)
 
 
 def host_launches(n, levels, channels, host_threads, fb):
@@ -101,24 +82,17 @@ def pinned():
     pin.free()
 
 
-class Settings:
-    """Solve mode and host threads of the shared context, restored afterwards."""
+@contextlib.contextmanager
+def settings(ctx, kind, host_threads=0):
+    """The shared context in the "exact" or "fast" solve and with `host_threads` host threads, both restored afterwards."""
+    from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST
 
-    def __init__(self, ctx, solve, host_threads=0):
-        self.ctx, self.solve, self.threads = ctx, solve, host_threads
-
-    def __enter__(self):
-        from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST
-
-        self.ctx.solve = SOLVE_FAST if self.solve == "fast" else SOLVE_EXACT
-        self.ctx.host_threads = self.threads
-        return self.ctx
-
-    def __exit__(self, *exc):
-        from cuda_optical_flow_2_b200 import SOLVE_EXACT
-
-        self.ctx.solve = SOLVE_EXACT
-        self.ctx.host_threads = 0
+    with solve(ctx, SOLVE_FAST if kind == "fast" else SOLVE_EXACT):
+        ctx.host_threads = host_threads
+        try:
+            yield ctx
+        finally:
+            ctx.host_threads = 0
 
 
 def gray_pairs(oracle, w, h, n, seed):
@@ -156,16 +130,16 @@ def _host_id(c):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", HOST_CASES, ids=[_host_id(c) for c in HOST_CASES])
-def test_fb_host_equals_fb_device(ctx, oracle, fb_oracle, pinned, case):
+def test_fb_host_equals_fb_device(ctx, oracle, fbo, pinned, case):
     from cuda_optical_flow_2_b200 import planar_to_device
 
-    channels, threads, pin, n, w, h, levels, win, mode, solve, want_bwd, want_err2, s = case
+    channels, threads, pin, n, w, h, levels, win, mode, kind, want_bwd, want_err2, s = case
     prevs, nexts = gray_pairs(oracle, w, h, n, seed=40 + n)
     rng = np.random.default_rng(n)
     hp, hn = (prevs, nexts) if channels == 1 else (with_channels(prevs, rng), with_channels(nexts, rng))
     if pin:
         hp, hn = pinned.copy(hp), pinned.copy(hn)
-    with Settings(ctx, solve, threads):
+    with settings(ctx, kind, threads):
         before = ctx.launch_count
         fwd, bwd, st, e2 = ctx.flow_pairs_fb_host(hp, hn, levels, win, warp_mode=mode, flow_scale=s, want_bwd=want_bwd,
                                                   want_err2=want_err2)
@@ -174,17 +148,17 @@ def test_fb_host_equals_fb_device(ctx, oracle, fb_oracle, pinned, case):
                                        flow_scale=s, want_err2=True)
     rf, rb, rst, re2 = (t.cpu().numpy() for t in ref)
     assert launches == host_launches(n, levels, channels, threads, fb=True)
-    same_bits(fwd, rf, "forward total")
-    same_bits(st, rst, "status")
+    assert_same_bytes(fwd, rf, "forward total")
+    assert_same_bytes(st, rst, "status")
     assert (bwd is not None) == want_bwd and (e2 is not None) == want_err2
     if want_bwd:
-        same_bits(bwd, rb, "backward total")
-        ost, oe2 = fb_oracle.fb_check(fwd, bwd, s)
-        same_bits(st, ost, "status against orc_fb_check")
+        assert_same_bytes(bwd, rb, "backward total")
+        ost, oe2 = fbo.fb_check(fwd, bwd, s)
+        assert_same_bytes(st, ost, "status against orc_fb_check")
         if want_err2:
-            same_bits(e2, oe2, "err2 against orc_fb_check")
+            assert_same_bytes(e2, oe2, "err2 against orc_fb_check")
     if want_err2:
-        same_bits(e2, re2, "err2")
+        assert_same_bytes(e2, re2, "err2")
 
 
 EX_CASES = [(1, 0, 53, 96, 64, 3), (3, 0, 7, 160, 120, 4), (3, 4, 24, 97, 61, 2), (1, 0, 1, 96, 64, 1), (3, 4, 3, 64, 48, 1)]
@@ -203,7 +177,7 @@ def test_host_ex_bytes_and_launches_unchanged(ctx, oracle, channels, threads, n,
     prevs, nexts = gray_pairs(oracle, w, h, n, seed=700 + n)
     rng = np.random.default_rng(n + 1)
     hp, hn = (prevs, nexts) if channels == 1 else (with_channels(prevs, rng), with_channels(nexts, rng))
-    with Settings(ctx, "exact", threads):
+    with settings(ctx, "exact", threads):
         c0 = ctx.launch_count
         total = ctx.total_flow_pairs_host(hp, hn, levels, win)
         c1 = ctx.launch_count
@@ -214,9 +188,9 @@ def test_host_ex_bytes_and_launches_unchanged(ctx, oracle, channels, threads, n,
     expect = host_launches(n, levels, channels, threads, fb=False)
     assert (c1 - c0, c2 - c1) == (expect, expect)
     for k in range(levels):
-        same_bits(flows[k], ref[k].cpu().numpy(), f"level {k}")
+        assert_same_bytes(flows[k], ref[k].cpu().numpy(), f"level {k}")
     # (one level: the host call downloads the residual flow as the total, the kernel has nothing to compose)
-    same_bits(total, (ref_total if levels > 1 else ref[0]).cpu().numpy(), "total flow")
+    assert_same_bytes(total, (ref_total if levels > 1 else ref[0]).cpu().numpy(), "total flow")
 
 
 @pytest.mark.gpu
@@ -267,13 +241,6 @@ def test_fb_host_bad_arguments_enqueue_nothing(ctx):
 
 
 # ------------------------------------------------------------------------------------ GPU: the frame stream
-SHIFTS = [(0.0, 0.0), (1.5, -0.5), (2.25, 0.75), (0.5, 2.0), (-1.0, 1.25), (3.0, -1.5)]
-
-
-def bgr_sequence(oracle, w, h, seed=61):
-    return [oracle.make_bgr_frame(w, h, dx, dy, 8, seed) for dx, dy in SHIFTS]
-
-
 def preprocessed(ctx, oracle, frame, bil):
     """The stream's level 0 of a frame as a (1, h, pitch) device tensor: the oracle's grayscale, then optionally the
     bilateral filter on the device."""
@@ -295,12 +262,12 @@ STREAM_CASES = [
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("w,h,levels,win,mode,bil,solve,s", STREAM_CASES)
-def test_stream_fb_equals_fb_device(ctx, oracle, fb_oracle, w, h, levels, win, mode, bil, solve, s):
+@pytest.mark.parametrize("w,h,levels,win,mode,bil,kind,s", STREAM_CASES)
+def test_stream_fb_equals_fb_device(ctx, oracle, fbo, w, h, levels, win, mode, bil, kind, s):
     """Every push after the first against ofb_flow_pairs_fb_device on the previous and current preprocessed frames, and
     the forward outputs against a second stream's plain push."""
     frames = bgr_sequence(oracle, w, h)
-    with Settings(ctx, solve):
+    with settings(ctx, kind):
         fb = ctx.open_stream(w, h, levels, win, warp_mode=mode, flow_scale=s, bil_win=bil)
         plain = ctx.open_stream(w, h, levels, win, warp_mode=mode, flow_scale=s, bil_win=bil)
         try:
@@ -312,14 +279,14 @@ def test_stream_fb_equals_fb_device(ctx, oracle, fb_oracle, w, h, levels, win, m
                 cur = preprocessed(ctx, oracle, frames[t], bil)
                 rf, rb, rst, re2 = (x[0].cpu().numpy() for x in ctx.flow_pairs_fb_device(prev, cur, w, levels, win, warp_mode=mode,
                                                                                          flow_scale=s, want_err2=True))
-                same_bits(got["fwd_total"], rf, f"push {t} forward total")
-                same_bits(got["bwd_total"], rb, f"push {t} backward total")
-                same_bits(got["status"], rst, f"push {t} status")
-                same_bits(got["err2"], re2, f"push {t} err2")
-                same_bits(got["status"], fb_oracle.fb_check(got["fwd_total"], got["bwd_total"], s)[0], f"push {t} orc_fb_check")
-                same_bits(got["fwd_total"], total, f"push {t} forward total against push")
+                assert_same_bytes(got["fwd_total"], rf, f"push {t} forward total")
+                assert_same_bytes(got["bwd_total"], rb, f"push {t} backward total")
+                assert_same_bytes(got["status"], rst, f"push {t} status")
+                assert_same_bytes(got["err2"], re2, f"push {t} err2")
+                assert_same_bytes(got["status"], fbo.fb_check(got["fwd_total"], got["bwd_total"], s)[0], f"push {t} orc_fb_check")
+                assert_same_bytes(got["fwd_total"], total, f"push {t} forward total against push")
                 for k in range(levels):
-                    same_bits(got["levels"][k], flows[k], f"push {t} level {k} against push")
+                    assert_same_bytes(got["levels"][k], flows[k], f"push {t} level {k} against push")
                 prev = cur
         finally:
             fb.close()
@@ -346,17 +313,17 @@ def test_stream_mixed_pushes(ctx, oracle):
                     assert m is None
                     continue
                 for k in range(levels):
-                    same_bits(m[0][k], a[0][k], f"frame {t} level {k}")
-                same_bits(m[1], a[1], f"frame {t} total")
+                    assert_same_bytes(m[0][k], a[0][k], f"frame {t} level {k}")
+                assert_same_bytes(m[1], a[1], f"frame {t} total")
             else:
                 m = mixed.push_fb(f, want_levels=True, want_bwd=True, want_err2=True)
                 if b is None:
                     assert m is None
                     continue
                 for key in ("fwd_total", "bwd_total", "status", "err2"):
-                    same_bits(m[key], b[key], f"frame {t} {key}")
+                    assert_same_bytes(m[key], b[key], f"frame {t} {key}")
                 for k in range(levels):
-                    same_bits(m["levels"][k], b["levels"][k], f"frame {t} level {k}")
+                    assert_same_bytes(m["levels"][k], b["levels"][k], f"frame {t} level {k}")
     finally:
         for s in (mixed, only_plain, only_fb):
             s.close()
@@ -438,4 +405,4 @@ def test_stream_serial_override_gives_the_same_bytes(oracle, tmp_path):
         res[serial] = np.load(out)
     assert sorted(res[False].files) == sorted(res[True].files) and len(res[False].files) == 5 * (4 + levels)
     for key in res[False].files:
-        same_bits(res[True][key], res[False][key], key)
+        assert_same_bytes(res[True][key], res[False][key], key)

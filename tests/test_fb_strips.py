@@ -15,8 +15,8 @@ import os
 import numpy as np
 import pytest
 
-from test_fb_consistency import (F32, FB_BWD_NONFINITE, FB_CONSISTENT, FB_FWD_NONFINITE, FB_INCONSISTENT, FB_OUTSIDE, S815,
-                                 assert_same_bits, assert_status_equal, fbo, np_fb_check)  # noqa: F401 (fbo is a fixture)
+from support import (F32, FB_BWD_NONFINITE, FB_CONSISTENT, FB_FWD_NONFINITE, FB_INCONSISTENT, FB_OUTSIDE, S815,
+                     assert_same_bits, assert_status_equal, fbo, np_fb_check, solve)  # noqa: F401 (fbo is a fixture)
 
 FB_UNCHECKED = 5
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -170,14 +170,6 @@ def _frames(oracle, W, H, seed, dx, dy):
     return planar_to_device(prev[None]), planar_to_device(nxt[None])
 
 
-def _same(got, ref):
-    """NaN positions equal, every other value bit for bit."""
-    import torch
-
-    ng, nr = torch.isnan(got), torch.isnan(ref)
-    return bool(torch.equal(ng, nr)) and bool(torch.equal(got[~ng].view(torch.int32), ref[~nr].view(torch.int32)))
-
-
 def _inputs(ranks, dp, dn):
     out = []
     for ns in ranks:
@@ -199,12 +191,12 @@ def _assert_equals_whole(ranks, whole, want_err2, what):
         _, out = tap_rows_outside(fwd[0, y0:y1].cpu().numpy(), y0, ns.h, b0, b1, ns.flow_scale)
         out = torch.from_numpy(out).to(st.device)
         gf, gb, gs, ge = ns.own_fb()
-        assert _same(gf, fwd[0, y0:y1]), f"{what} rank {ns.rank}: forward total"
-        assert _same(gb, bwd[0, y0:y1]), f"{what} rank {ns.rank}: backward total"
+        assert_same_bits(gf, fwd[0, y0:y1], f"{what} rank {ns.rank}: forward total")
+        assert_same_bits(gb, bwd[0, y0:y1], f"{what} rank {ns.rank}: backward total")
         ref_st = torch.where(out, torch.full_like(st[0, y0:y1], FB_UNCHECKED), st[0, y0:y1])
         assert bool((gs == ref_st).all()), f"{what} rank {ns.rank}: status ({int((gs != ref_st).sum())} differ)"
         if want_err2:
-            assert _same(ge, torch.where(out, torch.full_like(ge, float("nan")), e2[0, y0:y1])), f"{what} rank {ns.rank}: err2"
+            assert_same_bits(ge, torch.where(out, torch.full_like(ge, float("nan")), e2[0, y0:y1]), f"{what} rank {ns.rank}: err2")
 
 
 EQUIV = [(640, 480, 3, 9, 1, 2), (640, 480, 3, 9, 2, 1), (640, 480, 3, 5, 4, 2), (640, 480, 1, 9, 3, 2), (322, 406, 2, 5, 3, 2),
@@ -214,9 +206,9 @@ EQUIV = [(640, 480, 3, 9, 1, 2), (640, 480, 3, 9, 2, 1), (640, 480, 3, 5, 4, 2),
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("fused", [True, False])
-@pytest.mark.parametrize("solve", ["exact", "fast"])
+@pytest.mark.parametrize("kind", ["exact", "fast"])
 @pytest.mark.parametrize("W,H,levels,win,world,mode", EQUIV)
-def test_checked_pair_equals_whole_frame(ctx, oracle, W, H, levels, win, world, mode, solve, fused):
+def test_checked_pair_equals_whole_frame(ctx, oracle, W, H, levels, win, world, mode, kind, fused):
     """Three checked pairs back to back on the same handles (err2 on, off, on), every output bit-identical to the
     whole-frame ofb_flow_pairs_fb_device rows, NaN positions included."""
     import torch
@@ -224,22 +216,21 @@ def test_checked_pair_equals_whole_frame(ctx, oracle, W, H, levels, win, world, 
     from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST
     from cuda_optical_flow_2_b200.dist import NativeStrips
 
-    ctx.solve = SOLVE_FAST if solve == "fast" else SOLVE_EXACT
-    ranks = _make_ranks(ctx, W, H, levels, win, world, mode, fb_reach=16)
-    try:
-        for ns in ranks:
-            ns.set_fused(fused)
-        for trial, (dx, dy) in enumerate([(2.25, -1.5), (-3.0, 0.75), (0.5, 2.0)]):
-            want_err2 = trial != 1
-            dp, dn = _frames(oracle, W, H, 700 + trial, dx, dy)
-            whole = ctx.flow_pairs_fb_device(dp, dn, W, levels, win, warp_mode=mode, want_err2=want_err2)
-            torch.cuda.synchronize()
-            NativeStrips.run_local_sequenced_fb(ranks, _inputs(ranks, dp, dn), want_err2=want_err2,
-                                                stream=torch.cuda.current_stream().cuda_stream)
-            _assert_equals_whole(ranks, whole, want_err2, f"pair {trial}")
-    finally:
-        ctx.solve = SOLVE_EXACT
-        _close(ranks)
+    with solve(ctx, SOLVE_FAST if kind == "fast" else SOLVE_EXACT):
+        ranks = _make_ranks(ctx, W, H, levels, win, world, mode, fb_reach=16)
+        try:
+            for ns in ranks:
+                ns.set_fused(fused)
+            for trial, (dx, dy) in enumerate([(2.25, -1.5), (-3.0, 0.75), (0.5, 2.0)]):
+                want_err2 = trial != 1
+                dp, dn = _frames(oracle, W, H, 700 + trial, dx, dy)
+                whole = ctx.flow_pairs_fb_device(dp, dn, W, levels, win, warp_mode=mode, want_err2=want_err2)
+                torch.cuda.synchronize()
+                NativeStrips.run_local_sequenced_fb(ranks, _inputs(ranks, dp, dn), want_err2=want_err2,
+                                                    stream=torch.cuda.current_stream().cuda_stream)
+                _assert_equals_whole(ranks, whole, want_err2, f"pair {trial}")
+        finally:
+            _close(ranks)
 
 
 @pytest.mark.gpu
@@ -318,8 +309,8 @@ def test_plain_and_checked_pairs_alternate(ctx, oracle, world, fb_reach):
                 a.check()
                 b.check()
                 for k in range(levels):
-                    assert _same(b.own_flow(k), a.own_flow(k)), f"step {step} rank {a.rank} level {k}"
-                assert _same(b.own_flow(0, total=True), a.own_flow(0, total=True)), f"step {step} rank {a.rank} total"
+                    assert_same_bits(b.own_flow(k), a.own_flow(k), f"step {step} rank {a.rank} level {k}")
+                assert_same_bits(b.own_flow(0, total=True), a.own_flow(0, total=True), f"step {step} rank {a.rank} total")
     finally:
         _close(fb + plain)
 

@@ -12,10 +12,10 @@ import numpy as np
 import pytest
 
 from oracle.make_golden import MULTI, SINGLE, WINDOWS, load
+from support import TOL_ABS, TOL_REL, assert_values_equal
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_gpu_b200.npz")
-TOL_ABS, TOL_REL = 1e-4, 1e-5
 
 
 @pytest.fixture(scope="module")
@@ -28,8 +28,7 @@ def compare(got, ref, exact, what, mask=None):
         mask = np.ones(ref.shape[:2], bool)
     g, r = got[mask], ref[mask]
     if exact:
-        same = (g == r) | (np.isnan(g) & np.isnan(r))
-        assert same.all(), f"{what}: {(~same).sum()} values differ, max |d| {np.nanmax(np.abs(g - r)):.3e}"
+        assert_values_equal(g, r, what)
         return
     both = np.isfinite(g) & np.isfinite(r)
     assert (np.isfinite(g) == np.isfinite(r)).mean() > 0.9999, what

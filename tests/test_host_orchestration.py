@@ -21,7 +21,7 @@ import sys
 import numpy as np
 import pytest
 
-from test_fb_host_stream import BIL, NEAR, bgr_sequence, pyramid_launches, same_bits
+from support import BIL, NEAR, assert_same_bytes, bgr_sequence, pyramid_launches
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -42,7 +42,7 @@ def test_stream_push_without_total_composes_bit_identically(ctx, oracle, w, h, l
             cur = oracle.grayscale_c3(frames[t])[:, :, 0]
             ref = oracle.flow_pair(np.ascontiguousarray(prev), np.ascontiguousarray(cur), levels, win, mode, oracle.SUMS_EXACT)
             for k in range(levels):
-                same_bits(flows[k], ref_flows[k], f"push {t} level {k} against the push with the total")
+                assert_same_bytes(flows[k], ref_flows[k], f"push {t} level {k} against the push with the total")
                 r = np.asarray(ref[k]).reshape(flows[k].shape)
                 assert np.array_equal(np.isnan(flows[k]), np.isnan(r)), f"push {t} level {k}: NaN masks differ from the oracle"
                 m = ~np.isnan(r)

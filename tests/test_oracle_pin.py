@@ -15,6 +15,7 @@ import numpy as np
 import pytest
 
 from oracle.make_golden import DERIVATIVES, MULTI, SINGLE, WINDOWS, load
+from support import assert_values_equal
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_gpu_b200.npz")
 
@@ -53,10 +54,6 @@ def test_golden_file_decodes(gold):
         assert np.array_equal(direct, gold["a_sums_w5"][k]), f"sum {k}"
 
 
-def bits_equal(a, b):
-    return a.shape == b.shape and np.array_equal(np.isnan(a), np.isnan(b)) and np.array_equal(a[~np.isnan(a)], b[~np.isnan(b)])
-
-
 @pytest.mark.parametrize("case", SINGLE, ids=[c[0] for c in SINGLE])
 def test_derivatives_match_reference_gpu(oracle, gold, case):
     name, w, h, dx, dy, cell, seed = case
@@ -84,11 +81,11 @@ def test_window_sums_solve_and_level_match_reference_gpu(oracle, gold, case, win
         if np.abs(ref_sums[k]).max() < 2 ** 24:
             assert np.array_equal(oracle.srm_exact(a, b, win, win), ref_sums[k].astype(np.int64))
     ref_flow = gold[f"{name}_flow_w{win}"]
-    assert bits_equal(oracle.solve_f32(*ref_sums), ref_flow)
-    assert bits_equal(oracle.lk_level(prev, nxt, win, oracle.SUMS_F32_SEQUENTIAL), ref_flow)
+    assert_values_equal(oracle.solve_f32(*ref_sums), ref_flow)
+    assert_values_equal(oracle.lk_level(prev, nxt, win, oracle.SUMS_F32_SEQUENTIAL), ref_flow)
     exact = oracle.lk_level(prev, nxt, win, oracle.SUMS_EXACT)
     if np.abs(ref_sums).max() < 2 ** 24:
-        assert bits_equal(exact, ref_flow)
+        assert_values_equal(exact, ref_flow)
     else:  # fp32 rounding of the reference's sums: stated tolerance of the parity tests
         both = np.isfinite(exact) & np.isfinite(ref_flow)
         assert np.abs(exact[both] - ref_flow[both]).max() <= 1e-4
@@ -100,7 +97,7 @@ def test_entry_point_single_level(oracle, gold, case):
     name, w, h, dx, dy, cell, seed = case
     prev = oracle.make_frame(w, h, 0, 0, cell, seed)
     nxt = oracle.make_frame(w, h, dx, dy, cell, seed)
-    assert bits_equal(oracle.lk_level(prev, nxt, 19, oracle.SUMS_F32_SEQUENTIAL), gold[f"{name}_entry_flow"])
+    assert_values_equal(oracle.lk_level(prev, nxt, 19, oracle.SUMS_F32_SEQUENTIAL), gold[f"{name}_entry_flow"])
 
 
 def test_pyramid_and_coarse_to_fine_loop_match_reference_gpu(oracle, gold):

@@ -26,9 +26,8 @@ F. the pyramid's rows per thread (launch_pyr_roll) at each of its five values, a
 import numpy as np
 import pytest
 
-from test_adversarial_content import PAIRS
-from test_crafted_flow import c_for, noise_pair, oracle_warp
-from test_gpu_parity import assert_flow_identical, assert_flow_within_tolerance
+from support import (PAIRS, assert_flow_within_tolerance, assert_values_equal, bits_differ, c_for, noise_pair, oracle_warp,
+                     reach_flag, requested_rows, solve, values_differ)
 
 WINDOWS = [3, 5, 7, 9, 11, 13, 15, 17, 19]
 SHAPES_A = [(256, 160), (262, 150), (256, 161)]  # even; odd coarser width (no tensor map); 161 = 10 * 16 + 1 = 5 * 32 + 1
@@ -60,93 +59,10 @@ def test_rpb_values_reach_the_edges():
 
 
 # --------------------------------------------------------------------------------------- D: the reach rule in numpy
-def cta_rows(out_y0g, out_y1g, win):
-    """Global rows [yw0, ylim) whose 2x2 blocks some CTA of a strip launch gathers: the first CTA stages from its first
-    output row minus R + 1, lowered to an even global row; the last needs rows up to its last output row plus R + 1.
-    (Every CTA in between covers a sub-range of this one, and the rule below is the same in each, so the union does not
-    depend on the split.)"""
-    r = win // 2
-    yw0 = out_y0g - r - 1
-    yw0 -= yw0 & 1
-    return yw0, out_y1g + r + 1
-
-
 def window_rows(out_y0g, out_y1g, win, h):
     """Rows of prev and next the window sums of the output rows read: the caller must hold these (ofb200.h)."""
     r = win // 2
     return max(out_y0g - r - 1, 0), min(out_y1g + r + 1, h)
-
-
-def requested_rows(cum, w, h, mode, out_y0g, out_y1g, win, s=1.0):
-    """The rows lk_warp_block_general (csrc/lk_level.cuh) asks for, over every 2x2 block a strip launch gathers:
-    (mask of image rows (h,), mask of coarser rows (h >> 1,)).
-
-    Per block at even global (xe, ye), inside the image and before the CTA's ylim, with coarser vector
-    cf = cum[min(ye >> 1, ch - 1), min(xe >> 1, cw - 1)] (that coarser row is requested):
-      bilinear: U, V = rint(cf * 512 s); if both are in range (|.| < 2^23) and any target of the block is inside the image,
-                the three tap rows ye + (V >> 8) + 0..2, clamped to the image (the third also when its weight is 0);
-      nearest:  per pixel the truncated target row int(y + v) of a target inside the image;
-      both:     the pixel's own row for a pixel inside the image and before ylim whose target is skipped."""
-    ch, cw = h >> 1, w >> 1
-    yw0, ylim = cta_rows(out_y0g, out_y1g, win)
-    ye = np.arange(max(yw0, 0), min(ylim, h), 2)
-    xe = np.arange(0, w, 2)
-    img = np.zeros(h, bool)
-    crow = np.zeros(ch, bool)
-    if ye.size == 0:
-        return img, crow
-    cy = np.minimum(ye >> 1, ch - 1)
-    cx = np.minimum(xe >> 1, cw - 1)
-    crow[cy] = True
-    cf = cum[cy[:, None], cx[None, :]]  # (blocks rows, block columns, 2)
-    YE, XE = np.broadcast_arrays(ye[:, None], xe[None, :])
-    with np.errstate(invalid="ignore", over="ignore"):
-        if mode == 2:
-            s512 = np.float32(512.0) * np.float32(s)
-            fu, fv = (cf[..., 0] * s512).astype(np.float32), (cf[..., 1] * s512).astype(np.float32)
-            ranged = (np.abs(fu) < 8388608.0) & (np.abs(fv) < 8388608.0)
-            U = np.where(ranged, np.rint(fu), 0).astype(np.int64)
-            V = np.where(ranged, np.rint(fv), 0).astype(np.int64)
-            anyt = np.zeros(YE.shape, bool)
-            done = {}
-            for r in range(2):
-                for c in range(2):
-                    inimg = (XE + c < w) & (YE + r < h) & (YE + r < ylim)
-                    X, Y = ((XE + c) << 8) + U, ((YE + r) << 8) + V
-                    d = ranged & inimg & (X >= 0) & (X <= (w - 1) << 8) & (Y >= 0) & (Y <= (h - 1) << 8)
-                    done[r, c] = (inimg, d)
-                    anyt |= d
-            for k in range(3):
-                img[np.clip(YE + (V >> 8) + k, 0, h - 1)[anyt]] = True
-            for r in range(2):
-                for c in range(2):
-                    inimg, d = done[r, c]
-                    img[(YE + r)[inimg & ~d]] = True
-        else:
-            s2 = np.float32(2.0) * np.float32(s)
-            u, v = (cf[..., 0] * s2).astype(np.float32), (cf[..., 1] * s2).astype(np.float32)
-            for r in range(2):
-                for c in range(2):
-                    inimg = (XE + c < w) & (YE + r < h) & (YE + r < ylim)
-                    fx = ((XE + c).astype(np.float32) + u).astype(np.float32)
-                    fy = ((YE + r).astype(np.float32) + v).astype(np.float32)
-                    inr = (fx > -2147483648.0) & (fx < 2147483648.0) & (fy > -2147483648.0) & (fy < 2147483648.0)
-                    nx = np.where(inr, np.trunc(fx), -1).astype(np.int64)
-                    ny = np.where(inr, np.trunc(fy), -1).astype(np.int64)
-                    d = inimg & inr & (nx >= 0) & (nx < w) & (ny >= 0) & (ny < h)
-                    img[ny[d]] = True
-                    img[(YE + r)[inimg & ~d]] = True
-    return img, crow
-
-
-def reach_flag(req, y_off, h_local, cum_y_off, cum_h_local):
-    """The strip kernel's reach flag as the rule predicts it: a requested row outside the rows held."""
-    img, crow = req
-    held = np.zeros(img.size, bool)
-    held[y_off:y_off + h_local] = True
-    cheld = np.zeros(crow.size, bool)
-    cheld[cum_y_off:cum_y_off + cum_h_local] = True
-    return bool((img & ~held).any() or (crow & ~cheld).any())
 
 
 STRIP_SHAPES = [(200, 91), (202, 91)]  # coarser width 100 (tensor map) and 101 (copied tile); odd height: clamped coarse row
@@ -292,42 +208,6 @@ def test_pyramid_batch_sizes_reach_every_rows_per_thread(sw, sh, sm_count):
 
 
 # =================================================================================================== GPU
-def _torch():
-    import torch
-
-    return torch
-
-
-def _ident(got, ref):
-    """Oracle bar on the device: same NaN and finite masks, equal values (as assert_flow_identical); '' when they match."""
-    torch = _torch()
-    fg, fr = torch.isfinite(got), torch.isfinite(ref)
-    if not torch.equal(fg, fr) or not torch.equal(torch.isnan(got), torch.isnan(ref)):
-        return "non-finite masks differ"
-    bad = fg & (got != ref)
-    if bool(bad.any()):
-        i = torch.nonzero(bad)[0].tolist()
-        return f"{int(bad.sum())} values differ, first at {i}: {got[tuple(i)].item()!r} vs {ref[tuple(i)].item()!r}"
-    inf = ~fg & ~torch.isnan(got)
-    if not torch.equal(got[inf], ref[inf]):
-        return "infinities differ in sign"
-    return ""
-
-
-def _bits(got, ref):
-    """Bit-identical (NaN positions equal, every other value bit for bit); '' when they match."""
-    torch = _torch()
-    ng, nr = torch.isnan(got), torch.isnan(ref)
-    if not torch.equal(ng, nr):
-        return f"NaN masks differ at {int((ng != nr).sum())} values"
-    d = got.view(torch.int32) != ref.view(torch.int32)
-    d &= ~ng
-    if bool(d.any()):
-        i = torch.nonzero(d)[0].tolist()
-        return f"{int(d.sum())} values differ, first at {i}: {got[tuple(i)].item()!r} vs {ref[tuple(i)].item()!r}"
-    return ""
-
-
 @pytest.fixture
 def rows(monkeypatch):
     """set(n): force n rows per CTA on every following launch; set(None): the cost model's own split."""
@@ -342,29 +222,17 @@ def rows(monkeypatch):
     return set_rows
 
 
-@pytest.fixture
-def solve_mode(ctx):
-    from cuda_optical_flow_2_b200 import SOLVE_EXACT
-
-    assert ctx.solve == SOLVE_EXACT
-
-    def set_solve(m):
-        ctx.solve = m
-
-    yield set_solve
-    ctx.solve = SOLVE_EXACT
-
-
 # --------------------------------------------------------------------------------------- A
 @pytest.mark.gpu
 @pytest.mark.parametrize("w,h", SHAPES_A)
 @pytest.mark.parametrize("win", WINDOWS)
-def test_one_level_at_every_rows_per_cta(ctx, oracle, rows, solve_mode, win, w, h):
+def test_one_level_at_every_rows_per_cta(ctx, oracle, rows, win, w, h):
     """The coarsest level and the warped level in all three warp modes (on the oracle's cumulative flow of the coarser
     level), each with and without cum_out, at every forced rows per CTA.  Exact solve: bit-identical to the oracle; fast
     solve: every pair bit-identical to the cost model's split and, there, within the tolerance bar of the oracle.  At rows
     per CTA up to 5 a batch of three distinct pairs, so that row blocks and pairs interleave in the grid."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST, planar_to_device
 
     npair = 3
@@ -391,32 +259,32 @@ def test_one_level_at_every_rows_per_cta(ctx, oracle, rows, solve_mode, win, w, 
         return flow, cum_out
 
     cases = [(m, c) for m in (None, 0, 1, 2) for c in (False, True)]
-    for solve in (SOLVE_EXACT, SOLVE_FAST):
-        solve_mode(solve)
-        rows(None)
-        base = {}
-        for mode, want_cum in cases:
-            base[mode, want_cum] = run(mode, want_cum, npair)
-            if solve == SOLVE_FAST:
-                torch.cuda.synchronize()
-                for i in range(npair):
-                    got = base[mode, want_cum][0][i].cpu().numpy()
-                    assert_flow_within_tolerance(got, refs[mode][i], f"fast solve, mode {mode}, pair {i}, default split")
-        for rpb in rpb_values(win, h):
-            rows(rpb)
+    for sm in (SOLVE_EXACT, SOLVE_FAST):
+        with solve(ctx, sm):
+            rows(None)
+            base = {}
             for mode, want_cum in cases:
-                n = npair if rpb <= 5 else 1
-                flow, cum_out = run(mode, want_cum, n)
-                what = f"rows per CTA {rpb}, mode {mode}, cum_out {want_cum}, solve {solve}"
-                if solve == SOLVE_EXACT:
-                    assert not (e := _ident(flow, dev[mode][:n])), f"{what}: flow: {e}"
-                    if want_cum:
-                        assert not (e := _ident(cum_out, dev_cum[mode][:n])), f"{what}: cum_out: {e}"
-                else:
-                    e = _bits(flow, base[mode, want_cum][0][:n])
-                    assert not e, f"{what}: flow against the default split: {e}"
-                    if want_cum:
-                        assert not (e := _bits(cum_out, base[mode, want_cum][1][:n])), f"{what}: cum_out: {e}"
+                base[mode, want_cum] = run(mode, want_cum, npair)
+                if sm == SOLVE_FAST:
+                    torch.cuda.synchronize()
+                    for i in range(npair):
+                        got = base[mode, want_cum][0][i].cpu().numpy()
+                        assert_flow_within_tolerance(got, refs[mode][i], f"fast solve, mode {mode}, pair {i}, default split")
+            for rpb in rpb_values(win, h):
+                rows(rpb)
+                for mode, want_cum in cases:
+                    n = npair if rpb <= 5 else 1
+                    flow, cum_out = run(mode, want_cum, n)
+                    what = f"rows per CTA {rpb}, mode {mode}, cum_out {want_cum}, solve {sm}"
+                    if sm == SOLVE_EXACT:
+                        assert not (e := values_differ(flow, dev[mode][:n])), f"{what}: flow: {e}"
+                        if want_cum:
+                            assert not (e := values_differ(cum_out, dev_cum[mode][:n])), f"{what}: cum_out: {e}"
+                    else:
+                        e = bits_differ(flow, base[mode, want_cum][0][:n])
+                        assert not e, f"{what}: flow against the default split: {e}"
+                        if want_cum:
+                            assert not (e := bits_differ(cum_out, base[mode, want_cum][1][:n])), f"{what}: cum_out: {e}"
 
 
 # --------------------------------------------------------------------------------------- B
@@ -438,11 +306,12 @@ PIPE_RPB = [1, 2, 3, 5, 8, 9, 16, 17, 33]
 @pytest.mark.parametrize("win", [5, 9, 15])
 @pytest.mark.parametrize("content", ["smooth", "far_shift", "split_motion", "binary_noise", "diag6"])
 @pytest.mark.parametrize("w,h,want_total", [(256, 160, False), (256, 160, True), (262, 150, False)])
-def test_pipeline_at_every_rows_per_cta(ctx, oracle, rows, solve_mode, w, h, want_total, content, win):
+def test_pipeline_at_every_rows_per_cta(ctx, oracle, rows, w, h, want_total, content, win):
     """flow_pairs_device, 3 levels, every warp mode, the forced rows per CTA applying to every level: 256x160 without the
     total flow (level 0 composes the coarser cumulative flow on the fly), with it, and 262x150 (odd coarser sizes).  Exact:
     every level and the total flow bit-identical to the oracle; fast: bit-identical to the cost model's split."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST, planar_to_device
 
     levels = 3
@@ -457,21 +326,21 @@ def test_pipeline_at_every_rows_per_cta(ctx, oracle, rows, solve_mode, w, h, wan
             total = torch.empty((1, h, w, 2), dtype=torch.float32, device="cuda") if want_total else None
             return ctx.flow_pairs_device(dp, dn, w, levels, win, warp_mode=mode, total_flow=total), total
 
-        for solve in (SOLVE_EXACT, SOLVE_FAST):
-            solve_mode(solve)
-            rows(None)
-            base, base_total = run()
-            for rpb in PIPE_RPB:
-                rows(rpb)
-                flows, total = run()
-                what = f"mode {mode}, rows per CTA {rpb}, solve {solve}"
-                for k in range(levels):
-                    e = _ident(flows[k], dref[k]) if solve == SOLVE_EXACT else _bits(flows[k], base[k])
-                    assert not e, f"{what}, level {k}: {e}"
-                if want_total:
-                    e = _ident(total, dtot) if solve == SOLVE_EXACT else _bits(total, base_total)
-                    assert not e, f"{what}, total flow: {e}"
-            rows(None)
+        for sm in (SOLVE_EXACT, SOLVE_FAST):
+            with solve(ctx, sm):
+                rows(None)
+                base, base_total = run()
+                for rpb in PIPE_RPB:
+                    rows(rpb)
+                    flows, total = run()
+                    what = f"mode {mode}, rows per CTA {rpb}, solve {sm}"
+                    for k in range(levels):
+                        e = values_differ(flows[k], dref[k]) if sm == SOLVE_EXACT else bits_differ(flows[k], base[k])
+                        assert not e, f"{what}, level {k}: {e}"
+                    if want_total:
+                        e = values_differ(total, dtot) if sm == SOLVE_EXACT else bits_differ(total, base_total)
+                        assert not e, f"{what}, total flow: {e}"
+                rows(None)
 
 
 # --------------------------------------------------------------------------------------- C
@@ -533,15 +402,16 @@ def test_tail_batch_engages_the_tail_on_every_level(sm_count):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("solve", [0, 1])
-def test_batch_tail_at_every_shift_and_length(ctx, oracle, monkeypatch, solve_mode, solve):
+@pytest.mark.parametrize("mode", [0, 1])
+def test_batch_tail_at_every_shift_and_length(ctx, oracle, monkeypatch, mode):
     """A batch big enough that the launcher cuts its last pairs into 2^shift short row blocks, on a frame of one column
     strip whose 532 rows are not a multiple of 16, 3 levels, bilinear warp, no total flow (level 0 composes).  Every level
     is forced to one row block (the tail needs that), so that the tail engages at level 0 for every shift (tail rows 266,
     133, 67 and 34), at level 1 for shifts 1-3 and at level 2 for shifts 1-2 -- asserted from the restated switch with this
     GPU's SM count.  Every OFB_LK_TAIL in 1..4 and tail length 1, 10 and 30 tenths of a wave: bit-identical to the launch
     without a tail; exact solve: every copy of every prototype equals the oracle."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     w, h, win, distinct, levels = TAIL_W, TAIL_H, TAIL_WIN, TAIL_DISTINCT, 3
@@ -552,31 +422,33 @@ def test_batch_tail_at_every_shift_and_length(ctx, oracle, monkeypatch, solve_mo
     nexts = np.stack([oracle.make_frame(w, h, 1.25 - i, 0.5 + 0.75 * i, 6, 880 + i) for i in range(distinct)])
     dp = planar_to_device(prevs).repeat(n // distinct, 1, 1)
     dn = planar_to_device(nexts).repeat(n // distinct, 1, 1)
-    solve_mode(solve)
-    monkeypatch.setenv("OFB_LK_ROWS", str(h))  # clamped to each level's rows: one row block per level
-    monkeypatch.setenv("OFB_LK_TAIL", "0")
-    plain = [f.clone() for f in ctx.flow_pairs_device(dp, dn, w, levels, win)]
-    refs = None
-    if solve == 0:
-        refs = []
-        per = [oracle.flow_pair(prevs[i], nexts[i], levels, win, 2, oracle.SUMS_EXACT) for i in range(distinct)]
-        for k in range(levels):
-            refs.append(torch.from_numpy(np.stack([p[k] for p in per])).cuda())
-        for k in range(levels):
-            e = _ident(plain[k].view(n // distinct, distinct, h >> k, w >> k, 2), refs[k].expand(n // distinct, -1, -1, -1, -1))
-            assert not e, f"no tail, level {k}: {e}"
-    for shift in (1, 2, 3, 4):
-        for waves in (1, 10, 30):
-            monkeypatch.setenv("OFB_LK_TAIL", str(shift))
-            monkeypatch.setenv("OFB_LK_TAIL_WAVES", str(waves))
-            flows = ctx.flow_pairs_device(dp, dn, w, levels, win)
+    with solve(ctx, mode):
+        monkeypatch.setenv("OFB_LK_ROWS", str(h))  # clamped to each level's rows: one row block per level
+        monkeypatch.setenv("OFB_LK_TAIL", "0")
+        plain = [f.clone() for f in ctx.flow_pairs_device(dp, dn, w, levels, win)]
+        refs = None
+        if mode == 0:
+            refs = []
+            per = [oracle.flow_pair(prevs[i], nexts[i], levels, win, 2, oracle.SUMS_EXACT) for i in range(distinct)]
             for k in range(levels):
-                assert not (e := _bits(flows[k], plain[k])), f"tail {shift}, waves {waves}, level {k}: against no tail: {e}"
-                if refs is not None:  # every copy, those of the tail included
-                    e = _ident(flows[k].view(n // distinct, distinct, h >> k, w >> k, 2),
-                               refs[k].expand(n // distinct, -1, -1, -1, -1))
-                    assert not e, f"tail {shift}, waves {waves}, level {k}: against the oracle: {e}"
-            del flows
+                refs.append(torch.from_numpy(np.stack([p[k] for p in per])).cuda())
+            for k in range(levels):
+                e = values_differ(plain[k].view(n // distinct, distinct, h >> k, w >> k, 2),
+                                  refs[k].expand(n // distinct, -1, -1, -1, -1))
+                assert not e, f"no tail, level {k}: {e}"
+        for shift in (1, 2, 3, 4):
+            for waves in (1, 10, 30):
+                monkeypatch.setenv("OFB_LK_TAIL", str(shift))
+                monkeypatch.setenv("OFB_LK_TAIL_WAVES", str(waves))
+                flows = ctx.flow_pairs_device(dp, dn, w, levels, win)
+                for k in range(levels):
+                    e = bits_differ(flows[k], plain[k])
+                    assert not e, f"tail {shift}, waves {waves}, level {k}: against no tail: {e}"
+                    if refs is not None:  # every copy, those of the tail included
+                        e = values_differ(flows[k].view(n // distinct, distinct, h >> k, w >> k, 2),
+                                          refs[k].expand(n // distinct, -1, -1, -1, -1))
+                        assert not e, f"tail {shift}, waves {waves}, level {k}: against the oracle: {e}"
+                del flows
 
 
 # --------------------------------------------------------------------------------------- D
@@ -592,7 +464,8 @@ def test_strip_windows_bit_identical_unless_flagged(ctx, oracle, rows, w, h, mod
     is not raised, flow and cum_out rows equal lk_level_device on the whole frame bit for bit.  Rows outside what a call
     holds are filled with other bytes and other flow, so that a read of them shows; rows outside the output window must
     stay untouched."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     prev, nxt = noise_pair(w, h, 77 + w)
@@ -604,7 +477,7 @@ def test_strip_windows_bit_identical_unless_flagged(ctx, oracle, rows, w, h, mod
     whole = ctx.lk_level_device(P, N, w, win, warp_mode=mode, cum_in=cum_d, cum_out=whole_cum)
     torch.cuda.synchronize()
     ref = oracle.lk_level(prev, oracle_warp(oracle, nxt, cum, mode, 1.0), win, oracle.SUMS_EXACT)
-    assert_flow_identical(whole[0].cpu().numpy(), ref, "whole frame")
+    assert_values_equal(whole[0].cpu().numpy(), ref, "whole frame")
     # garbage copies: other bytes / other flow everywhere a call does not hold
     Pg, Ng = planar_to_device((255 - prev)[None])[0], planar_to_device(np.roll(nxt, 7, 1)[None])[0]
     cum_g = torch.from_numpy(np.ascontiguousarray(cum[::-1] * np.float32(-1.5) + np.float32(3.25))).cuda()
@@ -640,7 +513,7 @@ def test_strip_windows_bit_identical_unless_flagged(ctx, oracle, rows, w, h, mod
                             continue
                         assert bool((t[:lo] == sentinel).all() and (t[hi:] == sentinel).all()), f"{what}: wrote outside its rows"
                         if not expect:
-                            assert not (e := _bits(t[lo:hi], ref[0, y0:y1])), f"{what}: {e}"
+                            assert not (e := bits_differ(t[lo:hi], ref[0, y0:y1])), f"{what}: {e}"
     assert counts[False] > 0 and counts[True] > 0
 
 
@@ -653,7 +526,8 @@ def test_peer_memory_strips_at_other_splits(ctx, oracle, rows, world, rpb):
     the forced rows per CTA: many row blocks, the pushing blocks scheduled first (permuted order) and the push counters
     sized from the split.  Two pairs back to back, every level and the total flow bit-identical to the whole frame, and no
     flag (neither a timed-out neighbour nor a reach overflow)."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import WARP_BILINEAR, planar_to_device
     from cuda_optical_flow_2_b200.dist import NativeStrips
 
@@ -682,9 +556,9 @@ def test_peer_memory_strips_at_other_splits(ctx, oracle, rows, world, rpb):
             for ns in ranks:
                 for k in range(levels):
                     y0, y1 = ns.own_rows(k)
-                    assert not (e := _bits(ns.own_flow(k), whole[k][0, y0:y1])), f"pair {trial} rank {ns.rank} level {k}: {e}"
+                    assert not (e := bits_differ(ns.own_flow(k), whole[k][0, y0:y1])), f"pair {trial} rank {ns.rank} level {k}: {e}"
                 y0, y1 = ns.own_rows(0)
-                assert not (e := _bits(ns.own_flow(0, total=True), total[0, y0:y1])), f"pair {trial} rank {ns.rank} total: {e}"
+                assert not (e := bits_differ(ns.own_flow(0, total=True), total[0, y0:y1])), f"pair {trial} rank {ns.rank} total: {e}"
     finally:
         torch.cuda.synchronize()
         for ns in ranks:
@@ -695,7 +569,8 @@ def test_peer_memory_strips_at_other_splits(ctx, oracle, rows, world, rpb):
 def test_checked_peer_memory_strips_at_three_rows_per_cta(ctx, oracle, rows):
     """A checked pair (both directions and the forward-backward check) on three ranks at 3 rows per CTA: every output
     bit-identical to the whole-frame ofb_flow_pairs_fb_device rows, no flag."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
     from cuda_optical_flow_2_b200.dist import NativeStrips
 
@@ -717,10 +592,10 @@ def test_checked_peer_memory_strips_at_three_rows_per_cta(ctx, oracle, rows):
             ns.check()
             y0, y1 = ns.own_rows(0)
             gf, gb, gs, ge = ns.own_fb()
-            assert not (e := _bits(gf, fwd[0, y0:y1])), f"rank {ns.rank} forward total: {e}"
-            assert not (e := _bits(gb, bwd[0, y0:y1])), f"rank {ns.rank} backward total: {e}"
+            assert not (e := bits_differ(gf, fwd[0, y0:y1])), f"rank {ns.rank} forward total: {e}"
+            assert not (e := bits_differ(gb, bwd[0, y0:y1])), f"rank {ns.rank} backward total: {e}"
             assert torch.equal(gs, st[0, y0:y1]), f"rank {ns.rank} status"
-            assert not (e := _bits(ge, e2[0, y0:y1])), f"rank {ns.rank} err2: {e}"
+            assert not (e := bits_differ(ge, e2[0, y0:y1])), f"rank {ns.rank} err2: {e}"
     finally:
         torch.cuda.synchronize()
         for ns in ranks:
@@ -735,7 +610,8 @@ def test_pyramid_at_every_rows_per_thread(ctx, oracle, sw, sh):
     thread (restated above), byte-exact against the oracle for every image.  The two-step entry passes the context's SM
     count to launch_pyr_roll; the one-step entry goes through launch_pyr_down, which passes none (launch_pyr_roll then
     assumes 148 SMs), so each is sized with the count its launcher uses."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     distinct = 3
@@ -765,7 +641,8 @@ def test_pyramid_strip_on_minimal_source_rows(ctx, oracle, sw, sh):
     """ofb_pyr_down_strip_device with exactly source rows 2y0-1 .. 2y1-1 held (odd src_y_off except at the top), single
     destination rows at the top, in the interior and at the bottom, and longer runs; the rows around the held ones hold
     other bytes, so that a read past them shows.  Byte-exact against the oracle."""
-    torch = _torch()
+    import torch
+
     from cuda_optical_flow_2_b200 import planar_to_device
 
     img = oracle.make_frame(sw, sh, 0, 0, 3, 970 + sw)

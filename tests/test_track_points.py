@@ -10,90 +10,16 @@ GPU tests: the kernel against the restatement over windows, levels, sizes, batch
 flow scales; against the dense path itself; CUDA graph replay; argument refusals.
 """
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-PT_TRACKED, PT_NONFINITE, PT_LOW_TEXTURE, PT_OUTSIDE = 0, 1, 2, 3
-F32 = np.float32
-S815 = 8 / 15  # px per flow unit of the reference's masks (Sobel gain 8, Dt gain 15)
-
-
-class TrackOracle:
-    """tests/track_oracle.c (orc_track_points) through ctypes, on oracle.gauss_pyramid levels."""
-
-    def __init__(self, so_path, oracle):
-        self._lib = C.CDLL(so_path)
-        self._lib.orc_track_points.restype = None
-        self._lib.orc_track_points.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p,
-                                               C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_void_p]
-        self.O = oracle
-
-    def track(self, prev, nxt, levels, win, points, flow_scale=1.0, iters=30, eps=0.01, min_eig=0.0):
-        """One pair: prev / next (h, w) uint8, points (m, 2) float32 -> (flow (m, 2) float32, status (m,) uint8)."""
-        h, w = prev.shape
-        pp = self.O.gauss_pyramid(prev, levels)
-        pn = self.O.gauss_pyramid(nxt, levels)
-        arr = lambda lv: (C.c_void_p * levels)(*[a.ctypes.data for a in lv])
-        pts = np.ascontiguousarray(points, F32).reshape(-1, 2)
-        flow = np.empty_like(pts)
-        status = np.empty(len(pts), np.uint8)
-        self._lib.orc_track_points(arr(pp), arr(pn), w, h, levels, win, flow_scale, pts.ctypes.data, len(pts), iters, eps,
-                                   min_eig, flow.ctypes.data, status.ctypes.data)
-        return flow, status
-
-
-@pytest.fixture(scope="session")
-def tro(oracle, tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("track_oracle") / "libtrackoracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "track_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return TrackOracle(so, oracle)
-
-
-def assert_same_bits(got, ref, what=""):
-    """Equal NaN positions, every other value bit for bit (signed zeros and infinities included)."""
-    got, ref = np.asarray(got, F32), np.asarray(ref, F32)
-    assert got.shape == ref.shape, what
-    ng, nr = np.isnan(got), np.isnan(ref)
-    assert np.array_equal(ng, nr), f"{what}: NaN positions differ at {np.argwhere(ng != nr)[:5].tolist()}"
-    bad = got.view(np.uint32)[~ng] != ref.view(np.uint32)[~nr]
-    assert not bad.any(), f"{what}: {bad.sum()} values differ: got {got[~ng][bad][:4]} ref {ref[~nr][bad][:4]}"
-
-
-def assert_status_equal(got, ref, what=""):
-    bad = np.asarray(got) != np.asarray(ref)
-    assert not bad.any(), f"{what}: {bad.sum()} statuses differ, first at {np.argwhere(bad)[:3].tolist()}: " \
-                          f"got {np.asarray(got)[bad][:3]} ref {np.asarray(ref)[bad][:3]}"
+from support import (F32, PT_LOW_TEXTURE, PT_NONFINITE, PT_OUTSIDE, PT_TRACKED, S815, assert_same_bits, assert_status_equal,
+                     assert_values_equal, border_points, random_points, solve, to_device, tro)  # noqa: F401 (tro is a fixture)
 
 
 def frames(oracle, w, h, dx=1.5, dy=-0.75, cell=4, seed=1234):
     return oracle.make_frame(w, h, 0, 0, cell, seed), oracle.make_frame(w, h, dx, dy, cell, seed)
-
-
-def border_points(w, h):
-    """Every pixel of the four borders (corners included), as integer (x, y)."""
-    xs = np.arange(w)
-    ys = np.arange(1, h - 1)
-    pts = [np.stack([xs, np.zeros_like(xs)], 1), np.stack([xs, np.full_like(xs, h - 1)], 1),
-           np.stack([np.zeros_like(ys), ys], 1), np.stack([np.full_like(ys, w - 1), ys], 1)]
-    return np.concatenate(pts).astype(F32)
-
-
-def random_points(w, h, m, seed, margin=2.0):
-    """m sub-pixel points over [-margin, w-1+margin] x [-margin, h-1+margin] (some start outside), the first ones replaced
-    by the corners, exact last row / column, a NaN, an inf, a point 1/256 px past the last column and half-to-even ties
-    of x * 256 / 2^k at levels 0..3."""
-    rng = np.random.default_rng(seed)
-    pts = np.stack([rng.uniform(-margin, w - 1 + margin, m), rng.uniform(-margin, h - 1 + margin, m)], 1).astype(F32)
-    special = [(0, 0), (w - 1, h - 1), (w - 1, 0), (0, h - 1), (np.nan, 3), (4, np.inf), (w - 1 + 1 / 256, 2),
-               (10.5 / 256, 2.5 / 256 + 3), (16.5 / 128, 9 + 0.5 / 128), (7.5 / 64 + 5, 3.5 / 64 + 1), (1.5 / 32 + 2, 0.5 / 32 + 4)]
-    k = min(m, len(special))
-    pts[:k] = np.array(special[:k], F32)
-    return pts
 
 
 # ------------------------------------------------------------------------------------ CPU: the tie to the pinned oracle
@@ -101,15 +27,13 @@ def random_points(w, h, m, seed, margin=2.0):
 def test_single_level_single_iteration_is_the_dense_oracle(tro, oracle, win):
     """levels = 1, iters = 1, integer points, min_eig = 0: every sample is the field value and the solve is the dense one, so
     the flow of a point is oracle.lk_level at its pixel; on every border pixel and corner of an odd-sized frame."""
-    from test_gpu_parity import assert_flow_identical
-
     w, h = 37, 29
     prev, nxt = frames(oracle, w, h, 1.3, -0.6)
     pts = np.concatenate([border_points(w, h), np.array([[w // 2, h // 2], [5, 7], [30, 20]], F32)])
     flow, st = tro.track(prev, nxt, 1, win, pts, 1.0, iters=1, eps=0.0)
     dense = oracle.lk_level(prev, nxt, win)
     ref = dense[pts[:, 1].astype(int), pts[:, 0].astype(int)]
-    assert_flow_identical(flow, ref, f"win {win}")
+    assert_values_equal(flow, ref, f"win {win}")
     fin = np.isfinite(flow).all(1)
     assert (st[~fin] == PT_NONFINITE).all() and np.isin(st[fin], [PT_TRACKED, PT_OUTSIDE]).all()
 
@@ -272,12 +196,6 @@ def test_null_context_is_rejected():
 
 
 # ------------------------------------------------------------------------------------ GPU
-def _dev(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
 def _batch(oracle, w, h, n, seed):
     prevs = np.stack([oracle.make_frame(w, h, 0, 0, 4, seed + i) for i in range(n)])
     nexts = np.stack([oracle.make_frame(w, h, 1.2 + 0.37 * (i % 7), -0.8 + 0.21 * (i % 5), 4, seed + i) for i in range(n)])
@@ -287,7 +205,7 @@ def _batch(oracle, w, h, n, seed):
 def _run_gpu(ctx, prevs, nexts, w, levels, win, pts, **kw):
     from cuda_optical_flow_2_b200 import planar_to_device
 
-    flow, st = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, _dev(pts), **kw)
+    flow, st = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, to_device(pts), **kw)
     return flow.cpu().numpy(), st.cpu().numpy()
 
 
@@ -395,8 +313,6 @@ def test_single_level_single_iteration_is_the_dense_path(ctx, oracle, win):
     """levels = 1, iters = 1, integer points: the flow is flow_pairs_device's (EXACT solve) at those pixels, compared with no
     restatement in between; setting the context to SOLVE_FAST changes nothing in the tracker."""
     from cuda_optical_flow_2_b200 import SOLVE_EXACT, SOLVE_FAST, planar_to_device
-    from test_gpu_parity import assert_flow_identical
-
     w, h, n = 83, 61, 2
     prevs, nexts = _batch(oracle, w, h, n, 50 + win)
     p, q = planar_to_device(prevs), planar_to_device(nexts)
@@ -405,18 +321,15 @@ def test_single_level_single_iteration_is_the_dense_path(ctx, oracle, win):
     rng = np.random.default_rng(win)
     pts = np.stack([np.concatenate([border_points(w, h), np.stack([rng.integers(0, w, 200), rng.integers(0, h, 200)], 1)])
                     for _ in range(n)]).astype(F32)
-    flow, st = ctx.track_points_device(p, q, w, 1, win, _dev(pts), iters=1, eps=0.0)
+    flow, st = ctx.track_points_device(p, q, w, 1, win, to_device(pts), iters=1, eps=0.0)
     flow = flow.cpu().numpy()
     for i in range(n):
         ref = dense[i][pts[i, :, 1].astype(int), pts[i, :, 0].astype(int)]
-        assert_flow_identical(flow[i], ref, f"pair {i}")
-    ctx.solve = SOLVE_FAST
-    try:
-        f2, s2 = ctx.track_points_device(p, q, w, 1, win, _dev(pts), iters=1, eps=0.0)
-        f3, s3 = ctx.track_points_device(p, q, w, 3, win, _dev(pts), flow_scale=S815)
-    finally:
-        ctx.solve = SOLVE_EXACT
-    f4, s4 = ctx.track_points_device(p, q, w, 3, win, _dev(pts), flow_scale=S815)
+        assert_values_equal(flow[i], ref, f"pair {i}")
+    with solve(ctx, SOLVE_FAST):
+        f2, s2 = ctx.track_points_device(p, q, w, 1, win, to_device(pts), iters=1, eps=0.0)
+        f3, s3 = ctx.track_points_device(p, q, w, 3, win, to_device(pts), flow_scale=S815)
+    f4, s4 = ctx.track_points_device(p, q, w, 3, win, to_device(pts), flow_scale=S815)
     assert_same_bits(f2.cpu().numpy(), flow)
     assert np.array_equal(s2.cpu().numpy(), st.cpu().numpy())
     assert_same_bits(f3.cpu().numpy(), f4.cpu().numpy())
@@ -436,7 +349,7 @@ def test_cuda_graph_replay(ctx, oracle):
     rounds = [(_batch(oracle, w, h, n, 900 + 10 * r), np.stack([random_points(w, h, m, 77 * r + i) for i in range(n)]))
               for r in range(3)]
     (p0, q0), pts0 = rounds[0]
-    p, q, pts = planar_to_device(p0), planar_to_device(q0), _dev(pts0)
+    p, q, pts = planar_to_device(p0), planar_to_device(q0), to_device(pts0)
     side = torch.cuda.Stream()
     side.wait_stream(torch.cuda.current_stream())
     with torch.cuda.stream(side):
@@ -449,10 +362,10 @@ def test_cuda_graph_replay(ctx, oracle):
     for (prevs, nexts), pr in rounds[1:]:
         p.copy_(planar_to_device(prevs))
         q.copy_(planar_to_device(nexts))
-        pts.copy_(_dev(pr))
+        pts.copy_(to_device(pr))
         g.replay()
         torch.cuda.synchronize()
-        eager = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, _dev(pr), S815)
+        eager = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, to_device(pr), S815)
         torch.cuda.synchronize()
         for got, ref in zip(out, eager):
             assert np.array_equal(got.cpu().numpy().view(np.uint8), ref.cpu().numpy().view(np.uint8))

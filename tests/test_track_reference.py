@@ -14,29 +14,17 @@ shared by both would pass there.  Here:
     flow scales 3 and 0.01, 2^24 points and 65535 pairs.
 """
 import ctypes as C
-import os
-import subprocess
 from fractions import Fraction
 
 import numpy as np
 import pytest
 from scipy.ndimage import map_coordinates
 
-from test_adversarial_content import PAIRS, vertical_stripes
-from test_track_points import (F32, PT_LOW_TEXTURE, PT_NONFINITE, PT_OUTSIDE, PT_TRACKED, S815, TrackOracle,
-                               assert_same_bits, assert_status_equal, border_points, random_points)
+from support import (F32, PAIRS, PT_LOW_TEXTURE, PT_NONFINITE, PT_OUTSIDE, PT_TRACKED, S815, assert_same_bits, assert_status_equal,
+                     border_points, device_frames, random_points, to_device, tro, vertical_stripes)  # noqa: F401 (tro: a fixture)
 
 WINDOWS = [3, 5, 7, 9, 11, 13, 15, 17, 19]
 I32 = 2 ** 31
-
-
-@pytest.fixture(scope="session")
-def tro(oracle, tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("track_oracle_ref") / "libtrackoracle.so")
-    src = os.path.join(os.path.dirname(os.path.abspath(__file__)), "track_oracle.c")
-    subprocess.check_call(["gcc", "-O2", "-fPIC", "-std=c11", "-ffp-contract=off", "-fno-fast-math", "-Wall", "-Wextra",
-                           "-shared", "-o", so, src, "-lm"])
-    return TrackOracle(so, oracle)
 
 
 # ------------------------------------------------------------------------------------ references
@@ -387,17 +375,11 @@ def test_one_dimensional_window_is_low_texture_at_any_min_eig(tro, oracle):
 
 
 # ------------------------------------------------------------------------------------ GPU
-def _dev(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a)).cuda()
-
-
 def _track(ctx, prevs, nexts, w, levels, win, pts, **kw):
     """The kernel through Context.track_points_device on planar_to_device frames (64-byte pitch, zero padding)."""
     from cuda_optical_flow_2_b200 import planar_to_device
 
-    flow, st = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, _dev(pts), **kw)
+    flow, st = ctx.track_points_device(planar_to_device(prevs), planar_to_device(nexts), w, levels, win, to_device(pts), **kw)
     return flow.cpu().numpy(), st.cpu().numpy()
 
 
@@ -472,7 +454,6 @@ def test_caller_frame_layouts(ctx, tro, oracle, w, h, levels):
     from cuda_optical_flow_2_b200 import OfbParams
     from cuda_optical_flow_2_b200.api import align_up
     from cuda_optical_flow_2_b200._lib import check
-    from test_adversarial_content import _padded_device
 
     win, fs = 9, S815
     pitch = align_up(w, 16) if w % 16 else w + 16
@@ -483,8 +464,8 @@ def test_caller_frame_layouts(ctx, tro, oracle, w, h, levels):
     n = len(pairs)
     pts = np.stack([np.concatenate([random_points(w, h, 100, 60 + i), border_points(w, h)]) for i in range(n)])
     plain_f, plain_s = _track(ctx, prevs, nexts, w, levels, win, pts, flow_scale=fs, iters=5, eps=0.0)
-    bp, bn = _padded_device(prevs, pitch, stride), _padded_device(nexts, pitch, stride)
-    dpts = _dev(pts)
+    bp, bn = device_frames(prevs, pitch, stride, 0xFF)[0], device_frames(nexts, pitch, stride, 0xFF)[0]
+    dpts = to_device(pts)
     flow = torch.empty(pts.shape, dtype=torch.float32, device="cuda")
     st = torch.empty(pts.shape[:2], dtype=torch.uint8, device="cuda")
     p = OfbParams(w, h, levels, win, 2, fs, n)
