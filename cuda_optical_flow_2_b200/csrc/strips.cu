@@ -16,6 +16,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstdio>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -161,6 +162,51 @@ static void exchange_rows(const StripPlan &pl, int x, int rank, int *o0, int *o1
 struct HaloRows {
     int peer, lo, hi, base;
 };
+// The halo-row table of one rank, per exchange x in [0, nx) (numbering: ArenaLayout): the rows it sends and receives,
+// the ranks it pushes to in either kind of pair (they acknowledge through done[], the teardown drains them) and the
+// ranks that push to it (told at the end of a pair that their rows have been used; the check-row senders first, so
+// that the handshake kernel's flags keep their order).
+struct HaloTable {
+    std::vector<std::vector<HaloRows>> send, recv;
+    std::vector<int> done_from, sources;
+};
+static void add_unique(std::vector<int> &v, int x)
+{
+    if (std::find(v.begin(), v.end(), x) == v.end()) v.push_back(x);
+}
+// Sender and receiver lists come from the same exchange_rows, so they agree; the backward exchanges repeat the forward
+// ones.  Every window holds its rank's own rows and both ends of a window grow with the rank, so the peers of an
+// exchange are a run of ranks around `rank`: the scan stops at the first rank either side that shares no rows.
+static HaloTable halo_table(const StripPlan &pl, int nx, int rank)
+{
+    HaloTable t;
+    t.send.assign(nx, {});
+    t.recv.assign(nx, {});
+    for (int x = 0; x < nx; x++) {
+        int m0, m1, mw0, mw1;
+        exchange_rows(pl, x, rank, &m0, &m1, &mw0, &mw1);
+        auto shares = [&](int peer, bool add) {
+            int p0, p1, pw0, pw1;
+            exchange_rows(pl, x, peer, &p0, &p1, &pw0, &pw1);
+            // my own rows in the peer's window, and the peer's own rows in mine
+            const int s0 = std::max(m0, pw0), s1 = std::min(m1, pw1), r0 = std::max(p0, mw0), r1 = std::min(p1, mw1);
+            if (add && s0 < s1) t.send[x].push_back({peer, s0, s1, pw0});
+            if (add && r0 < r1) t.recv[x].push_back({peer, r0, r1, mw0});
+            return s0 < s1 || r0 < r1;
+        };
+        int first = rank, last = rank;
+        while (first > 0 && shares(first - 1, false)) first--;
+        while (last + 1 < pl.world && shares(last + 1, false)) last++;
+        for (int peer = first; peer <= last; peer++)
+            if (peer != rank) shares(peer, true);
+        for (const HaloRows &e : t.send[x]) add_unique(t.done_from, e.peer);
+    }
+    if (nx > pl.levels)
+        for (const HaloRows &e : t.recv[nx - 1]) add_unique(t.sources, e.peer);
+    for (int x = 0; x < nx; x++)
+        for (const HaloRows &e : t.recv[x]) add_unique(t.sources, e.peer);
+    return t;
+}
 
 struct PeerSeg {
     const void *src;
@@ -321,13 +367,6 @@ int dev_alloc(ofb_strips *st, void **p, size_t bytes)
 }
 // pixels of the own rows of level 0
 inline size_t s_own_px(const ofb_strips *st) { return (size_t)st->s[0].w * (st->s[0].y1 - st->s[0].y0); }
-// rows [lo, hi) that `owner` owns and `peer`'s buffer [b0, b1) holds
-inline bool overlap(int own0, int own1, int b0, int b1, int *lo, int *hi)
-{
-    *lo = std::max(own0, b0);
-    *hi = std::min(own1, b1);
-    return *lo < *hi;
-}
 
 // ---- peer memory: one exchange ---------------------------------------------------------------------------------------
 struct PeerSend {
@@ -394,12 +433,11 @@ int peer_exchange(ofb_strips *st, int x, const std::vector<PeerSend> &sends, cud
     }
     return OFB_OK;
 }
-void add_unique(std::vector<int> &v, int x)
-{
-    if (std::find(v.begin(), v.end(), x) == v.end()) v.push_back(x);
-}
 // The schedule of a w x h pair of `levels` levels cut into `world` strips (arguments checked by the caller); refuses a
-// coarsest level with fewer rows than strips.
+// coarsest level with fewer rows than strips, and strips so thin that some rank's halo rows come from, or go to, more
+// ranks than one exchange carries (PEER_MAX_DST ranks, PEER_MAX_SEG copy segments; 2 PEER_MAX_DST ranks in the
+// end-of-pair handshake).  The table of EVERY rank is checked, so that every rank refuses the same plan: a rank whose own
+// exchanges fit must not go on alone into the peer set-up.
 int make_plan(int w, int h, int levels, int win, int world, int reach, int fb_reach, StripPlan *pl)
 {
     const int hc = h >> (levels - 1);
@@ -412,6 +450,34 @@ int make_plan(int w, int h, int levels, int win, int world, int reach, int fb_re
     pl->r = win / 2;
     // image halo: 3x3 stencil + window radius + one row of even-row alignment + warp reach + bilinear tap
     pl->img_halo = pl->r + 2 + reach + 2;
+    const int nx = fb_reach >= 0 ? 2 * levels : levels;
+    for (int rank = 0; rank < world; rank++) {
+        HaloTable t;
+        try { // (std::vector growth must not throw across the C ABI)
+            t = halo_table(*pl, nx, rank);
+        } catch (const std::bad_alloc &) {
+            set_error("strips: out of host memory");
+            return OFB_ERR_NOMEM;
+        }
+        // (what is over the limit, the exchange or -1 for the whole pair, the count, the limit)
+        const char *what = nullptr;
+        int x = -1, n = 0, limit = 0;
+        for (int e = 0; e < nx && !what; e++) {
+            if ((n = (int)t.send[e].size()) > PEER_MAX_DST) what = "sends rows to %d ranks", x = e, limit = PEER_MAX_DST;
+            else if ((n = (int)t.recv[e].size()) > PEER_MAX_DST) what = "receives rows from %d ranks", x = e, limit = PEER_MAX_DST;
+        }
+        if (!what && (n = 2 * (int)t.send[0].size()) > PEER_MAX_SEG) what = "copies %d segments", x = 0, limit = PEER_MAX_SEG;
+        if (!what && (n = (int)t.sources.size()) > 2 * PEER_MAX_DST) what = "receives rows from %d ranks", limit = 2 * PEER_MAX_DST;
+        if (!what && (n = (int)t.done_from.size()) > 2 * PEER_MAX_DST) what = "sends rows to %d ranks", limit = 2 * PEER_MAX_DST;
+        if (what) {
+            char ex[40] = "the exchanges of a pair", msg[64];
+            if (x >= 0) snprintf(ex, sizeof ex, "exchange %d", x);
+            snprintf(msg, sizeof msg, what, n);
+            set_error("strips thinner than their halo: in %s rank %d %s, more than the limit of %d; use fewer ranks, fewer levels "
+                      "or a smaller reach / fb_reach", ex, rank, msg, limit);
+            return OFB_ERR_UNSUPPORTED;
+        }
+    }
     return OFB_OK;
 }
 } // namespace
@@ -471,27 +537,13 @@ static int strips_create_impl(ofb_ctx *ctx, int w, int h, int levels, int win, i
     st->s = pl.strips(rank);
     // what neighbours write into (level-0 image rows, coarser cumulative-flow rows, flags): one allocation, the arena
     st->lay = arena_layout(pl, rank);
-    // The halo-row table.  Sender and receiver lists come from the same exchange_rows, so they agree; the backward
-    // exchanges repeat the forward ones.  The end-of-pair handshake and the teardown drain cover every rank that can
-    // push to / be pushed to by this one in either kind of pair.
-    st->send.assign(st->lay.nx, {});
-    st->recv.assign(st->lay.nx, {});
-    for (int x = 0; x < st->lay.nx; x++) {
-        int m0, m1, mw0, mw1;
-        exchange_rows(pl, x, rank, &m0, &m1, &mw0, &mw1);
-        for (int peer = 0; peer < world; peer++) {
-            int p0, p1, pw0, pw1, lo, hi;
-            if (peer == rank) continue;
-            exchange_rows(pl, x, peer, &p0, &p1, &pw0, &pw1);
-            if (overlap(m0, m1, pw0, pw1, &lo, &hi)) st->send[x].push_back({peer, lo, hi, pw0});
-            if (overlap(p0, p1, mw0, mw1, &lo, &hi)) st->recv[x].push_back({peer, lo, hi, mw0});
-        }
-        for (const HaloRows &e : st->send[x]) add_unique(st->done_from, e.peer);
+    {
+        HaloTable t = halo_table(pl, st->lay.nx, rank);
+        st->send = std::move(t.send);
+        st->recv = std::move(t.recv);
+        st->done_from = std::move(t.done_from);
+        st->sources = std::move(t.sources);
     }
-    if (fb_reach >= 0) // (the check-row senders first: the handshake kernel's flags keep their order)
-        for (const HaloRows &e : st->recv[2 * levels - 1]) add_unique(st->sources, e.peer);
-    for (int x = 0; x < st->lay.nx; x++)
-        for (const HaloRows &e : st->recv[x]) add_unique(st->sources, e.peer);
     {
         void *p = nullptr;
         rc = dev_alloc(st, &p, st->lay.bytes);

@@ -254,7 +254,15 @@ int ofb_stream_destroy(ofb_stream *s);
  * sender's kernels into the receiver's memory over NVLink plus an epoch flag raised there, and a wait for that flag on the
  * receiver's stream.  ofb_strips_peer_connect_local does the same for ranks living in one process.
  *   ofb_strips_plan_query     : host only, no device: the rows {y0, y1, by0, by1, cy0, cy1, eb0, eb1} of a level on a rank
- *   ofb_strips_check          : synchronises; *overflow bit 0 = a warp sample reached past the halo rows, bit 1 = a
+ *   plans refused (ofb_strips_plan_query, _create, _create_fb alike, on every rank): OFB_ERR_INVALID when the coarsest
+ *                               level has fewer rows than ranks (or no column); OFB_ERR_UNSUPPORTED when strips are so
+ *                               much thinner than their halo that, on ANY rank, one exchange of a pair would send rows to
+ *                               or receive rows from more than 4 ranks, the image exchange would copy more than 8 row
+ *                               segments, or more than 8 ranks would push to, or be pushed to by, one rank over a pair
+ *                               (_create_fb: with its check-row and backward exchanges).  ofb_last_error names the
+ *                               exchange, the rank and the count; fewer ranks, fewer levels or a smaller reach / fb_reach
+ *                               help.  Plans whose coarsest strips are 1 or 2 rows are refused on more than 5 ranks
+ *   ofb_strips_check        : synchronises; *overflow bit 0 = a warp sample reached past the halo rows, bit 1 = a
  *                               neighbour's rows did not arrive within 4 s, bit 2 = a checked pair's check needed a
  *                               backward tap outside the rows the rank holds (OFB_FB_UNCHECKED pixels: raise fb_reach).
  *                               The flag is sticky: it covers every pair since the previous check, which clears it
@@ -301,7 +309,9 @@ int ofb_strips_peer_connect_local(ofb_strips *s, void *const *arenas_d);
  *                          fb_reach + 1)).  The arena also holds the backward direction's regions, so a handle that runs
  *                          checked pairs is created this way (before ofb_strips_peer_handle / _connect).  flow_scale > 0.
  *                          Plain pairs (ofb_strips_run_device) run on it unchanged, and plain and
- *                          checked pairs may alternate; all ranks must be created with the same fb_reach.
+ *                          checked pairs may alternate; all ranks must be created with the same fb_reach.  Refuses
+ *                          the plans ofb_strips_create refuses, and those whose check-row exchange or handshake goes
+ *                          past the same limits (see the plans refused above).
  *   ofb_strips_run_fb_device : one checked pair; alpha >= 0, beta >= 0 as in ofb_flow_pairs_fb_device; want_err2 = 0 leaves
  *                          the err2 buffer untouched.  Bad arguments are refused before anything is enqueued.
  *   ofb_strips_run_fb_phase_device : one of its 4L + 1 phases (L = levels; ranks of one process on one stream, as

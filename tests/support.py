@@ -633,6 +633,72 @@ def reach_flag(req, y_off, h_local, cum_y_off, cum_h_local):
     return bool((img & ~held).any() or (crow & ~cheld).any())
 
 
+@pytest.fixture
+def rows(monkeypatch):
+    """set(n): force n rows per CTA on every following launch (OFB_LK_ROWS, read by csrc/lk_win.cu on every launch);
+    set(None): the cost model's own split."""
+
+    def set_rows(n):
+        if n is None:
+            monkeypatch.delenv("OFB_LK_ROWS", raising=False)
+        else:
+            monkeypatch.setenv("OFB_LK_ROWS", str(n))
+
+    set_rows(None)
+    return set_rows
+
+
+# ------------------------------------------------------------------------------------ checked pairs on row strips
+FB_UNCHECKED = 5
+
+
+def held_rows(y0, y1, h, fb_reach):
+    """Rows of the level-0 backward total a strip's check holds: its own rows [y0, y1) and fb_reach more either side."""
+    return max(0, y0 - fb_reach), min(h, y1 + fb_reach + 1)
+
+
+def tap_rows_outside(fwd, y0, h, b0, b1, s):
+    """For own rows fwd ((rows, w, 2), global rows y0 ..) of a frame h rows high: which pixels read backward taps at all
+    (their whole-frame status is CONSISTENT, INCONSISTENT or BWD_NONFINITE) and which of those have a tap of non-zero
+    weight outside rows [b0, b1)."""
+    s = F32(s)
+    rows, w = fwd.shape[:2]
+    u, v = fwd[..., 0], fwd[..., 1]
+    ii, jj = np.meshgrid(np.arange(y0, y0 + rows, dtype=np.int64), np.arange(w, dtype=np.int64), indexing="ij")
+    with np.errstate(all="ignore"):
+        fin = np.isfinite(u) & np.isfinite(v)
+        du, dv = s * u, s * v
+        ranged = fin & (np.abs(du) < F32(32768)) & (np.abs(dv) < F32(32768))
+        X = jj * 256 + np.where(ranged, np.rint(du * F32(256)), F32(0)).astype(np.int64)
+        Y = ii * 256 + np.where(ranged, np.rint(dv * F32(256)), F32(0)).astype(np.int64)
+    reads = ranged & (X >= 0) & (X <= (w - 1) * 256) & (Y >= 0) & (Y <= (h - 1) * 256)
+    ty0 = Y >> 8
+    ty1 = np.where(Y & 255, ty0 + 1, ty0)
+    return reads, reads & ((ty0 < b0) | (ty1 >= b1))
+
+
+def assert_equals_whole(ranks, whole, want_err2, what):
+    """Checks the flags (bit 2 allowed) and every rank's outputs of a checked pair (dist.NativeStrips made with fb_reach)
+    against its rows of the whole-frame result `whole` (Context.flow_pairs_fb_device), with the pixels whose taps leave
+    the held rows -- predicted from the whole-frame forward total -- UNCHECKED and err2 NaN."""
+    import torch
+
+    fwd, bwd, st, e2 = whole
+    for ns in ranks:
+        ns.check(allow_unchecked=True)
+        y0, y1 = ns.own_rows(0)
+        b0, b1 = held_rows(y0, y1, ns.h, ns.fb_reach)
+        _, out = tap_rows_outside(fwd[0, y0:y1].cpu().numpy(), y0, ns.h, b0, b1, ns.flow_scale)
+        out = torch.from_numpy(out).to(st.device)
+        gf, gb, gs, ge = ns.own_fb()
+        assert_same_bits(gf, fwd[0, y0:y1], f"{what} rank {ns.rank}: forward total")
+        assert_same_bits(gb, bwd[0, y0:y1], f"{what} rank {ns.rank}: backward total")
+        ref_st = torch.where(out, torch.full_like(st[0, y0:y1], FB_UNCHECKED), st[0, y0:y1])
+        assert bool((gs == ref_st).all()), f"{what} rank {ns.rank}: status ({int((gs != ref_st).sum())} differ)"
+        if want_err2:
+            assert_same_bits(ge, torch.where(out, torch.full_like(ge, float("nan")), e2[0, y0:y1]), f"{what} rank {ns.rank}: err2")
+
+
 # ------------------------------------------------------------------------------------ the frame stream
 _STREAM_SHIFTS = [(0.0, 0.0), (1.5, -0.5), (2.25, 0.75), (0.5, 2.0), (-1.0, 1.25), (3.0, -1.5)]
 

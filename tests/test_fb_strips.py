@@ -15,38 +15,14 @@ import os
 import numpy as np
 import pytest
 
-from support import (F32, FB_BWD_NONFINITE, FB_CONSISTENT, FB_FWD_NONFINITE, FB_INCONSISTENT, FB_OUTSIDE, S815,
-                     assert_same_bits, assert_status_equal, fbo, np_fb_check, solve)  # noqa: F401 (fbo is a fixture)
+from support import (F32, FB_BWD_NONFINITE, FB_CONSISTENT, FB_FWD_NONFINITE, FB_INCONSISTENT, FB_OUTSIDE, FB_UNCHECKED, S815,
+                     assert_equals_whole, assert_same_bits, assert_status_equal, fbo, held_rows, np_fb_check, solve,
+                     tap_rows_outside)  # noqa: F401 (fbo is a fixture)
 
-FB_UNCHECKED = 5
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 # ------------------------------------------------------------------------------------ numpy restatement of the strip rule
-def held_rows(y0, y1, h, fb_reach):
-    return max(0, y0 - fb_reach), min(h, y1 + fb_reach + 1)
-
-
-def tap_rows_outside(fwd, y0, h, b0, b1, s):
-    """For own rows fwd ((rows, w, 2), global rows y0 ..) of a frame h rows high: which pixels read backward taps at all
-    (their whole-frame status is CONSISTENT, INCONSISTENT or BWD_NONFINITE) and which of those have a tap of non-zero
-    weight outside rows [b0, b1)."""
-    s = F32(s)
-    rows, w = fwd.shape[:2]
-    u, v = fwd[..., 0], fwd[..., 1]
-    ii, jj = np.meshgrid(np.arange(y0, y0 + rows, dtype=np.int64), np.arange(w, dtype=np.int64), indexing="ij")
-    with np.errstate(all="ignore"):
-        fin = np.isfinite(u) & np.isfinite(v)
-        du, dv = s * u, s * v
-        ranged = fin & (np.abs(du) < F32(32768)) & (np.abs(dv) < F32(32768))
-        X = jj * 256 + np.where(ranged, np.rint(du * F32(256)), F32(0)).astype(np.int64)
-        Y = ii * 256 + np.where(ranged, np.rint(dv * F32(256)), F32(0)).astype(np.int64)
-    reads = ranged & (X >= 0) & (X <= (w - 1) * 256) & (Y >= 0) & (Y <= (h - 1) * 256)
-    ty0 = Y >> 8
-    ty1 = np.where(Y & 255, ty0 + 1, ty0)
-    return reads, reads & ((ty0 < b0) | (ty1 >= b1))
-
-
 def np_fb_check_strip(fwd_own, bwd_held, y0, h, b0, b1, s, alpha=0.01, beta=0.5):
     """The strip check from what a rank holds: its own forward rows and backward rows [b0, b1)."""
     rows, w = fwd_own.shape[:2]
@@ -178,27 +154,6 @@ def _inputs(ranks, dp, dn):
     return out
 
 
-def _assert_equals_whole(ranks, whole, want_err2, what):
-    """Checks the flags (bit 2 allowed) and every rank's outputs against its rows of the whole-frame result, with the
-    pixels whose taps leave the held rows -- predicted from the whole-frame forward total -- UNCHECKED and err2 NaN."""
-    import torch
-
-    fwd, bwd, st, e2 = whole
-    for ns in ranks:
-        ns.check(allow_unchecked=True)
-        y0, y1 = ns.own_rows(0)
-        b0, b1 = held_rows(y0, y1, ns.h, ns.fb_reach)
-        _, out = tap_rows_outside(fwd[0, y0:y1].cpu().numpy(), y0, ns.h, b0, b1, ns.flow_scale)
-        out = torch.from_numpy(out).to(st.device)
-        gf, gb, gs, ge = ns.own_fb()
-        assert_same_bits(gf, fwd[0, y0:y1], f"{what} rank {ns.rank}: forward total")
-        assert_same_bits(gb, bwd[0, y0:y1], f"{what} rank {ns.rank}: backward total")
-        ref_st = torch.where(out, torch.full_like(st[0, y0:y1], FB_UNCHECKED), st[0, y0:y1])
-        assert bool((gs == ref_st).all()), f"{what} rank {ns.rank}: status ({int((gs != ref_st).sum())} differ)"
-        if want_err2:
-            assert_same_bits(ge, torch.where(out, torch.full_like(ge, float("nan")), e2[0, y0:y1]), f"{what} rank {ns.rank}: err2")
-
-
 EQUIV = [(640, 480, 3, 9, 1, 2), (640, 480, 3, 9, 2, 1), (640, 480, 3, 5, 4, 2), (640, 480, 1, 9, 3, 2), (322, 406, 2, 5, 3, 2),
          (322, 406, 2, 15, 2, 1), (322, 406, 3, 9, 4, 2), (1920, 1080, 3, 9, 8, 2), (1920, 1080, 4, 15, 4, 1),
          (7680, 4320, 4, 9, 8, 2), (7680, 4320, 4, 9, 2, 1)]
@@ -228,7 +183,7 @@ def test_checked_pair_equals_whole_frame(ctx, oracle, W, H, levels, win, world, 
                 torch.cuda.synchronize()
                 NativeStrips.run_local_sequenced_fb(ranks, _inputs(ranks, dp, dn), want_err2=want_err2,
                                                     stream=torch.cuda.current_stream().cuda_stream)
-                _assert_equals_whole(ranks, whole, want_err2, f"pair {trial}")
+                assert_equals_whole(ranks, whole, want_err2, f"pair {trial}")
         finally:
             _close(ranks)
 
@@ -297,7 +252,7 @@ def test_plain_and_checked_pairs_alternate(ctx, oracle, world, fb_reach):
             if kind == "c":
                 whole = ctx.flow_pairs_fb_device(dp, dn, W, levels, win, want_err2=True)
                 NativeStrips.run_local_sequenced_fb(fb, _inputs(fb, dp, dn), want_err2=True)
-                _assert_equals_whole(fb, whole, True, f"step {step}")
+                assert_equals_whole(fb, whole, True, f"step {step}")
                 continue
             n0 = ctx.launch_count
             NativeStrips.run_local_sequenced(plain, _inputs(plain, dp, dn))
@@ -349,7 +304,7 @@ def test_checked_pair_replays_as_cuda_graph(ctx, oracle):
             with torch.cuda.stream(side):
                 g.replay()
             torch.cuda.synchronize()
-            _assert_equals_whole(ranks, whole, True, f"replay {trial}")
+            assert_equals_whole(ranks, whole, True, f"replay {trial}")
     finally:
         _close(ranks)
 

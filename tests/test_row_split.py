@@ -27,7 +27,7 @@ import numpy as np
 import pytest
 
 from support import (PAIRS, assert_flow_within_tolerance, assert_values_equal, bits_differ, c_for, noise_pair, oracle_warp,
-                     reach_flag, requested_rows, solve, values_differ)
+                     reach_flag, requested_rows, rows, solve, values_differ)  # noqa: F401 (rows is a fixture)
 
 WINDOWS = [3, 5, 7, 9, 11, 13, 15, 17, 19]
 SHAPES_A = [(256, 160), (262, 150), (256, 161)]  # even; odd coarser width (no tensor map); 161 = 10 * 16 + 1 = 5 * 32 + 1
@@ -208,20 +208,6 @@ def test_pyramid_batch_sizes_reach_every_rows_per_thread(sw, sh, sm_count):
 
 
 # =================================================================================================== GPU
-@pytest.fixture
-def rows(monkeypatch):
-    """set(n): force n rows per CTA on every following launch; set(None): the cost model's own split."""
-
-    def set_rows(n):
-        if n is None:
-            monkeypatch.delenv("OFB_LK_ROWS", raising=False)
-        else:
-            monkeypatch.setenv("OFB_LK_ROWS", str(n))
-
-    set_rows(None)
-    return set_rows
-
-
 # --------------------------------------------------------------------------------------- A
 @pytest.mark.gpu
 @pytest.mark.parametrize("w,h", SHAPES_A)
